@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W     # the reference algorithm on the host CPU cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's image as DIR/rgb_map.npy
 
 Workload (BASELINE.json configs[1]): one step = one full 450x450 HeadNeRF frame, 202 500 rays,
 64 coarse + 128 importance samples (256 FaceNeRF evaluations per ray), random-init FaceNeRF
@@ -21,6 +22,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -458,12 +460,15 @@ def run_ours(args):
     frames = world                                   # frames per step (weak scaling: 202 500 rays per rank per step)
     lo, hi = band(N_RAYS, rank, world)
 
+    last = {}
+
     @torch.no_grad()
     def step_resident():
         """`frames` frames, each ray-sharded over the ranks; the band all-gather of frame i overlaps the kernels of frame i+1."""
         hs = [fr_r.render_frame(res["pose"], res["aud"], res["expr"], res["latent"], res["bc"], perturb=1.0, async_op=True)
               for _ in range(frames)]
-        return [h.wait() for h in hs][-1]
+        last["rgb_map"] = [h.wait() for h in hs][-1]
+        return last["rgb_map"]
 
     out_h = torch.empty((N_RAYS, 3)).pin_memory()
     h2d = sum(host[k].numel() * 4 for k in host)
@@ -510,6 +515,11 @@ def run_ours(args):
     total_ms = timed(step_resident, args.steps)          # the headline: no per-kernel events inside this region
     launches = ops.LAUNCHES["count"]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # the image the last timed step returned, before the passes below reuse its buffers; with the same arguments the inputs, the
+        # weights and the Philox seed / offsets are the same in every run, so two builds can be compared output for output
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "rgb_map.npy"), last["rgb_map"].float().cpu().numpy())
     # second, identical pass with a CUDA-event pair around every launch (on the launching stream) for the roofline / breakdown; under
     # kernel_timing the renderer takes the stage-by-stage entry points (one event pair per kernel), so that path gets its own warm-up
     with ops.kernel_timing():
@@ -727,7 +737,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-train", dest="no_train", action="store_true")
     ap.add_argument("--no-extra", dest="no_extra", action="store_true", help="skip the fp32-mode render, parity and config-4 keys")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the image the last timed step rendered to DIR/rgb_map.npy ((202500, 3) float32, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl in ("reference", "reference-gpu"):
         run_reference(args)
     else:

@@ -228,31 +228,67 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
-def _reference_head():
+def test_network_layout_matches_reference_network(M):
+    """The 'optimizer' entry of head.tar indexes the reference's per-parameter Adam state by position in list(Network.parameters()), so
+    the parameter order is part of the file format.  Name and shape of every parameter, in order (feature_linear and ds_aud_net
+    included), against the reference's Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128): from tests/golden/head_tar_layout.npz
+    (tests/golden/make_golden_head_tar.py) when it is committed, else from the reference tree when oracle/ref_import.py finds one."""
+    import numpy as np
     from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("neither /root/reference nor oracle/_ref is present")
-    return ref_import.import_head(force_cpu=True)
+    path = os.path.join(ROOT, "tests", "golden", "head_tar_layout.npz")
+    if os.path.exists(path):
+        with np.load(path) as z:
+            ref = [(str(n), tuple(int(d) for d in s[1:1 + s[0]])) for n, s in zip(z["names"], z["shapes"])]
+    elif ref_import.available():
+        head = ref_import.import_head(force_cpu=True)
+        ref = [(n, tuple(p.shape)) for n, p in head.Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128).named_parameters()]
+    else:
+        pytest.skip("neither tests/golden/head_tar_layout.npz nor the reference tree is present")
+    net = M.Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128)
+    assert [(n, tuple(p.shape)) for n, p in net.named_parameters()] == ref
+
+
+def test_network_parameter_order_matches_reference(M, golden):
+    """Parameter order (see test_network_layout_matches_reference_network) against what the committed fixtures made from the reference's
+    own modules record: the order of the FaceNeRF parameters that receive a gradient (train_step.npz; feature_linear receives none and is
+    not in it) and of AudioNet(64) / AudioAttNet (audio_nets.npz).  The positions of feature_linear and of ds_aud_net are not in these
+    fixtures; test_network_layout_matches_reference_network pins them."""
+    net = M.Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128)
+    names = [n for n, _ in net.named_parameters()]
+    assert list(net.state_dict()) == names                                     # no buffers: state_dict order == parameter order
+    modules = list(dict.fromkeys(n.split(".")[0] for n in names))
+    assert modules == ["face_nerf_coarse", "face_nerf_fine", "aud_net", "aud_att_net", "ds_aud_net"]
+    tr, au = golden("train_step"), golden("audio_nets")
+    for tag, mod in (("c", "face_nerf_coarse"), ("f", "face_nerf_fine")):
+        ref = [k[len(f"norm:{tag}."):] for k in tr if k.startswith(f"norm:{tag}.")]
+        ours = [n[len(mod) + 1:] for n in names if n.startswith(mod + ".")]
+        assert len(ref) == 26 and [n for n in ours if n in ref] == ref, mod
+        assert [n for n in ours if n not in ref] == ["feature_linear.weight", "feature_linear.bias"]      # unused by the forward: no gradient
+    for tag, mod in (("an64", "aud_net"), ("att", "aud_att_net")):
+        ref = [k[len(tag) + 1:] for k in au if k.startswith(tag + ".") and k.endswith((".weight", ".bias"))]
+        assert [n[len(mod) + 1:] for n in names if n.startswith(mod + ".")] == ref, mod
+        assert all(tuple(net.state_dict()[f"{mod}.{k}"].shape) == au[f"{tag}.{k}"].shape for k in ref)
 
 
 def test_head_tar_interchange_with_reference_adam(M, tmp_path):
-    """head.tar both ways (audio_exp_nerf.py:516-525 resume, :584-591 save) against the UNMODIFIED reference classes: a checkpoint written
-    by the reference's Network + per-parameter torch.optim.Adam loads into a live train.TrainStep with strict keys, IN PLACE (latent codes
-    and weights stay views of the flat Adam buffer -- ADVICE r1), the next update equals the reference's next update bit for bit, and the
-    file TrainStep.save() writes resumes the reference's own optimiser the same way."""
+    """head.tar both ways (audio_exp_nerf.py:516-525 resume, :584-591 save) with the reference's optimiser, a per-parameter
+    torch.optim.Adam over list(network.parameters()) + [latent codes] (:487-489): a checkpoint written by a Network + that optimiser
+    loads into a live train.TrainStep with strict keys, IN PLACE (latent codes and weights stay views of the flat Adam buffer), the next
+    update equals the per-parameter optimiser's next update bit for bit, and the file TrainStep.save() writes resumes the
+    per-parameter optimiser the same way.  Writer and reader are both this project's Network here, so the parameter order that indexes
+    the per-parameter state is checked against the reference's by the two tests above, not by this one."""
     from ideal_nerf_b200.train import TrainStep
-    head = _reference_head()
     torch.manual_seed(0)
 
     def ref_setup():
-        net = head.Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128)
+        net = M.Network(450, 450, 1200., 0.57, 1.17, 8192, None, 64, 128)
         lat = torch.ones(5, 32)
         lat.requires_grad = True
         tp = list(net.parameters()) + [lat]                                   # :487-489
         return net, lat, tp, torch.optim.Adam(params=tp, lr=3e-4, betas=(0.9, 0.999))
 
     ref, lat_ref, tp, opt_ref = ref_setup()
-    ref.apply(head.init_weights)
+    ref.apply(M.init_weights)
     g = torch.Generator().manual_seed(1)
 
     def fake_grads(params_list):
@@ -276,8 +312,7 @@ def test_head_tar_interchange_with_reference_adam(M, tmp_path):
     flat = ts.flat.flat
     for p in ts.flat.params:                                                   # still views of the flat buffer after the load
         assert flat.data_ptr() <= p.data_ptr() < flat.data_ptr() + flat.numel() * 4
-    assert list(ref.state_dict()) == list(ours.state_dict())
-    assert all(torch.equal(a, b) for a, b in zip(ref.state_dict().values(), ours.state_dict().values()))
+    assert all(torch.equal(a, b) for a, b in zip(ref.state_dict().values(), ours.state_dict().values()))      # the weights of the file
     assert torch.equal(lat.data, lat_ref.data)
     before = lat.detach().clone()
     fake_grads([tp, ts.flat.params])
