@@ -18,7 +18,7 @@ SOURCES = ["api.cu", "rays.cu", "composite.cu", "sample_pdf.cu", "mlp_fp32.cu", 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--shared"]
 
-INERF_MLP_FP32, INERF_MLP_BF16, INERF_MLP_BF16_BWD, INERF_MLP_F16X2 = 0, 1, 2, 3
+INERF_MLP_FP32, INERF_MLP_BF16, INERF_MLP_BF16_BWD, INERF_MLP_F16X2, INERF_MLP_BF16_EMB = 0, 1, 2, 3, 4
 INERF_PDF_EXACT_TORCH_CPU, INERF_PDF_FAST = 0, 1
 N_PARAMS = 26
 
@@ -96,6 +96,7 @@ SIGNATURES = {
     "inerf_mlp_bwd": (_I, [_DIMS, _PARAMS, _PARAMS, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P]),
     "inerf_mlp_train_sizes_bf16": (_I, [_DIMS, _L, _SZP, _SZP, _SZP, _SZP]),
     "inerf_mlp_fwd_train_bf16": (_I, [_DIMS, _PARAMS, _P, _P, _P, _I, _P, _I, _I, _P, _P, _P, _P]),
+    "inerf_mlp_fwd_train_bf16_embedded": (_I, [_DIMS, _PARAMS, _P, _P, _P, _L, _P, _P, _P, _P]),
     "inerf_mlp_bwd_bf16": (_I, [_DIMS, _PARAMS, _P, _PARAMS, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P]),
     "inerf_audio_net_fwd": (_I, [_PARAMS, _P, _I, _I, _P, _P]),
     "inerf_audio_att_fwd": (_I, [_PARAMS, _P, _I, _I, _I, _P, _P]),

@@ -27,6 +27,11 @@
 //   * alpha_linear (256->1) and rgb_linear (128->3) are fp32 dot products inside the L7 / V2 epilogues.
 // Weights are pre-packed (inerf_mlp_pack) as the exact shared-memory image of every stage: bf16,
 // K-major, 128-byte swizzle, in MMA issue order, so a stage is ONE contiguous bulk copy.
+//
+// Embedded-row variant (template parameter EMB, FaceNeRF.forward's x (P, 63+27)): the rows carry their own gamma(v), so there is no
+// per-ray view bias.  The 27 view columns of views_linears.0 run as one more K-block at the end of each V0 half, its A operand a
+// gamma(v) image that the producer warps write into the PE buffer once L5 (the last reader of gamma(p)) has completed; the commit after
+// the last V0 view MMA hands the buffer back for the next iteration's gamma(p).  Packed blob: INERF_MLP_BF16_EMB (two more stages).
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -80,6 +85,8 @@ struct Schedule {
 };
 
 __constant__ Step c_steps[MAX_STEPS];
+__constant__ Step c_steps_emb[MAX_STEPS];      // the embedded-row schedule (one more K-block per V0 half)
+template <bool EMB> __device__ __forceinline__ const Step& step_at(int s) { return EMB ? c_steps_emb[s] : c_steps[s]; }
 
 // smem map (bytes from the 1024-aligned base)
 constexpr int OFF_ACT = 0;                               // [2][4][16384]
@@ -207,6 +214,7 @@ __device__ __forceinline__ void epi_convert(const uint32_t (&r)[32], uint32_t* _
 __host__ __device__ constexpr int lay_N(int l) { return l < 8 ? 256 : 128; }
 __host__ __device__ constexpr int lay_act_kb(int l) { return l == 0 ? 0 : (l <= 8 ? 4 : 2); }     // activation K-blocks (64 wide)
 __host__ __device__ constexpr bool lay_pe(int l) { return l == 0 || l == 5; }                     // + the gamma(p) K-block
+__host__ __device__ constexpr bool lay_x(int l, bool emb) { return lay_pe(l) || (emb && l == 8); }   // + a PE-buffer K-block (gamma(p) or gamma(v))
 __host__ __device__ constexpr int lay_prev_N(int l) { return l == 0 ? 128 : lay_N(l - 1); }       // L0 follows V2 of the previous iteration
 
 __device__ __forceinline__ bool elect_one() {
@@ -269,10 +277,12 @@ struct IssueCtx {
 // constant of (L, half, K-block), so a step costs ~10 uniform-datapath instructions per tcgen05.mma instead of a table decode.
 // (The table-driven form was issue-latency bound: ~150 dependent SASS instructions per 8-MMA step on ONE thread, ~1000 cycles
 // against the 512 the tensor pipe needs -- profiles/r01_mlp_ablation.txt.)
-template <int L, bool TRACE, int ABL, bool PAIR>
+// EMB: the embedded-row schedule.  pe_ready and pe_free then complete twice per iteration (gamma(p) for L0 / L5, gamma(v) for V0), so
+// the issuer's waits have fixed parities: 0 before L0, 1 before V0's view K-block.
+template <int L, bool TRACE, int ABL, bool PAIR, bool EMB = false>
 __device__ __forceinline__ void issue_layer(IssueCtx& c) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
-    constexpr int N = lay_N(L), NH = N / 2, NKB = lay_act_kb(L), CNT = NKB + (lay_pe(L) ? 1 : 0);
+    constexpr int N = lay_N(L), NH = N / 2, NKB = lay_act_kb(L), CNT = NKB + (lay_x(L, EMB) ? 1 : 0);
     constexpr int KB_PER_HALF_PREV = lay_prev_N(L) / 128;     // activation K-blocks written by ONE half of the previous epilogue
     constexpr int N_OUT_H0 = NH / 64;                          // K-blocks epi(h0) of THIS layer overwrites
     constexpr int N_FIRST = NKB < N_OUT_H0 ? NKB : N_OUT_H0;   // leading K-blocks of h1 that epi(h0) will overwrite
@@ -300,7 +310,8 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
                 }
             }
             if constexpr (TRACE) { const long long c1 = clock64(); c.t_e += c1 - c0; c.t_e_layer[c.layer_ctr % 11] += c1 - c0; c0 = c1; }
-            if (L == 0 && h == 0 && i == 0) wait_ev<TRACE, PAIR>(&bars->pe_ready, c.iter_ctr & 1, 203, L, (int)c.iter_ctr);
+            if (L == 0 && h == 0 && i == 0) wait_ev<TRACE, PAIR>(&bars->pe_ready, EMB ? 0u : c.iter_ctr & 1, 203, L, (int)c.iter_ctr);
+            if (EMB && L == 8 && h == 0 && is_pe) wait_ev<TRACE, PAIR>(&bars->pe_ready, 1u, 206, L, (int)c.iter_ctr);
             if constexpr (TRACE) { const long long c1 = clock64(); c.t_pe += c1 - c0; c0 = c1; }
             if (!(ABL & 2) || (c.layer_ctr == 0 && L == 0 && h * CNT + i < NSTAGE)) {
                 const long long p0 = PH_CLK();
@@ -336,7 +347,7 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
                 if (h == 0 && last) commit_any<PAIR>(&bars->cbar[0]);
                 if (h == 1 && (N_FIRST > 0 ? i == N_FIRST - 1 : last)) commit_any<PAIR>(&bars->cbar[1]);
                 if (h == 1 && last) commit_any<PAIR>(&bars->cbar[2]);
-                if (h == 1 && last && L == 5) commit_any<PAIR>(&bars->pe_free);
+                if (h == 1 && last && (L == 5 || (EMB && L == 8))) commit_any<PAIR>(&bars->pe_free);
             }
             __syncwarp();
             if (i == 0) { c.bslot ^= 1; if (c.bslot == 0) c.bpar ^= 1; }
@@ -438,10 +449,11 @@ __device__ int g_save_abl;      // profiling builds: switch parts of the activat
 // bytes.  Schedule, layouts, packed blob and epilogue are the single-CTA kernel's: a pair iteration is two 256-point chunks, CTA r takes
 // chunk 2 it + r.  Cross-CTA protocol: commits are multicast to both CTAs' barriers; the peer's epilogue / positional-encoding warps
 // arrive remotely on the LEADER's event barriers; the peer's (otherwise idle) warp 1 relays "my half of the stage has landed".
-template <bool TRACE, int ABL = 0, bool SAVE = false, bool PAIR = false>
+template <bool TRACE, int ABL = 0, bool SAVE = false, bool PAIR = false, bool EMB = false>
 __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, int n_steps, int n_rays, float* __restrict__ trace) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
     static_assert(!(PAIR && (TRACE || ABL != 0)), "the pair build has no trace / ablation variants");
+    static_assert(!(EMB && (TRACE || ABL != 0)), "the embedded-row build has no trace / ablation variants");
     // Dynamic shared memory is the only shared allocation of this kernel, so it starts at offset 0 of the CTA's
     // window: 1024-byte aligned as the 128B-swizzle atoms need.  (No pointer re-alignment arithmetic here: it would
     // make the compiler lose the shared address space and emit generic LD/ST for every epilogue access.)
@@ -505,9 +517,9 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             for (long long it = it_first; it < n_iter; it += it_step) {
                 for (int s = 0; s < n_steps; ++s, ++g) {
                     const uint32_t stage = g % NSTAGE, round = g / NSTAGE;
-                    if (c_steps[s].first) {            // first step of a (layer, half): its bias tile
-                        const uint32_t slot = bh & 1, l = c_steps[s].layer, h = c_steps[s].acc_col ? 1u : 0u;
-                        const uint32_t bytes = (uint32_t)c_steps[s].n8 * 8u * 32u / SPLIT;
+                    if (step_at<EMB>(s).first) {       // first step of a (layer, half): its bias tile
+                        const uint32_t slot = bh & 1, l = step_at<EMB>(s).layer, h = step_at<EMB>(s).acc_col ? 1u : 0u;
+                        const uint32_t bytes = (uint32_t)step_at<EMB>(s).n8 * 8u * 32u / SPLIT;
                         const uint32_t off = (l < 8 ? (2 * l + h) * 4096u : 65536u + (2 * (l - 8) + h) * 2048u) + rank * bytes;
                         wait_or_report<TRACE>(&bars->bempty[slot], ((bh >> 1) & 1) ^ 1, 102, s, (int)bh);
                         mbar_arrive_expect_tx(&bars->bfull[slot], bytes);
@@ -516,9 +528,9 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                     }
                     if ((ABL & 2) && g >= NSTAGE) continue;
                     wait_or_report<TRACE>(&bars->wempty[stage], (round & 1) ^ 1, 101, s, (int)g);
-                    const uint32_t bytes = (uint32_t)c_steps[s].n8 * 8u * 128u / SPLIT;
+                    const uint32_t bytes = (uint32_t)step_at<EMB>(s).n8 * 8u * 128u / SPLIT;
                     mbar_arrive_expect_tx(&bars->wfull[stage], bytes);
-                    bulk_g2s(sm + OFF_W + stage * STAGE_BYTES, blob + c_steps[s].offset + rank * bytes, bytes, &bars->wfull[stage]);
+                    bulk_g2s(sm + OFF_W + stage * STAGE_BYTES, blob + step_at<EMB>(s).offset + rank * bytes, bytes, &bars->wfull[stage]);
                 }
             }
         }
@@ -528,7 +540,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             uint32_t g = 0, bh = 0;
             for (long long it = it_first; it < n_iter; it += it_step)
                 for (int s = 0; s < n_steps; ++s, ++g) {
-                    if (c_steps[s].first) {
+                    if (step_at<EMB>(s).first) {
                         mbar_wait(&bars->bfull[bh & 1], (bh >> 1) & 1);
                         mbar_arrive_remote(&bars->pbfull[bh & 1], 0);
                         ++bh;
@@ -559,16 +571,16 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             // Layers of equal geometry share ONE copy of the straight-line issue code (L1-L4, L6, L7 are 256 x 256 after a 256-wide
             // layer; V1, V2 are 128 x 128 after a 128-wide one): 11 inlined copies were 78 KB of SASS streamed once per iteration, which
             // together with the epilogue and PE code overflowed the instruction cache the epilogue warps live in (ncu: stall_no_inst).
-            issue_layer<0, TRACE, ABL, PAIR>(c);
+            issue_layer<0, TRACE, ABL, PAIR, EMB>(c);
 #pragma unroll 1
             for (int seg = 0; seg < 2; ++seg) {
 #pragma unroll 1
-                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, TRACE, ABL, PAIR>(c);
-                if (seg == 0) issue_layer<5, TRACE, ABL, PAIR>(c);
+                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, TRACE, ABL, PAIR, EMB>(c);
+                if (seg == 0) issue_layer<5, TRACE, ABL, PAIR, EMB>(c);
             }
-            issue_layer<8, TRACE, ABL, PAIR>(c);
+            issue_layer<8, TRACE, ABL, PAIR, EMB>(c);
 #pragma unroll 1
-            for (int r = 0; r < 2; ++r) issue_layer<9, TRACE, ABL, PAIR>(c);
+            for (int r = 0; r < 2; ++r) issue_layer<9, TRACE, ABL, PAIR, EMB>(c);
         }
 #ifdef INERF_PHASE_TIMERS
         if (lane == 0) {
@@ -606,7 +618,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             long long p = p0 + row;
             const bool in_range = p < a.P;
             if (!in_range) p = a.P - 1;
-            const int ray_local = (int)(p / a.s - min(p0, a.P - 1) / a.s);
+            const int ray_local = EMB ? 0 : (int)(p / a.s - min(p0, a.P - 1) / a.s);      // embedded rows: no per-ray view bias
             float alpha = 0.f, rgb0 = 0.f, rgb1 = 0.f, rgb2 = 0.f;
             for (int l = 0; l < 11; ++l, ++layer_ctr) {
                 const LayerInfo li = layer_info(l);
@@ -619,9 +631,9 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         if (l >= 1) { ph_wait[0] += phl[0]; ph_dur[0] += phl[1]; ph_wait[1] += phl[2]; ph_dur[1] += phl[3]; ph_c1 += phl[4]; }
                         continue;
                     }
-                    if (l == 9) { epi_plain_layer<64, PAIR>(bars, par, t_lane, act_row_u32, soff, lane, phl); continue; }
+                    if (l == 9 || (EMB && l == 8)) { epi_plain_layer<64, PAIR>(bars, par, t_lane, act_row_u32, soff, lane, phl); continue; }
                 }
-                if (l == 8) wait_or_report<TRACE>(&bars->dirb_ready, iter_ctr & 1, 301, l, (int)iter_ctr);
+                if (!EMB && l == 8) wait_or_report<TRACE>(&bars->dirb_ready, iter_ctr & 1, 301, l, (int)iter_ctr);
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
                     long long q0 = 0;
@@ -659,7 +671,10 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                             const bool dump = TRACE && chunk == 0;
                             switch (l) {                                    // layer kind is warp-uniform: one specialised body per chunk
                                 case 7: epi_convert<1, TRACE, SAVE>(r, &packed[c * 16], nullptr, s_aw + f0, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
-                                case 8: epi_convert<2, TRACE, SAVE>(r, &packed[c * 16], s_dirb + (slot * RMAX + ray_local) * 128 + f0, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
+                                case 8:
+                                    if constexpr (EMB) epi_convert<0, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg);
+                                    else epi_convert<2, TRACE, SAVE>(r, &packed[c * 16], s_dirb + (slot * RMAX + ray_local) * 128 + f0, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg);
+                                    break;
                                 case 10: epi_convert<3, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, s_rw + f0, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
                                 default: epi_convert<0, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
                             }
@@ -725,7 +740,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                     if (l >= 1 && l <= 7) { const long long ph3 = PH_CLK(); ph_wait[h] += ph1 - ph0; ph_dur[h] += ph3 - ph1; }
                     if constexpr (TRACE) te_st += clock64() - q0;
                 }
-                if (l == 8) {
+                if (!EMB && l == 8) {
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&bars->dirb_free);
                 }
@@ -752,6 +767,83 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             if (warp == 4 && lane == 0) {
                 float* t = trace + (size_t)11 * 256 * 256 + (148 + blockIdx.x) * 8;
                 t[0] = (float)te_wait; t[1] = (float)te_ld; t[2] = (float)te_c1; t[3] = (float)te_st; t[4] = (float)iter_ctr;
+            }
+        }
+    } else if (EMB && warp >= 12) {
+        // ================= embedded rows: gamma(p), then gamma(v), of row t of both slots, copied from x into the PE buffer ======
+        // A row of x is 90 floats (360 B; 8-byte aligned when x is 16-byte aligned): gamma(p) = columns 0..62 (image column 63 zero),
+        // gamma(v) = columns 63..89 (image columns 27..63 zero).  Each block is in registers before the wait for the buffer, so only the
+        // shared-memory stores lie between its release and the pe_ready arrival.  pe_free parities: 0 = L5 has read gamma(p) of this
+        // iteration, 1 = V0 has read gamma(v) of the previous one.
+        const int t = tid - 12 * 32;
+        const uint32_t row_img = (t >> 3) * 1024 + (t & 7) * 128;
+        auto store_img = [&](uint8_t* img, const uint32_t* w, int n_chunks) {      // one 128-byte row of a swizzled image, zero-padded
+#pragma unroll
+            for (int q = 0; q < 8; ++q)
+                *reinterpret_cast<uint4*>(img + row_img + ((q ^ (t & 7)) << 4)) =
+                    q < n_chunks ? make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]) : make_uint4(0u, 0u, 0u, 0u);
+        };
+        auto arrive_ready = [&] {
+            fence_proxy_async_smem();
+            if constexpr (PAIR) {
+                __syncwarp();
+                if (lane == 0) mbar_arrive_remote(&bars->pe_ready, 0);
+            } else {
+                mbar_arrive(&bars->pe_ready);
+            }
+        };
+        for (long long it = it_first; it < n_iter; it += it_step) {
+            const long long chunk = CHUNK_OF(it);
+            const bool chunk_ok = !PAIR || chunk * 256 < a.P;
+            const float* xr[2];
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl) {
+                long long p = chunk * 256 + sl * 128 + t;
+                if (p > a.P - 1) p = a.P - 1;
+                xr[sl] = a.x + p * 90;
+            }
+            uint32_t pk[2][32];
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl) {
+#pragma unroll
+                for (int j = 0; j < 31; ++j) {
+                    const float2 v = __ldg(reinterpret_cast<const float2*>(xr[sl]) + j);
+                    pk[sl][j] = pack_bf16x2(v.x, v.y);
+                }
+                pk[sl][31] = pack_bf16x2(__ldg(xr[sl] + 62), 0.f);
+            }
+            if (it != it_first) wait_or_report<TRACE>(&bars->pe_free, 1u, 401, 0, 0);
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl) store_img(sm + OFF_PE + sl * 16384, pk[sl], 8);
+            arrive_ready();
+            if (SAVE && chunk_ok) {          // training: gamma(p) is the X operand of dW for pts_linears.0 / .5
+#pragma unroll
+                for (int sl = 0; sl < 2; ++sl)
+                    store_img(a.save_img + (((size_t)chunk * 2 + sl) * TRAIN_IMGS + TRAIN_IMG_PE) * 16384, pk[sl], 8);
+            }
+            uint32_t pv[2][16];
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl) {
+                float g[28];
+                g[0] = __ldg(xr[sl] + 63);
+#pragma unroll
+                for (int j = 0; j < 13; ++j) {
+                    const float2 v = __ldg(reinterpret_cast<const float2*>(xr[sl] + 64) + j);
+                    g[1 + 2 * j] = v.x; g[2 + 2 * j] = v.y;
+                }
+                g[27] = 0.f;
+#pragma unroll
+                for (int j = 0; j < 14; ++j) pv[sl][j] = pack_bf16x2(g[2 * j], g[2 * j + 1]);
+                pv[sl][14] = pv[sl][15] = 0u;
+            }
+            wait_or_report<TRACE>(&bars->pe_free, 0u, 402, 0, 0);
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl) store_img(sm + OFF_PE + sl * 16384, pv[sl], 4);
+            arrive_ready();
+            if (SAVE && chunk_ok) {          // training: gamma(v) per point, the X operand of dW for the view columns of views_linears.0
+#pragma unroll
+                for (int sl = 0; sl < 2; ++sl)
+                    store_img(a.save_img + (((size_t)chunk * 2 + sl) * TRAIN_IMGS + TRAIN_IMG_DIR) * 16384, pv[sl], 4);
             }
         }
     } else if (warp >= 12) {
@@ -905,13 +997,15 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 // ---------------------------------------------------------------------------------------------
 struct LayerDesc { int N, n_act_kb; bool has_pe; int w_index; int ldw, wcol_act; };
 
-Schedule build_schedule(const InerfNetDims* d) {
+// emb: the embedded-row schedule -- V0 gains a last K-block per half, the view columns 256..282 of views_linears.0 (kmax = 27) against
+// the gamma(v) image in the PE buffer; every other step, and the order of all steps, is the fused-entry schedule's.
+Schedule build_schedule(const InerfNetDims* d, bool emb = false) {
     const int C = d->dim_aud + d->dim_expr + d->dim_latent, E = d->dim_expr;
     LayerDesc L[11];
     L[0] = {256, 0, true, 0, 63 + C, 0};
     for (int l = 1; l < 8; ++l) L[l] = {256, 4, false, 2 * l, 256, 0};
     L[5] = {256, 4, true, 10, 319 + C, 63 + C};
-    L[8] = {128, 4, false, P_VIEWS_W, 283 + E, 0};
+    L[8] = {128, 4, emb, P_VIEWS_W, 283 + E, 0};
     L[9] = {128, 2, false, P_VIEWS_W + 2, 128, 0};
     L[10] = {128, 2, false, P_VIEWS_W + 4, 128, 0};
     Schedule S{};
@@ -948,6 +1042,8 @@ Schedule build_schedule(const InerfNetDims* d) {
                     st.wait = (order[i] < kb_per_half) ? W_E0 : W_E1;
                 } else if (l == 0) {
                     st.wait = W_PE | W_E0 | W_E1;             // new iteration: PE ready and both accumulator halves drained
+                } else if (l == 8 && h == 0) {
+                    st.wait = W_PE;                           // embedded rows: the gamma(v) image is in the PE buffer
                 }
                 st.commit = 0;
                 const bool last = (i == cnt - 1);
@@ -955,11 +1051,11 @@ Schedule build_schedule(const InerfNetDims* d) {
                 if (h == 1) {
                     if (n_first > 0 ? (i == n_first - 1) : last) st.commit |= C_C1;
                     if (last) st.commit |= C_C2;
-                    if (last && l == 5) st.commit |= C_PEFREE;
+                    if (last && (l == 5 || l == 8)) st.commit |= C_PEFREE;
                 }
                 st.offset = off;
                 pk.w_index = L[l].w_index; pk.ldw = L[l].ldw; pk.n0 = h * NH; pk.rows = NH; pk.offset = off;
-                if (order[i] == 4) { pk.wcol = 0; pk.kmax = 63; }
+                if (order[i] == 4) { pk.wcol = l == 8 ? 256 : 0; pk.kmax = l == 8 ? 27 : 63; }
                 else { pk.wcol = L[l].wcol_act + order[i] * 64; pk.kmax = 64; }
                 off += (uint32_t)NH * 128u;
                 ++n;
@@ -994,15 +1090,15 @@ __global__ void pack_kernel(const __grid_constant__ PackArgs pa) {
 
 namespace inerf {
 
-int mlp_bf16_packed_bytes(const InerfNetDims* d, size_t* bytes) {
-    Schedule S = build_schedule(d);
+int mlp_bf16_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded) {
+    Schedule S = build_schedule(d, embedded);
     *bytes = (size_t)S.total_bytes;
     return INERF_OK;
 }
 
-int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st) {
+int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded) {
     if ((uintptr_t)packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_pack: packed must be 16-byte aligned");
-    Schedule S = build_schedule(d);
+    Schedule S = build_schedule(d, embedded);
     PackArgs pa{};
     for (int i = 0; i < INERF_N_PARAMS; ++i) pa.w[i] = params_host[i];
     for (int i = 0; i < S.n_steps; ++i) pa.st[i] = S.pack[i];
@@ -1037,11 +1133,11 @@ int mlp_bf16_hang_info(int32_t* out8) {
     return INERF_OK;
 }
 
-template <bool SAVE>
+template <bool SAVE, bool EMB = false>
 static int launch_pair(const MlpArgs& a, int n_steps, int n_rays, int dev, cudaStream_t st) {
     static thread_local int pair_dev = -1;
     if (pair_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, SAVE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
+        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, SAVE, true, EMB>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
         if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
         pair_dev = dev;
     }
@@ -1057,14 +1153,47 @@ static int launch_pair(const MlpArgs& a, int n_steps, int n_rays, int dev, cudaS
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, mlp_bf16_kernel<false, 0, SAVE, true>, a, n_steps, n_rays, (float*)nullptr);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, mlp_bf16_kernel<false, 0, SAVE, true, EMB>, a, n_steps, n_rays, (float*)nullptr);
     if (e != cudaSuccess) { set_error("inerf_mlp_fwd[bf16 pair]: %s", cudaGetErrorString(e)); return (int)e; }
     return check_launch(SAVE ? "inerf_mlp_fwd_train[bf16 pair]" : "inerf_mlp_fwd[bf16 pair]");
 }
 
+// the CTA-pair build (clusters of two) runs the inference and the activation-saving forward; INERF_MLP_PAIR=0 (read once) keeps the
+// single-CTA kernels for A/B runs, which also serve the trace / ablation builds
+static bool pair_enabled() {
+    static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
+    return pair_env && num_sms() >= 2;
+}
+
+// FaceNeRF.forward on embedded rows x (P, 90): a.packed is an INERF_MLP_BF16_EMB blob, a.save_img != NULL selects the saving build
+static int launch_embedded(const MlpArgs& a, cudaStream_t st) {
+    if (((uintptr_t)a.packed | (uintptr_t)a.x) & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd_embedded: packed weights and x must be 16-byte aligned");
+    if (a.save_img && !a.save_mask) return fail(INERF_E_ARG, "mlp_bf16: save_mask is NULL");
+    static thread_local int configured_dev = -1;
+    static const Schedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_schedule(&d, true); }();
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (configured_dev != dev) {
+        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
+        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_steps_emb, S.steps, sizeof(Step) * MAX_STEPS);
+        if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
+        configured_dev = dev;
+    }
+    if (pair_enabled())
+        return a.save_img ? launch_pair<true, true>(a, S.n_steps, 0, dev, st) : launch_pair<false, true>(a, S.n_steps, 0, dev, st);
+    const long long n_iter = (a.P + 255) / 256;
+    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
+    if (a.save_img) {
+        mlp_bf16_kernel<false, 0, true, false, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, 0, nullptr);
+        return check_launch("inerf_mlp_fwd_train_bf16_embedded");
+    }
+    mlp_bf16_kernel<false, 0, false, false, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, 0, nullptr);
+    return check_launch("inerf_mlp_fwd_embedded[bf16]");
+}
+
 int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
-    if (embedded)
-        return fail(INERF_E_UNSUPPORTED, "bf16 mode is built for the fused (rays, z) entry; FaceNeRF.forward on embedded rows runs in fp32 mode");
+    if (embedded) return launch_embedded(a, st);
     if (a.s < 43) return fail(INERF_E_UNSUPPORTED, "bf16 mode needs at least 43 samples per ray (a 128-row slot may touch at most 4 rays)");
     if ((uintptr_t)a.packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: packed weights must be 16-byte aligned");
     static thread_local int configured_dev = -1;
@@ -1082,10 +1211,7 @@ int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
     const long long n_iter = (a.P + 255) / 256;
     const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
     const int n_rays = (int)(a.P / a.s);
-    // the CTA-pair build (clusters of two) runs the inference and the activation-saving forward; INERF_MLP_PAIR=0 (read once) keeps the
-    // single-CTA kernels for A/B runs, which also serve the trace / ablation builds
-    static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
-    const bool use_pair = pair_env && num_sms() >= 2 && !a.trace;
+    const bool use_pair = pair_enabled() && !a.trace;
     if (a.trace) {
         if (!g_hang_host) {
             int* dptr = nullptr;

@@ -40,7 +40,8 @@ __host__ __device__ constexpr int train_img_of(int l) { return l < 8 ? 4 * l : 3
 __host__ __device__ constexpr int train_mask_of(int l) { return l < 8 ? 8 * l : 64 + 4 * (l - 8); }
 
 int mlp_fp32_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
-int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st);     // a.save_img != NULL: the activation-saving build
+// embedded: rows of a.x (P, 90) with an INERF_MLP_BF16_EMB blob; otherwise points of rays/z.  a.save_img != NULL: the activation-saving build
+int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
 int mlp_fp32_bwd_launch(const InerfNetDims* dims, const float* const* params_host, float* const* grads_host,
                         const float* aud, const float* expr, const float* latent, const float* acts, float* deltas,
                         const float* d_raw, long long P, float* d_cond, void* dw_args_dev, cudaStream_t st);
@@ -60,7 +61,8 @@ int mlp_bf16_dw_launch(const InerfNetDims* dims, float* const* grads_host, const
                        long long n_tiles, void* scratch, cudaStream_t st);
 int mlp_bwd_cond_launch(const InerfNetDims* dims, const float* const* params_host, float* const* grads_host, const float* aud,
                         const float* expr, const float* latent, float* d_cond, cudaStream_t st);
-int mlp_bf16_packed_bytes(const InerfNetDims* d, size_t* bytes);
-int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st);
+// embedded: the INERF_MLP_BF16_EMB blob of FaceNeRF.forward's embedded-row kernel instead of the fused entry's INERF_MLP_BF16 blob
+int mlp_bf16_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded = false);
+int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded = false);
 
 }  // namespace inerf

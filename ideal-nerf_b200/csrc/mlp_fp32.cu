@@ -362,6 +362,7 @@ extern "C" int inerf_mlp_packed_bytes(int mode, const InerfNetDims* dims, size_t
     if (!bytes) return fail(INERF_E_ARG, "inerf_mlp_packed_bytes: NULL");
     if (mode == INERF_MLP_FP32) { *bytes = 0; return INERF_OK; }
     if (mode == INERF_MLP_BF16) return mlp_bf16_packed_bytes(dims, bytes);
+    if (mode == INERF_MLP_BF16_EMB) return mlp_bf16_packed_bytes(dims, bytes, true);
     if (mode == INERF_MLP_BF16_BWD) return mlp_bf16_bwd_packed_bytes(dims, bytes);
     if (mode == INERF_MLP_F16X2) return mlp_f16x2_packed_bytes(dims, bytes);
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_packed_bytes: unknown mode");
@@ -375,6 +376,10 @@ extern "C" int inerf_mlp_pack(int mode, const InerfNetDims* dims, const float* c
     if (mode == INERF_MLP_BF16) {
         if (!params_host || !packed) return fail(INERF_E_ARG, "inerf_mlp_pack: NULL pointer");
         return mlp_bf16_pack(dims, params_host, packed, as_stream(stream));
+    }
+    if (mode == INERF_MLP_BF16_EMB) {
+        if (!params_host || !packed) return fail(INERF_E_ARG, "inerf_mlp_pack: NULL pointer");
+        return mlp_bf16_pack(dims, params_host, packed, as_stream(stream), true);
     }
     if (mode == INERF_MLP_BF16_BWD) {
         if (!params_host || !packed) return fail(INERF_E_ARG, "inerf_mlp_pack: NULL pointer");
@@ -495,7 +500,7 @@ extern "C" int inerf_mlp_fwd_embedded(int mode, const InerfNetDims* dims, const 
     a.x = x; a.P = p; a.out = out; a.packed = packed; a.s = 1;
     if (mode == INERF_MLP_FP32) return mlp_fp32_launch(a, true, as_stream(stream));
     if (mode == INERF_MLP_BF16) {
-        if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd_embedded: bf16 mode needs packed weights");
+        if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd_embedded: bf16 mode needs packed weights (INERF_MLP_BF16_EMB)");
         return mlp_bf16_launch(a, true, as_stream(stream));
     }
     if (mode == INERF_MLP_F16X2)
@@ -531,6 +536,22 @@ extern "C" int inerf_mlp_fwd_train_bf16(const InerfNetDims* dims, const float* c
     a.rays = rays; a.ray_stride = ray_stride; a.z = z; a.s = s; a.P = (long long)n * s; a.out = raw; a.packed = packed;
     a.save_img = reinterpret_cast<uint8_t*>(acts); a.save_mask = reinterpret_cast<uint32_t*>(mask);
     return mlp_bf16_launch(a, false, as_stream(stream));
+}
+
+extern "C" int inerf_mlp_fwd_train_bf16_embedded(const InerfNetDims* dims, const float* const* params_host, const void* packed,
+                                                 const float* cond, const float* x, int64_t p, float* raw, void* acts, void* mask,
+                                                 void* stream) {
+    MlpArgs a{};
+    int rc = fill_args(a, dims, params_host, cond);
+    if (rc) return rc;
+    if (p < 0) return fail(INERF_E_SHAPE, "inerf_mlp_fwd_train_bf16_embedded: p < 0");
+    if (p == 0) return INERF_OK;
+    if (!x || !raw || !packed || !acts || !mask) return fail(INERF_E_ARG, "inerf_mlp_fwd_train_bf16_embedded: NULL pointer");
+    if (((uintptr_t)x | (uintptr_t)raw | (uintptr_t)acts | (uintptr_t)mask) & 15)
+        return fail(INERF_E_ALIGN, "inerf_mlp_fwd_train_bf16_embedded: x/raw/acts/mask must be 16-byte aligned");
+    a.x = x; a.P = p; a.s = 1; a.out = raw; a.packed = packed;
+    a.save_img = reinterpret_cast<uint8_t*>(acts); a.save_mask = reinterpret_cast<uint32_t*>(mask);
+    return mlp_bf16_launch(a, true, as_stream(stream));
 }
 
 extern "C" int inerf_mlp_bwd_bf16(const InerfNetDims* dims, const float* const* params_host, const void* packed_t,

@@ -11,8 +11,9 @@ import torch.nn as nn
 
 from . import _lib, ops
 
-# "fp16x2": tensor cores at fp32-gate accuracy (fp16 hi/lo operand pairs, three MMA passes); inference kernel -- training in this mode
-# runs the fp32 kernels, like "fp32"
+# "bf16": tcgen05 kernels for inference and training, on both entries -- query(rays, z) and forward(x) on embedded rows (the latter with
+# its own packed blob, INERF_MLP_BF16_EMB).  "fp16x2": tensor cores at fp32-gate accuracy (fp16 hi/lo operand pairs, three MMA passes)
+# on query(); inference kernel -- training in this mode, and forward(x) on embedded rows, run the fp32 kernels, like "fp32"
 MODES = {"fp32": _lib.INERF_MLP_FP32, "bf16": _lib.INERF_MLP_BF16, "fp16x2": _lib.INERF_MLP_F16X2}
 
 
@@ -46,6 +47,8 @@ class FaceNeRF(nn.Module):
         self._packed_key = None
         self._packed_t = None
         self._packed_t_key = None
+        self._packed_e = None
+        self._packed_e_key = None
 
     # -- plumbing -------------------------------------------------------------------------------
     def kernel_params(self):
@@ -70,6 +73,7 @@ class FaceNeRF(nn.Module):
         re-packs on every call and invalidates afterwards) and train() / eval() switches drop it as well."""
         self._packed = self._packed_key = None
         self._packed_t = self._packed_t_key = None
+        self._packed_e = self._packed_e_key = None
 
     def train(self, mode=True):
         self.invalidate_packed()
@@ -93,6 +97,14 @@ class FaceNeRF(nn.Module):
             self._packed_t = ops.pack_weights(_lib.INERF_MLP_BF16_BWD, self._dims, [p.detach() for p in params])
             self._packed_t_key = key
         return self._packed_t
+
+    def packed_weights_emb(self, params):
+        """bf16 stage images of the embedded-row kernel (FaceNeRF.forward), re-packed when a parameter changed."""
+        key = tuple((p.data_ptr(), p._version) for p in params)
+        if key != self._packed_e_key:
+            self._packed_e = ops.pack_weights(_lib.INERF_MLP_BF16_EMB, self._dims, [p.detach() for p in params])
+            self._packed_e_key = key
+        return self._packed_e
 
     def _prep(self, aud, expr, latent_code):
         params = self.kernel_params()
@@ -140,10 +152,11 @@ class _MlpFn(torch.autograd.Function):
             ctx.net, ctx.has = net, (aud is not None, expr is not None, latent is not None)
             ctx.cond_shapes = tuple(None if t is None else t.shape for t in (aud, expr, latent))
             if mode == _lib.INERF_MLP_BF16:
-                if embedded:
-                    raise NotImplementedError("bf16 training runs through the fused (rays, z) entry; FaceNeRF.forward on embedded rows trains in mlp_mode='fp32'")
                 net.invalidate_packed()                       # optimiser steps may not bump parameter versions (fused Adam)
-                out, acts, mask, n_points = ops.mlp_fwd_train_bf16(net._dims, pd, net.packed_weights(params), cond, a, b)
+                if embedded:
+                    out, acts, mask, n_points = ops.mlp_fwd_train_bf16(net._dims, pd, net.packed_weights_emb(params), cond, x=a)
+                else:
+                    out, acts, mask, n_points = ops.mlp_fwd_train_bf16(net._dims, pd, net.packed_weights(params), cond, a, b)
                 ctx.n_points, ctx.bf16 = n_points, True
                 ctx.save_for_backward(acts, mask, *[t for t in (aud_d, expr_d, lat_d) if t is not None], *pd)
                 ctx.packed_t = net.packed_weights_bwd(params)
@@ -155,6 +168,8 @@ class _MlpFn(torch.autograd.Function):
             ctx.n_points, ctx.bf16 = n_points, False
             ctx.save_for_backward(acts, *[t for t in (aud_d, expr_d, lat_d) if t is not None], *pd)
             return out
+        if embedded and mode == _lib.INERF_MLP_BF16:
+            return ops.mlp_fwd_embedded(mode, net._dims, pd, net.packed_weights_emb(params), cond, a)
         packed = net.packed_weights(params)
         if embedded:                                         # FaceNeRF.forward on embedded rows: fp16x2 shares the fp32 kernel there
             m = _lib.INERF_MLP_FP32 if mode == _lib.INERF_MLP_F16X2 else mode

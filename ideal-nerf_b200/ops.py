@@ -599,19 +599,28 @@ def _train_sizes_bf16(dims, n_points):
     return [v.value for v in sizes]          # acts, mask, deltas, scratch (bytes)
 
 
-def mlp_fwd_train_bf16(dims, params, packed, cond, rays, z):
-    """bf16 tensor-core forward that keeps the activation images + ReLU masks for mlp_bwd_bf16.  Returns (raw, acts, mask, n_points)."""
-    rays, z = f32c(rays, "rays"), f32c(z, "z_vals")
-    n, s = z.shape
-    n_points, dev = n * s, z.device
+def mlp_fwd_train_bf16(dims, params, packed, cond, rays=None, z=None, x=None):
+    """bf16 tensor-core forward that keeps the activation images + ReLU masks for mlp_bwd_bf16.  Returns (raw, acts, mask, n_points).
+    rays (n,11) / z (n,s) with the INERF_MLP_BF16 blob, or embedded rows x (P, 90) with the INERF_MLP_BF16_EMB blob."""
+    if x is None:
+        rays, z = f32c(rays, "rays"), f32c(z, "z_vals")
+        n, s = z.shape
+        n_points, dev, out_shape = n * s, z.device, (n, s, 4)
+    else:
+        x = _rows90(x)
+        n_points, dev, out_shape = x.shape[0], x.device, (x.shape[0], 4)
     acts_b, mask_b, _, _ = _train_sizes_bf16(dims, n_points)
-    raw = torch.empty((n, s, 4), device=dev)
+    raw = torch.empty(out_shape, device=dev)
     acts = torch.empty((acts_b,), device=dev, dtype=torch.uint8)
     mask = torch.empty((mask_b,), device=dev, dtype=torch.uint8)
     arr = param_array(params)
     with torch.cuda.device(dev):
-        call("inerf_mlp_fwd_train", _lib.lib().inerf_mlp_fwd_train_bf16, ctypes.byref(dims), arr, ptr(packed), ptr(cond), ptr(rays),
-             rays.shape[1], ptr(z), n, s, ptr(raw), ptr(acts), ptr(mask), stream())
+        if x is None:
+            call("inerf_mlp_fwd_train", _lib.lib().inerf_mlp_fwd_train_bf16, ctypes.byref(dims), arr, ptr(packed), ptr(cond), ptr(rays),
+                 rays.shape[1], ptr(z), n, s, ptr(raw), ptr(acts), ptr(mask), stream())
+        else:
+            call("inerf_mlp_fwd_train_bf16_embedded", _lib.lib().inerf_mlp_fwd_train_bf16_embedded, ctypes.byref(dims), arr, ptr(packed),
+                 ptr(cond), ptr(x), n_points, ptr(raw), ptr(acts), ptr(mask), stream())
     return raw, acts, mask, n_points
 
 
@@ -657,9 +666,17 @@ def mlp_fwd_trace(mode, dims, params, packed, cond, rays, z):
     return raw, trace[:11 * 256 * 256].reshape(11, 256, 256)
 
 
-def mlp_fwd_embedded(mode, dims, params, packed, cond, x):
+def _rows90(x):
+    """x as the embedded-row kernels read it: contiguous fp32 (P, 90), 16-byte aligned as the bf16 kernel needs (a row slice may start off
+    alignment)."""
     x = f32c(x, "x")
     assert x.dim() == 2 and x.shape[1] == 90, "x must be (P, 63+27)"
+    return x if x.data_ptr() % 16 == 0 else x.clone()
+
+
+def mlp_fwd_embedded(mode, dims, params, packed, cond, x):
+    """FaceNeRF.forward on embedded rows x (P, 90) -> (P, 4).  bf16 mode takes the INERF_MLP_BF16_EMB blob."""
+    x = _rows90(x)
     out = torch.empty((x.shape[0], 4), device=x.device)
     arr = param_array(params)
     with torch.cuda.device(x.device):

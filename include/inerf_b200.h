@@ -20,9 +20,10 @@
  * Limits (every one is reported as INERF_E_UNSUPPORTED / INERF_E_SHAPE with a message, never silently worked around):
  *   - FaceNeRF geometry: D = 8, W = 256, skips = [4], in_xyz = 63, in_views = 27, use_viewdirs (the configuration of every reference
  *     script); conditioning dims are free (head 64 + 76 + 32, torso 106 + 0 + 0, ...);
- *   - the tensor-core modes (INERF_MLP_BF16, INERF_MLP_F16X2) need s >= 43 samples per ray (a 128-row slot may touch at most four
- *     rays) and exist for the fused (rays, z) entry inerf_mlp_fwd; inerf_mlp_fwd_embedded runs INERF_MLP_FP32 only;
- *   - training entry points exist for INERF_MLP_FP32 and INERF_MLP_BF16 (INERF_MLP_F16X2 is an inference mode);
+ *   - on the fused (rays, z) entry inerf_mlp_fwd the tensor-core modes (INERF_MLP_BF16, INERF_MLP_F16X2) need s >= 43 samples per
+ *     ray (a 128-row slot may touch at most four rays); inerf_mlp_fwd_embedded runs INERF_MLP_FP32 and INERF_MLP_BF16 on any number
+ *     of rows (INERF_MLP_F16X2 is built for the fused entry only);
+ *   - training entry points exist for INERF_MLP_FP32 and INERF_MLP_BF16, on both entries (INERF_MLP_F16X2 is an inference mode);
  *   - sample_pdf: 2 <= n_bins <= 1024, n_imp <= 1024, the per-ray working set within 48 KB of shared memory; s <= 4096 elsewhere.
  */
 #ifndef INERF_B200_H
@@ -51,8 +52,11 @@ enum {
     INERF_MLP_FP32 = 0, /* fp32 FFMA, weights read in nn.Linear layout                         */
     INERF_MLP_BF16 = 1, /* bf16 operands, fp32 accumulate in TMEM, tcgen05.mma (packed weights) */
     INERF_MLP_BF16_BWD = 2, /* inerf_mlp_packed_bytes / inerf_mlp_pack only: the TRANSPOSED stage images of the bf16 backward chain */
-    INERF_MLP_F16X2 = 3 /* fp32-gate tensor-core mode: every operand an fp16 (hi, lo) pair, three tcgen05 passes per product
+    INERF_MLP_F16X2 = 3, /* fp32-gate tensor-core mode: every operand an fp16 (hi, lo) pair, three tcgen05 passes per product
                            (hi.hi + lo.hi + hi.lo), fp32 accumulate in TMEM -- meets the <= 1e-3 max-abs gate (inference entry only) */
+    INERF_MLP_BF16_EMB = 4 /* inerf_mlp_packed_bytes / inerf_mlp_pack only: the stage images of the bf16 kernel on EMBEDDED rows
+                              (inerf_mlp_fwd_embedded, inerf_mlp_fwd_train_bf16_embedded): the INERF_MLP_BF16 schedule plus one
+                              K-block per half of views_linears.0 for its 27 view columns */
 };
 
 /* sample_pdf summation policies (SURVEY.md 7-1) */
@@ -340,12 +344,18 @@ int inerf_mlp_bwd(const InerfNetDims* dims, const float* const* params_host, flo
  * Same contract as the fp32 pair above, with bf16 operands on tcgen05: the forward keeps every post-ReLU activation as the 16 KB
  * shared-memory images of its own A operands plus one ReLU-mask bit per activation; the backward is a fused chain kernel
  * (delta_{l-1} = delta_l . W_l * mask, weights streamed TRANSPOSED, inerf_mlp_pack mode INERF_MLP_BF16_BWD), one long-K tcgen05 GEMM
- * per weight matrix for dW / db straight from those images, and the fp32 conditioning kernel.  Needs n*s points with s >= 43. */
+ * per weight matrix for dW / db straight from those images, and the fp32 conditioning kernel.  The fused entry needs n*s points with
+ * s >= 43; the embedded-row entry takes any number of rows. */
 int inerf_mlp_train_sizes_bf16(const InerfNetDims* dims, int64_t n_points, size_t* acts_bytes, size_t* mask_bytes,
                                size_t* deltas_bytes, size_t* scratch_bytes);
 int inerf_mlp_fwd_train_bf16(const InerfNetDims* dims, const float* const* params_host, const void* packed, const float* cond,
                              const float* rays, int ray_stride, const float* z, int n, int s, float* raw, void* acts, void* mask,
                              void* stream);
+/* inerf_mlp_fwd_train_bf16 on embedded rows x (p, in_xyz+in_views), FaceNeRF.forward's input: packed is an INERF_MLP_BF16_EMB blob;
+ * acts / mask are sized by inerf_mlp_train_sizes_bf16(dims, p, ...) and hold the same images, so inerf_mlp_bwd_bf16 (n_points = p)
+ * is the backward.  Any p >= 0 (0 enqueues nothing); x, raw (p, 4), acts and mask 16-byte aligned. */
+int inerf_mlp_fwd_train_bf16_embedded(const InerfNetDims* dims, const float* const* params_host, const void* packed, const float* cond,
+                                      const float* x, int64_t p, float* raw, void* acts, void* mask, void* stream);
 /* grads_host: ZERO-INITIALISED gradient tensors (nn.Linear layout, fp32); d_cond as in inerf_mlp_bwd. */
 int inerf_mlp_bwd_bf16(const InerfNetDims* dims, const float* const* params_host, const void* packed_t, float* const* grads_host,
                        const float* aud, const float* expr, const float* latent, const void* acts, const void* mask, void* deltas,
@@ -377,7 +387,9 @@ int inerf_audio_att_bwd(const float* const* params_host, float* const* grads_hos
 int inerf_debug_hang_info(int32_t* out8);
 
 /* FaceNeRF.forward on already-embedded inputs x (p, in_xyz+in_views) -- the reference module's own
- * call signature (face_nerf.py:40).  out (p, 4). */
+ * call signature (face_nerf.py:40).  out (p, 4).  Any p >= 0 (0 enqueues nothing).
+ * INERF_MLP_FP32: packed is ignored.  INERF_MLP_BF16: the tcgen05 kernel; packed must be an INERF_MLP_BF16_EMB blob (not the
+ * INERF_MLP_BF16 blob of inerf_mlp_fwd) and x 16-byte aligned.  INERF_MLP_F16X2: INERF_E_UNSUPPORTED. */
 int inerf_mlp_fwd_embedded(int mode, const InerfNetDims* dims, const float* const* params_host,
                            const void* packed, const float* cond, const float* x, int64_t p, float* out,
                            void* stream);
