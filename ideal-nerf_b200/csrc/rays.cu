@@ -249,11 +249,18 @@ extern "C" int inerf_flag_nonfinite(const float* const* xs_host, const int64_t* 
 // ---------------------------------------------------------------------------------------------
 // head/torso blend.  train_torso.py:269-270
 // ---------------------------------------------------------------------------------------------
+// one value of rgb_head * last_weight_torso[..., None] + rgb_fg_torso; shared by blend_kernel and head_torso_to8b_kernel so that both
+// entry points round the same way
+__device__ __forceinline__ float blend_value(float head, float lw, float fg) { return __fadd_rn(__fmul_rn(head, lw), fg); }
+
+// (255 * clip(x, 0, 1)).astype(uint8): float -> int truncates like astype
+__device__ __forceinline__ uint8_t to8b_value(float x) { return (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(x, 0.f), 1.f)); }
+
 __global__ void blend_kernel(const float* __restrict__ rgb_head, const float* __restrict__ lw,
                              const float* __restrict__ fg, int n, float* __restrict__ rgb) {
     int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= n * 3) return;
-    rgb[idx] = __fadd_rn(__fmul_rn(rgb_head[idx], lw[idx / 3]), fg[idx]);
+    rgb[idx] = blend_value(rgb_head[idx], lw[idx / 3], fg[idx]);
 }
 
 extern "C" int inerf_head_torso_blend(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso,
@@ -274,14 +281,9 @@ __global__ void to8b_kernel(const float* __restrict__ x, long long n, uint8_t* _
     if (i >= n) return;
     if (i + 3 < n && ((uintptr_t)(x + i) & 15) == 0 && ((uintptr_t)(out + i) & 3) == 0) {
         const float4 v = *reinterpret_cast<const float4*>(x + i);
-        uchar4 o;
-        o.x = (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(v.x, 0.f), 1.f));      // float -> int truncates like astype
-        o.y = (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(v.y, 0.f), 1.f));
-        o.z = (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(v.z, 0.f), 1.f));
-        o.w = (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(v.w, 0.f), 1.f));
-        *reinterpret_cast<uchar4*>(out + i) = o;
+        *reinterpret_cast<uchar4*>(out + i) = make_uchar4(to8b_value(v.x), to8b_value(v.y), to8b_value(v.z), to8b_value(v.w));
     } else {
-        for (long long j = i; j < n && j < i + 4; ++j) out[j] = (uint8_t)(int)__fmul_rn(255.f, fminf(fmaxf(x[j], 0.f), 1.f));
+        for (long long j = i; j < n && j < i + 4; ++j) out[j] = to8b_value(x[j]);
     }
 }
 
@@ -292,4 +294,44 @@ extern "C" int inerf_to8b(const float* x, int64_t n, uint8_t* out, void* stream)
     const long long threads = (n + 3) / 4;
     to8b_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, as_stream(stream)>>>(x, n, out);
     return check_launch("inerf_to8b");
+}
+
+// ---------------------------------------------------------------------------------------------
+// blend + to8b in one pass: the composited head + torso frame of test_torso.py:523-524 leaves a band as bytes.  Four values per thread
+// like to8b_kernel; value i belongs to ray i / 3.  out_rgb (optional) receives the fp32 blend.
+// ---------------------------------------------------------------------------------------------
+__global__ void head_torso_to8b_kernel(const float* __restrict__ rgb_head, const float* __restrict__ lw, const float* __restrict__ fg,
+                                       long long n_values, uint8_t* __restrict__ out, float* __restrict__ rgb) {
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
+    if (i >= n_values) return;
+    if (i + 3 < n_values && (((uintptr_t)(rgb_head + i) | (uintptr_t)(fg + i) | (rgb ? (uintptr_t)(rgb + i) : 0)) & 15) == 0 &&
+        ((uintptr_t)(out + i) & 3) == 0) {
+        // values i .. i + 3 span rays `ray` (value i) and `ray + 1` (value i + 3, always: i + 3 - 3 * ray >= 3)
+        const long long ray = i / 3;
+        const int m = (int)(i - ray * 3);
+        const float4 h = *reinterpret_cast<const float4*>(rgb_head + i), f = *reinterpret_cast<const float4*>(fg + i);
+        const float w0 = lw[ray], w1 = lw[ray + 1];
+        const float4 c = make_float4(blend_value(h.x, w0, f.x), blend_value(h.y, m + 1 < 3 ? w0 : w1, f.y),
+                                     blend_value(h.z, m + 2 < 3 ? w0 : w1, f.z), blend_value(h.w, w1, f.w));
+        if (rgb) *reinterpret_cast<float4*>(rgb + i) = c;
+        *reinterpret_cast<uchar4*>(out + i) = make_uchar4(to8b_value(c.x), to8b_value(c.y), to8b_value(c.z), to8b_value(c.w));
+    } else {
+        for (long long j = i; j < n_values && j < i + 4; ++j) {
+            const float c = blend_value(rgb_head[j], lw[j / 3], fg[j]);
+            if (rgb) rgb[j] = c;
+            out[j] = to8b_value(c);
+        }
+    }
+}
+
+extern "C" int inerf_head_torso_to8b(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso, int64_t n,
+                                     uint8_t* out_u8, float* out_rgb, void* stream) {
+    if (n < 0) return fail(INERF_E_SHAPE, "inerf_head_torso_to8b: n < 0");
+    if (n > 0x7fffffffLL * 256 * 4 / 3) return fail(INERF_E_SHAPE, "inerf_head_torso_to8b: too many rays for one launch");
+    if (n == 0) return INERF_OK;
+    if (!rgb_head || !last_weight_torso || !rgb_fg_torso || !out_u8) return fail(INERF_E_ARG, "inerf_head_torso_to8b: NULL pointer");
+    const long long threads = (3 * n + 3) / 4;
+    head_torso_to8b_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, as_stream(stream)>>>(rgb_head, last_weight_torso, rgb_fg_torso,
+                                                                                           3 * n, out_u8, out_rgb);
+    return check_launch("inerf_head_torso_to8b");
 }

@@ -352,6 +352,26 @@ def head_torso_blend(rgb_head, last_weight_torso, rgb_fg_torso):
     return _Blend.apply(rgb_head, last_weight_torso, rgb_fg_torso)
 
 
+def head_torso_to8b(rgb_head, last_weight_torso, rgb_fg_torso, out=None, out_rgb=None):
+    """to8b(head_torso_blend(...)) in one kernel (test_torso.py:523-524), no autograd: (n, 3) uint8 for n rays, written into `out` when
+    given.  out_rgb: None, or a contiguous float32 tensor of 3n values that receives the fp32 blend."""
+    a, b, c = f32c(rgb_head.detach(), "rgb_head"), f32c(last_weight_torso.detach(), "last_weight"), f32c(rgb_fg_torso.detach(), "rgb_fg")
+    n = a.numel() // 3
+    if a.numel() != 3 * n or b.numel() != n or c.numel() != 3 * n:
+        raise ValueError(f"head_torso_to8b: rgb_head {tuple(a.shape)}, last_weight {tuple(b.shape)}, rgb_fg {tuple(c.shape)} are not "
+                         "(n,3), (n), (n,3)")
+    if out is None:
+        out = torch.empty((n, 3), device=a.device, dtype=torch.uint8)
+    for t, dt, name in ((out, torch.uint8, "out"), (out_rgb, torch.float32, "out_rgb")):
+        if t is not None:
+            _need_cuda(t, name)
+            if t.dtype != dt or t.numel() != 3 * n or not t.is_contiguous():
+                raise ValueError(f"head_torso_to8b: `{name}` must be a contiguous {dt} tensor of {3 * n} values")
+    with torch.cuda.device(a.device):
+        call("inerf_head_torso_to8b", _lib.lib().inerf_head_torso_to8b, ptr(a), ptr(b), ptr(c), n, ptr(out), ptr(out_rgb), stream())
+    return out
+
+
 # ------------------------------------------------------------------------------------------------
 # importance sampling
 # ------------------------------------------------------------------------------------------------

@@ -184,6 +184,12 @@ int inerf_mse_pair(const float* rgb, const float* rgb0, const float* target, int
 int inerf_head_torso_blend(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso,
                            int n, float* rgb, void* stream);
 
+/* The blend followed by to8b in one pass, for n rays: out_u8 (n,3) bytes = inerf_to8b(inerf_head_torso_blend(...)) bit for bit, and
+ * out_rgb (n,3) = the fp32 blend, or NULL to skip it.  Replaces test_torso.py:523-524 on the rendered frame: a band of the composited
+ * head + torso image leaves the GPU as 3n bytes.  Any alignment (16-byte aligned pointers take the vector path); n == 0 enqueues nothing. */
+int inerf_head_torso_to8b(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso, int64_t n,
+                          uint8_t* out_u8, float* out_rgb, void* stream);
+
 /* ---- importance sampling -------------------------------------------------------------------- */
 
 /* sample_pdf.  Replaces helper.py:269-313.
