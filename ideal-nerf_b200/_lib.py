@@ -18,7 +18,7 @@ SOURCES = ["api.cu", "rays.cu", "composite.cu", "sample_pdf.cu", "mlp_fp32.cu", 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--shared"]
 
-INERF_MLP_FP32, INERF_MLP_BF16, INERF_MLP_BF16_BWD, INERF_MLP_F16X2, INERF_MLP_BF16_EMB = 0, 1, 2, 3, 4
+INERF_MLP_FP32, INERF_MLP_BF16, INERF_MLP_BF16_BWD, INERF_MLP_F16X2, INERF_MLP_BF16_EMB, INERF_MLP_F16X2_EMB = 0, 1, 2, 3, 4, 5
 INERF_PDF_EXACT_TORCH_CPU, INERF_PDF_FAST = 0, 1
 N_PARAMS = 26
 

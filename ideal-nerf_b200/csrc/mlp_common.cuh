@@ -46,9 +46,11 @@ int mlp_fp32_bwd_launch(const InerfNetDims* dims, const float* const* params_hos
                         const float* aud, const float* expr, const float* latent, const float* acts, float* deltas,
                         const float* d_raw, long long P, float* d_cond, void* dw_args_dev, cudaStream_t st);
 size_t mlp_fp32_bwd_args_bytes();
-int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes);                                     // fp32-gate tensor-core mode (mlp_f16x2.cu)
-int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st);
-int mlp_f16x2_launch(const MlpArgs& a, cudaStream_t st);
+// fp32-gate tensor-core mode (mlp_f16x2.cu).  embedded: the INERF_MLP_F16X2_EMB blob / rows of a.x (P, 90) instead of the fused entry's
+// INERF_MLP_F16X2 blob / points of rays, z
+int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded = false);
+int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded = false);
+int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
 int mlp_bf16_hang_info(int32_t* out8);
 void mlp_bf16_stage_offsets(uint32_t (*off)[2][5]);      // [11 layers][half][K-block index in issue order] -> byte offset in the packed blob
 // bf16 training path (mlp_bf16_bwd.cu, mlp_bf16_dw.cu, mlp_fp32_bwd.cu)

@@ -30,6 +30,13 @@
 //   * gamma(p): one sincosf per coordinate and octave (30 per point; the bf16 kernel's angle doubling is 6e-5 accurate, not enough
 //     here), split into hi / lo like the activations; gamma(viewdir) as a per-ray fp32 bias vector, as in the bf16 kernel.
 // Every mbarrier wait is bounded (~2 s) and traps instead of hanging the GPU.
+//
+// Embedded-row variant (template parameter EMB, FaceNeRF.forward's x (P, 63+27); inference only): mlp_bf16.cu's embedded-row build in
+// hi / lo form.  The producer warps split gamma(p) = x[:, 0:63] and gamma(v) = x[:, 63:90] of their row with split_rn2 instead of
+// computing them, so any row count works.  There is no per-ray view bias: the 27 view columns of views_linears.0 run as one more K-block
+// (W_hi, W_lo stages, 12 MMAs) at the end of each V0 half, its A operand the gamma(v) hi / lo image that the producers write into the PE
+// buffer once L5 (the last reader of gamma(p)) has completed; the commit after the last V0 view MMA hands the buffer back for the next
+// iteration's gamma(p).  pe_ready / pe_free therefore complete twice per iteration.  Packed blob: INERF_MLP_F16X2_EMB (four more stages).
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -46,7 +53,7 @@ constexpr int STAGE_BYTES = 16384;
 // CTA-pair build (PAIR = true, see mlp_bf16.cu): each CTA of a cluster of two holds HALF of the rows of every weight stage; the same 48 KB
 // ring is six stages deep
 template <bool PAIR> struct RingOf { static constexpr int N = PAIR ? 6 : 3, BYTES = PAIR ? 8192 : 16384; };
-constexpr int MAX_FSTAGES = 160;     // 76 K-block steps x (hi, lo)
+constexpr int MAX_FSTAGES = 160;     // 76 K-block steps x (hi, lo); the embedded-row schedule has 78
 constexpr int RMAX = 4;              // rays a 128-row slot can touch (s >= 43)
 constexpr int NTHREADS = 512;
 constexpr int N_EPI = 256, N_PE = 128;
@@ -71,6 +78,8 @@ struct FSchedule {
 };
 
 __constant__ FStage c_fstages[MAX_FSTAGES];
+__constant__ FStage c_fstages_emb[MAX_FSTAGES];     // the embedded-row schedule (one more K-block per V0 half)
+template <bool EMB> __device__ __forceinline__ const FStage& fstage_at(int s) { return EMB ? c_fstages_emb[s] : c_fstages[s]; }
 
 // smem map (bytes from the 1024-aligned base) -- mlp_bf16.cu's, with [hi|lo] where it has [slot 0|slot 1]
 constexpr int OFF_ACT = 0;                               // [2: hi, lo][4 K-blocks][16384]
@@ -117,6 +126,7 @@ __device__ __forceinline__ void wait_b(uint64_t* bar, uint32_t parity) {
 __host__ __device__ constexpr int lay_N(int l) { return l < 8 ? 256 : 128; }
 __host__ __device__ constexpr int lay_act_kb(int l) { return l == 0 ? 0 : (l <= 8 ? 4 : 2); }
 __host__ __device__ constexpr bool lay_pe(int l) { return l == 0 || l == 5; }
+__host__ __device__ constexpr bool lay_x(int l, bool emb) { return lay_pe(l) || (emb && l == 8); }   // + a PE-buffer K-block (gamma(p) or gamma(v))
 __host__ __device__ constexpr int lay_prev_N(int l) { return l == 0 ? 128 : lay_N(l - 1); }
 
 // kind::f16 instruction descriptor with fp16 A / B (format 0), fp32 D
@@ -215,10 +225,12 @@ struct IssueCtx {
 };
 
 // All MMAs of layer L, straight-line: every descriptor offset, wait and commit is a compile-time constant of (L, half, K-block).
-template <int L, bool PAIR>
+// EMB: the embedded-row schedule.  pe_ready and pe_free then complete twice per iteration (gamma(p) for L0 / L5, gamma(v) for V0), so
+// the issuer's waits have fixed parities: 0 before L0, 1 before V0's view K-block.
+template <int L, bool PAIR, bool EMB = false>
 __device__ __forceinline__ void issue_layer(IssueCtx& c) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
-    constexpr int N = lay_N(L), NH = N / 2, NKB = lay_act_kb(L), CNT = NKB + (lay_pe(L) ? 1 : 0);
+    constexpr int N = lay_N(L), NH = N / 2, NKB = lay_act_kb(L), CNT = NKB + (lay_x(L, EMB) ? 1 : 0);
     constexpr int KB_PER_HALF_PREV = lay_prev_N(L) / 128;
     constexpr int N_OUT_H0 = NH / 64;
     constexpr int N_FIRST = NKB < N_OUT_H0 ? NKB : N_OUT_H0;
@@ -238,7 +250,8 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
                     if (i == KB_PER_HALF_PREV) wait_ev<PAIR>(&bars->ebar[1], par_prev);
                 }
             }
-            if (L == 0 && h == 0 && i == 0) wait_ev<PAIR>(&bars->pe_ready, c.iter_ctr & 1);
+            if (L == 0 && h == 0 && i == 0) wait_ev<PAIR>(&bars->pe_ready, EMB ? 0u : c.iter_ctr & 1);
+            if (EMB && L == 8 && h == 0 && is_pe) wait_ev<PAIR>(&bars->pe_ready, 1u);
             const uint32_t d = c.tmem_base + h * NH, dc = d + CORR_COL;      // main / correction accumulator
             const uint32_t a_hi = is_pe ? c.pe_lo : c.a_lo + i * (16384 >> 4);
             const uint32_t a_lo = is_pe ? c.pe_lo + (16384 >> 4) : c.a_lo + (65536 >> 4) + i * (16384 >> 4);
@@ -278,7 +291,7 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
                 if (h == 0 && last) commit_any<PAIR>(&bars->cbar[0]);
                 if (h == 1 && (N_FIRST > 0 ? i == N_FIRST - 1 : last)) commit_any<PAIR>(&bars->cbar[1]);
                 if (h == 1 && last) commit_any<PAIR>(&bars->cbar[2]);
-                if (h == 1 && last && L == 5) commit_any<PAIR>(&bars->pe_free);
+                if (h == 1 && last && (L == 5 || (EMB && L == 8))) commit_any<PAIR>(&bars->pe_free);
             }
             __syncwarp();
             if (++c.stage == NSTAGE) { c.stage = 0; c.wpar ^= 1; }
@@ -324,7 +337,8 @@ __device__ __forceinline__ void epi16(const uint32_t (&r)[16], const uint32_t (&
 // epilogue keeps its barrier protocol but skips the TMEM loads / conversion / stores, bit 2 = the positional-encoding warps skip sincosf
 // PAIR = true: clusters of two CTAs, one tcgen05.mma.cta_group::2 over the 2 x 128 rows of the pair, the weight stages split across the
 // pair (the bf16 kernel's pair build, mlp_bf16.cu; a pair iteration is two 128-point slots, CTA r takes slot 2 it + r).
-template <bool PAIR>
+// EMB = true: rows of a.x (P, 90) with the INERF_MLP_F16X2_EMB schedule (see the header); launched with abl = 0.
+template <bool PAIR, bool EMB = false>
 __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n_stages, int n_rays, int abl) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
     extern __shared__ __align__(1024) uint8_t sm[];
@@ -385,7 +399,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
             for (long long it = it_first; it < n_iter; it += it_step) {
                 for (int s = 0; s < n_stages; ++s, ++g) {
                     const uint32_t stage = g % NSTAGE, round = g / NSTAGE;
-                    const FStage fs = c_fstages[s];
+                    const FStage fs = fstage_at<EMB>(s);
                     if (fs.bias) {
                         const uint32_t slot = bh & 1, l = fs.layer, h = fs.half;
                         const uint32_t bytes = (uint32_t)fs.n8 * 8u * 32u / SPLIT;
@@ -409,7 +423,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
             uint32_t g = 0, bh = 0;
             for (long long it = it_first; it < n_iter; it += it_step)
                 for (int s = 0; s < n_stages; ++s, ++g) {
-                    if (c_fstages[s].bias) {
+                    if (fstage_at<EMB>(s).bias) {
                         mbar_wait(&bars->bfull[bh & 1], (bh >> 1) & 1);
                         mbar_arrive_remote(&bars->pbfull[bh & 1], 0);
                         ++bh;
@@ -432,16 +446,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
         c.bslot = 0; c.bpar = 0;
         c.stage = 0; c.wpar = 0; c.layer_ctr = 0; c.iter_ctr = 0;
         for (long long it = it_first; it < n_iter; it += it_step, ++c.iter_ctr) {
-            issue_layer<0, PAIR>(c);
+            issue_layer<0, PAIR, EMB>(c);
 #pragma unroll 1
             for (int seg = 0; seg < 2; ++seg) {
 #pragma unroll 1
-                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, PAIR>(c);
-                if (seg == 0) issue_layer<5, PAIR>(c);
+                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, PAIR, EMB>(c);
+                if (seg == 0) issue_layer<5, PAIR, EMB>(c);
             }
-            issue_layer<8, PAIR>(c);
+            issue_layer<8, PAIR, EMB>(c);
 #pragma unroll 1
-            for (int r = 0; r < 2; ++r) issue_layer<9, PAIR>(c);
+            for (int r = 0; r < 2; ++r) issue_layer<9, PAIR, EMB>(c);
         }
     } else if (warp >= 4 && warp < 12) {
         // ================= epilogue: one row per thread, the two warp groups split the column chunks ======================
@@ -457,14 +471,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
             long long p = p0 + row;
             const bool in_range = p < a.P;
             if (!in_range) p = a.P - 1;
-            const int ray_local = (int)(p / a.s - min(p0, a.P - 1) / a.s);
+            const int ray_local = EMB ? 0 : (int)(p / a.s - min(p0, a.P - 1) / a.s);      // embedded rows: no per-ray view bias
             float alpha = 0.f, rgb0 = 0.f, rgb1 = 0.f, rgb2 = 0.f;
             for (int l = 0; l < 11; ++l, ++layer_ctr) {
                 const int NH = (l < 8 ? 256 : 128) >> 1;
                 const int npg = NH >> 6;                       // chunks per group and half: 2 (N = 256) or 1 (N = 128)
                 const uint32_t par = layer_ctr & 1;
                 const float ms = a.tc_comp >= 0.f ? 1.0f + a.tc_comp : 1.0f + a.tc_ulps[l == 0 ? 0 : (l < 8 ? 1 : (l == 8 ? 2 : 3))] * 1.1920928955078125e-07f;
-                if (l == 8) wait_b(&bars->dirb_ready, iter_ctr & 1);
+                if (!EMB && l == 8) wait_b(&bars->dirb_ready, iter_ctr & 1);
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
                     wait_b(&bars->cbar[h == 0 ? 0 : 2], par);
@@ -486,7 +500,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                                 uint32_t* ol = &pl[cc * 16 + q16 * 8];
                                 switch (l) {
                                     case 7: epi16<1>(r, rc, oh, ol, nullptr, s_aw + f, nullptr, alpha, rgb0, rgb1, rgb2, ms); break;
-                                    case 8: epi16<2>(r, rc, oh, ol, s_dirb + ray_local * 128 + f, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, ms); break;
+                                    case 8:
+                                        if constexpr (EMB) epi16<0>(r, rc, oh, ol, nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, ms);
+                                        else epi16<2>(r, rc, oh, ol, s_dirb + ray_local * 128 + f, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, ms);
+                                        break;
                                     case 10: epi16<3>(r, rc, oh, ol, nullptr, nullptr, s_rw + f, alpha, rgb0, rgb1, rgb2, ms); break;
                                     default: epi16<0>(r, rc, oh, ol, nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, ms); break;
                                 }
@@ -518,7 +535,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                     __syncwarp();
                     if (lane == 0) { if constexpr (PAIR) mbar_arrive_remote(&bars->ebar[h], 0); else mbar_arrive(&bars->ebar[h]); }
                 }
-                if (l == 8) {
+                if (!EMB && l == 8) {
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&bars->dirb_free);
                 }
@@ -538,6 +555,61 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                 o.w = (alpha + q.w) + s_sb[0];
                 reinterpret_cast<float4*>(a.out)[p] = o;
             }
+        }
+    } else if (EMB && warp >= 12) {
+        // ================= embedded rows: gamma(p), then gamma(v), of row t of the slot, split from x into the PE buffer ==========
+        // A row of x is 90 floats (360 B; 8-byte aligned when x is 16-byte aligned): gamma(p) = columns 0..62 (image column 63 zero),
+        // gamma(v) = columns 63..89 (image columns 27..63 zero); each value is split into its fp16 hi / lo pair.  Each block is in
+        // registers before the wait for the buffer, so only the shared-memory stores lie between its release and the pe_ready arrival.
+        // pe_free parities: 0 = L5 has read gamma(p) of this iteration, 1 = V0 has read gamma(v) of the previous one.
+        const int t = tid - 12 * 32;
+        uint8_t* dst = sm + OFF_PE + (t >> 3) * 1024 + (t & 7) * 128;
+        auto store_and_arrive = [&](const uint32_t* wh, const uint32_t* wl, int n_chunks) {      // one row of both images, zero-padded
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const uint32_t o = (q ^ (t & 7)) << 4;
+                const bool v = q < n_chunks;
+                *reinterpret_cast<uint4*>(dst + o) = v ? make_uint4(wh[4 * q], wh[4 * q + 1], wh[4 * q + 2], wh[4 * q + 3]) : make_uint4(0u, 0u, 0u, 0u);
+                *reinterpret_cast<uint4*>(dst + 16384 + o) =
+                    v ? make_uint4(wl[4 * q], wl[4 * q + 1], wl[4 * q + 2], wl[4 * q + 3]) : make_uint4(0u, 0u, 0u, 0u);
+            }
+            fence_proxy_async_smem();
+            if constexpr (PAIR) {
+                __syncwarp();
+                if (lane == 0) mbar_arrive_remote(&bars->pe_ready, 0);
+            } else {
+                mbar_arrive(&bars->pe_ready);
+            }
+        };
+        for (long long it = it_first; it < n_iter; it += it_step) {
+            long long p = SLOT_OF(it) * 128 + t;
+            if (p > a.P - 1) p = a.P - 1;
+            const float* xr = a.x + p * 90;
+            uint32_t pkh[32], pkl[32];
+#pragma unroll
+            for (int j = 0; j < 31; ++j) {
+                const float2 v = __ldg(reinterpret_cast<const float2*>(xr) + j);
+                split_rn2(v.x, v.y, pkh[j], pkl[j]);
+            }
+            split_rn2(__ldg(xr + 62), 0.f, pkh[31], pkl[31]);
+            if (it != it_first) wait_b(&bars->pe_free, 1u);
+            store_and_arrive(pkh, pkl, 8);
+            uint32_t pvh[16], pvl[16];
+            {
+                float g[28];
+                g[0] = __ldg(xr + 63);
+#pragma unroll
+                for (int j = 0; j < 13; ++j) {
+                    const float2 v = __ldg(reinterpret_cast<const float2*>(xr + 64) + j);
+                    g[1 + 2 * j] = v.x; g[2 + 2 * j] = v.y;
+                }
+                g[27] = 0.f;
+#pragma unroll
+                for (int j = 0; j < 14; ++j) split_rn2(g[2 * j], g[2 * j + 1], pvh[j], pvl[j]);
+                pvh[14] = pvh[15] = pvl[14] = pvl[15] = 0u;
+            }
+            wait_b(&bars->pe_free, 0u);
+            store_and_arrive(pvh, pvl, 4);
         }
     } else if (warp >= 12) {
         // ================= positional encoding + per-ray view bias producers ==================
@@ -644,13 +716,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
 // ---------------------------------------------------------------------------------------------
 struct LayerDesc { int N, n_act_kb; bool has_pe; int w_index; int ldw, wcol_act; };
 
-FSchedule build_fschedule(const InerfNetDims* d) {
+// emb: the embedded-row schedule -- V0 gains a last K-block per half, (hi, lo) stages of the view columns 256..282 of views_linears.0
+// (kmax = 27) against the gamma(v) image in the PE buffer; every other stage, and the order of all stages, is the fused-entry schedule's.
+FSchedule build_fschedule(const InerfNetDims* d, bool emb = false) {
     const int C = d->dim_aud + d->dim_expr + d->dim_latent, E = d->dim_expr;
     LayerDesc L[11];
     L[0] = {256, 0, true, 0, 63 + C, 0};
     for (int l = 1; l < 8; ++l) L[l] = {256, 4, false, 2 * l, 256, 0};
     L[5] = {256, 4, true, 10, 319 + C, 63 + C};
-    L[8] = {128, 4, false, P_VIEWS_W, 283 + E, 0};
+    L[8] = {128, 4, emb, P_VIEWS_W, 283 + E, 0};
     L[9] = {128, 2, false, P_VIEWS_W + 2, 128, 0};
     L[10] = {128, 2, false, P_VIEWS_W + 4, 128, 0};
     FSchedule S{};
@@ -667,7 +741,7 @@ FSchedule build_fschedule(const InerfNetDims* d) {
                     FPack& pk = S.pack[n];
                     st.offset = off; st.n8 = (uint8_t)(NH / 8); st.bias = (uint8_t)(i == 0 && part == 0); st.layer = (uint8_t)l; st.half = (uint8_t)h;
                     pk.w_index = L[l].w_index; pk.ldw = L[l].ldw; pk.n0 = h * NH; pk.rows = NH; pk.offset = off; pk.lo = part;
-                    if (pe) { pk.wcol = 0; pk.kmax = 63; }
+                    if (pe) { pk.wcol = l == 8 ? 256 : 0; pk.kmax = l == 8 ? 27 : 63; }
                     else { pk.wcol = L[l].wcol_act + i * 64; pk.kmax = 64; }
                     off += (uint32_t)NH * 128u;
                     ++n;
@@ -680,7 +754,7 @@ FSchedule build_fschedule(const InerfNetDims* d) {
     return S;
 }
 
-// 152 stages x 32 B would not fit the 4 KB parameter space next to the 26 weight pointers: the pack table is split over two launches
+// 152 (156) stages x 32 B would not fit the 4 KB parameter space next to the 26 weight pointers: the pack table is split over two launches
 constexpr int PACK_PER_LAUNCH = 80;
 struct FPackArgs {
     const float* w[INERF_N_PARAMS];
@@ -705,15 +779,15 @@ __global__ void f16x2_pack_kernel(const __grid_constant__ FPackArgs pa) {
 
 namespace inerf {
 
-int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes) {
-    FSchedule S = build_fschedule(d);
+int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded) {
+    FSchedule S = build_fschedule(d, embedded);
     *bytes = (size_t)S.total_bytes;
     return INERF_OK;
 }
 
-int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st) {
+int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded) {
     if ((uintptr_t)packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_pack: packed must be 16-byte aligned");
-    FSchedule S = build_fschedule(d);
+    FSchedule S = build_fschedule(d, embedded);
     for (int first = 0; first < S.n_stages; first += PACK_PER_LAUNCH) {
         FPackArgs pa{};
         for (int i = 0; i < INERF_N_PARAMS; ++i) pa.w[i] = params_host[i];
@@ -727,17 +801,26 @@ int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void*
     return INERF_OK;
 }
 
-int mlp_f16x2_launch(const MlpArgs& a, cudaStream_t st) {
-    if (a.s < 43) return fail(INERF_E_UNSUPPORTED, "fp16x2 mode needs at least 43 samples per ray (a 128-row slot may touch at most 4 rays)");
-    if ((uintptr_t)a.packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: packed weights must be 16-byte aligned");
+int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
+    if (embedded) {
+        if (((uintptr_t)a.packed | (uintptr_t)a.x) & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd_embedded: packed weights and x must be 16-byte aligned");
+    } else {
+        if (a.s < 43) return fail(INERF_E_UNSUPPORTED, "fp16x2 mode needs at least 43 samples per ray (a 128-row slot may touch at most 4 rays)");
+        if ((uintptr_t)a.packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: packed weights must be 16-byte aligned");
+    }
     static thread_local int configured_dev = -1;
-    static const FSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_fschedule(&d); }();      // offsets do not depend on the conditioning dims
+    // offsets do not depend on the conditioning dims
+    static const FSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_fschedule(&d); }();
+    static const FSchedule SE = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_fschedule(&d, true); }();
     int dev = 0;
     cudaGetDevice(&dev);
     if (configured_dev != dev) {
         cudaError_t e = cudaFuncSetAttribute(mlp_f16x2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
         if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_fstages, S.st, sizeof(FStage) * MAX_FSTAGES);
+        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_fstages_emb, SE.st, sizeof(FStage) * MAX_FSTAGES);
         if (e != cudaSuccess) { set_error("mlp_f16x2: setup: %s", cudaGetErrorString(e)); return (int)e; }
         configured_dev = dev;
     }
@@ -749,7 +832,9 @@ int mlp_f16x2_launch(const MlpArgs& a, cudaStream_t st) {
     if (const char* e = getenv("INERF_F16X2_COMP")) b.tc_comp = (float)atof(e);      // calibration sweeps (tests/native/f16x2_comp_sweep.py)
     if (const char* e = getenv("INERF_F16X2_ULPS")) sscanf(e, "%f,%f,%f,%f", &b.tc_ulps[0], &b.tc_ulps[1], &b.tc_ulps[2], &b.tc_ulps[3]);
     int abl = 0;
-    if (const char* e = getenv("INERF_F16X2_ABL")) abl = atoi(e);
+    if (const char* e = getenv("INERF_F16X2_ABL"); e && !embedded) abl = atoi(e);   // the embedded-row build has no ablation variants
+    const int n_stages = embedded ? SE.n_stages : S.n_stages;
+    const int n_rays = embedded ? 0 : (int)(a.P / a.s);
     // the CTA-pair build by default; INERF_MLP_PAIR=0 (read once) keeps the single-CTA kernel for A/B runs
     static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
     if (pair_env && num_sms() >= 2) {
@@ -765,11 +850,16 @@ int mlp_f16x2_launch(const MlpArgs& a, cudaStream_t st) {
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        cudaError_t e = cudaLaunchKernelEx(&cfg, mlp_f16x2_kernel<true>, b, S.n_stages, (int)(a.P / a.s), abl);
-        if (e != cudaSuccess) { set_error("inerf_mlp_fwd[fp16x2 pair]: %s", cudaGetErrorString(e)); return (int)e; }
-        return check_launch("inerf_mlp_fwd[fp16x2 pair]");
+        const char* what = embedded ? "inerf_mlp_fwd_embedded[fp16x2 pair]" : "inerf_mlp_fwd[fp16x2 pair]";
+        cudaError_t e = cudaLaunchKernelEx(&cfg, embedded ? mlp_f16x2_kernel<true, true> : mlp_f16x2_kernel<true>, b, n_stages, n_rays, abl);
+        if (e != cudaSuccess) { set_error("%s: %s", what, cudaGetErrorString(e)); return (int)e; }
+        return check_launch(what);
     }
-    mlp_f16x2_kernel<false><<<grid, NTHREADS, SMEM_BYTES, st>>>(b, S.n_stages, (int)(a.P / a.s), abl);
+    if (embedded) {
+        mlp_f16x2_kernel<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(b, n_stages, n_rays, abl);
+        return check_launch("inerf_mlp_fwd_embedded[fp16x2]");
+    }
+    mlp_f16x2_kernel<false><<<grid, NTHREADS, SMEM_BYTES, st>>>(b, n_stages, n_rays, abl);
     return check_launch("inerf_mlp_fwd[fp16x2]");
 }
 

@@ -365,6 +365,7 @@ extern "C" int inerf_mlp_packed_bytes(int mode, const InerfNetDims* dims, size_t
     if (mode == INERF_MLP_BF16_EMB) return mlp_bf16_packed_bytes(dims, bytes, true);
     if (mode == INERF_MLP_BF16_BWD) return mlp_bf16_bwd_packed_bytes(dims, bytes);
     if (mode == INERF_MLP_F16X2) return mlp_f16x2_packed_bytes(dims, bytes);
+    if (mode == INERF_MLP_F16X2_EMB) return mlp_f16x2_packed_bytes(dims, bytes, true);
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_packed_bytes: unknown mode");
 }
 
@@ -389,6 +390,10 @@ extern "C" int inerf_mlp_pack(int mode, const InerfNetDims* dims, const float* c
         if (!params_host || !packed) return fail(INERF_E_ARG, "inerf_mlp_pack: NULL pointer");
         return mlp_f16x2_pack(dims, params_host, packed, as_stream(stream));
     }
+    if (mode == INERF_MLP_F16X2_EMB) {
+        if (!params_host || !packed) return fail(INERF_E_ARG, "inerf_mlp_pack: NULL pointer");
+        return mlp_f16x2_pack(dims, params_host, packed, as_stream(stream), true);
+    }
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_pack: unknown mode");
 }
 
@@ -411,8 +416,10 @@ extern "C" int inerf_mlp_fwd(int mode, const InerfNetDims* dims, const float* co
     }
     if (mode == INERF_MLP_F16X2) {
         if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd: fp16x2 mode needs packed weights");
-        return mlp_f16x2_launch(a, as_stream(stream));
+        return mlp_f16x2_launch(a, false, as_stream(stream));
     }
+    if (mode == INERF_MLP_F16X2_EMB)
+        return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd: INERF_MLP_F16X2_EMB is the embedded-row mode of inerf_mlp_fwd_embedded; use INERF_MLP_F16X2");
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd: unknown mode");
 }
 
@@ -503,8 +510,12 @@ extern "C" int inerf_mlp_fwd_embedded(int mode, const InerfNetDims* dims, const 
         if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd_embedded: bf16 mode needs packed weights (INERF_MLP_BF16_EMB)");
         return mlp_bf16_launch(a, true, as_stream(stream));
     }
-    if (mode == INERF_MLP_F16X2)
-        return fail(INERF_E_UNSUPPORTED, "fp16x2 mode is built for the fused (rays, z) entry; FaceNeRF.forward on embedded rows runs in fp32 mode");
+    if (mode == INERF_MLP_F16X2_EMB) {
+        if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd_embedded: fp16x2 mode needs packed weights (INERF_MLP_F16X2_EMB)");
+        return mlp_f16x2_launch(a, true, as_stream(stream));
+    }
+    if (mode == INERF_MLP_F16X2)      // the two fp16x2 blobs cannot be told apart: embedded rows take the mode of their own blob
+        return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd_embedded: fp16x2 on embedded rows is mode INERF_MLP_F16X2_EMB, with that mode's packed blob");
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd_embedded: unknown mode");
 }
 

@@ -210,6 +210,8 @@ int render_rays_fused(const InerfRenderArgs* a, void* stream, cudaEvent_t* ev) {
     Workspace w{};
     int rc = plan(a, w);
     if (rc) return rc;
+    if (a->mode == INERF_MLP_F16X2_EMB)
+        return fail(INERF_E_UNSUPPORTED, "inerf_render_rays_fused: INERF_MLP_F16X2_EMB is an embedded-row mode; the fused render takes INERF_MLP_F16X2");
     if (a->n == 0) return INERF_OK;
     if (!a->workspace || a->workspace_bytes < w.total) return fail(INERF_E_ARG, "inerf_render_rays_fused: workspace missing or smaller than inerf_render_workspace_bytes");
     if ((uintptr_t)a->workspace & 255) return fail(INERF_E_ALIGN, "inerf_render_rays_fused: workspace must be 256-byte aligned");

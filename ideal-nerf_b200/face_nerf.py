@@ -13,7 +13,8 @@ from . import _lib, ops
 
 # "bf16": tcgen05 kernels for inference and training, on both entries -- query(rays, z) and forward(x) on embedded rows (the latter with
 # its own packed blob, INERF_MLP_BF16_EMB).  "fp16x2": tensor cores at fp32-gate accuracy (fp16 hi/lo operand pairs, three MMA passes)
-# on query(); inference kernel -- training in this mode, and forward(x) on embedded rows, run the fp32 kernels, like "fp32"
+# for inference on both entries (forward(x) with its own blob and mode, INERF_MLP_F16X2_EMB); training in this mode runs the fp32
+# kernels, like "fp32"
 MODES = {"fp32": _lib.INERF_MLP_FP32, "bf16": _lib.INERF_MLP_BF16, "fp16x2": _lib.INERF_MLP_F16X2}
 
 
@@ -99,10 +100,12 @@ class FaceNeRF(nn.Module):
         return self._packed_t
 
     def packed_weights_emb(self, params):
-        """bf16 stage images of the embedded-row kernel (FaceNeRF.forward), re-packed when a parameter changed."""
-        key = tuple((p.data_ptr(), p._version) for p in params)
+        """Stage images of the embedded-row kernel (FaceNeRF.forward) of the current tensor-core mode -- INERF_MLP_BF16_EMB or
+        INERF_MLP_F16X2_EMB -- re-packed when a parameter or the mode changed."""
+        mode = _lib.INERF_MLP_F16X2_EMB if self._mode() == _lib.INERF_MLP_F16X2 else _lib.INERF_MLP_BF16_EMB
+        key = (mode, tuple((p.data_ptr(), p._version) for p in params))
         if key != self._packed_e_key:
-            self._packed_e = ops.pack_weights(_lib.INERF_MLP_BF16_EMB, self._dims, [p.detach() for p in params])
+            self._packed_e = ops.pack_weights(mode, self._dims, [p.detach() for p in params])
             self._packed_e_key = key
         return self._packed_e
 
@@ -170,10 +173,11 @@ class _MlpFn(torch.autograd.Function):
             return out
         if embedded and mode == _lib.INERF_MLP_BF16:
             return ops.mlp_fwd_embedded(mode, net._dims, pd, net.packed_weights_emb(params), cond, a)
+        if embedded and mode == _lib.INERF_MLP_F16X2:       # the embedded-row kernel has its own mode value: the blobs differ
+            return ops.mlp_fwd_embedded(_lib.INERF_MLP_F16X2_EMB, net._dims, pd, net.packed_weights_emb(params), cond, a)
         packed = net.packed_weights(params)
-        if embedded:                                         # FaceNeRF.forward on embedded rows: fp16x2 shares the fp32 kernel there
-            m = _lib.INERF_MLP_FP32 if mode == _lib.INERF_MLP_F16X2 else mode
-            return ops.mlp_fwd_embedded(m, net._dims, pd, packed, cond, a)
+        if embedded:
+            return ops.mlp_fwd_embedded(mode, net._dims, pd, packed, cond, a)
         return ops.mlp_fwd(mode, net._dims, pd, packed, cond, a, b)
 
     @staticmethod

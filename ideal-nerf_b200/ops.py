@@ -695,7 +695,8 @@ def _rows90(x):
 
 
 def mlp_fwd_embedded(mode, dims, params, packed, cond, x):
-    """FaceNeRF.forward on embedded rows x (P, 90) -> (P, 4).  bf16 mode takes the INERF_MLP_BF16_EMB blob."""
+    """FaceNeRF.forward on embedded rows x (P, 90) -> (P, 4).  bf16 mode takes the INERF_MLP_BF16_EMB blob; fp16x2 runs as mode
+    INERF_MLP_F16X2_EMB with that mode's blob."""
     x = _rows90(x)
     out = torch.empty((x.shape[0], 4), device=x.device)
     arr = param_array(params)

@@ -21,8 +21,8 @@
  *   - FaceNeRF geometry: D = 8, W = 256, skips = [4], in_xyz = 63, in_views = 27, use_viewdirs (the configuration of every reference
  *     script); conditioning dims are free (head 64 + 76 + 32, torso 106 + 0 + 0, ...);
  *   - on the fused (rays, z) entry inerf_mlp_fwd the tensor-core modes (INERF_MLP_BF16, INERF_MLP_F16X2) need s >= 43 samples per
- *     ray (a 128-row slot may touch at most four rays); inerf_mlp_fwd_embedded runs INERF_MLP_FP32 and INERF_MLP_BF16 on any number
- *     of rows (INERF_MLP_F16X2 is built for the fused entry only);
+ *     ray (a 128-row slot may touch at most four rays); inerf_mlp_fwd_embedded runs INERF_MLP_FP32, INERF_MLP_BF16 and
+ *     INERF_MLP_F16X2_EMB on any number of rows (each tensor-core mode with its embedded-row blob);
  *   - training entry points exist for INERF_MLP_FP32 and INERF_MLP_BF16, on both entries (INERF_MLP_F16X2 is an inference mode);
  *   - sample_pdf: 2 <= n_bins <= 1024, n_imp <= 1024, the per-ray working set within 48 KB of shared memory; s <= 4096 elsewhere.
  */
@@ -54,9 +54,12 @@ enum {
     INERF_MLP_BF16_BWD = 2, /* inerf_mlp_packed_bytes / inerf_mlp_pack only: the TRANSPOSED stage images of the bf16 backward chain */
     INERF_MLP_F16X2 = 3, /* fp32-gate tensor-core mode: every operand an fp16 (hi, lo) pair, three tcgen05 passes per product
                            (hi.hi + lo.hi + hi.lo), fp32 accumulate in TMEM -- meets the <= 1e-3 max-abs gate (inference entry only) */
-    INERF_MLP_BF16_EMB = 4 /* inerf_mlp_packed_bytes / inerf_mlp_pack only: the stage images of the bf16 kernel on EMBEDDED rows
+    INERF_MLP_BF16_EMB = 4, /* inerf_mlp_packed_bytes / inerf_mlp_pack only: the stage images of the bf16 kernel on EMBEDDED rows
                               (inerf_mlp_fwd_embedded, inerf_mlp_fwd_train_bf16_embedded): the INERF_MLP_BF16 schedule plus one
                               K-block per half of views_linears.0 for its 27 view columns */
+    INERF_MLP_F16X2_EMB = 5 /* the fp16x2 mode on EMBEDDED rows (inference only): the mode of inerf_mlp_fwd_embedded and of its blob
+                               (inerf_mlp_packed_bytes / inerf_mlp_pack), the INERF_MLP_F16X2 schedule plus one (hi, lo) K-block per half
+                               of views_linears.0 for its 27 view columns; inerf_mlp_fwd and InerfRenderArgs reject it */
 };
 
 /* sample_pdf summation policies (SURVEY.md 7-1) */
@@ -248,7 +251,7 @@ enum {
 };
 
 typedef struct InerfRenderArgs {
-    int32_t mode;                    /* INERF_MLP_FP32 / _BF16 / _F16X2, both nets                                        */
+    int32_t mode;                    /* INERF_MLP_FP32 / _BF16 / _F16X2, both nets (not _F16X2_EMB: INERF_E_UNSUPPORTED) */
     int32_t n;                       /* rays                                                                               */
     int32_t n_samples, n_importance; /* args.N_samples, args.N_importance                                                  */
     int32_t perturb;                 /* 0: deterministic depths; 1: stratified jitter and importance draws made in-kernel  */
@@ -395,7 +398,9 @@ int inerf_debug_hang_info(int32_t* out8);
 /* FaceNeRF.forward on already-embedded inputs x (p, in_xyz+in_views) -- the reference module's own
  * call signature (face_nerf.py:40).  out (p, 4).  Any p >= 0 (0 enqueues nothing).
  * INERF_MLP_FP32: packed is ignored.  INERF_MLP_BF16: the tcgen05 kernel; packed must be an INERF_MLP_BF16_EMB blob (not the
- * INERF_MLP_BF16 blob of inerf_mlp_fwd) and x 16-byte aligned.  INERF_MLP_F16X2: INERF_E_UNSUPPORTED. */
+ * INERF_MLP_BF16 blob of inerf_mlp_fwd) and x 16-byte aligned.  INERF_MLP_F16X2_EMB: the fp16x2 tcgen05 kernel at fp32-gate accuracy;
+ * packed must be an INERF_MLP_F16X2_EMB blob and x 16-byte aligned.  INERF_MLP_F16X2: INERF_E_UNSUPPORTED (its blob is the fused
+ * entry's; the two cannot be told apart). */
 int inerf_mlp_fwd_embedded(int mode, const InerfNetDims* dims, const float* const* params_host,
                            const void* packed, const float* cond, const float* x, int64_t p, float* out,
                            void* stream);

@@ -1,17 +1,18 @@
 """FaceNeRF.forward on embedded rows (x (P, 63+27), the reference module's own signature) against the fused (rays, z) entry.
 
-    python profiles/embedded_mlp.py                      # card, power limit, points/s of the four paths below, query hash
-    python profiles/embedded_mlp.py --hash-only --root T # only the sha256 of the bf16 fused-query raw, with the package of tree T
+    python profiles/embedded_mlp.py                      # card, power limit, points/s of the paths below, query hashes
+    python profiles/embedded_mlp.py --hash-only --root T # only the sha256 of the bf16 and fp16x2 fused-query raw, with the package of tree T
 
 On P = 202 500 x 64 rows (one 450 x 450 frame, 64 samples per ray; x is 4.7 GB, far larger than L2, and read once per call):
-  * FaceNeRF.forward(x), mlp_mode="fp32" (FFMA kernel) and "bf16" (tcgen05 embedded-row kernel);
-  * FaceNeRF.query(rays, z) in bf16 on the same points (fused gamma, per-ray view bias);
+  * FaceNeRF.forward(x), mlp_mode="fp32" (FFMA kernel), "bf16" and "fp16x2" (tcgen05 embedded-row kernels);
+  * FaceNeRF.query(rays, z) in bf16 and in fp16x2 on the same points (fused gamma, per-ray view bias);
   * Network.run_network at the reference's netchunk = 65 536 (embedding + FaceNeRF.forward per 65 536-row piece), and the forward calls
     alone on the pre-embedded pieces.
 Times are CUDA-event times of whole calls after a warm-up.  TFLOP/s are algorithmic: 560 640 MAC per point for the fused form (view
-columns folded into a per-ray bias), 560 640 + 3 456 for the embedded form, against the sustained cuBLAS bf16 figure of DESIGN.md §3.
-The hash is of raw from a seeded bf16 FaceNeRF.query (137 rays x {64, 192} samples): equal hashes from two trees = the fused path is
-unchanged bit for bit.
+columns folded into a per-ray bias), 560 640 + 3 456 for the embedded form, against the sustained cuBLAS bf16 figure of DESIGN.md §3;
+for fp16x2 the issued rate of its three MMA passes (hi.hi + lo.hi + hi.lo) is printed as well.
+The hashes are of raw from a seeded FaceNeRF.query (137 rays x {64, 192} samples) in bf16 and in fp16x2: equal hashes from two trees =
+the fused paths are unchanged bit for bit.
 """
 import argparse
 import hashlib
@@ -47,9 +48,9 @@ cam, fr = S.camera(), S.frame_inputs(0)
 aud, expr, lat = fr["aud"].to(dev), fr["expr"].to(dev), fr["latent"].to(dev)
 
 
-def query_hash():
+def query_hash(mode):
     torch.manual_seed(3)
-    net = M.FaceNeRF(dim_aud=64, dim_latent=32, dim_expr=76, mlp_mode="bf16").apply(M.init_weights).to(dev)
+    net = M.FaceNeRF(dim_aud=64, dim_latent=32, dim_expr=76, mlp_mode=mode).apply(M.init_weights).to(dev)
     rays = ops.get_rays_range(450, 450, cam["focal"], cam["c2w"].to(dev), S.NEAR, S.FAR, 90000, 137)
     h = hashlib.sha256()
     with torch.no_grad():
@@ -59,7 +60,8 @@ def query_hash():
     return h.hexdigest()
 
 
-say(f"query_raw_sha256 {query_hash()}  (package of {os.path.abspath(args.root)})")
+say(f"query_raw_sha256 {query_hash('bf16')}  (package of {os.path.abspath(args.root)})")
+say(f"query_raw_sha256_fp16x2 {query_hash('fp16x2')}  (package of {os.path.abspath(args.root)})")
 if args.hash_only:
     sys.exit(0)
 
@@ -83,10 +85,11 @@ def timed(fn, reps):
     return a.elapsed_time(b) / reps
 
 
-def report(name, ms, n_pts, flop_per_pt):
+def report(name, ms, n_pts, flop_per_pt, passes=1):
     tf = n_pts * flop_per_pt / (ms * 1e-3) / 1e12
+    issued = f";  {passes * tf:7.1f} TFLOP/s issued ({passes} passes) = {passes * tf / SUSTAINED_BF16_TFLOPS:.3f}" if passes > 1 else ""
     say(f"{name:52s} {ms:9.3f} ms  {n_pts / (ms * 1e-3) / 1e6:9.1f} M points/s  {tf:7.1f} TFLOP/s algorithmic "
-        f"= {tf / SUSTAINED_BF16_TFLOPS:.3f} of sustained bf16")
+        f"= {tf / SUSTAINED_BF16_TFLOPS:.3f} of sustained bf16{issued}")
     return n_pts / (ms * 1e-3)
 
 
@@ -108,6 +111,16 @@ host = M.Network(450, 450, 1200., S.NEAR, S.FAR, 8192, None, 64, 128, args=M.def
 with torch.no_grad():
     net.mlp_mode = "fp32"
     r32 = report("FaceNeRF.forward(x)  fp32", timed(lambda: net(x, aud, expr, lat), 2), P, FLOP_EMB)
+    out32 = net(x, aud, expr, lat)
+    net.mlp_mode = "fp16x2"
+    rx = report("FaceNeRF.forward(x)  fp16x2", timed(lambda: net(x, aud, expr, lat), 5), P, FLOP_EMB, passes=3)
+    rxq = report("FaceNeRF.query(rays, z)  fp16x2 (same points)", timed(lambda: net.query(rays, z, aud, expr, lat), 5), P, FLOP_FUSED,
+                 passes=3)
+    outx = net(x, aud, expr, lat)
+    scale = out32.abs().amax(0)
+    dx32 = ((outx - out32).abs().amax(0) / scale).tolist()
+    dxq = ((outx - net.query(rays, z, aud, expr, lat).reshape(-1, 4)).abs().amax(0) / scale).tolist()
+    del outx
     net.mlp_mode = "bf16"
     r16 = report("FaceNeRF.forward(x)  bf16", timed(lambda: net(x, aud, expr, lat), 10), P, FLOP_EMB)
     rq = report("FaceNeRF.query(rays, z)  bf16 (same points)", timed(lambda: net.query(rays, z, aud, expr, lat), 10), P, FLOP_FUSED)
@@ -119,6 +132,9 @@ with torch.no_grad():
 say(f"bf16 embedded / bf16 fused: {r16 / rq:.3f};  bf16 embedded / fp32 embedded: {r16 / r32:.1f}x;  "
     f"run_network(netchunk 65536) / bf16 embedded: {rn / r16:.3f} (forward pieces alone {rp / r16:.3f})")
 say(f"max |embedded - fused| per channel (r, g, b, sigma): {[f'{v:.2e}' for v in d.tolist()]}")
+say(f"fp16x2 embedded / fp16x2 fused: {rx / rxq:.3f};  fp16x2 embedded / fp32 embedded: {rx / r32:.1f}x")
+say(f"fp16x2 embedded, max-abs / scale of the fp32 kernel's raw per channel (r, g, b, sigma): vs fp32 embedded "
+    f"{[f'{v:.2e}' for v in dx32]}, vs fp16x2 fused {[f'{v:.2e}' for v in dxq]}")
 if args.out:
     with open(args.out, "w") as f:
         f.write("\n".join(lines) + "\n")
