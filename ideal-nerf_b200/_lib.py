@@ -80,6 +80,7 @@ SIGNATURES = {
     "inerf_composite_bwd": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "inerf_mse_pair": (_I, [_P, _P, _P, _L, _P, _P, _P, _P]),
     "inerf_head_torso_blend": (_I, [_P, _P, _P, _I, _P, _P]),
+    "inerf_head_torso_mse_pair": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _P, _P]),
     "inerf_head_torso_to8b": (_I, [_P, _P, _P, _L, _P, _P, _P]),
     "inerf_sample_pdf": (_I, [_P, _I, _P, _I, _I, _I, _I, _P, _I, _I, _P, _P, _P, _I, _P, _P, _P]),
     "inerf_importance_sample": (_I, [_P, _P, _I, _I, _I, _P, _I, _I, _P, _P, _P, _P, _P]),

@@ -7,6 +7,8 @@
 * fine-tune source (--ft_path, :498-514): {'network_fn_state_dict', 'network_fine_state_dict', 'network_audnet_state_dict',
       'network_audattnet_state_dict'}; the reference drops pts_linears.0 / pts_linears.5 / views_linears.0 weights (their input
       widths depend on dim_aud / dim_expr) and loads the rest with strict=False.
+* the start of the torso stage (NeRFs/TorsoNeRF/train_torso.py): load_head_into_torso copies a head.tar's head pair into a TorsoNetwork;
+      train.TorsoTrainStep.save / load write and resume the torso stage itself.
 Pure host I/O: nothing here launches a kernel."""
 import torch
 
@@ -58,3 +60,31 @@ def load_finetune_checkpoint(path, network, map_location=None):
     if "network_audattnet_state_dict" in ckpt:
         network.aud_att_net.load_state_dict(ckpt["network_audattnet_state_dict"], strict=False)
     return 0
+
+
+def load_head_into_torso(path, torso_network, map_location=None):
+    """The start of the torso stage: copy the head pair of a head.tar (the reference's keys, as load_head_checkpoint reads them) into
+    torso_network.face_nerf_coarse / face_nerf_fine, in place.  The torso pair is left alone and the head pair's packed weight blobs are
+    dropped.  Returns the head's latent codes (n_frames, 32), or None when the file has none.
+
+    Every key of the head pair must be present with this network's shape; otherwise ValueError names the key and both shapes before
+    anything is copied.  TorsoNetwork defaults to dim_expr=79, so a head trained with another expression width fails here."""
+    ckpt = torch.load(path, map_location=map_location, weights_only=False)
+    sd = ckpt["model_state_dict"]
+    pairs = []
+    for name in ("face_nerf_coarse", "face_nerf_fine"):
+        for k, v in getattr(torso_network, name).state_dict().items():
+            key = f"{name}.{k}"
+            if key not in sd:
+                raise ValueError(f"load_head_into_torso: {path} has no '{key}': not a head.tar of the reference's Network")
+            if tuple(sd[key].shape) != tuple(v.shape):
+                raise ValueError(f"load_head_into_torso: '{key}' is {tuple(sd[key].shape)} in {path} but {tuple(v.shape)} in this "
+                                 "TorsoNetwork: the head was trained with other conditioning widths (dim_aud / dim_expr / dim_latent; "
+                                 "TorsoNetwork(dim_expr=...) must match the head's)")
+            pairs.append((v, sd[key]))
+    with torch.no_grad():
+        for dst, src in pairs:
+            dst.copy_(src.to(dst.device))
+    for m in (torso_network.face_nerf_coarse, torso_network.face_nerf_fine):
+        m.invalidate_packed()
+    return ckpt.get("latent_codes")

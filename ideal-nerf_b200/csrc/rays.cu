@@ -274,6 +274,64 @@ extern "C" int inerf_head_torso_blend(const float* rgb_head, const float* last_w
 }
 
 // ---------------------------------------------------------------------------------------------
+// torso-stage loss seed: the two composites of train_torso.py:269-270, their mean squared errors and the gradients that reach the torso
+// pair, in one pass.  The composite is blend_value (the bits of blend_kernel), the per-value gradient the expression of mse_pair_kernel;
+// one thread per ray, so last_weight's gradient is summed over the ray's three values in registers.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) head_torso_mse_pair_kernel(
+    const float* __restrict__ head, const float* __restrict__ head0, const float* __restrict__ lw, const float* __restrict__ lw0,
+    const float* __restrict__ fg, const float* __restrict__ fg0, const float* __restrict__ tgt, long long n, float inv_m,
+    float* __restrict__ g_lw, float* __restrict__ g_lw0, float* __restrict__ g_fg, float* __restrict__ g_fg0, float* __restrict__ loss) {
+    float s0 = 0.f, s1 = 0.f;
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (long long)gridDim.x * blockDim.x) {
+        const float w = lw[r], w0 = lw0[r];
+        float gw = 0.f, gw0 = 0.f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const long long i = 3 * r + c;
+            const float t = tgt[i], h = head[i], h0 = head0[i];
+            const float d0 = blend_value(h, w, fg[i]) - t, d1 = blend_value(h0, w0, fg0[i]) - t;
+            s0 = fmaf(d0, d0, s0);
+            s1 = fmaf(d1, d1, s1);
+            const float g0 = 2.0f * d0 * inv_m, g1 = 2.0f * d1 * inv_m;
+            g_fg[i] = g0;
+            g_fg0[i] = g1;
+            gw = __fadd_rn(gw, __fmul_rn(g0, h));
+            gw0 = __fadd_rn(gw0, __fmul_rn(g1, h0));
+        }
+        g_lw[r] = gw;
+        g_lw0[r] = gw0;
+    }
+    s0 = warp_sum(s0);
+    s1 = warp_sum(s1);
+    __shared__ float sh[2][8];
+    const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
+    if (lane == 0) { sh[0][wi] = s0; sh[1][wi] = s1; }
+    __syncthreads();
+    if (threadIdx.x < 2) {
+        float t = 0.f;
+        for (int j = 0; j < 8; ++j) t += sh[threadIdx.x][j];
+        atomicAdd(loss + threadIdx.x, t * inv_m);
+    }
+}
+
+extern "C" int inerf_head_torso_mse_pair(const float* rgb_head, const float* rgb_head0, const float* last_weight, const float* last_weight0,
+                                         const float* rgb_fg, const float* rgb_fg0, const float* target, int64_t n, float* g_last_weight,
+                                         float* g_last_weight0, float* g_rgb_fg, float* g_rgb_fg0, float* loss2, void* stream) {
+    if (n <= 0) return fail(INERF_E_SHAPE, "inerf_head_torso_mse_pair: need at least one ray");
+    if (!rgb_head || !rgb_head0 || !last_weight || !last_weight0 || !rgb_fg || !rgb_fg0 || !target || !g_last_weight || !g_last_weight0 ||
+        !g_rgb_fg || !g_rgb_fg0 || !loss2)
+        return fail(INERF_E_ARG, "inerf_head_torso_mse_pair: NULL pointer");
+    cudaError_t e = cudaMemsetAsync(loss2, 0, 2 * sizeof(float), as_stream(stream));
+    if (e != cudaSuccess) { set_error("inerf_head_torso_mse_pair: %s", cudaGetErrorString(e)); return (int)e; }
+    const int grid = (int)((n + 255) / 256 < 4 * (long long)num_sms() ? (n + 255) / 256 : 4 * (long long)num_sms());
+    head_torso_mse_pair_kernel<<<grid, 256, 0, as_stream(stream)>>>(rgb_head, rgb_head0, last_weight, last_weight0, rgb_fg, rgb_fg0, target, n,
+                                                                   1.0f / (float)(3 * n), g_last_weight, g_last_weight0, g_rgb_fg, g_rgb_fg0,
+                                                                   loss2);
+    return check_launch("inerf_head_torso_mse_pair");
+}
+
+// ---------------------------------------------------------------------------------------------
 // to8b: (255 * clip(x, 0, 1)).astype(uint8)   helper.py:154 (used on every rendered frame, eval_aud_exp_nerf.py:490)
 // ---------------------------------------------------------------------------------------------
 __global__ void to8b_kernel(const float* __restrict__ x, long long n, uint8_t* __restrict__ out) {

@@ -80,14 +80,15 @@ class FaceNeRF(nn.Module):
         self.invalidate_packed()
         return super().train(mode)
 
-    def packed_weights(self, params):
-        """Mode-specific packed weights, re-packed whenever a parameter was updated in place."""
+    def packed_weights(self, params, out=None):
+        """Mode-specific packed weights, re-packed whenever a parameter was updated in place.  out: a blob of this mode's size that must
+        hold them (a captured CUDA graph reads it): the weights are packed into it unless it already is the current cached blob."""
         mode = self._mode()
         if mode == _lib.INERF_MLP_FP32:
             return None
         key = (mode, tuple((p.data_ptr(), p._version) for p in params))
-        if key != self._packed_key:
-            self._packed = ops.pack_weights(mode, self._dims, [p.detach() for p in params])
+        if key != self._packed_key or (out is not None and self._packed is not out):
+            self._packed = ops.pack_weights(mode, self._dims, [p.detach() for p in params], out=out)
             self._packed_key = key
         return self._packed
 

@@ -352,6 +352,45 @@ def head_torso_blend(rgb_head, last_weight_torso, rgb_fg_torso):
     return _Blend.apply(rgb_head, last_weight_torso, rgb_fg_torso)
 
 
+class _HeadTorsoMsePair(torch.autograd.Function):
+    """img_loss + img_loss0 of the torso stage: both composites, both losses and the gradients reaching the torso pair in one kernel."""
+
+    @staticmethod
+    def forward(ctx, rgb_head, rgb_head0, lw, lw0, fg, fg0, target):
+        h, h0 = f32c(rgb_head, "rgb_head"), f32c(rgb_head0, "rgb_head0")
+        w, w0 = f32c(lw, "last_weight"), f32c(lw0, "last_weight0")
+        f, f0, t = f32c(fg, "rgb_fg"), f32c(fg0, "rgb_fg0"), f32c(target, "target")
+        n = w.numel()
+        if not (h.numel() == h0.numel() == f.numel() == f0.numel() == t.numel() == 3 * n and w0.numel() == n):
+            raise ValueError(f"head_torso_mse_pair: rgb_head {tuple(h.shape)}, rgb_head0 {tuple(h0.shape)}, last_weight {tuple(w.shape)}, "
+                             f"last_weight0 {tuple(w0.shape)}, rgb_fg {tuple(f.shape)}, rgb_fg0 {tuple(f0.shape)}, target {tuple(t.shape)} "
+                             "are not (n,3) x 2, (n) x 2, (n,3) x 3")
+        g_w, g_w0, g_f, g_f0 = torch.empty_like(w), torch.empty_like(w0), torch.empty_like(f), torch.empty_like(f0)
+        loss2 = torch.empty((2,), device=w.device)
+        with torch.cuda.device(w.device):
+            call("inerf_head_torso_mse_pair", _lib.lib().inerf_head_torso_mse_pair, ptr(h), ptr(h0), ptr(w), ptr(w0), ptr(f), ptr(f0), ptr(t),
+                 n, ptr(g_w), ptr(g_w0), ptr(g_f), ptr(g_f0), ptr(loss2), stream())
+        ctx.save_for_backward(g_w, g_w0, g_f, g_f0)
+        ctx.shapes = (lw.shape, lw0.shape, fg.shape, fg0.shape)
+        return loss2
+
+    @staticmethod
+    def backward(ctx, g):
+        g_w, g_w0, g_f, g_f0 = ctx.saved_tensors
+        s = ctx.shapes
+        return (None, None, (g_w * g[0]).view(s[0]), (g_w0 * g[1]).view(s[1]), (g_f * g[0]).view(s[2]), (g_f0 * g[1]).view(s[3]), None)
+
+
+def head_torso_mse_pair(rgb_head, rgb_head0, last_weight, last_weight0, rgb_fg, rgb_fg0, target):
+    """(F.mse_loss(head_torso_blend(rgb_head, last_weight, rgb_fg), target), the same for the coarse set) as a 2-vector, differentiable
+    in last_weight, last_weight0, rgb_fg and rgb_fg0 (train_torso.py:269-271).  The head is frozen in the torso stage and the kernel
+    computes no gradient for it, so a head image that requires grad raises instead of silently losing its gradient."""
+    if (isinstance(rgb_head, torch.Tensor) and rgb_head.requires_grad) or (isinstance(rgb_head0, torch.Tensor) and rgb_head0.requires_grad):
+        raise ValueError("head_torso_mse_pair: rgb_head / rgb_head0 require grad, but no gradient w.r.t. the head image is computed; "
+                         "render the head pair under torch.no_grad() or pass .detach()")
+    return _HeadTorsoMsePair.apply(rgb_head, rgb_head0, last_weight, last_weight0, rgb_fg, rgb_fg0, target)
+
+
 def head_torso_to8b(rgb_head, last_weight_torso, rgb_fg_torso, out=None, out_rgb=None):
     """to8b(head_torso_blend(...)) in one kernel (test_torso.py:523-524), no autograd: (n, 3) uint8 for n rays, written into `out` when
     given.  out_rgb: None, or a contiguous float32 tensor of 3n values that receives the fp32 blend."""
@@ -550,13 +589,19 @@ def fold_cond(dims, params, aud, expr, latent):
     return cond
 
 
-def pack_weights(mode, dims, params):
+def pack_weights(mode, dims, params, out=None):
+    """The packed weight blob of `mode` (None when the mode has none), written into `out` when given (a uint8 tensor of exactly that
+    size), else into a new tensor."""
     nb = ctypes.c_size_t()
     check(_lib.lib().inerf_mlp_packed_bytes(mode, ctypes.byref(dims), ctypes.byref(nb)), "inerf_mlp_packed_bytes")
     if nb.value == 0:
         return None
     dev = params[0].device
-    packed = torch.empty((nb.value,), device=dev, dtype=torch.uint8)
+    if out is not None:
+        _need_cuda(out, "out")
+        if out.dtype != torch.uint8 or out.numel() != nb.value or not out.is_contiguous() or out.device != dev:
+            raise ValueError(f"pack_weights: `out` must be a contiguous uint8 tensor of {nb.value} bytes on {dev}")
+    packed = torch.empty((nb.value,), device=dev, dtype=torch.uint8) if out is None else out
     arr = param_array(params)
     with torch.cuda.device(dev):
         call("inerf_mlp_pack", _lib.lib().inerf_mlp_pack, mode, ctypes.byref(dims), arr, ptr(packed), stream())

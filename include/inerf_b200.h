@@ -187,6 +187,16 @@ int inerf_mse_pair(const float* rgb, const float* rgb0, const float* target, int
 int inerf_head_torso_blend(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso,
                            int n, float* rgb, void* stream);
 
+/* Torso-stage loss seed, the counterpart of inerf_mse_pair for the composites of train_torso.py:269-270, for n rays:
+ * com = rgb_head * last_weight[:,None] + rgb_fg (the bits of inerf_head_torso_blend), loss2[0] = mean((com - target)^2) over 3n values,
+ * loss2[1] the same for the coarse set (rgb_head0, last_weight0, rgb_fg0);  g_com = 2 (com - target) / (3n);  g_rgb_fg = g_com;
+ * g_last_weight[i] = sum_c g_com[i,c] * rgb_head[i,c]  (and the "0" set).  The head is frozen in this stage: no gradient w.r.t. rgb_head.
+ * All (n,3) / (n) fp32 contiguous, any alignment; loss2: 2 floats (zeroed here).  n <= 0 is a shape error. */
+int inerf_head_torso_mse_pair(const float* rgb_head, const float* rgb_head0, const float* last_weight, const float* last_weight0,
+                              const float* rgb_fg, const float* rgb_fg0, const float* target, int64_t n,
+                              float* g_last_weight, float* g_last_weight0, float* g_rgb_fg, float* g_rgb_fg0,
+                              float* loss2, void* stream);
+
 /* The blend followed by to8b in one pass, for n rays: out_u8 (n,3) bytes = inerf_to8b(inerf_head_torso_blend(...)) bit for bit, and
  * out_rgb (n,3) = the fp32 blend, or NULL to skip it.  Replaces test_torso.py:523-524 on the rendered frame: a band of the composited
  * head + torso image leaves the GPU as 3n bytes.  Any alignment (16-byte aligned pointers take the vector path); n == 0 enqueues nothing. */
