@@ -14,7 +14,7 @@ REPO_ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 SO_PATH = os.environ.get("INERF_SO") or os.path.join(PKG_DIR, "libinerf_b200.so")     # INERF_SO: profiling builds only
 SOURCES = ["api.cu", "rays.cu", "composite.cu", "sample_pdf.cu", "mlp_fp32.cu", "mlp_fp32_bwd.cu", "mlp_bf16.cu", "mlp_bf16_bwd.cu",
-           "mlp_bf16_dw.cu", "mlp_f16x2.cu", "audio_net.cu", "render_fused.cu"]
+           "mlp_bf16_dw.cu", "mlp_f16x2.cu", "audio_net.cu", "render_fused.cu", "pixel_sampler.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--shared"]
 
@@ -52,6 +52,16 @@ class InerfRenderArgs(ctypes.Structure):
                                                 "weights", "z_vals", "rgb_map_fg", "rgb_map_fg0", "last_weight0", "nonfinite", "workspace")] +
                 [("workspace_bytes", ctypes.c_size_t)])
 
+
+class InerfPixelSampleArgs(ctypes.Structure):
+    _fields_ = ([(k, ctypes.c_int32) for k in ("H", "W", "n_frames")] + [("k", ctypes.c_int32 * 4)] +
+                [(k, ctypes.c_int32) for k in ("first", "count")] + [(k, ctypes.c_float) for k in ("focal", "cx", "cy", "near_", "far_")] +
+                [(k, ctypes.c_void_p) for k in ("frame_index", "bounds", "torso_bits", "poses", "frames", "bc_img", "rng_state", "rays", "target",
+                                                "bc_rgb", "coords")])
+
+
+INERF_PIXEL_SAMPLER_MAX_K = 4096
+INERF_PIXEL_SAMPLER_MAX_PIXELS = 1 << 22
 
 NF_BITS = {"rgb_map": 1, "disp_map": 2, "acc_map": 4, "rgb0": 8, "disp0": 16, "acc0": 32, "z_std": 64, "last_weight": 128}     # INERF_NF_*
 
@@ -106,6 +116,8 @@ SIGNATURES = {
     "inerf_audio_att_bwd": (_I, [_PARAMS, _PARAMS, _P, _P, _I, _I, _I, _P, _P]),
     "inerf_debug_hang_info": (_I, [ctypes.POINTER(ctypes.c_int32)]),
     "inerf_mlp_fwd_embedded": (_I, [_I, _DIMS, _PARAMS, _P, _P, _P, _L, _P, _P]),
+    "inerf_pixel_sampler_workspace_bytes": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _SZP]),
+    "inerf_sample_train_pixels": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _P, ctypes.c_size_t, _P]),
 }
 
 _lib = None
@@ -169,7 +181,7 @@ def lib():
         for name, (res, args) in SIGNATURES.items():
             fn = getattr(L, name)           # AttributeError here = header/library mismatch
             fn.restype, fn.argtypes = res, args
-        for which, struct in enumerate((InerfNetDims, InerfRenderNet, InerfRenderArgs)):      # the ctypes mirrors must match the header
+        for which, struct in ((0, InerfNetDims), (1, InerfRenderNet), (2, InerfRenderArgs), (4, InerfPixelSampleArgs)):      # the ctypes mirrors must match the header
             if L.inerf_sizeof(which) != ctypes.sizeof(struct):
                 raise RuntimeError(f"{struct.__name__}: ctypes layout ({ctypes.sizeof(struct)} B) differs from the library's "
                                    f"({L.inerf_sizeof(which)} B); rebuild libinerf_b200.so")

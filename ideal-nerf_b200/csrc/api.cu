@@ -24,6 +24,7 @@ extern "C" size_t inerf_sizeof(int which) {
         case 0: return sizeof(InerfNetDims);
         case 1: return sizeof(InerfRenderNet);
         case 2: return sizeof(InerfRenderArgs);
+        case 4: return sizeof(InerfPixelSampleArgs);
         default: return 0;
     }
 }

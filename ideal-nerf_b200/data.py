@@ -9,15 +9,16 @@ data_util/process_data.py:253-288:
     <data_dir>/ori_imgs/<img_id>.lms              68 x 2 landmarks; rows 48.. are the mouth
     <data_dir>/parsing/<img_id>.png               face parsing; pure red = torso
 
-Host side only (json / numpy / PIL), except that the N_rand training rays are generated on the device for the SELECTED pixels
-(ops.get_rays_at) instead of building the 450 x 450 ray grid per sample and indexing it (:123-139,189-191)."""
+HeadDataset is host side (json / numpy / PIL), except that the N_rand training rays are generated on the device for the SELECTED pixels
+(ops.get_rays_at) instead of building the 450 x 450 ray grid per sample and indexing it (:123-139,189-191).  DeviceHeadDataset decodes
+every frame once and draws each batch on the device (ops.sample_train_pixels): no host work per step."""
 import json
 import os
 
 import numpy as np
 import torch
 
-from . import ops
+from . import _lib, ops
 
 
 def _imread_rgb(path):
@@ -95,3 +96,144 @@ class HeadDataset(torch.utils.data.Dataset):
         bc_rgb = self.background_img[sel[:, 0], sel[:, 1]] if self.mode == "train" else self.background_img
         exp = torch.tensor(self.all_exprs[index], dtype=torch.float32)
         return batch_rays, target_s, bc_rgb, self.auds, raw_img, pose, exp, index
+
+
+# ---- the device-resident dataset -------------------------------------------------------------------------------------------------
+REGIONS = ("rect", "norect", "mouth", "torso")          # the output order of sample_pixels and of inerf_sample_train_pixels
+
+
+def region_budgets(args):
+    """(rect, norect, mouth, torso) rows of sample_pixels: mouth_rays, torso_rays, int((N_rand - mouth - torso) * sample_rate), the rest."""
+    mouth, torso = int(args.mouth_rays), int(args.torso_rays)
+    sample_num = int(args.N_rand) - mouth - torso
+    rect = int(sample_num * args.sample_rate)
+    k = (rect, sample_num - rect, mouth, torso)
+    if min(k) < 0:
+        raise ValueError(f"negative region budget {dict(zip(REGIONS, k))} from N_rand={args.N_rand}, mouth_rays={args.mouth_rays}, "
+                         f"torso_rays={args.torso_rays}, sample_rate={args.sample_rate}")
+    return k
+
+
+def _lower(v, n):
+    """Smallest integer i in [0, n] with i >= v (n: none of 0..n-1 qualifies)."""
+    return n if np.isnan(v) else int(np.clip(np.ceil(v), 0, n))
+
+
+def _upper(v, n):
+    """Largest integer i in [-1, n-1] with i <= v (-1: none of 0..n-1 qualifies)."""
+    return -1 if np.isnan(v) else int(np.clip(np.floor(v), -1, n - 1))
+
+
+def region_bounds(face_rect, landmark, H, W):
+    """int32 (8,) = inclusive (row lo, row hi, col lo, col hi) of the face rectangle, then of the mouth box, such that integer tests on
+    (row, col) select exactly the pixels of sample_pixels' predicates (the mouth's row against the landmarks' x range and its column
+    against their y range, as the reference compares them; float thresholds rounded inwards)."""
+    lm = np.asarray(landmark, dtype=np.float64)[48:]
+    fr = [int(v) for v in face_rect]
+    mr0, mr1 = np.min(lm[:, 0]) - 20, np.max(lm[:, 0]) + 20
+    mc0, mc1 = np.min(lm[:, 1]) - 20, np.max(lm[:, 1]) + 20
+    return np.array([_lower(fr[0], H), _upper(fr[0] + fr[2], H), _lower(fr[1], W), _upper(fr[1] + fr[3], W),
+                     _lower(mr0, H), _upper(mr1, H), _lower(mc0, W), _upper(mc1, W)], dtype=np.int32)
+
+
+def torso_bits(parse_img):
+    """uint32 (ceil(H*W/32),): bit p & 31 of word p >> 5 is set where parsing pixel p = row * W + col is pure red (255, 0, 0)."""
+    t = ((parse_img[:, :, 0] == 255) & (parse_img[:, :, 1] == 0) & (parse_img[:, :, 2] == 0)).reshape(-1)
+    t = np.concatenate([t, np.zeros((-t.size) % 32, bool)])
+    return (t.reshape(-1, 32).astype(np.uint64) << np.arange(32, dtype=np.uint64)).sum(1).astype(np.uint32)
+
+
+def region_sizes(bounds, n_torso, H, W):
+    """Members of (rect, norect, mouth, torso) of each frame: bounds (F, 8) as region_bounds, n_torso (F,) -> int64 (F, 4)."""
+    b = np.asarray(bounds, dtype=np.int64)
+
+    def area(r0, r1, c0, c1):
+        return np.maximum(r1 - r0 + 1, 0) * np.maximum(c1 - c0 + 1, 0)
+
+    rect = area(b[:, 0], b[:, 1], b[:, 2], b[:, 3])
+    mouth = area(b[:, 4], b[:, 5], b[:, 6], b[:, 7])
+    both = area(np.maximum(b[:, 0], b[:, 4]), np.minimum(b[:, 1], b[:, 5]), np.maximum(b[:, 2], b[:, 6]), np.minimum(b[:, 3], b[:, 7]))
+    return np.stack([rect - both, H * W - rect, mouth, np.asarray(n_torso, dtype=np.int64)], 1)
+
+
+def check_region_sizes(sizes, budgets, names=None):
+    """ValueError naming the first frame and region with fewer members than its budget (np.random.choice(replace=False) would raise there
+    in the middle of training)."""
+    short = np.argwhere(np.asarray(sizes) < np.asarray(budgets)[None, :])
+    if len(short):
+        f, r = (int(v) for v in short[0])
+        name = names[f] if names is not None else str(f)
+        raise ValueError(f"frame {f} ({name}): region '{REGIONS[r]}' has {int(sizes[f][r])} pixels, fewer than its budget of {budgets[r]} rays")
+
+
+class DeviceHeadDataset(HeadDataset):
+    """HeadDataset with every frame decoded once and kept on the device (BGR uint8), and each training batch drawn there.
+
+    sample(index) draws the batch with the region budgets of sample_pixels -- from the same distribution, not the same numbers: the draw
+    is the Philox contract of inerf_sample_train_pixels (include/inerf_b200.h) -- and builds rays, targets, bc_rgb, the audio window, the
+    expression and the pose without a host synchronise, so `index` may be an int64 device tensor and the call may sit in a CUDA graph.
+    Memory: F * H * W * 3 bytes of frames (5 000 frames of 450 x 450: 3.0 GB) plus small per-frame tables."""
+
+    def __init__(self, data_dir, aud_file, mode, args, skip=1, device="cuda"):
+        super().__init__(data_dir, aud_file, mode, args, skip, device)
+        self.budgets = region_budgets(args)
+        imgs = [_imread_rgb(p)[:, :, ::-1] for p in self.all_imgs]              # cv2.imread order: BGR
+        shapes = {im.shape for im in imgs}
+        if len(shapes) != 1:
+            raise ValueError(f"frames differ in size: {sorted(shapes)}")
+        H, W = imgs[0].shape[:2]
+        if tuple(self.background_img.shape[:2]) != (H, W):
+            raise ValueError(f"bc.jpg is {tuple(self.background_img.shape[:2])}, the frames are {(H, W)}")
+        if H * W > _lib.INERF_PIXEL_SAMPLER_MAX_PIXELS:
+            raise ValueError(f"{H} x {W} frames exceed the sampler's {_lib.INERF_PIXEL_SAMPLER_MAX_PIXELS} pixels")
+        self.H, self.W = H, W
+        bounds, bits, n_torso = [], [], []
+        for rect, lms, parse in zip(self.all_face_rects, self.all_landmarks, self.all_parse_imgs):
+            bounds.append(region_bounds(rect, np.loadtxt(lms), H, W))
+            b = torso_bits(_imread_rgb(parse))
+            bits.append(b)
+            n_torso.append(int(np.unpackbits(b.view(np.uint8)).sum()))
+        check_region_sizes(region_sizes(np.stack(bounds), n_torso, H, W), self.budgets, [os.path.basename(p) for p in self.all_imgs])
+        dev = self.device
+        self.frames = torch.from_numpy(np.ascontiguousarray(np.stack(imgs))).to(dev)
+        self.bounds = torch.from_numpy(np.stack(bounds)).to(dev)
+        self.torso_bits = torch.from_numpy(np.stack(bits).view(np.int32)).to(dev)
+        self.poses = torch.tensor(np.stack(self.all_poses)[:, :3, :4], dtype=torch.float32, device=dev)
+        self.exprs = torch.tensor(np.asarray(self.all_exprs), dtype=torch.float32, device=dev)
+        self.bc_img = self.background_img.float().contiguous()
+        half = int(getattr(args, "smo_size", 8) / 2)
+        pad = torch.zeros((half,) + tuple(self.auds.shape[1:]), dtype=self.auds.dtype, device=dev)
+        self.auds_padded = torch.cat([pad, self.auds, pad], 0)
+        self._win = torch.arange(2 * half, dtype=torch.int64, device=dev)
+        self._index = torch.zeros((), dtype=torch.int64, device=dev)
+
+    def sample(self, index, rank=0, world=1):
+        """The training batch of frame `index` (host int or int64 device scalar), rows frame.band(N_rand, rank, world) of it: a dict with
+        rays (n, 11) packed with args.near / args.far, target (n, 3), bc_rgb (n, 3), aud_window (smo_size, 16, 29) =
+        Network.audio_window(auds, index, len(self)), expr, pose (3, 4).  Advances the Philox offset by one."""
+        from .frame import band
+        if torch.is_tensor(index):
+            idx = index.reshape(())
+            if idx.dtype != torch.int64 or idx.device != self.frames.device:
+                raise ValueError(f"a tensor index must be an int64 scalar on {self.frames.device}")
+        else:
+            if not 0 <= int(index) < self.data_size:
+                raise IndexError(f"frame {index} outside [0, {self.data_size})")
+            idx = self._index.fill_(int(index))
+        lo, hi = band(sum(self.budgets), rank, world)
+        rays, target, bc_rgb, _ = ops.sample_train_pixels(idx, self.budgets, self.bounds, self.torso_bits, self.poses, self.frames,
+                                                          self.bc_img, self.focal, self.cx, self.cy, self.args.near, self.args.far,
+                                                          first=lo, count=hi - lo)
+        i1 = idx.reshape(1)
+        return {"rays": rays, "target": target, "bc_rgb": bc_rgb, "aud_window": self.auds_padded.index_select(0, i1 + self._win),
+                "expr": self.exprs.index_select(0, i1)[0], "pose": self.poses.index_select(0, i1)[0]}
+
+    def __getitem__(self, index):
+        """HeadDataset's tuple (batch_rays (2, N_rand, 3), target_s, bc_rgb, auds, raw_img, pose, exp, index) built from sample(): raw_img
+        is the device frame (BGR uint8), bc_rgb fp32."""
+        if index is None:
+            index = np.random.choice(self.data_size)
+        b = self.sample(index)
+        rays = b["rays"]
+        batch_rays = torch.stack([rays[:, 0:3], rays[:, 3:6]], 0)
+        return batch_rays, b["target"], b["bc_rgb"], self.auds, self.frames[index], self.all_poses[index][:3, :4], b["expr"], index

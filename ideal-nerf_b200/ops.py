@@ -171,7 +171,7 @@ def sample_coarse(rays, n_samples, t_rand=None, lindisp=False):
 # ------------------------------------------------------------------------------------------------
 # in-kernel random draws (perturb > 0): Philox state per device, {seed, offset} in device memory
 # ------------------------------------------------------------------------------------------------
-RNG_STREAM_COARSE, RNG_STREAM_PDF = 1, 2
+RNG_STREAM_COARSE, RNG_STREAM_PDF, RNG_STREAM_PIXELS = 1, 2, 3
 _rng_states = {}
 
 
@@ -228,6 +228,44 @@ def importance_sample_rng(z_coarse, w_coarse, n_importance, state=None, stream_i
     if advance:
         rng_advance(state)
     return zs, zm, zstd
+
+
+def sample_train_pixels(frame_index, budgets, bounds, torso_bits, poses, frames, bc_img, focal, cx, cy, near, far, first=0, count=None,
+                        state=None, want_coords=False, advance=True):
+    """The training batch of frame `frame_index` (int64 device scalar) drawn on the device (include/inerf_b200.h, inerf_sample_train_pixels):
+    budgets = (rect, norect, mouth, torso) rows; bounds (F, 8) int32, torso_bits (F, ceil(H*W/32)) int32 / uint32 bits, poses (F, 3, 4)
+    fp32, frames (F, H, W, 3) uint8, bc_img (H, W, 3) fp32.  Returns (rays (count, 11), target (count, 3), bc_rgb (count, 3),
+    coords (count, 2) int64 or None) for the rows [first, first + count) of the N_rand = sum(budgets) rows.  Draws from `state` (default:
+    the device's Philox state), whose offset is advanced afterwards when `advance`."""
+    dev = frames.device
+    for t, name, dt in ((frame_index, "frame_index", torch.int64), (bounds, "bounds", torch.int32), (torso_bits, "torso_bits", torch.int32),
+                        (poses, "poses", torch.float32), (frames, "frames", torch.uint8), (bc_img, "bc_img", torch.float32)):
+        _need_cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"sample_train_pixels: `{name}` must be a contiguous {dt} tensor on {dev}")
+    F, H, W = frames.shape[0], frames.shape[1], frames.shape[2]
+    n_rand = sum(int(k) for k in budgets)
+    count = n_rand - int(first) if count is None else int(count)
+    state = rng_state(dev) if state is None else state
+    rays = torch.empty((count, 11), device=dev, dtype=torch.float32)
+    target = torch.empty((count, 3), device=dev, dtype=torch.float32)
+    bc_rgb = torch.empty((count, 3), device=dev, dtype=torch.float32)
+    coords = torch.empty((count, 2), device=dev, dtype=torch.int64) if want_coords else None
+    a = _lib.InerfPixelSampleArgs(H=H, W=W, n_frames=F, k=(ctypes.c_int32 * 4)(*[int(k) for k in budgets]), first=int(first), count=count,
+                                  focal=float(focal), cx=float(cx), cy=float(cy), near_=float(near), far_=float(far),
+                                  frame_index=frame_index.data_ptr(), bounds=bounds.data_ptr(), torso_bits=torso_bits.data_ptr(),
+                                  poses=poses.data_ptr(), frames=frames.data_ptr(), bc_img=bc_img.data_ptr(), rng_state=state.data_ptr(),
+                                  rays=rays.data_ptr(), target=target.data_ptr(), bc_rgb=bc_rgb.data_ptr(),
+                                  coords=coords.data_ptr() if want_coords else None)
+    L = _lib.lib()
+    nbytes = ctypes.c_size_t(0)
+    check(L.inerf_pixel_sampler_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), "inerf_pixel_sampler_workspace_bytes")
+    ws = torch.empty((nbytes.value,), device=dev, dtype=torch.uint8)
+    with torch.cuda.device(dev):
+        call("inerf_sample_train_pixels", L.inerf_sample_train_pixels, ctypes.byref(a), ptr(ws), nbytes.value, stream(), launches=4)
+    if advance:
+        rng_advance(state)
+    return rays, target, bc_rgb, coords
 
 
 def flag_nonfinite(tensors, flags):

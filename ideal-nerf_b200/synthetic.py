@@ -1,7 +1,7 @@
 """Seeded synthetic inputs of the shapes BASELINE.json names (SURVEY.md 8d): camera, background,
 audio / expression / latent codes, random-init FaceNeRF weights with the normalised-density preset.
 
-Used by bench.py and __graft_entry__.smoke(); there is no dataset or checkpoint in this environment.
+Used by bench.py and __graft_entry__.smoke(); write_head_subject writes a small subject on disk for the dataset classes.
 The tensors follow the same generator sequence as the test oracle's synthetic_frame so both arms of
 the benchmark see the same data, but nothing here imports the test infrastructure.
 """
@@ -49,3 +49,36 @@ def normalise_density_(net, rays, aud, expr, latent, n_samples=64, target_std=8.
     net.alpha_linear.weight.mul_(k)
     net.alpha_linear.bias.copy_((net.alpha_linear.bias - float(s.mean())) * k + 0.01)
     return net
+
+
+def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, constant_rgb=None, n_aud=None):
+    """A seeded synthetic subject in the reference's on-disk layout (data.py): random JPEG frames (or one constant colour), parsing maps
+    whose last `torso_rows` rows are torso, landmarks that give a mouth box near the centre, a face rectangle, bc.jpg, aud.npy and
+    transforms_exp_train.json.  Returns the args a HeadDataset needs for it (gt_dirs = head_imgs)."""
+    import json
+    import os
+
+    import numpy as np
+    from PIL import Image
+    for sub in ("head_imgs", "ori_imgs", "parsing"):
+        os.makedirs(os.path.join(d, sub), exist_ok=True)
+    rng = np.random.RandomState(seed)
+    frames = []
+    for i in range(n_frames):
+        img = np.empty((H, W, 3), np.uint8)
+        img[:] = constant_rgb if constant_rgb is not None else rng.randint(0, 255, (H, W, 3), dtype=np.uint8)
+        Image.fromarray(img).save(os.path.join(d, "head_imgs", f"{i}.jpg"), quality=95)
+        parse = np.zeros((H, W, 3), np.uint8)
+        parse[H - torso_rows:, :, 0] = 255
+        Image.fromarray(parse).save(os.path.join(d, "parsing", f"{i}.png"))
+        lms = rng.rand(68, 2) * 10 + H * 0.3
+        lms[48:] = rng.rand(20, 2) * 0.1 * min(H, W) + np.array([H * 0.55, W * 0.45])
+        np.savetxt(os.path.join(d, "ori_imgs", f"{i}.lms"), lms)
+        pose = np.eye(4)
+        pose[:3, 3] = [0.001 * i, -0.002, 0.7772]
+        frames.append({"img_id": i, "aud_id": i, "transform_matrix": pose.tolist(),
+                       "face_rect": [H // 8, W // 8, H * 5 // 8, W * 3 // 4], "exp": rng.randn(76).tolist()})
+    with open(os.path.join(d, "transforms_exp_train.json"), "w") as fp:
+        json.dump({"focal_len": 1200.0 * W / 450, "cx": W / 2, "cy": H / 2, "frames": frames}, fp)
+    np.save(os.path.join(d, "aud.npy"), rng.randn(n_aud or n_frames, 16, 29).astype(np.float32))
+    Image.fromarray(rng.randint(0, 255, (H, W, 3), dtype=np.uint8)).save(os.path.join(d, "bc.jpg"), quality=95)

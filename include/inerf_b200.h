@@ -93,8 +93,8 @@ int inerf_version(void);
 const char* inerf_last_error(void);
 /* 0 when the current CUDA device is compute capability 10.x, INERF_E_DEVICE otherwise. */
 int inerf_device_check(void);
-/* sizeof of the structs of this header as the library was compiled: 0 InerfNetDims, 1 InerfRenderNet, 2 InerfRenderArgs (0 for any
- * other value) -- lets a foreign-language binding check its struct layout at load time. */
+/* sizeof of the structs of this header as the library was compiled: 0 InerfNetDims, 1 InerfRenderNet, 2 InerfRenderArgs,
+ * 4 InerfPixelSampleArgs (0 for any other value, 3 included: bindings written against the three-struct header check that 3 reports 0) -- lets a foreign-language binding check its struct layout at load time. */
 size_t inerf_sizeof(int which);
 
 /* ---- rays ----------------------------------------------------------------------------------- */
@@ -144,6 +144,7 @@ int inerf_sample_coarse(const float* rays, int n, int ray_stride, int s, const f
  * inerf_rng_advance adds `increment` to the offset (one tiny launch, graph-capturable) so the next step draws fresh numbers. */
 #define INERF_RNG_STREAM_COARSE 1u /* stratified jitter of inerf_sample_coarse_rng */
 #define INERF_RNG_STREAM_PDF 2u    /* default stream of inerf_importance_sample_rng */
+#define INERF_RNG_STREAM_PIXELS 3u /* per-pixel keys of inerf_sample_train_pixels */
 int inerf_rng_advance(uint64_t* rng_state, uint64_t increment, void* stream);
 
 /* inerf_sample_coarse with t_rand = U[0,1) drawn in the kernel (word (i & 3) of Philox block (i >> 2), i = ray * s + sample; the
@@ -202,6 +203,59 @@ int inerf_head_torso_mse_pair(const float* rgb_head, const float* rgb_head0, con
  * head + torso image leaves the GPU as 3n bytes.  Any alignment (16-byte aligned pointers take the vector path); n == 0 enqueues nothing. */
 int inerf_head_torso_to8b(const float* rgb_head, const float* last_weight_torso, const float* rgb_fg_torso, int64_t n,
                           uint8_t* out_u8, float* out_rgb, void* stream);
+
+/* ---- training-batch pixel sampler -------------------------------------------------------------
+ * The pixel selection of the training sampler (audio_exp_nerf.py:141-187, data.HeadDataset.sample_pixels) and the batch built from
+ * it (:189-191), on the device.  It draws from the same distribution as sample_pixels (an ordered k-subset per region, uniformly at
+ * random, without replacement) but not the same numbers; the draw is fixed exactly by these rules:
+ *   - pixel p = row * W + col; its keys are the words (x, y, z, w) of philox_at(rng_state, index = p, INERF_RNG_STREAM_PIXELS);
+ *   - regions, from bounds[f] = {rr0, rr1, rc0, rc1, mr0, mr1, mc0, mc1} (inclusive int32) and the torso bitmask:
+ *       R = rr0 <= row <= rr1 && rc0 <= col <= rc1   (face_rect: rr0 = fr[0], rr1 = fr[0] + fr[2], rc0 = fr[1], rc1 = fr[1] + fr[3])
+ *       M = mr0 <= row <= mr1 && mc0 <= col <= mc1   (mouth: the row against the landmarks' x range, the column against their y range,
+ *                                                      as the reference compares them; ceil of the lower and floor of the upper float
+ *                                                      thresholds, so the integer tests equal its float64 ones)
+ *       T = bit (p & 31) of torso_bits[f][p >> 5]   (the parsing pixel is pure red)
+ *   - region r, its members and its key: 0 rect = R && !M, key x;  1 norect = !R, key x;  2 mouth = M, key y;  3 torso = T, key z
+ *     (overlapping regions use different words, so their draws are independent);
+ *   - selection: the k[r] members with the smallest (key << 32 | p), in ascending order of that value (ties in the key go to the lower
+ *     pixel index);
+ *   - output rows: rect, norect, mouth, torso, k[0] + k[1] + k[2] + k[3] = N_rand rows in all; the call writes the rows
+ *     [first, first + count) only, so ranks that share rng_state and each take a band of N_rand emit disjoint parts of one batch.
+ * Per output row: rays (count, 11) as inerf_get_rays_at writes them for that pixel and pose; target (count, 3) = the frame's bytes (BGR,
+ * as stored) times fl(1 / 255), the fp32 bits of torch's CUDA `u8.float() / 255.0`; bc_rgb (count, 3) = bc_img at the pixel; coords
+ * (count, 2) int64 (row, col), optional.
+ * Every input is read from device memory (the frame index too), so a captured CUDA graph draws a fresh batch on every replay once the
+ * offset of rng_state is advanced (inerf_rng_advance, not done here).  A frame index outside [0, n_frames) selects nothing and writes no
+ * output; a region with fewer than k[r] members leaves its last rows unwritten -- the caller rules both out (the library cannot read
+ * device data without a synchronise).
+ * Limits: k[r] <= INERF_PIXEL_SAMPLER_MAX_K (INERF_E_UNSUPPORTED above: one CTA sorts each region in shared memory), H * W <=
+ * INERF_PIXEL_SAMPLER_MAX_PIXELS (beyond it one of the 4096 histogram bins that bound the sort could overflow it). */
+#define INERF_PIXEL_SAMPLER_MAX_K 4096
+#define INERF_PIXEL_SAMPLER_MAX_PIXELS (1 << 22)
+
+typedef struct InerfPixelSampleArgs {
+    int32_t H, W, n_frames;
+    int32_t k[4];                  /* region budgets: rect, norect, mouth, torso                                              */
+    int32_t first, count;          /* the band of output rows                                                                 */
+    float focal, cx, cy, near_, far_;
+    const int64_t* frame_index;    /* device scalar                                                                           */
+    const int32_t* bounds;         /* (n_frames, 8)                                                                           */
+    const uint32_t* torso_bits;    /* (n_frames, ceil(H * W / 32))                                                            */
+    const float* poses;            /* (n_frames, 3, 4) camera-to-world                                                        */
+    const uint8_t* frames;         /* (n_frames, H, W, 3)                                                                     */
+    const float* bc_img;           /* (H, W, 3) background                                                                    */
+    const uint64_t* rng_state;     /* {seed, offset}                                                                          */
+    float* rays;                   /* outputs, `count` rows each                                                              */
+    float* target;
+    float* bc_rgb;
+    int64_t* coords;               /* NULL to skip                                                                            */
+} InerfPixelSampleArgs;
+
+/* Workspace of inerf_sample_train_pixels: the per-region key histograms, boundary bins and candidate buffers. */
+int inerf_pixel_sampler_workspace_bytes(const InerfPixelSampleArgs* args, size_t* bytes);
+/* workspace: 256-byte aligned, at least inerf_pixel_sampler_workspace_bytes.  Four kernels and one memset on `stream`; count == 0
+ * enqueues nothing.  Every argument error is returned before any device work. */
+int inerf_sample_train_pixels(const InerfPixelSampleArgs* args, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- importance sampling -------------------------------------------------------------------- */
 
