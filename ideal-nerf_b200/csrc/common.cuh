@@ -52,8 +52,17 @@ struct CondLayout {
     __host__ __device__ int views(int i) const { return 8 * W + i * H; }
     __host__ __device__ int alpha_b() const { return 8 * W + 3 * H; }
     __host__ __device__ int rgb_b() const { return 8 * W + 3 * H + 1; }
-    __host__ __device__ int total() const { return 8 * W + 3 * H + 4; }
+    __host__ __device__ constexpr int total() const { return 8 * W + 3 * H + 4; }
 };
+
+// `cond` of one call: the COND_FLOATS folded fp32 biases (CondLayout{256, 128}), then two bias-tile sets for the tensor-core kernels
+// (fold_cond.cuh): the bf16 set, then the fp16x2 set.  A set holds one tile per (layer, half): 4 KB for the 8 pts_linears (128 rows),
+// 2 KB for the 3 views_linears (64 rows).
+constexpr int COND_FLOATS = CondLayout{256, 128}.total();
+constexpr int BIAS_TILE_BYTES = 16 * 4096 + 6 * 2048;
+__host__ __device__ constexpr uint32_t bias_tile_offset(int layer, int half) {
+    return layer < 8 ? (2 * layer + half) * 4096u : 65536u + (2 * (layer - 8) + half) * 2048u;
+}
 
 inline int check_dims(const InerfNetDims* d) {
     if (!d) return fail(INERF_E_ARG, "dims is NULL");

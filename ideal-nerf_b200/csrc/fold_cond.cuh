@@ -1,7 +1,7 @@
 // Conditioning fold (SURVEY.md Appendix B; face_nerf.py:44-56,69): the per-call constant columns [aud | expr/3 | latent] of pts_linears.0 / .5 and
 // views_linears.0 become biases, written as fp32 (CondLayout) and as the operand tiles of the two tensor-core kernels.  The block body is
-// shared by inerf_mlp_fold_cond (mlp_fp32.cu: one net per launch) and the set-up kernel of inerf_render_rays_fused (render_fused.cu: both
-// nets of a render_rays call plus the rays and coarse depths in ONE launch).
+// shared by fold_cond_kernel (mlp_fp32.cu, launched by inerf_mlp_fold_cond: one net per launch) and the set-up kernel of
+// inerf_render_rays_fused (render_fused.cu: both nets of a render_rays call plus the rays and coarse depths in ONE launch).
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -16,6 +16,7 @@ struct FoldArgs {
     int da, de, dl;
     float* cond;
 };
+int mlp_fold_cond_launch(const FoldArgs& f, cudaStream_t st);      // mlp_fp32.cu
 
 // Row `r` of a bias tile for the tensor-core kernel (mlp_bf16.cu): K-major, non-swizzled [rows][16] bf16 stored as 8x8 core
 // matrices, columns (hi, lo, 0, ..., 0) with hi + lo = the fp32 bias to 16 mantissa bits.
@@ -41,12 +42,10 @@ __device__ __forceinline__ void write_bias_tile_row_f16x3(uint8_t* tile, int r, 
     *reinterpret_cast<uint4*>(p + 128) = make_uint4(0u, 0u, 0u, 0u);
 }
 
-constexpr int BIAS_TILE_BYTES = 16 * 4096 + 6 * 2048;      // per tile set: 8 layers x 2 halves x 4 KB + 3 layers x 2 halves x 2 KB
-
 // One block of the fold: bx in [0, 12) = layer (8 pts_linears, 3 views_linears, the two head biases), by in [0, 8) = row group; 256 threads;
 // c = 1024 floats of shared memory.
 __device__ __forceinline__ void fold_cond_block(const FoldArgs& f, int bx, int by, float* c) {
-    uint8_t* tiles = reinterpret_cast<uint8_t*>(f.cond + CondLayout{256, 128}.total());
+    uint8_t* tiles = reinterpret_cast<uint8_t*>(f.cond + COND_FLOATS);
     const int C = f.da + f.de + f.dl;
     for (int i = threadIdx.x; i < C; i += blockDim.x) {
         float v;
@@ -70,8 +69,8 @@ __device__ __forceinline__ void fold_cond_block(const FoldArgs& f, int bx, int b
             s = warp_sum(s);
             if (lane == 0) {
                 f.cond[cl.pts(b) + n] = B[n] + s;
-                write_bias_tile_row(tiles + (2 * b + (n >> 7)) * 4096, n & 127, B[n] + s);
-                write_bias_tile_row_f16x3(tiles + BIAS_TILE_BYTES + (2 * b + (n >> 7)) * 4096, n & 127, B[n] + s);
+                write_bias_tile_row(tiles + bias_tile_offset(b, n >> 7), n & 127, B[n] + s);
+                write_bias_tile_row_f16x3(tiles + BIAS_TILE_BYTES + bias_tile_offset(b, n >> 7), n & 127, B[n] + s);
             }
         }
     } else if (b < 11) {                          // views_linears.(b-8)
@@ -86,8 +85,8 @@ __device__ __forceinline__ void fold_cond_block(const FoldArgs& f, int bx, int b
             s = warp_sum(s);
             if (lane == 0) {
                 f.cond[cl.views(v) + n] = B[n] + s;
-                write_bias_tile_row(tiles + 65536 + (2 * v + (n >> 6)) * 2048, n & 63, B[n] + s);
-                write_bias_tile_row_f16x3(tiles + BIAS_TILE_BYTES + 65536 + (2 * v + (n >> 6)) * 2048, n & 63, B[n] + s);
+                write_bias_tile_row(tiles + bias_tile_offset(b, n >> 6), n & 63, B[n] + s);
+                write_bias_tile_row_f16x3(tiles + BIAS_TILE_BYTES + bias_tile_offset(b, n >> 6), n & 63, B[n] + s);
             }
         }
     } else if (threadIdx.x < 4 && by == 0) {

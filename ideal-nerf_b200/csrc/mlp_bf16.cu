@@ -35,8 +35,7 @@
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
-#include "mlp_common.cuh"
-#include "sm100_ptx.cuh"
+#include "mlp_tc.cuh"
 
 using namespace inerf;
 using namespace sm100;
@@ -47,46 +46,15 @@ constexpr int NSTAGE = 3;
 constexpr int STAGE_BYTES = 16384;
 // CTA-pair build (PAIR = true): every weight stage is split across the two CTAs of a cluster (each holds HALF of its rows), so the same
 // 48 KB ring is six stages deep
-constexpr int NSTAGE_PAIR = 6;
-constexpr int STAGE_BYTES_PAIR = 8192;
-template <bool PAIR> struct RingOf { static constexpr int N = PAIR ? NSTAGE_PAIR : NSTAGE, BYTES = PAIR ? STAGE_BYTES_PAIR : STAGE_BYTES; };
+template <bool PAIR> using RingOf = Ring<PAIR, NSTAGE>;
 constexpr int MAX_STEPS = 80;
 constexpr int RMAX = 4;            // rays a 128-row slot can touch (s >= 43)
 constexpr int NTHREADS_BF16 = 512;
 constexpr int N_EPI = 256, N_PE = 128;
 
-// event bits
-enum { W_E0 = 1, W_E1 = 2, W_PE = 4 };
-enum { C_C0 = 1, C_C1 = 2, C_C2 = 4, C_PEFREE = 8 };
-
-struct Step {
-    uint8_t a_kb;      // 0..3 activation K-block, 4 = positional-encoding block
-    uint8_t n8;        // MMA N / 8
-    uint8_t acc_col;   // accumulator column offset inside the slot (0, 64, 128)
-    uint8_t first;     // first MMA of its (layer, half): overwrite instead of accumulate
-    uint8_t wait;      // W_* bits
-    uint8_t commit;    // C_* bits
-    uint8_t layer;     // 0..10
-    uint8_t pad;
-    uint32_t offset;   // byte offset of this stage's image inside the packed blob
-};
-
-struct PackStep {
-    int w_index, ldw, n0, rows, wcol;   // weight rows [n0, n0+rows), columns wcol .. wcol+63 (kmax valid)
-    int kmax;
-    uint32_t offset;
-};
-
-struct Schedule {
-    int n_steps;
-    Step steps[MAX_STEPS];
-    PackStep pack[MAX_STEPS];
-    uint32_t total_bytes;
-};
-
-__constant__ Step c_steps[MAX_STEPS];
-__constant__ Step c_steps_emb[MAX_STEPS];      // the embedded-row schedule (one more K-block per V0 half)
-template <bool EMB> __device__ __forceinline__ const Step& step_at(int s) { return EMB ? c_steps_emb[s] : c_steps[s]; }
+__constant__ TcStage c_steps[MAX_STEPS];
+__constant__ TcStage c_steps_emb[MAX_STEPS];      // the embedded-row schedule (one more K-block per V0 half)
+template <bool EMB> __device__ __forceinline__ const TcStage& step_at(int s) { return EMB ? c_steps_emb[s] : c_steps[s]; }
 
 // smem map (bytes from the 1024-aligned base)
 constexpr int OFF_ACT = 0;                               // [2][4][16384]
@@ -99,14 +67,13 @@ constexpr int OFF_AW = OFF_SB + 16;                      // alpha_linear.weight 
 constexpr int OFF_RW = OFF_AW + 1024;                    // rgb_linear.weight 3x128 floats
 constexpr int OFF_DIRB = OFF_RW + 1536;                  // [2][RMAX][128] floats
 constexpr int OFF_BAR = OFF_DIRB + 2 * RMAX * 128 * 4;   // mbarriers
-constexpr int BIAS_TILE_BYTES_TOTAL = 16 * 4096 + 6 * 2048;   // per call, after the 2436 folded fp32 biases of `cond`
 constexpr int SMEM_BYTES = OFF_BAR + 320;
 constexpr int SMEM_ALLOC = SMEM_BYTES;
 static_assert(SMEM_ALLOC <= 232448, "shared memory budget");
 
 struct Bars {
-    uint64_t wfull[NSTAGE_PAIR], wempty[NSTAGE_PAIR];
-    uint64_t pfull[NSTAGE_PAIR];   // pair build, leader only: the PEER's half of the stage has landed (relayed by the peer's warp 1)
+    uint64_t wfull[RingOf<true>::N], wempty[RingOf<true>::N];
+    uint64_t pfull[RingOf<true>::N];   // pair build, leader only: the PEER's half of the stage has landed (relayed by the peer's warp 1)
     uint64_t cbar[3];        // C0, C1, C2   (tcgen05.commit, once per layer; pair build: multicast to both CTAs)
     uint64_t ebar[2];        // E0, E1       (8 epilogue warps, once per layer; pair build: the leader's, 8 + 8 warps)
     uint64_t pe_ready;       // 128 PE threads, once per iteration (pair build: the leader's, 4 + 4 warps)
@@ -156,8 +123,8 @@ __device__ unsigned long long g_phase[148][16];
 // issuer-side wait on an event whose arrivals may come from the peer CTA (pair build: cluster-scope acquire)
 template <bool DBG, bool PAIR>
 __device__ __forceinline__ void wait_ev(uint64_t* bar, uint32_t parity, int code, int aux0, int aux1) {
-    if constexpr (PAIR) mbar_wait_cluster(bar, parity);
-    else wait_or_report<DBG>(bar, parity, code, aux0, aux1);
+    if constexpr (DBG && !PAIR) wait_or_report<true>(bar, parity, code, aux0, aux1);
+    else sm100::wait_ev<PAIR>(bar, parity);
 }
 
 struct LayerInfo { int N, bias_off; };
@@ -207,59 +174,6 @@ __device__ __forceinline__ void epi_convert(const uint32_t (&r)[32], uint32_t* _
         }
     }
 }
-
-// ---------------------------------------------------------------------------------------------
-// compile-time layer geometry (must agree with build_schedule below, which lays out the packed blob)
-// ---------------------------------------------------------------------------------------------
-__host__ __device__ constexpr int lay_N(int l) { return l < 8 ? 256 : 128; }
-__host__ __device__ constexpr int lay_act_kb(int l) { return l == 0 ? 0 : (l <= 8 ? 4 : 2); }     // activation K-blocks (64 wide)
-__host__ __device__ constexpr bool lay_pe(int l) { return l == 0 || l == 5; }                     // + the gamma(p) K-block
-__host__ __device__ constexpr bool lay_x(int l, bool emb) { return lay_pe(l) || (emb && l == 8); }   // + a PE-buffer K-block (gamma(p) or gamma(v))
-__host__ __device__ constexpr int lay_prev_N(int l) { return l == 0 ? 128 : lay_N(l - 1); }       // L0 follows V2 of the previous iteration
-
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-
-// tcgen05.mma with the two smem descriptors given as (lo, hi) halves: lo = the 14-bit start-address field (+ LBO bit), advanced with
-// plain 32-bit adds of compile-time constants; hi is the same constant for every operand of this kernel.
-__device__ __forceinline__ void umma_bf16_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
-// The same for a CTA pair: M = 256 (128 rows from each CTA), the N rows of B split across the two CTAs; issued by the leader only.
-__device__ __forceinline__ void umma_bf16_lohi_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-template <bool PAIR>
-__device__ __forceinline__ void umma_any(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    if constexpr (PAIR) umma_bf16_lohi_pair(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
-    else umma_bf16_lohi(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
-}
-template <bool PAIR>
-__device__ __forceinline__ void commit_any(uint64_t* bar) {
-    if constexpr (PAIR) umma_commit_pair(bar);
-    else umma_commit(bar);
-}
-
-// Descriptor halves of a K-major, NON-swizzled 16-column (K = 16) bf16 tile stored as [row/8][k/8][row%8][k%8]: 8x8 core matrices of
-// 128 contiguous bytes, the two K halves 128 B apart (leading byte offset), 8-row groups 256 B apart (stride byte offset).
-constexpr uint32_t HI_NOSWZ = (256u >> 4) | (1u << 14);
-__device__ __forceinline__ uint32_t desc_lo_noswz(uint32_t smem_addr) { return ((smem_addr & 0x3FFFF) >> 4) | ((128u >> 4) << 16); }
 
 struct IssueCtx {
     Bars* bars;
@@ -509,7 +423,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
         // ================= weight producer ==================================================
         if (lane == 0) {
             const uint8_t* blob = reinterpret_cast<const uint8_t*>(a.packed);
-            const uint8_t* tiles = reinterpret_cast<const uint8_t*>(a.cond + 2436);
+            const uint8_t* tiles = reinterpret_cast<const uint8_t*>(a.cond + COND_FLOATS);
             uint32_t g = 0, bh = 0;
             // pair build: this CTA's HALF of the rows of every stage / bias tile (rows [rank * NH / 2, (rank + 1) * NH / 2) are the first /
             // second half of the image's bytes: 8-row groups are contiguous)
@@ -518,9 +432,9 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 for (int s = 0; s < n_steps; ++s, ++g) {
                     const uint32_t stage = g % NSTAGE, round = g / NSTAGE;
                     if (step_at<EMB>(s).first) {       // first step of a (layer, half): its bias tile
-                        const uint32_t slot = bh & 1, l = step_at<EMB>(s).layer, h = step_at<EMB>(s).acc_col ? 1u : 0u;
+                        const uint32_t slot = bh & 1, l = step_at<EMB>(s).layer, h = step_at<EMB>(s).half;
                         const uint32_t bytes = (uint32_t)step_at<EMB>(s).n8 * 8u * 32u / SPLIT;
-                        const uint32_t off = (l < 8 ? (2 * l + h) * 4096u : 65536u + (2 * (l - 8) + h) * 2048u) + rank * bytes;
+                        const uint32_t off = bias_tile_offset(l, h) + rank * bytes;
                         wait_or_report<TRACE>(&bars->bempty[slot], ((bh >> 1) & 1) ^ 1, 102, s, (int)bh);
                         mbar_arrive_expect_tx(&bars->bfull[slot], bytes);
                         bulk_g2s(sm + OFF_BT + slot * 4096, tiles + off, bytes, &bars->bfull[slot]);
@@ -992,129 +906,17 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 #undef CHUNK_OF
 }
 
-// ---------------------------------------------------------------------------------------------
-// schedule (host)
-// ---------------------------------------------------------------------------------------------
-struct LayerDesc { int N, n_act_kb; bool has_pe; int w_index; int ldw, wcol_act; };
-
-// emb: the embedded-row schedule -- V0 gains a last K-block per half, the view columns 256..282 of views_linears.0 (kmax = 27) against
-// the gamma(v) image in the PE buffer; every other step, and the order of all steps, is the fused-entry schedule's.
-Schedule build_schedule(const InerfNetDims* d, bool emb = false) {
-    const int C = d->dim_aud + d->dim_expr + d->dim_latent, E = d->dim_expr;
-    LayerDesc L[11];
-    L[0] = {256, 0, true, 0, 63 + C, 0};
-    for (int l = 1; l < 8; ++l) L[l] = {256, 4, false, 2 * l, 256, 0};
-    L[5] = {256, 4, true, 10, 319 + C, 63 + C};
-    L[8] = {128, 4, emb, P_VIEWS_W, 283 + E, 0};
-    L[9] = {128, 2, false, P_VIEWS_W + 2, 128, 0};
-    L[10] = {128, 2, false, P_VIEWS_W + 4, 128, 0};
-    Schedule S{};
-    uint32_t off = 0;
-    int n = 0;
-    for (int l = 0; l < 11; ++l) {
-        const int NH = L[l].N / 2;
-        const int prevN = l == 0 ? 128 : L[l - 1].N;          // L0 follows V2 of the previous iteration
-        const int n_out_h0 = NH / 64;                         // K-blocks epi(h0) overwrites: kb < n_out_h0
-        for (int h = 0; h < 2; ++h) {
-            int order[5], cnt = 0;                            // K-block order of this half (4 = PE)
-            if (h == 0) {
-                for (int kb = 0; kb < L[l].n_act_kb; ++kb) order[cnt++] = kb;
-                if (L[l].has_pe) order[cnt++] = 4;
-            } else {
-                for (int kb = 0; kb < L[l].n_act_kb; ++kb) if (kb < n_out_h0) order[cnt++] = kb;
-                for (int kb = 0; kb < L[l].n_act_kb; ++kb) if (kb >= n_out_h0) order[cnt++] = kb;
-                if (L[l].has_pe) order[cnt++] = 4;
-            }
-            int n_first = 0;                                  // how many leading K-blocks of h1 are "overwritten by h0" ones
-            if (h == 1) for (int i = 0; i < cnt; ++i) if (order[i] < 4 && order[i] < n_out_h0) ++n_first;
-            for (int i = 0; i < cnt; ++i) {
-                Step& st = S.steps[n];
-                PackStep& pk = S.pack[n];
-                st.a_kb = (uint8_t)order[i];
-                st.n8 = (uint8_t)(NH / 8);
-                st.acc_col = (uint8_t)(h * NH);
-                st.first = (i == 0);
-                st.layer = (uint8_t)l;
-                st.wait = 0;
-                if (order[i] < 4) {
-                    // which half of the previous layer's epilogue produced this K-block
-                    const int kb_per_half = prevN / 128;      // 2 for N=256, 1 for N=128
-                    st.wait = (order[i] < kb_per_half) ? W_E0 : W_E1;
-                } else if (l == 0) {
-                    st.wait = W_PE | W_E0 | W_E1;             // new iteration: PE ready and both accumulator halves drained
-                } else if (l == 8 && h == 0) {
-                    st.wait = W_PE;                           // embedded rows: the gamma(v) image is in the PE buffer
-                }
-                st.commit = 0;
-                const bool last = (i == cnt - 1);
-                if (h == 0 && last) st.commit |= C_C0;
-                if (h == 1) {
-                    if (n_first > 0 ? (i == n_first - 1) : last) st.commit |= C_C1;
-                    if (last) st.commit |= C_C2;
-                    if (last && (l == 5 || l == 8)) st.commit |= C_PEFREE;
-                }
-                st.offset = off;
-                pk.w_index = L[l].w_index; pk.ldw = L[l].ldw; pk.n0 = h * NH; pk.rows = NH; pk.offset = off;
-                if (order[i] == 4) { pk.wcol = l == 8 ? 256 : 0; pk.kmax = l == 8 ? 27 : 63; }
-                else { pk.wcol = L[l].wcol_act + order[i] * 64; pk.kmax = 64; }
-                off += (uint32_t)NH * 128u;
-                ++n;
-            }
-        }
-    }
-    S.n_steps = n;
-    S.total_bytes = off;
-    return S;
-}
-
-struct PackArgs {
-    const float* w[INERF_N_PARAMS];
-    PackStep st[MAX_STEPS];
-    uint8_t* blob;
-};
-
-// The argument table travels as a kernel parameter (2.4 KB, by value): nothing is copied from pageable host memory, so the launch can be
-// captured in a CUDA graph (train.TrainStep re-packs the weights after every optimiser step).
-static_assert(sizeof(PackArgs) <= 4000, "kernel parameter space");
-__global__ void pack_kernel(const __grid_constant__ PackArgs pa) {
-    const PackStep st = pa.st[blockIdx.x];
-    const float* W = pa.w[st.w_index];
-    for (int i = threadIdx.x; i < st.rows * 64; i += blockDim.x) {
-        const int r = i >> 6, c = i & 63;
-        const float v = (c < st.kmax) ? W[(size_t)(st.n0 + r) * st.ldw + st.wcol + c] : 0.f;
-        *reinterpret_cast<__nv_bfloat16*>(pa.blob + st.offset + sw128_offset(r, c)) = __float2bfloat16_rn(v);
-    }
-}
-
 }  // namespace
 
 namespace inerf {
 
 int mlp_bf16_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded) {
-    Schedule S = build_schedule(d, embedded);
-    *bytes = (size_t)S.total_bytes;
+    *bytes = (size_t)build_tc_schedule(d, embedded, 1).total_bytes;
     return INERF_OK;
 }
 
 int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded) {
-    if ((uintptr_t)packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_pack: packed must be 16-byte aligned");
-    Schedule S = build_schedule(d, embedded);
-    PackArgs pa{};
-    for (int i = 0; i < INERF_N_PARAMS; ++i) pa.w[i] = params_host[i];
-    for (int i = 0; i < S.n_steps; ++i) pa.st[i] = S.pack[i];
-    pa.blob = reinterpret_cast<uint8_t*>(packed);
-    pack_kernel<<<S.n_steps, 256, 0, st>>>(pa);
-    return check_launch("inerf_mlp_pack");
-}
-
-void mlp_bf16_stage_offsets(uint32_t (*off)[2][5]) {
-    InerfNetDims d{64, 76, 32, 256, 8, 63, 27};              // offsets do not depend on the conditioning dims
-    Schedule S = build_schedule(&d);
-    int idx[11][2] = {};
-    for (int n = 0; n < S.n_steps; ++n) {
-        const int l = S.steps[n].layer, h = S.steps[n].acc_col ? 1 : 0;
-        off[l][h][idx[l][h]++] = S.steps[n].offset;
-    }
+    return pack_tc_schedule<false>(build_tc_schedule(d, embedded, 1), params_host, packed, st, "inerf_mlp_pack");
 }
 
 #ifdef INERF_PHASE_TIMERS
@@ -1133,36 +935,11 @@ int mlp_bf16_hang_info(int32_t* out8) {
     return INERF_OK;
 }
 
-template <bool SAVE, bool EMB = false>
-static int launch_pair(const MlpArgs& a, int n_steps, int n_rays, int dev, cudaStream_t st) {
-    static thread_local int pair_dev = -1;
-    if (pair_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, SAVE, true, EMB>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-        if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        pair_dev = dev;
-    }
-    const long long n_pair_iter = (a.P + 511) / 512;
-    const long long max_pairs = num_sms() / 2;
-    const long long pairs = n_pair_iter < max_pairs ? n_pair_iter : max_pairs;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(2 * pairs));
-    cfg.blockDim = dim3(NTHREADS_BF16);
-    cfg.dynamicSmemBytes = SMEM_ALLOC;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, mlp_bf16_kernel<false, 0, SAVE, true, EMB>, a, n_steps, n_rays, (float*)nullptr);
-    if (e != cudaSuccess) { set_error("inerf_mlp_fwd[bf16 pair]: %s", cudaGetErrorString(e)); return (int)e; }
-    return check_launch(SAVE ? "inerf_mlp_fwd_train[bf16 pair]" : "inerf_mlp_fwd[bf16 pair]");
-}
-
-// the CTA-pair build (clusters of two) runs the inference and the activation-saving forward; INERF_MLP_PAIR=0 (read once) keeps the
-// single-CTA kernels for A/B runs, which also serve the trace / ablation builds
-static bool pair_enabled() {
-    static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
-    return pair_env && num_sms() >= 2;
+// the production builds: no trace, no ablation
+template <bool SAVE, bool PAIR, bool EMB>
+static int launch(const MlpArgs& a, int n_steps, int n_rays, cudaStream_t st, const char* what) {
+    return launch_tc(mlp_bf16_kernel<false, 0, SAVE, PAIR, EMB>, PAIR, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, what, a, n_steps, n_rays,
+                     (float*)nullptr);
 }
 
 // FaceNeRF.forward on embedded rows x (P, 90): a.packed is an INERF_MLP_BF16_EMB blob, a.save_img != NULL selects the saving build
@@ -1170,26 +947,17 @@ static int launch_embedded(const MlpArgs& a, cudaStream_t st) {
     if (((uintptr_t)a.packed | (uintptr_t)a.x) & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd_embedded: packed weights and x must be 16-byte aligned");
     if (a.save_img && !a.save_mask) return fail(INERF_E_ARG, "mlp_bf16: save_mask is NULL");
     static thread_local int configured_dev = -1;
-    static const Schedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_schedule(&d, true); }();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (configured_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_steps_emb, S.steps, sizeof(Step) * MAX_STEPS);
-        if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        configured_dev = dev;
-    }
-    if (pair_enabled())
-        return a.save_img ? launch_pair<true, true>(a, S.n_steps, 0, dev, st) : launch_pair<false, true>(a, S.n_steps, 0, dev, st);
-    const long long n_iter = (a.P + 255) / 256;
-    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
-    if (a.save_img) {
-        mlp_bf16_kernel<false, 0, true, false, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, 0, nullptr);
-        return check_launch("inerf_mlp_fwd_train_bf16_embedded");
-    }
-    mlp_bf16_kernel<false, 0, false, false, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, 0, nullptr);
-    return check_launch("inerf_mlp_fwd_embedded[bf16]");
+    static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, true, 1); }();
+    int rc = setup_once(configured_dev,
+                        {(const void*)mlp_bf16_kernel<false, 0, false, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, false, true>,
+                         (const void*)mlp_bf16_kernel<false, 0, false, true, true>, (const void*)mlp_bf16_kernel<false, 0, true, true, true>},
+                        SMEM_ALLOC, "mlp_bf16", [] { return cudaMemcpyToSymbol(c_steps_emb, S.st, sizeof(TcStage) * MAX_STEPS); });
+    if (rc) return rc;
+    if (mlp_pair_enabled())
+        return a.save_img ? launch<true, true, true>(a, S.n_stages, 0, st, "inerf_mlp_fwd_train[bf16 pair]")
+                          : launch<false, true, true>(a, S.n_stages, 0, st, "inerf_mlp_fwd[bf16 pair]");
+    return a.save_img ? launch<true, false, true>(a, S.n_stages, 0, st, "inerf_mlp_fwd_train_bf16_embedded")
+                      : launch<false, false, true>(a, S.n_stages, 0, st, "inerf_mlp_fwd_embedded[bf16]");
 }
 
 int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
@@ -1198,20 +966,14 @@ int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
     if ((uintptr_t)a.packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: packed weights must be 16-byte aligned");
     static thread_local int configured_dev = -1;
     // the step table does not depend on the conditioning dims; a function-local static is initialised once, thread-safely
-    static const Schedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_schedule(&d); }();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (configured_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_bf16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_steps, S.steps, sizeof(Step) * MAX_STEPS);
-        if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        configured_dev = dev;
-    }
-    const long long n_iter = (a.P + 255) / 256;
-    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
+    static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, false, 1); }();
+    int rc = setup_once(configured_dev,
+                        {(const void*)mlp_bf16_kernel<false>, (const void*)mlp_bf16_kernel<true>, (const void*)mlp_bf16_kernel<false, 0, true>,
+                         (const void*)mlp_bf16_kernel<false, 0, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, true>},
+                        SMEM_ALLOC, "mlp_bf16", [] { return cudaMemcpyToSymbol(c_steps, S.st, sizeof(TcStage) * MAX_STEPS); });
+    if (rc) return rc;
     const int n_rays = (int)(a.P / a.s);
-    const bool use_pair = pair_enabled() && !a.trace;
+    const bool use_pair = mlp_pair_enabled() && !a.trace;
     if (a.trace) {
         if (!g_hang_host) {
             int* dptr = nullptr;
@@ -1222,10 +984,12 @@ int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
         if (g_hang_host) for (int i = 0; i < 8; ++i) g_hang_host[i] = 0;
     }
 #ifdef INERF_ABLATION
+    const long long n_iter = (a.P + 255) / 256;
+    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
     if (const char* e = a.save_img ? nullptr : getenv("INERF_ABL")) {
         const int abl = atoi(e);
 #define ABL_CASE(N_) case N_: cudaFuncSetAttribute(mlp_bf16_kernel<false, N_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC); \
-                              mlp_bf16_kernel<false, N_><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, nullptr); break;
+                              mlp_bf16_kernel<false, N_><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); break;
         switch (abl) { ABL_CASE(1) ABL_CASE(2) ABL_CASE(3) ABL_CASE(4) ABL_CASE(5) ABL_CASE(6) ABL_CASE(7) ABL_CASE(8) ABL_CASE(16) ABL_CASE(24) default: break; }
 #undef ABL_CASE
         if (abl >= 1 && abl <= 24) return check_launch("inerf_mlp_fwd[bf16,ablation]");
@@ -1233,36 +997,27 @@ int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
 #endif
     if (a.save_img) {
         if (!a.save_mask) return fail(INERF_E_ARG, "mlp_bf16: save_mask is NULL");
-        static thread_local int save_dev = -1;
-        if (save_dev != dev) {
-            cudaError_t e = cudaFuncSetAttribute(mlp_bf16_kernel<false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-            if (e != cudaSuccess) { set_error("mlp_bf16: setup: %s", cudaGetErrorString(e)); return (int)e; }
-            save_dev = dev;
-        }
 #ifdef INERF_ABLATION
         { const char* e = getenv("INERF_SAVE_ABL"); const int v = e ? atoi(e) : 0; cudaMemcpyToSymbolAsync(g_save_abl, &v, sizeof(v), 0, cudaMemcpyHostToDevice, st); cudaStreamSynchronize(st); }
         if (const char* e = getenv("INERF_ABL")) {      // weight streaming (2) / sincosf (4) off on top of the saving switches
             const int abl = atoi(e);
             if (abl == 2 || abl == 4) {
                 if (abl == 2) { cudaFuncSetAttribute(mlp_bf16_kernel<false, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-                                mlp_bf16_kernel<false, 2, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, nullptr); }
+                                mlp_bf16_kernel<false, 2, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); }
                 else { cudaFuncSetAttribute(mlp_bf16_kernel<false, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-                       mlp_bf16_kernel<false, 4, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, nullptr); }
+                       mlp_bf16_kernel<false, 4, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); }
                 return check_launch("inerf_mlp_fwd_train[bf16,ablation]");
             }
         }
 #endif
-        if (use_pair) return launch_pair<true>(a, S.n_steps, n_rays, dev, st);
-        mlp_bf16_kernel<false, 0, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, nullptr);
-        return check_launch("inerf_mlp_fwd_train[bf16]");
+        return use_pair ? launch<true, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16 pair]")
+                        : launch<true, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16]");
     }
-    if (a.trace) {
-        mlp_bf16_kernel<true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, a.trace);
-        return check_launch("inerf_mlp_fwd[bf16]");
-    }
-    if (use_pair) return launch_pair<false>(a, S.n_steps, n_rays, dev, st);
-    mlp_bf16_kernel<false><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_steps, n_rays, nullptr);
-    return check_launch("inerf_mlp_fwd[bf16]");
+    if (a.trace)
+        return launch_tc(mlp_bf16_kernel<true>, false, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, "inerf_mlp_fwd[bf16]", a, S.n_stages, n_rays,
+                         a.trace);
+    return use_pair ? launch<false, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16 pair]")
+                    : launch<false, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16]");
 }
 
 }  // namespace inerf

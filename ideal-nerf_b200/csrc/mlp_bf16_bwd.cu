@@ -16,8 +16,7 @@
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
-#include "mlp_common.cuh"
-#include "sm100_ptx.cuh"
+#include "mlp_tc.cuh"
 
 using namespace inerf;
 using namespace sm100;
@@ -28,7 +27,7 @@ constexpr int NSTAGE = 4;
 constexpr int STAGE_BYTES = 16384;
 // CTA-pair build (PAIR = true, see mlp_bf16.cu): each CTA of a cluster of two holds HALF of the rows of every weight stage; the same 64 KB
 // ring is eight stages deep
-template <bool PAIR> struct RingOf { static constexpr int N = PAIR ? 8 : 4, BYTES = PAIR ? 8192 : 16384; };
+template <bool PAIR> using RingOf = Ring<PAIR, NSTAGE>;
 constexpr int NTH = 512;
 constexpr int N_EPI = 256, N_INIT = 128;
 constexpr int NLAY = 10;
@@ -79,49 +78,12 @@ __device__ __forceinline__ void bwait(uint64_t* bar, uint32_t parity) {
         if (clock64() - t0 > 8000000000LL) __trap();          // ~4 s: a lost arrival must not hang the GPU
 }
 
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-
-__device__ __forceinline__ void umma_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(acc)
-        : "memory");
-}
-__device__ __forceinline__ void umma_lohi_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t acc) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(acc)
-        : "memory");
-}
+// issuer-side wait on an event whose arrivals may come from the peer CTA; the single-CTA build waits with the bounded bwait
 template <bool PAIR>
-__device__ __forceinline__ void umma_any(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t acc) {
-    if constexpr (PAIR) umma_lohi_pair(tmem_d, a_lo, b_lo, hi, idesc, acc);
-    else umma_lohi(tmem_d, a_lo, b_lo, hi, idesc, acc);
-}
-template <bool PAIR>
-__device__ __forceinline__ void commit_any(uint64_t* bar) {
-    if constexpr (PAIR) umma_commit_pair(bar);
-    else umma_commit(bar);
-}
-// issuer-side wait on an event whose arrivals may come from the peer CTA
-template <bool PAIR>
-__device__ __forceinline__ void wait_ev(uint64_t* bar, uint32_t parity) {
+__device__ __forceinline__ void wait_ev_bounded(uint64_t* bar, uint32_t parity) {
     if constexpr (PAIR) mbar_wait_cluster(bar, parity);
     else bwait(bar, parity);
 }
-
-constexpr uint32_t HI_NOSWZ = (256u >> 4) | (1u << 14);
-__device__ __forceinline__ uint32_t desc_lo_noswz(uint32_t smem_addr) { return ((smem_addr & 0x3FFFF) >> 4) | ((128u >> 4) << 16); }
 
 struct IssueCtx {
     Bars* bars;
@@ -146,13 +108,13 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
             if (h == 0 && c.layer_ctr > 0) {
                 if (J == 0 || bl_N(J) > bl_prev_N(J)) {        // new iteration, or a layer WIDER than the previous one: its first half
                     // overwrites accumulator columns that both halves of the previous epilogue read
-                    if (i == 0) { wait_ev<PAIR>(&bars->ebar[0], par_prev); wait_ev<PAIR>(&bars->ebar[1], par_prev); }
+                    if (i == 0) { wait_ev_bounded<PAIR>(&bars->ebar[0], par_prev); wait_ev_bounded<PAIR>(&bars->ebar[1], par_prev); }
                 } else {
-                    if (i == 0) wait_ev<PAIR>(&bars->ebar[0], par_prev);
-                    if (i == KB_PER_HALF_PREV) wait_ev<PAIR>(&bars->ebar[1], par_prev);
+                    if (i == 0) wait_ev_bounded<PAIR>(&bars->ebar[0], par_prev);
+                    if (i == KB_PER_HALF_PREV) wait_ev_bounded<PAIR>(&bars->ebar[1], par_prev);
                 }
             }
-            if (J == 0 && h == 0 && i == 0) wait_ev<PAIR>(&bars->init_ready, c.iter_ctr & 1);
+            if (J == 0 && h == 0 && i == 0) wait_ev_bounded<PAIR>(&bars->init_ready, c.iter_ctr & 1);
             bwait(&bars->wfull[c.stage], c.wpar);
             if constexpr (PAIR) mbar_wait_cluster(&bars->pfull[c.stage], c.wpar);
             tc_fence_after();
@@ -551,41 +513,15 @@ int mlp_bf16_bwd_chain_launch(const InerfNetDims* dims, const float* const* para
     static thread_local int configured_dev = -1;
     // step sizes / offsets do not depend on the conditioning dims; a function-local static is initialised once, thread-safely
     static const BSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_bschedule(&d); }();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (configured_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_bwd_chain_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_bf16_bwd_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BWD);
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_bsteps, S.steps, sizeof(BStep) * MAX_BSTEPS);
-        if (e != cudaSuccess) { set_error("mlp_bf16_bwd: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        configured_dev = dev;
-    }
+    int rc = setup_once(configured_dev, {(const void*)mlp_bf16_bwd_chain_kernel<false>, (const void*)mlp_bf16_bwd_chain_kernel<true>}, SMEM_BWD,
+                        "mlp_bf16_bwd", [] { return cudaMemcpyToSymbol(c_bsteps, S.steps, sizeof(BStep) * MAX_BSTEPS); });
+    if (rc) return rc;
     BwdChainArgs a{};
     a.packed_t = packed_t; a.rgb_w = params_host[P_RGB_W]; a.mask = mask; a.d_raw = d_raw; a.delta_img = delta_img; a.P = P;
     a.n_stage_bytes_total = S.stage_bytes;
     const long long n_iter = (P + 255) / 256;
-    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
-    // the CTA-pair build by default; INERF_MLP_PAIR=0 (read once) keeps the single-CTA kernel for A/B runs
-    static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
-    if (pair_env && num_sms() >= 2) {
-        const long long n_pair_iter = (P + 511) / 512;
-        const long long max_pairs = num_sms() / 2;
-        const long long pairs = n_pair_iter < max_pairs ? n_pair_iter : max_pairs;
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(2 * pairs));
-        cfg.blockDim = dim3(NTH);
-        cfg.dynamicSmemBytes = SMEM_BWD;
-        cfg.stream = st;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        cudaError_t e = cudaLaunchKernelEx(&cfg, mlp_bf16_bwd_chain_kernel<true>, a, S.n_steps);
-        if (e != cudaSuccess) { set_error("inerf_mlp_bwd[bf16 chain pair]: %s", cudaGetErrorString(e)); return (int)e; }
-        return check_launch("inerf_mlp_bwd[bf16 chain pair]");
-    }
-    mlp_bf16_bwd_chain_kernel<false><<<grid, NTH, SMEM_BWD, st>>>(a, S.n_steps);
-    return check_launch("inerf_mlp_bwd[bf16 chain]");
+    return mlp_pair_enabled() ? launch_tc(mlp_bf16_bwd_chain_kernel<true>, true, n_iter, NTH, SMEM_BWD, st, "inerf_mlp_bwd[bf16 chain pair]", a, S.n_steps)
+                              : launch_tc(mlp_bf16_bwd_chain_kernel<false>, false, n_iter, NTH, SMEM_BWD, st, "inerf_mlp_bwd[bf16 chain]", a, S.n_steps);
 }
 
 }  // namespace inerf

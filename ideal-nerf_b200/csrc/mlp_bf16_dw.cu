@@ -47,7 +47,6 @@ struct DwArgs {
 
 __device__ __forceinline__ uint32_t desc_lo_mn(uint32_t smem_addr) { return ((smem_addr & 0x3FFFF) >> 4) | ((16384u >> 4) << 16); }
 constexpr uint32_t HI_MN_SW128 = (1024u >> 4) | (1u << 14) | ((uint32_t)SWIZZLE_128B << 29);
-constexpr uint32_t HI_NOSWZ = (256u >> 4) | (1u << 14);
 
 __device__ __forceinline__ void umma_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t acc) {
     asm volatile(
@@ -57,12 +56,6 @@ __device__ __forceinline__ void umma_lohi(uint32_t tmem_d, uint32_t a_lo, uint32
         "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}" ::"r"(tmem_d),
         "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc)
         : "memory");
-}
-
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
 }
 
 __device__ __forceinline__ void bounded_wait(uint64_t* bar, uint32_t parity) {
@@ -218,13 +211,8 @@ size_t mlp_bf16_dw_scratch_bytes() { return 16; }      // the work-item counter
 int mlp_bf16_dw_launch(const InerfNetDims* dims, float* const* grads_host, const uint8_t* delta_img, const uint8_t* acts_img,
                        long long n_tiles, void* scratch, cudaStream_t st) {
     static thread_local int configured_dev = -1;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (configured_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_bf16_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DW_SMEM);
-        if (e != cudaSuccess) { set_error("mlp_bf16_dw: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        configured_dev = dev;
-    }
+    int rc = setup_once(configured_dev, {(const void*)mlp_bf16_dw_kernel}, DW_SMEM, "mlp_bf16_dw");
+    if (rc) return rc;
     const int C = dims->dim_aud + dims->dim_expr + dims->dim_latent, E = dims->dim_expr;
     DwArgs d{};
     d.delta_img = delta_img; d.acts_img = acts_img; d.n_tiles = n_tiles;

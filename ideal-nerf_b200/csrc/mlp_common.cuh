@@ -1,5 +1,10 @@
 // Shared declarations of the FaceNeRF MLP kernels.
 #pragma once
+#include <stdlib.h>
+
+#include <initializer_list>
+#include <utility>
+
 #include "common.cuh"
 
 namespace inerf {
@@ -39,6 +44,51 @@ constexpr int TRAIN_IMGS = 40, TRAIN_IMG_PE = 38, TRAIN_IMG_DIR = 39, TRAIN_IMG_
 __host__ __device__ constexpr int train_img_of(int l) { return l < 8 ? 4 * l : 32 + 2 * (l - 8); }
 __host__ __device__ constexpr int train_mask_of(int l) { return l < 8 ? 8 * l : 64 + 4 * (l - 8); }
 
+// ---- launch plumbing of the tensor-core kernels ----------------------------------------------------------------------------------
+// The CTA-pair builds (clusters of two, tcgen05 cta_group::2) run by default; INERF_MLP_PAIR=0, read once per process, keeps the
+// single-CTA builds: the bit-exact reference of the pair builds, and what the trace / ablation builds run.
+inline bool mlp_pair_enabled() {
+    static const bool env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
+    return env && num_sms() >= 2;
+}
+
+// Once per device and host thread for each launch site (`configured_dev`: the site's thread_local, -1 at first): the dynamic
+// shared-memory limit of every kernel in `kernels`, then `more` (when given; e.g. a stage table to constant memory).  Errors read
+// "<what>: setup: ...".
+inline int setup_once(int& configured_dev, std::initializer_list<const void*> kernels, int smem_bytes, const char* what,
+                      cudaError_t (*more)() = nullptr) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (configured_dev == dev) return INERF_OK;
+    cudaError_t e = cudaSuccess;
+    for (const void* k : kernels)
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    if (e == cudaSuccess && more) e = more();
+    if (e != cudaSuccess) { set_error("%s: setup: %s", what, cudaGetErrorString(e)); return (int)e; }
+    configured_dev = dev;
+    return INERF_OK;
+}
+
+// Launches `kernel` for `n_iter` single-CTA iterations: as one CTA per iteration up to one per SM, or with `pair` as clusters of two
+// CTAs, one per two iterations, up to one per two SMs.  `what` names the launch in error messages.
+template <typename... KArgs, typename... Args>
+int launch_tc(void (*kernel)(KArgs...), bool pair, long long n_iter, int nthreads, int smem_bytes, cudaStream_t st, const char* what,
+              Args&&... args) {
+    const long long n = pair ? (n_iter + 1) / 2 : n_iter, cap = pair ? num_sms() / 2 : num_sms();
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((unsigned)((pair ? 2 : 1) * (n < cap ? n : cap)));
+    cfg.blockDim = dim3(nthreads);
+    cfg.dynamicSmemBytes = smem_bytes;
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = pair ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+    if (e != cudaSuccess) { set_error("%s: %s", what, cudaGetErrorString(e)); return (int)e; }
+    return check_launch(what);
+}
+
 int mlp_fp32_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
 // embedded: rows of a.x (P, 90) with an INERF_MLP_BF16_EMB blob; otherwise points of rays/z.  a.save_img != NULL: the activation-saving build
 int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
@@ -52,7 +102,6 @@ int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded =
 int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded = false);
 int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
 int mlp_bf16_hang_info(int32_t* out8);
-void mlp_bf16_stage_offsets(uint32_t (*off)[2][5]);      // [11 layers][half][K-block index in issue order] -> byte offset in the packed blob
 // bf16 training path (mlp_bf16_bwd.cu, mlp_bf16_dw.cu, mlp_fp32_bwd.cu)
 int mlp_bf16_bwd_packed_bytes(const InerfNetDims* d, size_t* bytes);
 int mlp_bf16_bwd_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st);

@@ -40,8 +40,7 @@
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
-#include "mlp_common.cuh"
-#include "sm100_ptx.cuh"
+#include "mlp_tc.cuh"
 
 using namespace inerf;
 using namespace sm100;
@@ -52,34 +51,15 @@ constexpr int NSTAGE = 3;
 constexpr int STAGE_BYTES = 16384;
 // CTA-pair build (PAIR = true, see mlp_bf16.cu): each CTA of a cluster of two holds HALF of the rows of every weight stage; the same 48 KB
 // ring is six stages deep
-template <bool PAIR> struct RingOf { static constexpr int N = PAIR ? 6 : 3, BYTES = PAIR ? 8192 : 16384; };
+template <bool PAIR> using RingOf = Ring<PAIR, NSTAGE>;
 constexpr int MAX_FSTAGES = 160;     // 76 K-block steps x (hi, lo); the embedded-row schedule has 78
 constexpr int RMAX = 4;              // rays a 128-row slot can touch (s >= 43)
 constexpr int NTHREADS = 512;
 constexpr int N_EPI = 256, N_PE = 128;
 
-struct FStage {
-    uint32_t offset;   // byte offset of the stage image in the packed blob
-    uint8_t n8;        // rows / 8 of the image (N of the MMA / 8)
-    uint8_t bias;      // 1: first stage of a (layer, half): its bias tile is streamed with it
-    uint8_t layer, half;
-};
-
-struct FPack {
-    int w_index, ldw, n0, rows, wcol, kmax, lo;   // weight rows [n0, n0+rows), columns wcol .. wcol+63 (kmax valid); lo: the low half
-    uint32_t offset;
-};
-
-struct FSchedule {
-    int n_stages;
-    FStage st[MAX_FSTAGES];
-    FPack pack[MAX_FSTAGES];
-    uint32_t total_bytes;
-};
-
-__constant__ FStage c_fstages[MAX_FSTAGES];
-__constant__ FStage c_fstages_emb[MAX_FSTAGES];     // the embedded-row schedule (one more K-block per V0 half)
-template <bool EMB> __device__ __forceinline__ const FStage& fstage_at(int s) { return EMB ? c_fstages_emb[s] : c_fstages[s]; }
+__constant__ TcStage c_fstages[MAX_FSTAGES];
+__constant__ TcStage c_fstages_emb[MAX_FSTAGES];     // the embedded-row schedule (one more K-block per V0 half)
+template <bool EMB> __device__ __forceinline__ const TcStage& fstage_at(int s) { return EMB ? c_fstages_emb[s] : c_fstages[s]; }
 
 // smem map (bytes from the 1024-aligned base) -- mlp_bf16.cu's, with [hi|lo] where it has [slot 0|slot 1]
 constexpr int OFF_ACT = 0;                               // [2: hi, lo][4 K-blocks][16384]
@@ -95,7 +75,6 @@ constexpr int OFF_PART = OFF_DIRB + RMAX * 128 * 4;      // [128 rows] float4: h
 constexpr int OFF_BAR = OFF_PART + 128 * 16;             // mbarriers
 constexpr int SMEM_BYTES = OFF_BAR + 320;
 static_assert(SMEM_BYTES <= 232448, "shared memory budget");
-constexpr int BF16_TILE_BYTES = 16 * 4096 + 6 * 2048;    // the bf16 kernel's bias tiles come first in `cond`; ours follow
 
 struct Bars {
     uint64_t wfull[6], wempty[6];
@@ -123,66 +102,8 @@ __device__ __forceinline__ void wait_b(uint64_t* bar, uint32_t parity) {
     }
 }
 
-__host__ __device__ constexpr int lay_N(int l) { return l < 8 ? 256 : 128; }
-__host__ __device__ constexpr int lay_act_kb(int l) { return l == 0 ? 0 : (l <= 8 ? 4 : 2); }
-__host__ __device__ constexpr bool lay_pe(int l) { return l == 0 || l == 5; }
-__host__ __device__ constexpr bool lay_x(int l, bool emb) { return lay_pe(l) || (emb && l == 8); }   // + a PE-buffer K-block (gamma(p) or gamma(v))
-__host__ __device__ constexpr int lay_prev_N(int l) { return l == 0 ? 128 : lay_N(l - 1); }
-
 // kind::f16 instruction descriptor with fp16 A / B (format 0), fp32 D
 __host__ __device__ constexpr uint32_t idesc_f16(int M, int N) { return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24); }
-
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-
-__device__ __forceinline__ void umma_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_lohi_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
-        "setp.ne.b32 p, %5, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
-        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-template <bool PAIR>
-__device__ __forceinline__ void umma_any(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
-    if constexpr (PAIR) umma_lohi_pair(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
-    else umma_lohi(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
-}
-template <bool PAIR>
-__device__ __forceinline__ void commit_any(uint64_t* bar) {
-    if constexpr (PAIR) umma_commit_pair(bar);
-    else umma_commit(bar);
-}
-// issuer-side wait on an event whose arrivals may come from the peer CTA
-template <bool PAIR>
-__device__ __forceinline__ void wait_ev(uint64_t* bar, uint32_t parity) {
-    if constexpr (PAIR) mbar_wait_cluster(bar, parity);
-    else mbar_wait(bar, parity);
-}
-
-// 32 lanes x 16 consecutive 32-bit columns
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr)
-        : "memory");
-}
 
 constexpr uint32_t CORR_COL = 256;      // first TMEM column of the correction accumulator
 // Compensation of the tensor core's accumulation rounding.  tcgen05.mma adds into its fp32 accumulator with round-toward-zero: each of
@@ -196,8 +117,6 @@ constexpr uint32_t CORR_COL = 256;      // first TMEM column of the correction a
 // brings raw to 2.0e-6 max / 5e-7 rms of scale, against 1.5e-6 / 3.3e-7 for the FFMA kernel and 3.5e-6 / 1.0e-6 uncompensated.
 // INERF_F16X2_COMP (uniform comp) / INERF_F16X2_ULPS ("l0,trunk,v0,v12") re-run the calibration (tests/native/f16x2_comp_sweep.py).
 __host__ __device__ constexpr float tc_comp_ulps(int l) { return l == 0 ? 1.0f : (l < 8 ? 4.0f : 2.0f); }
-constexpr uint32_t HI_NOSWZ = (256u >> 4) | (1u << 14);
-__device__ __forceinline__ uint32_t desc_lo_noswz(uint32_t smem_addr) { return ((smem_addr & 0x3FFFF) >> 4) | ((128u >> 4) << 16); }
 
 // (hi, lo) fp16x2 words of two fp32 values, ReLU applied: hi = the value truncated to 11 significant bits, lo = the exact remainder
 __device__ __forceinline__ void split_relu2(float v0, float v1, uint32_t& hi2, uint32_t& lo2) {
@@ -393,17 +312,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
         // ================= weight producer ==================================================
         if (lane == 0) {
             const uint8_t* blob = reinterpret_cast<const uint8_t*>(a.packed);
-            const uint8_t* tiles = reinterpret_cast<const uint8_t*>(a.cond + 2436) + BF16_TILE_BYTES;
+            const uint8_t* tiles = reinterpret_cast<const uint8_t*>(a.cond + COND_FLOATS) + BIAS_TILE_BYTES;      // after the bf16 tile set
             uint32_t g = 0, bh = 0;
             constexpr uint32_t SPLIT = PAIR ? 2u : 1u;      // pair build: this CTA's half of the rows of every stage / bias tile
             for (long long it = it_first; it < n_iter; it += it_step) {
                 for (int s = 0; s < n_stages; ++s, ++g) {
                     const uint32_t stage = g % NSTAGE, round = g / NSTAGE;
-                    const FStage fs = fstage_at<EMB>(s);
-                    if (fs.bias) {
+                    const TcStage fs = fstage_at<EMB>(s);
+                    if (fs.first) {
                         const uint32_t slot = bh & 1, l = fs.layer, h = fs.half;
                         const uint32_t bytes = (uint32_t)fs.n8 * 8u * 32u / SPLIT;
-                        const uint32_t off = (l < 8 ? (2 * l + h) * 4096u : 65536u + (2 * (l - 8) + h) * 2048u) + rank * bytes;
+                        const uint32_t off = bias_tile_offset(l, h) + rank * bytes;
                         wait_b(&bars->bempty[slot], ((bh >> 1) & 1) ^ 1);
                         mbar_arrive_expect_tx(&bars->bfull[slot], bytes);
                         bulk_g2s(sm + OFF_BT + slot * 4096, tiles + off, bytes, &bars->bfull[slot]);
@@ -423,7 +342,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
             uint32_t g = 0, bh = 0;
             for (long long it = it_first; it < n_iter; it += it_step)
                 for (int s = 0; s < n_stages; ++s, ++g) {
-                    if (fstage_at<EMB>(s).bias) {
+                    if (fstage_at<EMB>(s).first) {
                         mbar_wait(&bars->bfull[bh & 1], (bh >> 1) & 1);
                         mbar_arrive_remote(&bars->pbfull[bh & 1], 0);
                         ++bh;
@@ -711,94 +630,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
 #undef SLOT_OF
 }
 
-// ---------------------------------------------------------------------------------------------
-// schedule + packing (host)
-// ---------------------------------------------------------------------------------------------
-struct LayerDesc { int N, n_act_kb; bool has_pe; int w_index; int ldw, wcol_act; };
-
-// emb: the embedded-row schedule -- V0 gains a last K-block per half, (hi, lo) stages of the view columns 256..282 of views_linears.0
-// (kmax = 27) against the gamma(v) image in the PE buffer; every other stage, and the order of all stages, is the fused-entry schedule's.
-FSchedule build_fschedule(const InerfNetDims* d, bool emb = false) {
-    const int C = d->dim_aud + d->dim_expr + d->dim_latent, E = d->dim_expr;
-    LayerDesc L[11];
-    L[0] = {256, 0, true, 0, 63 + C, 0};
-    for (int l = 1; l < 8; ++l) L[l] = {256, 4, false, 2 * l, 256, 0};
-    L[5] = {256, 4, true, 10, 319 + C, 63 + C};
-    L[8] = {128, 4, emb, P_VIEWS_W, 283 + E, 0};
-    L[9] = {128, 2, false, P_VIEWS_W + 2, 128, 0};
-    L[10] = {128, 2, false, P_VIEWS_W + 4, 128, 0};
-    FSchedule S{};
-    uint32_t off = 0;
-    int n = 0;
-    for (int l = 0; l < 11; ++l) {
-        const int NH = L[l].N / 2;
-        for (int h = 0; h < 2; ++h) {
-            const int cnt = L[l].n_act_kb + (L[l].has_pe ? 1 : 0);
-            for (int i = 0; i < cnt; ++i) {
-                const bool pe = (i == L[l].n_act_kb);             // K-blocks in natural order, the gamma(p) block last
-                for (int part = 0; part < 2; ++part) {
-                    FStage& st = S.st[n];
-                    FPack& pk = S.pack[n];
-                    st.offset = off; st.n8 = (uint8_t)(NH / 8); st.bias = (uint8_t)(i == 0 && part == 0); st.layer = (uint8_t)l; st.half = (uint8_t)h;
-                    pk.w_index = L[l].w_index; pk.ldw = L[l].ldw; pk.n0 = h * NH; pk.rows = NH; pk.offset = off; pk.lo = part;
-                    if (pe) { pk.wcol = l == 8 ? 256 : 0; pk.kmax = l == 8 ? 27 : 63; }
-                    else { pk.wcol = L[l].wcol_act + i * 64; pk.kmax = 64; }
-                    off += (uint32_t)NH * 128u;
-                    ++n;
-                }
-            }
-        }
-    }
-    S.n_stages = n;
-    S.total_bytes = off;
-    return S;
-}
-
-// 152 (156) stages x 32 B would not fit the 4 KB parameter space next to the 26 weight pointers: the pack table is split over two launches
-constexpr int PACK_PER_LAUNCH = 80;
-struct FPackArgs {
-    const float* w[INERF_N_PARAMS];
-    FPack st[PACK_PER_LAUNCH];
-    uint8_t* blob;
-};
-static_assert(sizeof(FPackArgs) <= 4000, "kernel parameter space");
-
-__global__ void f16x2_pack_kernel(const __grid_constant__ FPackArgs pa) {
-    const FPack st = pa.st[blockIdx.x];
-    const float* W = pa.w[st.w_index];
-    for (int i = threadIdx.x; i < st.rows * 64; i += blockDim.x) {
-        const int r = i >> 6, c = i & 63;
-        const float v = (c < st.kmax) ? W[(size_t)(st.n0 + r) * st.ldw + st.wcol + c] : 0.f;
-        const __half hi = __float2half_rn(v);
-        const __half out = st.lo ? __float2half_rn(v - __half2float(hi)) : hi;
-        *reinterpret_cast<__half*>(pa.blob + st.offset + sw128_offset(r, c)) = out;
-    }
-}
-
 }  // namespace
 
 namespace inerf {
 
 int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded) {
-    FSchedule S = build_fschedule(d, embedded);
-    *bytes = (size_t)S.total_bytes;
+    *bytes = (size_t)build_tc_schedule(d, embedded, 2).total_bytes;
     return INERF_OK;
 }
 
 int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded) {
-    if ((uintptr_t)packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_pack: packed must be 16-byte aligned");
-    FSchedule S = build_fschedule(d, embedded);
-    for (int first = 0; first < S.n_stages; first += PACK_PER_LAUNCH) {
-        FPackArgs pa{};
-        for (int i = 0; i < INERF_N_PARAMS; ++i) pa.w[i] = params_host[i];
-        const int cnt = S.n_stages - first < PACK_PER_LAUNCH ? S.n_stages - first : PACK_PER_LAUNCH;
-        for (int i = 0; i < cnt; ++i) pa.st[i] = S.pack[first + i];
-        pa.blob = reinterpret_cast<uint8_t*>(packed);
-        f16x2_pack_kernel<<<cnt, 256, 0, st>>>(pa);
-        int rc = check_launch("inerf_mlp_pack[fp16x2]");
-        if (rc) return rc;
-    }
-    return INERF_OK;
+    return pack_tc_schedule<true>(build_tc_schedule(d, embedded, 2), params_host, packed, st, "inerf_mlp_pack[fp16x2]");
 }
 
 int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
@@ -810,22 +652,16 @@ int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
     }
     static thread_local int configured_dev = -1;
     // offsets do not depend on the conditioning dims
-    static const FSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_fschedule(&d); }();
-    static const FSchedule SE = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_fschedule(&d, true); }();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (configured_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(mlp_f16x2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_f16x2_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_fstages, S.st, sizeof(FStage) * MAX_FSTAGES);
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_fstages_emb, SE.st, sizeof(FStage) * MAX_FSTAGES);
-        if (e != cudaSuccess) { set_error("mlp_f16x2: setup: %s", cudaGetErrorString(e)); return (int)e; }
-        configured_dev = dev;
-    }
-    const long long n_iter = (a.P + 127) / 128;
-    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
+    static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, false, 2); }();
+    static const TcSchedule SE = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, true, 2); }();
+    int rc = setup_once(configured_dev,
+                        {(const void*)mlp_f16x2_kernel<false>, (const void*)mlp_f16x2_kernel<true>, (const void*)mlp_f16x2_kernel<false, true>,
+                         (const void*)mlp_f16x2_kernel<true, true>},
+                        SMEM_BYTES, "mlp_f16x2", [] {
+                            cudaError_t e = cudaMemcpyToSymbol(c_fstages, S.st, sizeof(TcStage) * MAX_FSTAGES);
+                            return e == cudaSuccess ? cudaMemcpyToSymbol(c_fstages_emb, SE.st, sizeof(TcStage) * MAX_FSTAGES) : e;
+                        });
+    if (rc) return rc;
     MlpArgs b = a;
     b.tc_comp = -1.0f;                                                                // < 0: the per-layer table tc_comp_ulps
     b.tc_ulps[0] = tc_comp_ulps(0); b.tc_ulps[1] = tc_comp_ulps(1); b.tc_ulps[2] = tc_comp_ulps(8); b.tc_ulps[3] = tc_comp_ulps(9);
@@ -835,32 +671,12 @@ int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
     if (const char* e = getenv("INERF_F16X2_ABL"); e && !embedded) abl = atoi(e);   // the embedded-row build has no ablation variants
     const int n_stages = embedded ? SE.n_stages : S.n_stages;
     const int n_rays = embedded ? 0 : (int)(a.P / a.s);
-    // the CTA-pair build by default; INERF_MLP_PAIR=0 (read once) keeps the single-CTA kernel for A/B runs
-    static const bool pair_env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
-    if (pair_env && num_sms() >= 2) {
-        const long long n_pair_iter = (a.P + 255) / 256;
-        const long long max_pairs = num_sms() / 2;
-        const long long pairs = n_pair_iter < max_pairs ? n_pair_iter : max_pairs;
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(2 * pairs));
-        cfg.blockDim = dim3(NTHREADS);
-        cfg.dynamicSmemBytes = SMEM_BYTES;
-        cfg.stream = st;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        const char* what = embedded ? "inerf_mlp_fwd_embedded[fp16x2 pair]" : "inerf_mlp_fwd[fp16x2 pair]";
-        cudaError_t e = cudaLaunchKernelEx(&cfg, embedded ? mlp_f16x2_kernel<true, true> : mlp_f16x2_kernel<true>, b, n_stages, n_rays, abl);
-        if (e != cudaSuccess) { set_error("%s: %s", what, cudaGetErrorString(e)); return (int)e; }
-        return check_launch(what);
-    }
-    if (embedded) {
-        mlp_f16x2_kernel<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(b, n_stages, n_rays, abl);
-        return check_launch("inerf_mlp_fwd_embedded[fp16x2]");
-    }
-    mlp_f16x2_kernel<false><<<grid, NTHREADS, SMEM_BYTES, st>>>(b, n_stages, n_rays, abl);
-    return check_launch("inerf_mlp_fwd[fp16x2]");
+    const bool pair = mlp_pair_enabled();
+    const auto kernel = pair ? (embedded ? mlp_f16x2_kernel<true, true> : mlp_f16x2_kernel<true>)
+                             : (embedded ? mlp_f16x2_kernel<false, true> : mlp_f16x2_kernel<false>);
+    const char* what = embedded ? (pair ? "inerf_mlp_fwd_embedded[fp16x2 pair]" : "inerf_mlp_fwd_embedded[fp16x2]")
+                                : (pair ? "inerf_mlp_fwd[fp16x2 pair]" : "inerf_mlp_fwd[fp16x2]");
+    return launch_tc(kernel, pair, (a.P + 127) / 128, NTHREADS, SMEM_BYTES, st, what, b, n_stages, n_rays, abl);
 }
 
 }  // namespace inerf

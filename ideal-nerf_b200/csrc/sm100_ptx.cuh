@@ -183,6 +183,67 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
                  : "memory");
 }
 
+// true in exactly one lane of the (fully active) warp
+__device__ __forceinline__ bool elect_one() {
+    uint32_t pred;
+    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
+    return pred != 0;
+}
+
+// 32 lanes x 16 consecutive 32-bit columns
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+        : "r"(taddr)
+        : "memory");
+}
+
+// tcgen05.mma with the two smem descriptors given as (lo, hi) halves: lo = the 14-bit start-address field (+ LBO bit), advanced with
+// plain 32-bit adds of compile-time constants; hi is the same constant for both operands.  Issued by ONE thread.
+__device__ __forceinline__ void umma_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
+        "setp.ne.b32 p, %5, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
+        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// The same for a CTA pair: M = 256 (128 rows from each CTA), the N rows of B split across the two CTAs; issued by the leader only.
+__device__ __forceinline__ void umma_lohi_pair(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+        "mov.b64 da, {%1, %3};\n\tmov.b64 db, {%2, %3};\n\t"
+        "setp.ne.b32 p, %5, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %4, p;\n\t}" ::"r"(tmem_d),
+        "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+template <bool PAIR>
+__device__ __forceinline__ void umma_any(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (PAIR) umma_lohi_pair(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
+    else umma_lohi(tmem_d, a_lo, b_lo, hi, idesc, accumulate);
+}
+template <bool PAIR>
+__device__ __forceinline__ void commit_any(uint64_t* bar) {
+    if constexpr (PAIR) umma_commit_pair(bar);
+    else umma_commit(bar);
+}
+// issuer-side wait on an event whose arrivals may come from the peer CTA
+template <bool PAIR>
+__device__ __forceinline__ void wait_ev(uint64_t* bar, uint32_t parity) {
+    if constexpr (PAIR) mbar_wait_cluster(bar, parity);
+    else mbar_wait(bar, parity);
+}
+
+// Descriptor halves of a K-major, NON-swizzled 16-column (K = 16) bf16 tile stored as [row/8][k/8][row%8][k%8]: 8x8 core matrices of
+// 128 contiguous bytes, the two K halves 128 B apart (leading byte offset), 8-row groups 256 B apart (stride byte offset).
+constexpr uint32_t HI_NOSWZ = (256u >> 4) | (1u << 14);
+__device__ __forceinline__ uint32_t desc_lo_noswz(uint32_t smem_addr) { return ((smem_addr & 0x3FFFF) >> 4) | ((128u >> 4) << 16); }
+
 // byte offset of element (row, col) of a [rows][64] bf16 K-major tile in the 128B-swizzled layout
 __host__ __device__ __forceinline__ uint32_t sw128_offset(uint32_t row, uint32_t col) {
     return (row >> 3) * 1024 + (row & 7) * 128 + ((((col >> 3) ^ row) & 7) << 4) + (col & 7) * 2;

@@ -32,6 +32,8 @@ def test_packed_sizes(L, dims):
     assert n.value == 1114112                       # the fused entry's blob is unchanged: 76 stages
     assert L.inerf_mlp_packed_bytes(_lib.INERF_MLP_BF16_EMB, ctypes.byref(d), ctypes.byref(e)) == 0
     assert e.value == n.value + 2 * 64 * 64 * 2     # + one 64-row x 64-column bf16 view K-block per half of views_linears.0
+    assert L.inerf_mlp_packed_bytes(_lib.INERF_MLP_BF16_BWD, ctypes.byref(d), ctypes.byref(n)) == 0
+    assert n.value == 1048576 + 2 * 4096            # the backward chain's transposed weight stages, then its two alpha tiles
     assert L.inerf_mlp_pack(_lib.INERF_MLP_BF16_EMB, ctypes.byref(d), None, None, None) == -1
 
 
