@@ -268,6 +268,38 @@ def sample_train_pixels(frame_index, budgets, bounds, torso_bits, poses, frames,
     return rays, target, bc_rgb, coords
 
 
+def image_metrics(pred_u8, gt_frames, frame_index, bounds=None):
+    """Scores of rendered frames against ground truth on the device (include/inerf_b200.h, inerf_image_metrics): pred_u8 (B, H, W, 3)
+    uint8, gt_frames (F, H, W, 3) uint8 (e.g. DeviceHeadDataset.frames), frame_index (B,) int64 device tensor selecting each row's ground
+    truth, bounds (F, 8) int32 face-rect / mouth boxes (DeviceHeadDataset.bounds) or None.  Returns device tensors {sse (B, 3) int64,
+    npix (B, 3) int64: full frame, face rect, mouth box (0 without bounds); ssim (B,) float64: the mean SSIM over the channels and the
+    (H - 10) x (W - 10) positions whose window lies inside the frame}.  A row whose index is outside [0, F) scores 0 everywhere.
+    One kernel and no host synchronise: the call may be captured in a CUDA graph."""
+    dev = gt_frames.device
+    for t, name, dt in ((pred_u8, "pred_u8", torch.uint8), (gt_frames, "gt_frames", torch.uint8), (frame_index, "frame_index", torch.int64),
+                        (bounds, "bounds", torch.int32)):
+        if t is None:
+            continue
+        _need_cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"image_metrics: `{name}` must be a contiguous {dt} tensor on {dev}")
+    if gt_frames.dim() != 4 or gt_frames.shape[3] != 3 or pred_u8.dim() != 4 or pred_u8.shape[1:] != gt_frames.shape[1:]:
+        raise ValueError(f"image_metrics: pred_u8 {tuple(pred_u8.shape)} and gt_frames {tuple(gt_frames.shape)} must be (B, H, W, 3) and "
+                         "(F, H, W, 3)")
+    B, F, H, W = pred_u8.shape[0], gt_frames.shape[0], gt_frames.shape[1], gt_frames.shape[2]
+    if frame_index.shape != (B,):
+        raise ValueError(f"image_metrics: frame_index {tuple(frame_index.shape)} must be ({B},)")
+    if bounds is not None and bounds.shape != (F, 8):
+        raise ValueError(f"image_metrics: bounds {tuple(bounds.shape)} must be ({F}, 8)")
+    new = torch.empty if bounds is not None else torch.zeros           # without bounds the kernel writes column 0 only
+    sse, npix = new((B, 3), device=dev, dtype=torch.int64), new((B, 3), device=dev, dtype=torch.int64)
+    ssim_sum = torch.empty((B,), device=dev, dtype=torch.float64)
+    with torch.cuda.device(dev):
+        call("inerf_image_metrics", _lib.lib().inerf_image_metrics, ptr(pred_u8), ptr(gt_frames), ptr(frame_index), ptr(bounds), B, H, W, F,
+             ptr(sse), ptr(npix), ptr(ssim_sum), stream())
+    return {"sse": sse, "npix": npix, "ssim": ssim_sum / (3 * (H - 10) * (W - 10))}
+
+
 def flag_nonfinite(tensors, flags):
     """OR bit i into the int32 device scalar `flags` when tensors[i] holds a NaN / Inf; ONE launch, no host synchronisation."""
     tensors = [f32c(t, "tensor") for t in tensors]

@@ -51,10 +51,12 @@ def normalise_density_(net, rays, aud, expr, latent, n_samples=64, target_std=8.
     return net
 
 
-def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, constant_rgb=None, n_aud=None):
+def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, constant_rgb=None, n_aud=None, val_frames=0):
     """A seeded synthetic subject in the reference's on-disk layout (data.py): random JPEG frames (or one constant colour), parsing maps
     whose last `torso_rows` rows are torso, landmarks that give a mouth box near the centre, a face rectangle, bc.jpg, aud.npy and
-    transforms_exp_train.json.  Returns the args a HeadDataset needs for it (gt_dirs = head_imgs)."""
+    transforms_exp_train.json.  With val_frames > 0 it also writes transforms_exp_val.json: `val_frames` held-out frames (img_id n_frames + j, aud_id
+    the train audio's length + j, poses continuing the train path) whose DeepSpeech windows are appended to aud.npy; every train file is the same as
+    with val_frames = 0 except that longer aud.npy.  Returns the args a HeadDataset needs for it (gt_dirs = head_imgs)."""
     import json
     import os
 
@@ -63,8 +65,8 @@ def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, cons
     for sub in ("head_imgs", "ori_imgs", "parsing"):
         os.makedirs(os.path.join(d, sub), exist_ok=True)
     rng = np.random.RandomState(seed)
-    frames = []
-    for i in range(n_frames):
+
+    def frame(i, aud_id):
         img = np.empty((H, W, 3), np.uint8)
         img[:] = constant_rgb if constant_rgb is not None else rng.randint(0, 255, (H, W, 3), dtype=np.uint8)
         Image.fromarray(img).save(os.path.join(d, "head_imgs", f"{i}.jpg"), quality=95)
@@ -76,9 +78,18 @@ def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, cons
         np.savetxt(os.path.join(d, "ori_imgs", f"{i}.lms"), lms)
         pose = np.eye(4)
         pose[:3, 3] = [0.001 * i, -0.002, 0.7772]
-        frames.append({"img_id": i, "aud_id": i, "transform_matrix": pose.tolist(),
-                       "face_rect": [H // 8, W // 8, H * 5 // 8, W * 3 // 4], "exp": rng.randn(76).tolist()})
-    with open(os.path.join(d, "transforms_exp_train.json"), "w") as fp:
-        json.dump({"focal_len": 1200.0 * W / 450, "cx": W / 2, "cy": H / 2, "frames": frames}, fp)
-    np.save(os.path.join(d, "aud.npy"), rng.randn(n_aud or n_frames, 16, 29).astype(np.float32))
+        return {"img_id": i, "aud_id": aud_id, "transform_matrix": pose.tolist(),
+                "face_rect": [H // 8, W // 8, H * 5 // 8, W * 3 // 4], "exp": rng.randn(76).tolist()}
+
+    def transforms(mode, frames):
+        with open(os.path.join(d, f"transforms_exp_{mode}.json"), "w") as fp:
+            json.dump({"focal_len": 1200.0 * W / 450, "cx": W / 2, "cy": H / 2, "frames": frames}, fp)
+
+    transforms("train", [frame(i, i) for i in range(n_frames)])
+    aud = rng.randn(n_aud or n_frames, 16, 29).astype(np.float32)
+    np.save(os.path.join(d, "aud.npy"), aud)
     Image.fromarray(rng.randint(0, 255, (H, W, 3), dtype=np.uint8)).save(os.path.join(d, "bc.jpg"), quality=95)
+    if val_frames > 0:                      # drawn after every train file, so those keep their bytes
+        n_aud_train = aud.shape[0]
+        transforms("val", [frame(n_frames + j, n_aud_train + j) for j in range(val_frames)])
+        np.save(os.path.join(d, "aud.npy"), np.concatenate([aud, rng.randn(val_frames, 16, 29).astype(np.float32)]))

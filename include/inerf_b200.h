@@ -257,6 +257,28 @@ int inerf_pixel_sampler_workspace_bytes(const InerfPixelSampleArgs* args, size_t
  * enqueues nothing.  Every argument error is returned before any device work. */
 int inerf_sample_train_pixels(const InerfPixelSampleArgs* args, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- image metrics ----------------------------------------------------------------------------------------------------------------
+ * Scores B rendered frames against ground-truth frames, both uint8 (H, W, 3) as to8b writes them, for held-out evaluation (the scores of
+ * the bytes a user sees in the video).  Row b of the batch is compared with gt_frames[frame_index[b]]; the index is read from device
+ * memory, so the call may sit in a CUDA graph.  The results are exactly these:
+ *   - sse[b] = {full, R, M}: the sum over the pixels of the region and over the 3 channels of (pred - gt)^2, exact in int64.  R and M are
+ *     the inclusive boxes {r0, r1, c0, c1} = bounds[f][0..3] (face rect) and bounds[f][4..7] (mouth), as inerf_sample_train_pixels reads
+ *     them; npix[b] = the number of frame pixels in the full frame, R and M.  When bounds is NULL only column 0 of sse and npix is written.
+ *   - ssim_sum[b]: the sum over the 3 channels and over the (H - 10) x (W - 10) positions whose 11 x 11 window lies inside the frame of
+ *       SSIM = ((2 mu_x mu_y + C1)(2 s_xy + C2)) / ((mu_x^2 + mu_y^2 + C1)(s_x^2 + s_y^2 + C2)),
+ *     with mu, E[x^2], E[xy] weighted by the normalised 11-tap Gaussian (sigma 1.5) in both directions, biased moments (s_x^2 = E[x^2] -
+ *     mu_x^2, s_xy = E[xy] - mu_x mu_y), C1 = (0.01 * 255)^2, C2 = (0.03 * 255)^2 (Wang et al. 2004; skimage's structural_similarity
+ *     with gaussian_weights=True, sigma=1.5, use_sample_covariance=False, data_range=255, channel_axis=-1).  The mean SSIM is
+ *     ssim_sum / (3 (H - 10)(W - 10)).  The moments are fp32 (each image shifted by a byte of its tile first); sse and npix are exact.
+ * pred (B, H, W, 3), gt_frames (n_frames, H, W, 3), frame_index (B) int64, bounds (n_frames, 8) int32 or NULL; outputs sse, npix (B, 3)
+ * int64 and ssim_sum (B) fp64.  A row whose frame index lies outside [0, n_frames) gets zeros in every output.
+ * Work: two memsets of the accumulators, then one kernel of one CTA per 32 x 32 tile per row.  Every argument error is returned before
+ * any device work: NULL pointers, B or n_frames < 0 (INERF_E_ARG); H or W < 11, H * W > INERF_IMAGE_METRICS_MAX_PIXELS (INERF_E_SHAPE).
+ * B == 0 enqueues nothing. */
+#define INERF_IMAGE_METRICS_MAX_PIXELS (1 << 24)
+int inerf_image_metrics(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const int32_t* bounds, int32_t B,
+                        int32_t H, int32_t W, int32_t n_frames, int64_t* sse, int64_t* npix, double* ssim_sum, void* stream);
+
 /* ---- importance sampling -------------------------------------------------------------------- */
 
 /* sample_pdf.  Replaces helper.py:269-313.
