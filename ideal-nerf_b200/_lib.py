@@ -120,6 +120,7 @@ SIGNATURES = {
     "inerf_pixel_sampler_workspace_bytes": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _SZP]),
     "inerf_sample_train_pixels": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _P, ctypes.c_size_t, _P]),
     "inerf_image_metrics": (_I, [_P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P, _P, _P, _P]),
+    "inerf_masked_sse": (_I, [_P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P, _P, _P]),
 }
 
 _lib = None

@@ -1,6 +1,7 @@
 // Image quality of rendered uint8 frames against ground-truth uint8 frames: exact SSE over three regions and the SSIM of Wang et al. 2004
 // (11-tap Gaussian, sigma 1.5), on the device and graph-capturable.  The contract is written down in include/inerf_b200.h above
-// inerf_image_metrics; oracle/image_metrics_ref.py restates it in numpy float64.
+// inerf_image_metrics; oracle/image_metrics_ref.py restates it in numpy float64.  inerf_masked_sse (end of the file; oracle/masked_sse_ref.py)
+// gives the exact SSE over a per-frame pixel mask instead of boxes: the torso region of data.torso_bits.
 //
 // One CTA scores one 32 x 32 tile of one frame.  It stages the tile plus its 5-pixel halo of both images in shared memory as bytes, sums
 // the tile's squared errors in integers, then per channel runs the separable filter -- a horizontal pass over the 42 halo rows, then a
@@ -169,6 +170,58 @@ __global__ void __launch_bounds__(kThreads) image_metrics_kernel(const uint8_t* 
     }
 }
 
+// ---- SSE over a per-frame pixel mask (inerf_masked_sse) ---------------------------------------------------------------------------------
+// One 256-thread CTA scores kMaskPixels consecutive pixels of one row of the batch; the 32 lanes of a warp read 32 consecutive pixels, whose
+// mask bits are one word (read once per warp, broadcast), so only pixels in the mask load their bytes.
+constexpr int kMaskThreads = 256;
+constexpr int kMaskPixels = 4 * kMaskThreads;
+
+__global__ void __launch_bounds__(kMaskThreads) masked_sse_kernel(const uint8_t* __restrict__ pred, const uint8_t* __restrict__ gt,
+                                                                  const int64_t* __restrict__ frame_index, const uint32_t* __restrict__ bits,
+                                                                  int hw, int words, int n_frames, int chunks, long long* sse,
+                                                                  long long* npix) {
+    __shared__ long long s_e[kMaskThreads / 32];
+    __shared__ int s_n[kMaskThreads / 32];
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int b = blockIdx.x / chunks, p0 = (blockIdx.x - b * chunks) * kMaskPixels;
+    const long long f = frame_index[b];
+    if (f < 0 || f >= n_frames) return;                 // sse and npix were zeroed before the launch
+    const uint8_t* pa = pred + (size_t)b * hw * 3;
+    const uint8_t* pb = gt + (size_t)f * hw * 3;
+    const uint32_t* m = bits + (size_t)f * words;
+    const int p1 = min(p0 + kMaskPixels, hw);
+    int e = 0, n = 0;                                   // at most 4 pixels x 3 x 255^2 per thread
+    for (int p = p0 + t; p < p1; p += kMaskThreads) {
+        if (!((__ldg(m + (p >> 5)) >> (p & 31)) & 1u)) continue;
+        const size_t o = (size_t)p * 3;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const int d = (int)pa[o + c] - (int)pb[o + c];
+            e += d * d;
+        }
+        ++n;
+    }
+    const long long w_e = warp_sum_ll(e);
+    int w_n = n;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) w_n += __shfl_xor_sync(0xffffffffu, w_n, o);
+    if (lane == 0) {
+        s_e[warp] = w_e;
+        s_n[warp] = w_n;
+    }
+    __syncthreads();
+    if (t == 0) {
+        long long te = 0, tn = 0;
+#pragma unroll
+        for (int w = 0; w < kMaskThreads / 32; ++w) {
+            te += s_e[w];
+            tn += s_n[w];
+        }
+        if (te) atomicAdd(reinterpret_cast<unsigned long long*>(sse + b), (unsigned long long)te);
+        if (tn) atomicAdd(reinterpret_cast<unsigned long long*>(npix + b), (unsigned long long)tn);
+    }
+}
+
 }  // namespace
 
 extern "C" int inerf_image_metrics(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const int32_t* bounds,
@@ -199,4 +252,27 @@ extern "C" int inerf_image_metrics(const uint8_t* pred, const uint8_t* gt_frames
                                                                     reinterpret_cast<long long*>(sse), reinterpret_cast<long long*>(npix),
                                                                     ssim_sum);
     return check_launch("inerf_image_metrics");
+}
+
+extern "C" int inerf_masked_sse(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const uint32_t* bits, int32_t B,
+                                int32_t H, int32_t W, int32_t n_frames, int64_t* sse, int64_t* npix, void* stream) {
+    if (!pred || !gt_frames || !frame_index || !bits || !sse || !npix) return fail(INERF_E_ARG, "inerf_masked_sse: NULL pointer");
+    if (B < 0 || n_frames < 0) return fail(INERF_E_ARG, "inerf_masked_sse: negative B or n_frames");
+    if (H < kTaps || W < kTaps || (int64_t)H * W > INERF_IMAGE_METRICS_MAX_PIXELS) {
+        set_error("inerf_masked_sse: %d x %d frames (need H, W >= %d and H * W <= %d)", H, W, kTaps, INERF_IMAGE_METRICS_MAX_PIXELS);
+        return INERF_E_SHAPE;
+    }
+    const int hw = H * W, chunks = (hw + kMaskPixels - 1) / kMaskPixels;
+    if ((int64_t)B * chunks > 0x7fffffff) return fail(INERF_E_SHAPE, "inerf_masked_sse: B * chunks exceeds the grid");
+    if (B == 0) return INERF_OK;
+    cudaStream_t s = as_stream(stream);
+    cudaError_t e = cudaMemsetAsync(sse, 0, (size_t)B * sizeof(int64_t), s);
+    if (e == cudaSuccess) e = cudaMemsetAsync(npix, 0, (size_t)B * sizeof(int64_t), s);
+    if (e != cudaSuccess) {
+        set_error("inerf_masked_sse: %s", cudaGetErrorString(e));
+        return (int)e;
+    }
+    masked_sse_kernel<<<(unsigned)(B * chunks), kMaskThreads, 0, s>>>(pred, gt_frames, frame_index, bits, hw, (hw + 31) / 32, n_frames, chunks,
+                                                                      reinterpret_cast<long long*>(sse), reinterpret_cast<long long*>(npix));
+    return check_launch("inerf_masked_sse");
 }

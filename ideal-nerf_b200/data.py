@@ -11,7 +11,8 @@ data_util/process_data.py:253-288:
 
 HeadDataset is host side (json / numpy / PIL), except that the N_rand training rays are generated on the device for the SELECTED pixels
 (ops.get_rays_at) instead of building the 450 x 450 ray grid per sample and indexing it (:123-139,189-191).  DeviceHeadDataset decodes
-every frame once and draws each batch on the device (ops.sample_train_pixels): no host work per step."""
+every frame once and draws each batch on the device (ops.sample_train_pixels): no host work per step.  DeviceTorsoDataset does the same
+for the torso stage: the head batch plus the torso rays of the same pixels and the frozen head's per-frame codes."""
 import json
 import os
 
@@ -207,10 +208,9 @@ class DeviceHeadDataset(HeadDataset):
         self._win = torch.arange(2 * half, dtype=torch.int64, device=dev)
         self._index = torch.zeros((), dtype=torch.int64, device=dev)
 
-    def sample(self, index, rank=0, world=1):
-        """The training batch of frame `index` (host int or int64 device scalar), rows frame.band(N_rand, rank, world) of it: a dict with
-        rays (n, 11) packed with args.near / args.far, target (n, 3), bc_rgb (n, 3), aud_window (smo_size, 16, 29) =
-        Network.audio_window(auds, index, len(self)), expr, pose (3, 4).  Advances the Philox offset by one."""
+    def _draw(self, index, rank, world, want_coords):
+        """(idx (1,) int64 device tensor, ops.sample_train_pixels' (rays, target, bc_rgb, coords)) of rows frame.band(N_rand, rank, world)
+        of frame `index`'s batch."""
         from .frame import band
         if torch.is_tensor(index):
             idx = index.reshape(())
@@ -221,10 +221,15 @@ class DeviceHeadDataset(HeadDataset):
                 raise IndexError(f"frame {index} outside [0, {self.data_size})")
             idx = self._index.fill_(int(index))
         lo, hi = band(sum(self.budgets), rank, world)
-        rays, target, bc_rgb, _ = ops.sample_train_pixels(idx, self.budgets, self.bounds, self.torso_bits, self.poses, self.frames,
-                                                          self.bc_img, self.focal, self.cx, self.cy, self.args.near, self.args.far,
-                                                          first=lo, count=hi - lo)
-        i1 = idx.reshape(1)
+        batch = ops.sample_train_pixels(idx, self.budgets, self.bounds, self.torso_bits, self.poses, self.frames, self.bc_img, self.focal,
+                                        self.cx, self.cy, self.args.near, self.args.far, first=lo, count=hi - lo, want_coords=want_coords)
+        return idx.reshape(1), batch
+
+    def sample(self, index, rank=0, world=1):
+        """The training batch of frame `index` (host int or int64 device scalar), rows frame.band(N_rand, rank, world) of it: a dict with
+        rays (n, 11) packed with args.near / args.far, target (n, 3), bc_rgb (n, 3), aud_window (smo_size, 16, 29) =
+        Network.audio_window(auds, index, len(self)), expr, pose (3, 4).  Advances the Philox offset by one."""
+        i1, (rays, target, bc_rgb, _) = self._draw(index, rank, world, False)
         return {"rays": rays, "target": target, "bc_rgb": bc_rgb, "aud_window": self.auds_padded.index_select(0, i1 + self._win),
                 "expr": self.exprs.index_select(0, i1)[0], "pose": self.poses.index_select(0, i1)[0]}
 
@@ -233,7 +238,61 @@ class DeviceHeadDataset(HeadDataset):
         is the device frame (BGR uint8), bc_rgb fp32."""
         if index is None:
             index = np.random.choice(self.data_size)
-        b = self.sample(index)
+        b = DeviceHeadDataset.sample(self, index)
         rays = b["rays"]
         batch_rays = torch.stack([rays[:, 0:3], rays[:, 3:6]], 0)
         return batch_rays, b["target"], b["bc_rgb"], self.auds, self.frames[index], self.all_poses[index][:3, :4], b["expr"], index
+
+
+class DeviceTorsoDataset(DeviceHeadDataset):
+    """The torso stage's batches (NeRFs/TorsoNeRF/train_torso.py) drawn on the device: DeviceHeadDataset's files, checks and region
+    budgets, with targets from args.gt_dirs (for this stage the composited head + torso frames, conventionally com_imgs), plus what
+    train.TorsoTrainStep takes besides the head batch.
+
+    The pixels are drawn with the head stage's region machinery (face rect, mouth box, torso mask and their budgets) on the gt_dirs frames.
+    The reference's train_torso.py loader was not available when this was written, so that it samples the same regions is not verified.
+
+    aud_codes: (F, args.dim_aud), row i = the frozen head's audio code of frame i, computed once, e.g. evaluate.audio_codes(head_network,
+    HeadDataset(...)) after checkpoint.load_head_checkpoint (the torso stage trains no audio net).  latent_codes: (F, 32), as
+    checkpoint.load_head_into_torso returns them; required for mode "train", optional otherwise (sample() then raises).  torso_pose: the
+    fixed camera of the torso pair, (3, 4) or (4, 4); default: the transform_matrix of the first frame of transforms_exp_train.json, for
+    every mode (the frame-0 camera of frame.HeadTorsoFrameRenderer: a val split is rendered from the camera the torso was trained with).
+    Kept as torso_pose (3, 4) fp32 on the device.  A table of the wrong shape raises ValueError here, naming it.
+
+    sample(index, rank=0, world=1) returns a dict keyed by TorsoTrainStep's parameters, so step(**ds.sample(i)) runs one iteration:
+    rays_head, target, bc_rgb are DeviceHeadDataset.sample's rays, target and bc_rgb for the same Philox state (one draw; the offset advances
+    once); rays_torso are the rays of the same pixels from torso_pose (ops.get_rays_at on the sampler's coordinates, the bits the sampler
+    writes for a pose); aud_feature, pose (3, 4), expr, latent_code are row `index` of the tables.  No host synchronise: `index` may be an
+    int64 device scalar and the call may sit in a CUDA graph.  __getitem__ keeps DeviceHeadDataset's tuple."""
+
+    def __init__(self, data_dir, aud_file, mode, args, aud_codes, latent_codes=None, torso_pose=None, skip=1, device="cuda"):
+        super().__init__(data_dir, aud_file, mode, args, skip, device)
+        if torso_pose is None:
+            with open(os.path.join(data_dir, "transforms_exp_train.json")) as fp:
+                torso_pose = json.load(fp)["frames"][0]["transform_matrix"]
+        pose = torch.as_tensor(torso_pose).detach()
+        if tuple(pose.shape) not in ((3, 4), (4, 4)):
+            raise ValueError(f"torso_pose is {tuple(pose.shape)}, not (3, 4) or (4, 4)")
+        self.torso_pose = pose[:3].to(self.device, torch.float32).contiguous()
+        self.aud_codes = self._table("aud_codes", aud_codes, int(args.dim_aud))
+        if latent_codes is None and mode == "train":
+            raise ValueError("latent_codes: the train split needs the head's (F, 32) latent codes")
+        self.latent_codes = None if latent_codes is None else self._table("latent_codes", latent_codes, 32)
+
+    def _table(self, name, t, width):
+        t = torch.as_tensor(t).detach()
+        if tuple(t.shape) != (self.data_size, width):
+            raise ValueError(f"{name} is {tuple(t.shape)}, this split needs ({self.data_size}, {width})")
+        return t.to(self.device, torch.float32).contiguous()
+
+    def sample(self, index, rank=0, world=1):
+        """The torso batch of frame `index` (host int or int64 device scalar), rows frame.band(N_rand, rank, world) of it: {rays_head,
+        rays_torso (n, 11), bc_rgb, target (n, 3), aud_feature (dim_aud,), pose (3, 4), expr, latent_code (32,)}.  Advances the Philox
+        offset by one."""
+        if self.latent_codes is None:
+            raise ValueError("DeviceTorsoDataset.sample needs latent_codes (given none for this split)")
+        i1, (rays, target, bc_rgb, coords) = self._draw(index, rank, world, True)
+        rays_torso = ops.get_rays_at(coords, self.focal, self.torso_pose, self.args.near, self.args.far, self.cx, self.cy)
+        return {"rays_head": rays, "rays_torso": rays_torso, "bc_rgb": bc_rgb, "target": target,
+                "aud_feature": self.aud_codes.index_select(0, i1)[0], "pose": self.poses.index_select(0, i1)[0],
+                "expr": self.exprs.index_select(0, i1)[0], "latent_code": self.latent_codes.index_select(0, i1)[0]}

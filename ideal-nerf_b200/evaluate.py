@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .data import DeviceTorsoDataset
 from .frame import HeadTorsoFrameRenderer, render_head_torso_video, render_video
 
 
@@ -46,17 +47,25 @@ def evaluate_split(renderer, dataset, latent, codes, perturb=0., keep_video=True
 
     Returns, on rank 0, a dict of host values: psnr (F, 3) float64 (full frame, face rect, mouth box), ssim (F,) float64, their means over
     the frames mean_psnr (3,) and mean_ssim, the exact sse / npix (F, 3) int64 behind the PSNR, and video (F, H, W, 3) uint8 (the rendered
-    bytes, the frames' channel order) when keep_video, else None.  Other ranks return None."""
+    bytes, the frames' channel order) when keep_video, else None.  Other ranks return None.
+
+    When dataset is a data.DeviceTorsoDataset (render it with HeadTorsoFrameRenderer(torso_net, dataset.torso_pose)), each frame is also
+    scored over its torso pixels (dataset.torso_bits, ops.masked_sse), the region the torso stage trains -- the head pair is frozen there,
+    so the face rect and mouth box measure the head, and the full frame is mostly background.  Extra keys: sse_torso, npix_torso (F,)
+    int64, psnr_torso (F,) float64 and mean_psnr_torso."""
     n = len(dataset)
     if codes.shape[0] != n:
         raise ValueError(f"evaluate_split: {codes.shape[0]} audio codes for {n} frames")
     dev = dataset.frames.device
     index = torch.arange(n, dtype=torch.int64, device=dev)
     frames = [(dataset.poses[i], codes[i], dataset.exprs[i]) for i in range(n)]
-    scores = []
+    torso = isinstance(dataset, DeviceTorsoDataset)
+    scores, torso_scores = [], []
 
     def on_frame(i, img):
         scores.append(ops.image_metrics(img[None], dataset.frames, index[i:i + 1], dataset.bounds))
+        if torso:
+            torso_scores.append(ops.masked_sse(img[None], dataset.frames, index[i:i + 1], dataset.torso_bits))
 
     drive = render_head_torso_video if isinstance(renderer, HeadTorsoFrameRenderer) else render_video
     video = drive(renderer, frames, latent, dataset.bc_img, perturb, on_frame=on_frame)
@@ -66,5 +75,11 @@ def evaluate_split(renderer, dataset, latent, codes, perturb=0., keep_video=True
     npix = torch.cat([s["npix"] for s in scores]).cpu().numpy()
     ssim = torch.cat([s["ssim"] for s in scores]).cpu().numpy()
     p = psnr(sse, npix).numpy()
-    return {"psnr": p, "ssim": ssim, "mean_psnr": p.mean(0), "mean_ssim": float(ssim.mean()), "sse": sse, "npix": npix,
-            "video": video.numpy() if keep_video else None}
+    res = {"psnr": p, "ssim": ssim, "mean_psnr": p.mean(0), "mean_ssim": float(ssim.mean()), "sse": sse, "npix": npix,
+           "video": video.numpy() if keep_video else None}
+    if torso:
+        sse_t = torch.cat([s for s, _ in torso_scores]).cpu().numpy()
+        npix_t = torch.cat([c for _, c in torso_scores]).cpu().numpy()
+        p_t = psnr(sse_t, npix_t).numpy()
+        res.update(sse_torso=sse_t, npix_torso=npix_t, psnr_torso=p_t, mean_psnr_torso=float(p_t.mean()))
+    return res

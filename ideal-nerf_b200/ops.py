@@ -300,6 +300,33 @@ def image_metrics(pred_u8, gt_frames, frame_index, bounds=None):
     return {"sse": sse, "npix": npix, "ssim": ssim_sum / (3 * (H - 10) * (W - 10))}
 
 
+def masked_sse(pred_u8, gt_frames, frame_index, bits):
+    """Squared error of rendered frames over a per-frame pixel mask on the device (include/inerf_b200.h, inerf_masked_sse): pred_u8
+    (B, H, W, 3) uint8, gt_frames (F, H, W, 3) uint8, frame_index (B,) int64 device tensor, bits (F, ceil(H*W/32)) int32 holding the uint32
+    words of data.torso_bits (e.g. DeviceTorsoDataset.torso_bits).  Returns device tensors (sse (B,) int64 over the 3 channels of the masked
+    pixels, npix (B,) int64 masked pixels); a row whose index is outside [0, F) gets zeros.  One kernel and no host synchronise: the call
+    may be captured in a CUDA graph."""
+    dev = gt_frames.device
+    for t, name, dt in ((pred_u8, "pred_u8", torch.uint8), (gt_frames, "gt_frames", torch.uint8), (frame_index, "frame_index", torch.int64),
+                        (bits, "bits", torch.int32)):
+        _need_cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"masked_sse: `{name}` must be a contiguous {dt} tensor on {dev}")
+    if gt_frames.dim() != 4 or gt_frames.shape[3] != 3 or pred_u8.dim() != 4 or pred_u8.shape[1:] != gt_frames.shape[1:]:
+        raise ValueError(f"masked_sse: pred_u8 {tuple(pred_u8.shape)} and gt_frames {tuple(gt_frames.shape)} must be (B, H, W, 3) and "
+                         "(F, H, W, 3)")
+    B, F, H, W = pred_u8.shape[0], gt_frames.shape[0], gt_frames.shape[1], gt_frames.shape[2]
+    if frame_index.shape != (B,):
+        raise ValueError(f"masked_sse: frame_index {tuple(frame_index.shape)} must be ({B},)")
+    if bits.shape != (F, (H * W + 31) // 32):
+        raise ValueError(f"masked_sse: bits {tuple(bits.shape)} must be ({F}, {(H * W + 31) // 32})")
+    sse, npix = torch.empty((B,), device=dev, dtype=torch.int64), torch.empty((B,), device=dev, dtype=torch.int64)
+    with torch.cuda.device(dev):
+        call("inerf_masked_sse", _lib.lib().inerf_masked_sse, ptr(pred_u8), ptr(gt_frames), ptr(frame_index), ptr(bits), B, H, W, F, ptr(sse),
+             ptr(npix), stream())
+    return sse, npix
+
+
 def flag_nonfinite(tensors, flags):
     """OR bit i into the int32 device scalar `flags` when tensors[i] holds a NaN / Inf; ONE launch, no host synchronisation."""
     tensors = [f32c(t, "tensor") for t in tensors]

@@ -11,6 +11,7 @@ from . import ops
 
 NEAR = 0.5772005200386048   # NeRFs/HeadNeRF/configs/audio_expr_nerf/may/paper_model/torso_bg.txt:11-12
 FAR = 1.1772005200386046
+TORSO_RGB = (40, 150, 90)   # the torso colour of write_head_subject's com_imgs
 
 
 def camera():
@@ -51,18 +52,20 @@ def normalise_density_(net, rays, aud, expr, latent, n_samples=64, target_std=8.
     return net
 
 
-def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, constant_rgb=None, n_aud=None, val_frames=0):
+def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, constant_rgb=None, n_aud=None, val_frames=0, com_imgs=False):
     """A seeded synthetic subject in the reference's on-disk layout (data.py): random JPEG frames (or one constant colour), parsing maps
     whose last `torso_rows` rows are torso, landmarks that give a mouth box near the centre, a face rectangle, bc.jpg, aud.npy and
     transforms_exp_train.json.  With val_frames > 0 it also writes transforms_exp_val.json: `val_frames` held-out frames (img_id n_frames + j, aud_id
     the train audio's length + j, poses continuing the train path) whose DeepSpeech windows are appended to aud.npy; every train file is the same as
-    with val_frames = 0 except that longer aud.npy.  Returns the args a HeadDataset needs for it (gt_dirs = head_imgs)."""
+    with val_frames = 0 except that longer aud.npy.  With com_imgs it also writes com_imgs/<img_id>.jpg, the torso stage's targets
+    (gt_dirs = com_imgs): each frame's head image with its last `torso_rows` rows painted TORSO_RGB (no draw from the generator, so every
+    other file keeps its bytes).  Returns the args a HeadDataset needs for it (gt_dirs = head_imgs)."""
     import json
     import os
 
     import numpy as np
     from PIL import Image
-    for sub in ("head_imgs", "ori_imgs", "parsing"):
+    for sub in ("head_imgs", "ori_imgs", "parsing") + (("com_imgs",) if com_imgs else ()):
         os.makedirs(os.path.join(d, sub), exist_ok=True)
     rng = np.random.RandomState(seed)
 
@@ -70,6 +73,9 @@ def write_head_subject(d, H=450, W=450, n_frames=64, seed=0, torso_rows=40, cons
         img = np.empty((H, W, 3), np.uint8)
         img[:] = constant_rgb if constant_rgb is not None else rng.randint(0, 255, (H, W, 3), dtype=np.uint8)
         Image.fromarray(img).save(os.path.join(d, "head_imgs", f"{i}.jpg"), quality=95)
+        if com_imgs:
+            img[H - torso_rows:] = TORSO_RGB
+            Image.fromarray(img).save(os.path.join(d, "com_imgs", f"{i}.jpg"), quality=95)
         parse = np.zeros((H, W, 3), np.uint8)
         parse[H - torso_rows:, :, 0] = 255
         Image.fromarray(parse).save(os.path.join(d, "parsing", f"{i}.png"))

@@ -279,6 +279,19 @@ int inerf_sample_train_pixels(const InerfPixelSampleArgs* args, void* workspace,
 int inerf_image_metrics(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const int32_t* bounds, int32_t B,
                         int32_t H, int32_t W, int32_t n_frames, int64_t* sse, int64_t* npix, double* ssim_sum, void* stream);
 
+/* The squared error of B rendered frames over a per-frame pixel mask, e.g. the torso region the torso stage trains (its pixels are the
+ * parsing map's pure red ones, the torso bitmask of inerf_sample_train_pixels).  Row b is compared with gt_frames[frame_index[b]] (index
+ * read from device memory, so the call may sit in a CUDA graph):
+ *   - sse[b] = the sum over the 3 channels and over the pixels p < H * W whose bit (p & 31) of bits[f][p >> 5] is set (p = row * W + col,
+ *     f = frame_index[b]) of (pred - gt)^2, exact in int64;  npix[b] = the number of those pixels.
+ * pred (B, H, W, 3) uint8, gt_frames (n_frames, H, W, 3) uint8, frame_index (B) int64, bits (n_frames, ceil(H * W / 32)) uint32 (the bits
+ * past H * W in the last word are ignored); outputs sse, npix (B) int64.  A row whose frame index lies outside [0, n_frames) gets zeros.
+ * Work: two memsets of the accumulators, then one kernel of one CTA per 1 024 pixels per row.  Every argument error is returned before any
+ * device work, with inerf_image_metrics' codes and limits: NULL pointers, B or n_frames < 0 (INERF_E_ARG); H or W < 11, H * W >
+ * INERF_IMAGE_METRICS_MAX_PIXELS (INERF_E_SHAPE).  B == 0 enqueues nothing. */
+int inerf_masked_sse(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const uint32_t* bits, int32_t B, int32_t H,
+                     int32_t W, int32_t n_frames, int64_t* sse, int64_t* npix, void* stream);
+
 /* ---- importance sampling -------------------------------------------------------------------- */
 
 /* sample_pdf.  Replaces helper.py:269-313.
