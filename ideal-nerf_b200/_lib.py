@@ -14,7 +14,8 @@ REPO_ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 SO_PATH = os.environ.get("INERF_SO") or os.path.join(PKG_DIR, "libinerf_b200.so")     # INERF_SO: profiling builds only
 SOURCES = ["api.cu", "rays.cu", "composite.cu", "sample_pdf.cu", "mlp_api.cu", "mlp_fp32.cu", "mlp_fp32_bwd.cu", "mlp_bf16.cu", "mlp_bf16_bwd.cu",
-           "mlp_bf16_dw.cu", "mlp_f16x2.cu", "audio_net.cu", "render_fused.cu", "pixel_sampler.cu", "image_metrics.cu"]
+           "mlp_bf16_dw.cu", "mlp_f16x2.cu", "audio_net.cu", "render_fused.cu", "pixel_sampler.cu", "image_metrics.cu",
+           "lpips.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--shared"]
 
@@ -63,6 +64,8 @@ class InerfPixelSampleArgs(ctypes.Structure):
 INERF_PIXEL_SAMPLER_MAX_K = 4096
 INERF_PIXEL_SAMPLER_MAX_PIXELS = 1 << 22
 INERF_IMAGE_METRICS_MAX_PIXELS = 1 << 24
+INERF_LPIPS_N_PARAMS = 15
+INERF_LPIPS_MAX_ROWS = 65535
 
 NF_BITS = {"rgb_map": 1, "disp_map": 2, "acc_map": 4, "rgb0": 8, "disp0": 16, "acc0": 32, "z_std": 64, "last_weight": 128}     # INERF_NF_*
 
@@ -121,6 +124,8 @@ SIGNATURES = {
     "inerf_sample_train_pixels": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _P, ctypes.c_size_t, _P]),
     "inerf_image_metrics": (_I, [_P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P, _P, _P, _P]),
     "inerf_masked_sse": (_I, [_P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P, _P, _P]),
+    "inerf_lpips_workspace_bytes": (_I, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _SZP]),
+    "inerf_lpips": (_I, [_PARAMS, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P, ctypes.c_size_t, _P, _P]),
 }
 
 _lib = None

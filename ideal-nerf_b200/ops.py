@@ -327,6 +327,50 @@ def masked_sse(pred_u8, gt_frames, frame_index, bits):
     return sse, npix
 
 
+# inerf_lpips' 15 parameters in ABI order: conv1..conv5 (weight, bias), then lin0..lin4
+LPIPS_CHANNELS = (64, 192, 384, 256, 256)
+LPIPS_SHAPES = ([s for cout, cin, k in zip(LPIPS_CHANNELS, (3, 64, 192, 384, 256), (11, 5, 3, 3, 3)) for s in ((cout, cin, k, k), (cout,))] +
+                [(c,) for c in LPIPS_CHANNELS])
+
+
+def lpips(pred_u8, gt_frames, frame_index, weights):
+    """LPIPS v0.1 (AlexNet trunk) of rendered frames against ground truth on the device (include/inerf_b200.h, inerf_lpips): pred_u8
+    (B, H, W, 3) uint8, gt_frames (F, H, W, 3) uint8 (BGR as stored, e.g. DeviceHeadDataset.frames), frame_index (B,) int64 device tensor
+    selecting each row's ground truth, weights the 15 fp32 device tensors of evaluate.load_lpips.  Returns (B,) float32 on the device,
+    what lpips.LPIPS(net='alex')(pred, gt) gives each row; a row whose index is outside [0, F) gets 0.  Frames need H, W >= 31.  One C
+    call, no host synchronise: the call may be captured in a CUDA graph (its workspace is allocated here, before the launches)."""
+    dev = gt_frames.device
+    for t, name, dt in ((pred_u8, "pred_u8", torch.uint8), (gt_frames, "gt_frames", torch.uint8), (frame_index, "frame_index", torch.int64)):
+        _need_cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"lpips: `{name}` must be a contiguous {dt} tensor on {dev}")
+    if gt_frames.dim() != 4 or gt_frames.shape[3] != 3 or pred_u8.dim() != 4 or pred_u8.shape[1:] != gt_frames.shape[1:]:
+        raise ValueError(f"lpips: pred_u8 {tuple(pred_u8.shape)} and gt_frames {tuple(gt_frames.shape)} must be (B, H, W, 3) and "
+                         "(F, H, W, 3)")
+    B, F, H, W = pred_u8.shape[0], gt_frames.shape[0], gt_frames.shape[1], gt_frames.shape[2]
+    if frame_index.shape != (B,):
+        raise ValueError(f"lpips: frame_index {tuple(frame_index.shape)} must be ({B},)")
+    if len(weights) != len(LPIPS_SHAPES):
+        raise ValueError(f"lpips: {len(weights)} weight tensors, need {len(LPIPS_SHAPES)} (evaluate.load_lpips)")
+    for i, (t, shape) in enumerate(zip(weights, LPIPS_SHAPES)):
+        _need_cuda(t, f"weights[{i}]")
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev or tuple(t.shape) != shape:
+            raise ValueError(f"lpips: weights[{i}] must be a contiguous float32 {shape} tensor on {dev}, got {t.dtype} "
+                             f"{tuple(t.shape)} on {t.device}")
+    L = _lib.lib()
+    out = torch.empty((B,), device=dev, dtype=torch.float32)
+    if B == 0:
+        return out
+    nbytes = ctypes.c_size_t(0)
+    check(L.inerf_lpips_workspace_bytes(B, H, W, ctypes.byref(nbytes)), "inerf_lpips_workspace_bytes")
+    ws = torch.empty((nbytes.value,), device=dev, dtype=torch.uint8)
+    params = (ctypes.c_void_p * len(weights))(*[t.data_ptr() for t in weights])
+    with torch.cuda.device(dev):
+        call("inerf_lpips", L.inerf_lpips, params, ptr(pred_u8), ptr(gt_frames), ptr(frame_index), B, H, W, F, ptr(ws), nbytes.value,
+             ptr(out), stream(), launches=13)
+    return out
+
+
 def flag_nonfinite(tensors, flags):
     """OR bit i into the int32 device scalar `flags` when tensors[i] holds a NaN / Inf; ONE launch, no host synchronisation."""
     tensors = [f32c(t, "tensor") for t in tensors]

@@ -292,6 +292,36 @@ int inerf_image_metrics(const uint8_t* pred, const uint8_t* gt_frames, const int
 int inerf_masked_sse(const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, const uint32_t* bits, int32_t B, int32_t H,
                      int32_t W, int32_t n_frames, int64_t* sse, int64_t* npix, void* stream);
 
+/* LPIPS v0.1 with the AlexNet trunk (Zhang et al. 2018) of B rendered frames: out[b] is what lpips.LPIPS(net='alex', version='0.1')(in0,
+ * in1) computes (normalize=False) for in0 = pred[b], in1 = gt_frames[frame_index[b]].  The frames are uint8 (H, W, 3) BGR as stored, so the
+ * bytes of a pixel are read as B, G, R and fed to AlexNet as R, G, B.
+ *   1. x = byte / 127.5 - 1 per channel (lpips' im2tensor), then the ScalingLayer (x - shift_c) / scale_c with shift = (-0.030, -0.088,
+ *      -0.188), scale = (0.458, 0.448, 0.450) in R, G, B order.  Convolution zero padding applies to these scaled values.
+ *   2. AlexNet features (torchvision layout): conv1 11 x 11 stride 4 pad 2, 3 -> 64, ReLU = f1; max pool 3 / 2; conv2 5 x 5 pad 2, 64 ->
+ *      192, ReLU = f2; max pool 3 / 2; conv3 3 x 3 pad 1, 192 -> 384, ReLU = f3; conv4 3 x 3 pad 1, 384 -> 256, ReLU = f4; conv5 3 x 3
+ *      pad 1, 256 -> 256, ReLU = f5.  (The final max pool is not used.)
+ *   3. Per layer k and output position, each image's feature vector is normalised over the channels, f / (sqrt(sum_c f^2) + 1e-10); the
+ *      squared difference of the two normalised vectors is dotted with lin_k (C_k weights, no bias); that is averaged over the layer's
+ *      h_k x w_k positions.
+ *   4. out[b] = the sum of the five layer means, added in layer order.
+ * For 450 x 450 frames the maps are 111^2 (f1), 55^2 (f2) and 27^2 (f3 - f5); every map is non-empty for H, W >= 31.
+ * params_host: host array of INERF_LPIPS_N_PARAMS device pointers to contiguous fp32, in this order: conv1.weight (64, 3, 11, 11),
+ * conv1.bias (64), conv2.weight (192, 64, 5, 5), conv2.bias, conv3.weight (384, 192, 3, 3), conv3.bias, conv4.weight (256, 384, 3, 3),
+ * conv4.bias, conv5.weight (256, 256, 3, 3), conv5.bias, lin0 (64), lin1 (192), lin2 (384), lin3 (256), lin4 (256) -- torchvision's
+ * features.{0,3,6,8,10} and lpips' lin{0..4}.model.1.weight.  pred (B, H, W, 3), gt_frames (n_frames, H, W, 3), frame_index (B) int64, read
+ * from device memory; out (B) fp32.  A row whose frame index lies outside [0, n_frames) gets 0.  The arithmetic is fp32 with every sum in
+ * a fixed order: results are bit-identical from call to call and between eager calls and CUDA-graph replay.
+ * workspace: device memory of at least inerf_lpips_workspace_bytes(B, H, W) bytes, 256-byte aligned (the fp32 feature maps of both images
+ * of every row, 26.3 MB per row at 450 x 450, and the per-CTA partial sums).  Work: 13 kernels on `stream`, no allocation, no copy and no
+ * synchronise, so the call may sit in a CUDA graph.  Every argument error is returned before any device work: NULL pointers, B or n_frames
+ * < 0 (INERF_E_ARG); H or W < 31, H * W > INERF_IMAGE_METRICS_MAX_PIXELS, B > INERF_LPIPS_MAX_ROWS, a workspace smaller than needed
+ * (INERF_E_SHAPE).  B == 0 enqueues nothing. */
+#define INERF_LPIPS_N_PARAMS 15
+#define INERF_LPIPS_MAX_ROWS 65535
+int inerf_lpips_workspace_bytes(int32_t B, int32_t H, int32_t W, size_t* bytes);
+int inerf_lpips(const float* const* params_host, const uint8_t* pred, const uint8_t* gt_frames, const int64_t* frame_index, int32_t B,
+                int32_t H, int32_t W, int32_t n_frames, void* workspace, size_t workspace_bytes, float* out, void* stream);
+
 /* ---- importance sampling -------------------------------------------------------------------- */
 
 /* sample_pdf.  Replaces helper.py:269-313.
