@@ -787,8 +787,12 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 #pragma unroll
                 for (int c = 0; c < 3; ++c) {
                     // one accurate sincosf per coordinate, then angle doubling: sin 2a = 2 sin a cos a, cos 2a = 1 - 2 sin^2 a.
-                    // The absolute error at most doubles per octave (~2^9 * 1e-7 = 6e-5 at 2^9 x), two orders below the bf16
-                    // rounding (2^-9) the operand gets anyway, and costs 27 short FMA chains instead of 27 range reductions.
+                    // An angle error doubles per octave, but an amplitude error (sin^2 + cos^2 != 1) is multiplied by 4 sin^2 a, so
+                    // the absolute error grows by up to ~3.1x per octave (two steps at most 9.5x): bounded by 3.1^f * 2^-22, ~1e-4 at
+                    // octave 7 and ~6e-3 at octave 9 (tests/test_bf16_operands.py measured 1.0e-4 and 9.7e-4 there).  Near a zero of sin / cos that is
+                    // many bf16 ulps of the value; against the bf16 rounding (2^-9 relative) of operands of magnitude ~1 it is small,
+                    // and it costs 27 short FMA chains instead of 27 range reductions.  (mlp_f16x2.cu and mlp_fp32.cu call sincosf
+                    // per octave.)
                     float sn, cs;
                     if constexpr (ABL & 4) { sn = v[c]; cs = zz; }
                     else sincosf(v[c], &sn, &cs);

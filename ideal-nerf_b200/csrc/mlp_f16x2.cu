@@ -27,8 +27,8 @@
 //     values, their per-group partial sums meet through shared memory once per iteration;
 //   * biases enter through one K = 16 MMA per layer half against a tile of fp16 ones with columns (hi, mid, lo) = the folded fp32
 //     bias split in three fp16 (exact to 2^-33);
-//   * gamma(p): one sincosf per coordinate and octave (30 per point; the bf16 kernel's angle doubling is 6e-5 accurate, not enough
-//     here), split into hi / lo like the activations; gamma(viewdir) as a per-ray fp32 bias vector, as in the bf16 kernel.
+//   * gamma(p): one sincosf per coordinate and octave (30 per point; the bf16 kernel's angle doubling is accurate to ~3.1^f * 2^-22
+//     at octave f, not enough here), split into hi / lo like the activations; gamma(viewdir) as a per-ray fp32 bias vector, as in the bf16 kernel.
 // Every mbarrier wait is bounded (~2 s) and traps instead of hanging the GPU.
 //
 // Embedded-row variant (template parameter EMB, FaceNeRF.forward's x (P, 63+27); inference only): mlp_bf16.cu's embedded-row build in
