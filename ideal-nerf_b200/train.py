@@ -70,11 +70,27 @@ def learning_rate(args, global_step):
     return args.lrate * (0.1 ** (global_step / (args.lrate_decay * 1500)))
 
 
+def _check_ranks_agree(key, group=None):
+    """Every rank of `group` passes the key of the CUDA graph it is about to capture; one eager all_gather_object compares them.  Returns
+    when all keys are equal, else raises RuntimeError on every rank (all ranks see the same list), naming each rank's key.  A rank that
+    captured a graph of other shapes or another perturb would still take part in every replay's all-reduce, and the run would go on
+    averaging gradients of different programs without an error."""
+    keys = [None] * dist.get_world_size(group)
+    dist.all_gather_object(keys, key, group=group)
+    if any(k != keys[0] for k in keys):
+        raise RuntimeError("cuda_graph=True: the ranks would capture different graphs; keys by rank: "
+                           + "; ".join(f"{r}: {k}" for r, k in enumerate(keys)))
+
+
 class _AdamStep:
     """What TrainStep and TorsoTrainStep share: the trained parameters as one FlatParams buffer under ONE Adam (torch's fused kernel;
     with cuda_graph=True its capturable form, the learning rate and the step count held in device tensors), the learning-rate schedule,
     the conversion of that Adam's state to and from the reference's per-parameter layout, and the capture / replay bookkeeping of the
-    CUDA-graph mode.  Subclasses name what a captured graph fixes in _FIXED."""
+    CUDA-graph mode.  Subclasses name what a captured graph fixes in _FIXED.
+
+    cuda_graph=True with world > 1 needs an NCCL process group: the all-reduce of the flat gradient is recorded in each rank's graph
+    (a gloo collective cannot be).  The ranks compare their graph keys once, on the capturing call (_check_ranks_agree); replays add no
+    collective and no host work."""
     _FIXED = "batch shapes and perturb"
 
     def __init__(self, params, args, world, group, cuda_graph):
@@ -85,10 +101,12 @@ class _AdamStep:
         name = type(self).__name__
         on_cuda = self.flat.flat.is_cuda
         if self.cuda_graph:
+            backend = dist.get_backend(group) if world > 1 else None
+            if backend not in (None, "nccl"):
+                raise ValueError(f"{name}(cuda_graph=True, world={world}) needs an NCCL process group, got the {backend!r} backend: a "
+                                 f"{backend} collective cannot be recorded in a CUDA graph")
             if not on_cuda:
                 raise RuntimeError(f"{name}(cuda_graph=True) needs CUDA tensors")
-            if world > 1:
-                raise NotImplementedError("cuda_graph=True is built for one process per model replica without a gradient all-reduce")
             dev = self.flat.flat.device
             self._lr_t = torch.tensor(float(args.lrate), device=dev)          # the learning rate and the step count live on the device
             self._gs_t = torch.zeros((), device=dev)
@@ -182,7 +200,10 @@ class _AdamStep:
         """One call of the CUDA-graph mode.  `key` is what a captured graph fixes; make_static() returns the static input buffers,
         fill(st) copies this call's inputs into them, body(st) is the iteration (its tensors are the outputs the replays refresh).  The
         learning-rate schedule runs on the device after body.  The first call runs eagerly (it initialises Adam's state and the kernels'
-        per-device constants), the second call captures, every later call replays."""
+        per-device constants; with world > 1 its eager all-reduce also sets up the NCCL communicator the capture records into), the
+        second call captures, every later call replays.  With world > 1 the capturing call first checks that every rank has the same key
+        (_check_ranks_agree); a key that changes on one rank after the capture raises on that rank only, and the other ranks then wait in
+        their next replay's all-reduce, as in any data-parallel program whose ranks stop taking the same steps."""
         if self._static is None or self._static["key"] != key:
             if self._static is not None:
                 name = type(self).__name__
@@ -203,15 +224,31 @@ class _AdamStep:
             st["out"] = run()                                        # eager: lazy initialisations happen here
         else:
             if st["graph"] is None:
+                if self.world > 1:
+                    _check_ranks_agree(key, self.group)
                 torch.cuda.synchronize()
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    st["out"] = run()
-                st["graph"] = g
+                st["graph"], st["out"], st["capture_mode"] = self._capture(run)
             st["graph"].replay()
         st["calls"] += 1
         self.global_step += 1
         return st["out"]
+
+    def _capture(self, run):
+        """(graph, outputs, capture_error_mode) of run() captured.  With world > 1 a capture that fails in torch's default "global" mode
+        is tried once more in "thread_local" mode, where CUDA calls of other threads (the process group's watchdog querying its events)
+        cannot invalidate it."""
+        def capture(mode):
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, capture_error_mode=mode):
+                out = run()
+            return g, out, mode
+
+        try:
+            return capture("global")
+        except RuntimeError:
+            if self.world == 1:
+                raise
+            return capture("thread_local")                          # a second failure is raised chained to the first
 
 
 class TrainStep(_AdamStep):
@@ -219,7 +256,18 @@ class TrainStep(_AdamStep):
 
     The optimiser is ONE Adam over the flat buffer; `optimizer_state_dict()` / `load_optimizer_state_dict()` convert to and from the
     reference's per-parameter Adam state (params = list(network.parameters()) + [latent_codes], audio_exp_nerf.py:487-493) so the
-    'optimizer' entry of head.tar moves both ways; `save()` / `load()` write and resume the reference's checkpoint (:516-525, :584-591)."""
+    'optimizer' entry of head.tar moves both ways; `save()` / `load()` write and resume the reference's checkpoint (:516-525, :584-591).
+
+    world > 1: one process per GPU, each stepping on its band of the batch (frame.band(N_rand, rank, world)); FlatParams.gather_grads
+    averages the flat gradient over the ranks with one all-reduce (the mean of the ranks' gradients, whatever their band sizes), so
+    identical replicas stay identical.  The returned losses are the rank's own.
+
+    cuda_graph=True: the first call runs eagerly, the second captures the whole iteration, later calls replay it; a graph fixes the
+    batch shapes, the aud_window / aud_feature choice and perturb (a change raises).  With world > 1 (NCCL only) each rank captures its
+    own graph with the all-reduce recorded in it, after the ranks have checked once that their keys agree -- so in this mode every rank
+    takes a band of the same shape.  For the ranks to draw complementary bands of one batch (DeviceHeadDataset.sample(i, rank, world)),
+    seed the in-kernel Philox stream the same way on every rank (ops.seed_rng(seed) on each rank's device) and make the same sequence of
+    stochastic calls."""
     _FIXED = "batch shapes, the aud_window / aud_feature choice and perturb"
 
     def __init__(self, network, latent_codes, args, world=1, group=None, cuda_graph=False):
@@ -326,8 +374,10 @@ class TorsoTrainStep(_AdamStep):
       schedule lines were not re-read: that they are the same is not verified.
     * cuda_graph=True works as in TrainStep: the first call runs eagerly, the second captures, later calls replay.  The inputs are copied
       into static buffers (pose, aud_feature, expr and latent_code included; torso_signal is computed inside the graph), the learning
-      rate and Adam's step count are device tensors, batch shapes and perturb are fixed per step (a change raises), and world == 1.
-      The step owns the head pair's packed blobs the graph reads; when the nets' caches were dropped (train() / eval(),
+      rate and Adam's step count are device tensors, batch shapes and perturb are fixed per step (a change raises).  With world > 1
+      (NCCL only) the gradient all-reduce is recorded in each rank's graph and the ranks' keys must agree at the capture, as in
+      TrainStep; seed the Philox stream alike on every rank for DeviceTorsoDataset.sample(i, rank, world) to give complementary bands.
+      Each rank's step owns the head pair's packed blobs its graph reads; when the nets' caches were dropped (train() / eval(),
       invalidate_packed(), checkpoint.load_head_into_torso) the next call re-packs the current head weights into that same memory.
       load() after the capture raises before it changes anything.
 
