@@ -101,7 +101,10 @@ __device__ __forceinline__ float2 ldg_stream2(const float* p) {
 // NULL (the fine pass of an inference render only needs its last entry); last_weight: NULL or (n).  z_c0 / w_c0 return the lane's two
 // depths / weights of chunk 0 (S = 64: the whole ray).  Returns a bit mask of the non-finite outputs this lane wrote
 // (1 rgb, 2 disp, 4 acc, 8 depth, 16 last_weight).
-template <int C>
+// SIG = 1 or 4: the sigma-only form (the coarse pass of a render that discards its colour).  Only the densities are read, sample i's at
+// ((const float*)raw)[i * SIG + SIG - 1] -- a density-only buffer (1) or the sigma lane of a full raw (4) -- and rgb, rgb_fg, bc_rgb
+// are not touched; weights, depth, disp, acc and last_weight are the bits of the full form (reduce8 sums each quantity on its own).
+template <int C, int SIG = 0>
 __device__ __forceinline__ uint32_t composite2_ray(
     const float4* __restrict__ raw, const float* __restrict__ z, const float* __restrict__ rays_d, int d_stride,
     const float* __restrict__ bc_rgb, const float* __restrict__ noise, int ray, int s, int white_bkgd,
@@ -116,7 +119,14 @@ __device__ __forceinline__ uint32_t composite2_ray(
         const int i = c * 64 + 2 * lane;                       // s is even: i < s  <=>  i + 1 < s
         const bool ok = i < s;
         if (ok) {
-            rv[c] = ldg_stream8(raw + base + i);
+            if constexpr (SIG == 0) {
+                rv[c] = ldg_stream8(raw + base + i);
+            } else {
+                const float* sg = reinterpret_cast<const float*>(raw) + (base + i) * SIG + (SIG - 1);
+                const float2 s2 = SIG == 1 ? ldg_stream2(sg) : make_float2(ldg_stream(sg), ldg_stream(sg + SIG));
+                rv[c].a = make_float4(0.f, 0.f, 0.f, s2.x);
+                rv[c].b = make_float4(0.f, 0.f, 0.f, s2.y);
+            }
             zv[c] = ldg_stream2(z + base + i);
             nv[c] = noise ? ldg_stream2(noise + base + i) : make_float2(0.f, 0.f);
         } else {
@@ -127,7 +137,7 @@ __device__ __forceinline__ uint32_t composite2_ray(
     const float* dptr = rays_d + (size_t)ray * d_stride;
     const float dx = dptr[0], dy = dptr[1], dz = dptr[2];
     const float norm = sqrtf(dx * dx + dy * dy + dz * dz);
-    const float bcr = bc_rgb[ray * 3], bcg = bc_rgb[ray * 3 + 1], bcb = bc_rgb[ray * 3 + 2];
+    const float bcr = SIG ? 0.f : bc_rgb[ray * 3], bcg = SIG ? 0.f : bc_rgb[ray * 3 + 1], bcb = SIG ? 0.f : bc_rgb[ray * 3 + 2];
 
     float carry = 1.0f;
     uint32_t bad = 0;
@@ -153,15 +163,17 @@ __device__ __forceinline__ uint32_t composite2_ray(
         if (valid && weights) *reinterpret_cast<float2*>(weights + base + i) = make_float2(wa, wb);
         if (last_b && last_weight) { last_weight[ray] = wb; if (!isfinite(wb)) bad |= 16u; }
         if (c == 0) { z_c0 = zv[0]; w_c0 = make_float2(wa, wb); }
-        const float ar = sigmoidf_(rv[c].a.x), ag = sigmoidf_(rv[c].a.y), ab = sigmoidf_(rv[c].a.z);
-        const float br = sigmoidf_(rv[c].b.x), bg = sigmoidf_(rv[c].b.y), bb = sigmoidf_(rv[c].b.z);
-        const float fr = wa * ar + (last_b ? 0.f : wb * br);   // foreground sums exclude the background sample
-        const float fg = wa * ag + (last_b ? 0.f : wb * bg);
-        const float fb = wa * ab + (last_b ? 0.f : wb * bb);
-        v[5] += fr; v[6] += fg; v[7] += fb;
-        v[0] += last_b ? fr + wb * bcr : fr;
-        v[1] += last_b ? fg + wb * bcg : fg;
-        v[2] += last_b ? fb + wb * bcb : fb;
+        if constexpr (SIG == 0) {
+            const float ar = sigmoidf_(rv[c].a.x), ag = sigmoidf_(rv[c].a.y), ab = sigmoidf_(rv[c].a.z);
+            const float br = sigmoidf_(rv[c].b.x), bg = sigmoidf_(rv[c].b.y), bb = sigmoidf_(rv[c].b.z);
+            const float fr = wa * ar + (last_b ? 0.f : wb * br);   // foreground sums exclude the background sample
+            const float fg = wa * ag + (last_b ? 0.f : wb * bg);
+            const float fb = wa * ab + (last_b ? 0.f : wb * bb);
+            v[5] += fr; v[6] += fg; v[7] += fb;
+            v[0] += last_b ? fr + wb * bcr : fr;
+            v[1] += last_b ? fg + wb * bcg : fg;
+            v[2] += last_b ? fb + wb * bcb : fb;
+        }
         v[3] += wa * zv[c].x + wb * zv[c].y;
         v[4] += wa + wb;
     }
@@ -171,9 +183,11 @@ __device__ __forceinline__ uint32_t composite2_ray(
     const int q = lane >> 2;
     if ((lane & 3) == 0) {
         if (q < 3) {
-            const float v_ = white_bkgd ? tot + (1.0f - acc_t) : tot;
-            rgb[ray * 3 + q] = v_;
-            if (!isfinite(v_)) bad |= 1u;
+            if constexpr (SIG == 0) {
+                const float v_ = white_bkgd ? tot + (1.0f - acc_t) : tot;
+                rgb[ray * 3 + q] = v_;
+                if (!isfinite(v_)) bad |= 1u;
+            }
         } else if (q == 3) {
             const float dp = __fdiv_rn(1.0f, fmaxf(1e-10f, __fdiv_rn(depth_t, acc_t)));
             depth[ray] = depth_t;
@@ -183,7 +197,7 @@ __device__ __forceinline__ uint32_t composite2_ray(
         } else if (q == 4) {
             acc[ray] = acc_t;
             if (!isfinite(acc_t)) bad |= 4u;
-        } else if (rgb_fg) rgb_fg[ray * 3 + (q - 5)] = tot;
+        } else if (!SIG && rgb_fg) rgb_fg[ray * 3 + (q - 5)] = tot;
     }
     return bad;
 }

@@ -98,18 +98,35 @@ extern "C" int inerf_mlp_pack(int mode, const InerfNetDims* dims, const float* c
     }
 }
 
-extern "C" int inerf_mlp_fwd(int mode, const InerfNetDims* dims, const float* const* params_host, const void* packed,
-                             const float* cond, const float* rays, int ray_stride, const float* z, int n, int s,
-                             float* raw, void* stream) {
-    MlpArgs a{};
+// The argument checks and MlpArgs of a forward over the points of rays / z (inerf_mlp_fwd, mlp_fwd_density); INERF_OK with a.P == 0: nothing to do
+static int fwd_args(MlpArgs& a, const InerfNetDims* dims, const float* const* params_host, const void* packed, const float* cond,
+                    const float* rays, int ray_stride, const float* z, int n, int s, float* out) {
     int rc = fill_args(a, dims, params_host, cond);
     if (rc) return rc;
     if (n < 0 || s <= 0 || ray_stride < 11) return fail(INERF_E_SHAPE, "inerf_mlp_fwd: bad n/s/ray_stride (rays need the viewdir columns)");
     if (n == 0) return INERF_OK;
-    if (!rays || !z || !raw) return fail(INERF_E_ARG, "inerf_mlp_fwd: NULL pointer");
-    if ((uintptr_t)raw & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: raw must be 16-byte aligned");
+    if (!rays || !z || !out) return fail(INERF_E_ARG, "inerf_mlp_fwd: NULL pointer");
+    if ((uintptr_t)out & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: raw must be 16-byte aligned");
     a.rays = rays; a.ray_stride = ray_stride; a.z = z; a.s = s;
-    a.P = (long long)n * s; a.out = raw; a.packed = packed;
+    a.P = (long long)n * s; a.out = out; a.packed = packed;
+    return INERF_OK;
+}
+
+int inerf::mlp_fwd_density(const InerfNetDims* dims, const float* const* params_host, const void* packed, const float* cond, const float* rays,
+                           int ray_stride, const float* z, int n, int s, float* sigma, cudaStream_t st) {
+    MlpArgs a{};
+    int rc = fwd_args(a, dims, params_host, packed, cond, rays, ray_stride, z, n, s, sigma);
+    if (rc || a.P == 0) return rc;
+    if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd: bf16 mode needs packed weights");
+    return mlp_bf16_launch(a, false, st, true);
+}
+
+extern "C" int inerf_mlp_fwd(int mode, const InerfNetDims* dims, const float* const* params_host, const void* packed,
+                             const float* cond, const float* rays, int ray_stride, const float* z, int n, int s,
+                             float* raw, void* stream) {
+    MlpArgs a{};
+    int rc = fwd_args(a, dims, params_host, packed, cond, rays, ray_stride, z, n, s, raw);
+    if (rc || a.P == 0) return rc;
     if (mode == INERF_MLP_FP32) return mlp_fp32_launch(a, false, as_stream(stream));
     if (mode == INERF_MLP_BF16) {
         if (!packed) return fail(INERF_E_ARG, "inerf_mlp_fwd: bf16 mode needs packed weights");

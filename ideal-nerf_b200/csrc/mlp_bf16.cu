@@ -341,6 +341,34 @@ __device__ __forceinline__ void epi_plain_layer(Bars* bars, uint32_t par, uint32
     ph[2] += p4 - p3; ph[3] += p5 - p4;
 }
 
+// Epilogue of L7 in the density-only build (DENS): the alpha head alone, in epi_convert<1>'s FMA order.  Nothing reads h7 (V0 does not
+// run), so it is neither converted nor stored and no C1 wait is needed; each half still arrives on its event once its TMEM loads are
+// done, because the next iteration's L0 overwrites those accumulators.
+template <bool PAIR>
+__device__ __forceinline__ void epi_alpha_layer(Bars* bars, uint32_t par, uint32_t t_lane, const float* __restrict__ aw, int lane, float& alpha) {
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        mbar_wait(&bars->cbar[h == 0 ? 0 : 2], par);
+        __syncwarp();
+        tc_fence_after();
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+            uint32_t r[32];
+            tmem_ld32(t_lane + h * 128 + c * 32, r);
+            tmem_wait_ld();
+#pragma unroll
+            for (int j = 0; j < 32; j += 4) {
+                const float4 w = *reinterpret_cast<const float4*>(aw + h * 128 + c * 32 + j);
+                alpha = fmaf(relu_nan(__uint_as_float(r[j])), w.x, alpha); alpha = fmaf(relu_nan(__uint_as_float(r[j + 1])), w.y, alpha);
+                alpha = fmaf(relu_nan(__uint_as_float(r[j + 2])), w.z, alpha); alpha = fmaf(relu_nan(__uint_as_float(r[j + 3])), w.w, alpha);
+            }
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) { if constexpr (PAIR) mbar_arrive_remote(&bars->ebar[h], 0); else mbar_arrive(&bars->ebar[h]); }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
@@ -363,11 +391,17 @@ __device__ int g_save_abl;      // profiling builds: switch parts of the activat
 // bytes.  Schedule, layouts, packed blob and epilogue are the single-CTA kernel's: a pair iteration is two 256-point chunks, CTA r takes
 // chunk 2 it + r.  Cross-CTA protocol: commits are multicast to both CTAs' barriers; the peer's epilogue / positional-encoding warps
 // arrive remotely on the LEADER's event barriers; the peer's (otherwise idle) warp 1 relays "my half of the stage has landed".
-template <bool TRACE, int ABL = 0, bool SAVE = false, bool PAIR = false, bool EMB = false>
+//
+// DENS = true (density-only build, inference only): the coarse pass of a render that discards the coarse colour needs sigma alone, which
+// depends on L0-L7 and the alpha head.  The issuer runs L0-L7 and starts the next iteration (L0 waits E0 / E1 of L7), producer and relay
+// stream the stages of L0-L7 -- the first n_steps of the same schedule and blob -- the PE warps skip the per-ray view bias, and the output
+// is one float per point, alpha + alpha_linear.bias: the .w of the full build, bit for bit.
+template <bool TRACE, int ABL = 0, bool SAVE = false, bool PAIR = false, bool EMB = false, bool DENS = false>
 __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, int n_steps, int n_rays, float* __restrict__ trace) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
     static_assert(!(PAIR && (TRACE || ABL != 0)), "the pair build has no trace / ablation variants");
     static_assert(!(EMB && (TRACE || ABL != 0)), "the embedded-row build has no trace / ablation variants");
+    static_assert(!(DENS && (TRACE || ABL != 0 || SAVE || EMB)), "the density-only build is an inference build of the fused entry");
     // Dynamic shared memory is the only shared allocation of this kernel, so it starts at offset 0 of the CTA's
     // window: 1024-byte aligned as the 128B-swizzle atoms need.  (No pointer re-alignment arithmetic here: it would
     // make the compiler lose the shared address space and emit generic LD/ST for every epilogue access.)
@@ -492,9 +526,11 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, TRACE, ABL, PAIR, EMB>(c);
                 if (seg == 0) issue_layer<5, TRACE, ABL, PAIR, EMB>(c);
             }
-            issue_layer<8, TRACE, ABL, PAIR, EMB>(c);
+            if constexpr (!DENS) {
+                issue_layer<8, TRACE, ABL, PAIR, EMB>(c);
 #pragma unroll 1
-            for (int r = 0; r < 2; ++r) issue_layer<9, TRACE, ABL, PAIR, EMB>(c);
+                for (int r = 0; r < 2; ++r) issue_layer<9, TRACE, ABL, PAIR, EMB>(c);
+            }
         }
 #ifdef INERF_PHASE_TIMERS
         if (lane == 0) {
@@ -534,7 +570,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
             if (!in_range) p = a.P - 1;
             const int ray_local = EMB ? 0 : (int)(p / a.s - min(p0, a.P - 1) / a.s);      // embedded rows: no per-ray view bias
             float alpha = 0.f, rgb0 = 0.f, rgb1 = 0.f, rgb2 = 0.f;
-            for (int l = 0; l < 11; ++l, ++layer_ctr) {
+            for (int l = 0; l < (DENS ? 8 : 11); ++l, ++layer_ctr) {
                 const LayerInfo li = layer_info(l);
                 const int NH = li.N >> 1;
                 const uint32_t par = layer_ctr & 1;
@@ -545,6 +581,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         if (l >= 1) { ph_wait[0] += phl[0]; ph_dur[0] += phl[1]; ph_wait[1] += phl[2]; ph_dur[1] += phl[3]; ph_c1 += phl[4]; }
                         continue;
                     }
+                    if constexpr (DENS) { epi_alpha_layer<PAIR>(bars, par, t_lane, s_aw, lane, alpha); continue; }
                     if (l == 9 || (EMB && l == 8)) { epi_plain_layer<64, PAIR>(bars, par, t_lane, act_row_u32, soff, lane, phl); continue; }
                 }
                 if (!EMB && l == 8) wait_or_report<TRACE>(&bars->dirb_ready, iter_ctr & 1, 301, l, (int)iter_ctr);
@@ -659,7 +696,9 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                     if (lane == 0) mbar_arrive(&bars->dirb_free);
                 }
             }
-            if (in_range) {
+            if (DENS && in_range) {
+                a.out[p] = alpha + s_sb[0];
+            } else if (in_range) {
                 float4 o;
                 o.x = rgb0 + s_sb[1];
                 o.y = rgb1 + s_sb[2];
@@ -764,7 +803,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
         // ================= positional encoding + per-ray view bias producers ==================
         const int t = tid - 12 * 32;                 // 0..127: row of both slots, and output feature of the view bias
         float wdir[27];                              // views_linears.0.weight[t, 256:283], resident in registers
-        {
+        if constexpr (!DENS) {
             const float* wrow = a.w[P_VIEWS_W] + (size_t)t * (283 + a.dim_expr) + 256;
 #pragma unroll
             for (int j = 0; j < 27; ++j) wdir[j] = wrow[j];
@@ -837,8 +876,8 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                             make_uint4(pk[sl][4 * q], pk[sl][4 * q + 1], pk[sl][4 * q + 2], pk[sl][4 * q + 3]);
                 }
             }
-            // ---- per-ray view bias: lane q < 2*RMAX encodes ray q, the warp shares it by shuffle ----
-            {
+            // ---- per-ray view bias: lane q < 2*RMAX encodes ray q, the warp shares it by shuffle (no V0 in the density-only build) ----
+            if constexpr (!DENS) {
                 float enc[27];
                 const int q = lane;
                 if (q < 2 * RMAX) {
@@ -940,9 +979,9 @@ int mlp_bf16_hang_info(int32_t* out8) {
 }
 
 // the production builds: no trace, no ablation
-template <bool SAVE, bool PAIR, bool EMB>
+template <bool SAVE, bool PAIR, bool EMB, bool DENS = false>
 static int launch(const MlpArgs& a, int n_steps, int n_rays, cudaStream_t st, const char* what) {
-    return launch_tc(mlp_bf16_kernel<false, 0, SAVE, PAIR, EMB>, PAIR, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, what, a, n_steps, n_rays,
+    return launch_tc(mlp_bf16_kernel<false, 0, SAVE, PAIR, EMB, DENS>, PAIR, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, what, a, n_steps, n_rays,
                      (float*)nullptr);
 }
 
@@ -964,20 +1003,28 @@ static int launch_embedded(const MlpArgs& a, cudaStream_t st) {
                       : launch<false, false, true>(a, S.n_stages, 0, st, "inerf_mlp_fwd_embedded[bf16]");
 }
 
-int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
+int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st, bool density) {
     if (embedded) return launch_embedded(a, st);
     if (a.s < 43) return fail(INERF_E_UNSUPPORTED, "bf16 mode needs at least 43 samples per ray (a 128-row slot may touch at most 4 rays)");
     if ((uintptr_t)a.packed & 15) return fail(INERF_E_ALIGN, "inerf_mlp_fwd: packed weights must be 16-byte aligned");
     static thread_local int configured_dev = -1;
     // the step table does not depend on the conditioning dims; a function-local static is initialised once, thread-safely
     static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, false, 1); }();
+    static const int n_steps_dens = tc_stages_before(S, 8);      // the stages of L0-L7
     int rc = setup_once(configured_dev,
                         {(const void*)mlp_bf16_kernel<false>, (const void*)mlp_bf16_kernel<true>, (const void*)mlp_bf16_kernel<false, 0, true>,
-                         (const void*)mlp_bf16_kernel<false, 0, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, true>},
+                         (const void*)mlp_bf16_kernel<false, 0, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, true>,
+                         (const void*)mlp_bf16_kernel<false, 0, false, false, false, true>,
+                         (const void*)mlp_bf16_kernel<false, 0, false, true, false, true>},
                         SMEM_ALLOC, "mlp_bf16", [] { return cudaMemcpyToSymbol(c_steps, S.st, sizeof(TcStage) * MAX_STEPS); });
     if (rc) return rc;
     const int n_rays = (int)(a.P / a.s);
     const bool use_pair = mlp_pair_enabled() && !a.trace;
+    if (density) {
+        if (a.trace || a.save_img) return fail(INERF_E_ARG, "mlp_bf16: the density-only build has no trace / saving form");
+        return use_pair ? launch<false, true, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16 pair, density only]")
+                        : launch<false, false, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16, density only]");
+    }
     if (a.trace) {
         if (!g_hang_host) {
             int* dptr = nullptr;

@@ -90,8 +90,13 @@ int launch_tc(void (*kernel)(KArgs...), bool pair, long long n_iter, int nthread
 }
 
 int mlp_fp32_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
-// embedded: rows of a.x (P, 90) with an INERF_MLP_BF16_EMB blob; otherwise points of rays/z.  a.save_img != NULL: the activation-saving build
-int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
+// embedded: rows of a.x (P, 90) with an INERF_MLP_BF16_EMB blob; otherwise points of rays/z.  a.save_img != NULL: the activation-saving build.
+// density: the density-only inference build (points of rays/z): a.out receives sigma alone, one float per point
+int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st, bool density = false);
+// inerf_mlp_fwd in bf16 mode with the density-only build: sigma (n * s floats, 16-byte aligned) instead of raw (the coarse pass of
+// inerf_render_rays_fused when no coarse colour is asked for)
+int mlp_fwd_density(const InerfNetDims* dims, const float* const* params_host, const void* packed, const float* cond, const float* rays,
+                    int ray_stride, const float* z, int n, int s, float* sigma, cudaStream_t st);
 int mlp_fp32_bwd_launch(const InerfNetDims* dims, const float* const* params_host, float* const* grads_host,
                         const float* aud, const float* expr, const float* latent, const float* acts, float* deltas,
                         const float* d_raw, long long P, float* d_cond, void* dw_args_dev, cudaStream_t st);

@@ -78,6 +78,14 @@ inline TcSchedule build_tc_schedule(const InerfNetDims* d, bool emb, int parts) 
     return S;
 }
 
+// Number of stages of layers [0, layer): a prefix of the schedule, which runs layer by layer (the density-only build of mlp_bf16.cu
+// streams the stages of L0-L7 of the unchanged blob)
+inline int tc_stages_before(const TcSchedule& S, int layer) {
+    int n = 0;
+    while (n < S.n_stages && S.st[n].layer < layer) ++n;
+    return n;
+}
+
 // ---- packing ------------------------------------------------------------------------------------------------------------------
 // The table travels as a kernel parameter (by value): nothing is copied from pageable host memory, so the launch can be captured in a
 // CUDA graph (train.TrainStep re-packs the weights after every optimiser step).  80 rows next to the 26 weight pointers fit the 4 KB

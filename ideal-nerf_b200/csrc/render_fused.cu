@@ -12,11 +12,15 @@
 //   * composite_final_kernel = raw2outputs of the fine pass writing the maps and last_weight only (the (n, 192) weights tensor is
 //                      optional: 768 B/ray less), OR-ing the NaN / Inf flags and bumping the RNG offset (was: composite_fwd +
 //                      rng_advance [+ flag_nonfinite]).
+// Without rgb0 (args->rgb0 == NULL: a frame or video render, which keeps only the fine colour) the coarse pass needs sigma alone: in bf16
+// mode the coarse net runs its density-only build (L0-L7 and the alpha head, one float per point), in the other modes the full net, and
+// the coarse compositor reads sigma only (composite2_ray's SIG form): the same weights, disp0, acc0, z_std and merged depths, bit for bit.
 // A rank that renders a 25 k-ray band of a frame (8 GPUs) spends as long in these small launches as in their work, so the count matters
 // there.  Every fused kernel runs the same device functions as its stand-alone twin: bit-identical outputs (tests/test_gpu_parity.py).
 #include "common.cuh"
 #include "composite_parts.cuh"
 #include "fold_cond.cuh"
+#include "mlp_common.cuh"
 #include "philox.cuh"
 #include "rays_parts.cuh"
 #include "sample_parts.cuh"
@@ -100,15 +104,17 @@ struct CompArgs {
     int* flags;
 };
 
-// coarse pass: raw2outputs (S = 64) + sample_pdf / merge / std (128 in-kernel draws); one warp per ray
+// coarse pass: raw2outputs (S = 64) + sample_pdf / merge / std (128 in-kernel draws); one warp per ray.  SIG: composite2_ray's
+// sigma-only form (1: density-only raw, 4: the sigma lane of a full raw) or 0, the full form with rgb0
+template <int SIG>
 __global__ void __launch_bounds__(256) composite_sample_64_128_kernel(const CompArgs a) {
     __shared__ __align__(16) float smem[8 * IMP64_WARP_FLOATS];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int ray = blockIdx.x * 8 + wib;
     if (ray >= a.n) return;
     float2 z2, w2;
-    const uint32_t bad = composite2_ray<1>(a.raw, a.z, a.rays + 3, a.ray_stride, a.bc_rgb, nullptr, ray, 64, a.white_bkgd, a.rgb, a.disp,
-                                           a.acc, a.depth, a.weights, a.rgb_fg, a.last_weight, lane, z2, w2);
+    const uint32_t bad = composite2_ray<1, SIG>(a.raw, a.z, a.rays + 3, a.ray_stride, a.bc_rgb, nullptr, ray, 64, a.white_bkgd, a.rgb, a.disp,
+                                                a.acc, a.depth, a.weights, a.rgb_fg, a.last_weight, lane, z2, w2);
     const float sd = importance_rng_64_128_ray(z2, w2, ray, lane, smem + wib * IMP64_WARP_FLOATS, a.rng_state, INERF_RNG_STREAM_PDF, nullptr,
                                                a.z_merged, a.z_std);
     if (a.flags) {
@@ -116,6 +122,27 @@ __global__ void __launch_bounds__(256) composite_sample_64_128_kernel(const Comp
         if (lane == 0 && !isfinite(sd)) f |= INERF_NF_Z_STD;
         if (f) atomicOr(a.flags, (int)f);
     }
+}
+
+// coarse pass of the general path without rgb0: raw2outputs of the densities alone (composite2_ray's SIG form) writing disp0, acc0,
+// depth0 and the weights that inerf_importance_sample reads -- the bits inerf_composite_fwd writes there
+template <int C, int SIG>
+__global__ void __launch_bounds__(256) composite_sigma_kernel(const CompArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int ray = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (ray >= a.n) return;
+    float2 z2, w2;
+    composite2_ray<C, SIG>(a.raw, a.z, a.rays + 3, a.ray_stride, nullptr, nullptr, ray, a.s, a.white_bkgd, nullptr, a.disp, a.acc, a.depth,
+                           a.weights, nullptr, nullptr, lane, z2, w2);
+}
+
+template <int SIG>
+void launch_composite_sigma(const CompArgs& a, cudaStream_t st) {
+    const int c2 = (a.s + 63) / 64;      // n_samples <= 254
+    if (c2 <= 1) composite_sigma_kernel<1, SIG><<<(a.n + 7) / 8, 256, 0, st>>>(a);
+    else if (c2 == 2) composite_sigma_kernel<2, SIG><<<(a.n + 7) / 8, 256, 0, st>>>(a);
+    else if (c2 == 3) composite_sigma_kernel<3, SIG><<<(a.n + 7) / 8, 256, 0, st>>>(a);
+    else composite_sigma_kernel<4, SIG><<<(a.n + 7) / 8, 256, 0, st>>>(a);
 }
 
 // fine pass: raw2outputs writing maps + last_weight (weights optional), the NaN / Inf flags, the RNG bump
@@ -160,13 +187,14 @@ int plan(const InerfRenderArgs* a, Workspace& w) {
     if (rc) return rc;
     const size_t n = (size_t)a->n, s1 = (size_t)a->n_samples, st = s1 + (size_t)a->n_importance;
     const bool fused_cs = a->perturb && a->n_samples == 64 && a->n_importance == 128;
+    const bool dens = !a->rgb0 && a->mode == INERF_MLP_BF16;      // the coarse net's density-only build: one float per point
     size_t o = 0;
     auto take = [&o](size_t bytes) { const size_t at = o; o += up256(bytes); return at; };
     w.rays = take(a->gen_rays ? n * 11 * 4 : 0);
     w.cond_c = take(cf * 4);
     w.cond_f = take(cf * 4);
     w.z_c = take(n * s1 * 4);
-    w.raw_c = take(n * s1 * 16);
+    w.raw_c = take(n * s1 * (dens ? 4 : 16));
     w.w_c = take(fused_cs ? 0 : n * s1 * 4);
     w.z_s = take(a->perturb ? 0 : n * (size_t)a->n_importance * 4);
     w.z_m = take(a->z_vals ? 0 : n * st * 4);
@@ -215,13 +243,14 @@ int render_rays_fused(const InerfRenderArgs* a, void* stream, cudaEvent_t* ev) {
     if (a->n == 0) return INERF_OK;
     if (!a->workspace || a->workspace_bytes < w.total) return fail(INERF_E_ARG, "inerf_render_rays_fused: workspace missing or smaller than inerf_render_workspace_bytes");
     if ((uintptr_t)a->workspace & 255) return fail(INERF_E_ALIGN, "inerf_render_rays_fused: workspace must be 256-byte aligned");
-    if (!a->bc_rgb || !a->t_vals || !a->rgb_map || !a->disp_map || !a->acc_map || !a->depth_map || !a->last_weight || !a->rgb0 || !a->disp0 ||
-        !a->acc0 || !a->z_std)
+    if (!a->bc_rgb || !a->t_vals || !a->rgb_map || !a->disp_map || !a->acc_map || !a->depth_map || !a->last_weight || !a->disp0 || !a->acc0 ||
+        !a->z_std)
         return fail(INERF_E_ARG, "inerf_render_rays_fused: NULL pointer");
     if (a->perturb ? !a->rng_state : !a->u_vals) return fail(INERF_E_ARG, "inerf_render_rays_fused: rng_state (perturb) / u_vals (deterministic) missing");
     const bool with_fg = a->rgb_map_fg != nullptr;
     if (with_fg != (a->rgb_map_fg0 != nullptr) || with_fg != (a->last_weight0 != nullptr))
         return fail(INERF_E_ARG, "inerf_render_rays_fused: rgb_map_fg, rgb_map_fg0 and last_weight0 are given together or not at all");
+    if (with_fg && !a->rgb0) return fail(INERF_E_ARG, "inerf_render_rays_fused: the torso extras need rgb0 (rgb_map_fg0 is a coarse colour)");
     if (a->gen_rays) {
         if (a->H <= 0 || a->W <= 0 || (int64_t)a->H * a->W > (1 << 30) || a->c2w_row_stride < 4 || a->first < 0 ||
             (int64_t)a->first + a->n > (int64_t)a->H * a->W)
@@ -274,7 +303,11 @@ int render_rays_fused(const InerfRenderArgs* a, void* stream, cudaEvent_t* ev) {
 
     mark(1);
     // ---- 2. coarse FaceNeRF ------------------------------------------------------------------------------------------------------
-    rc = inerf_mlp_fwd(a->mode, &a->coarse.dims, a->coarse.params_host, a->coarse.packed, F(w.cond_c), rays, stride, z_c, n, s1, F(w.raw_c), stream);
+    // without rgb0 the compositor reads sigma alone: the density-only buffer (bf16) or the sigma lane of the full raw
+    const int sig = a->rgb0 ? 0 : (a->mode == INERF_MLP_BF16 ? 1 : 4);
+    rc = sig == 1 ? mlp_fwd_density(&a->coarse.dims, a->coarse.params_host, a->coarse.packed, F(w.cond_c), rays, stride, z_c, n, s1, F(w.raw_c), st)
+                  : inerf_mlp_fwd(a->mode, &a->coarse.dims, a->coarse.params_host, a->coarse.packed, F(w.cond_c), rays, stride, z_c, n, s1, F(w.raw_c),
+                                  stream);
     if (rc) return rc;
 
     mark(2);
@@ -286,13 +319,21 @@ int render_rays_fused(const InerfRenderArgs* a, void* stream, cudaEvent_t* ev) {
     ca.weights = nullptr; ca.rgb_fg = a->rgb_map_fg0; ca.last_weight = a->last_weight0;
     ca.rng_state = rng; ca.z_merged = z_m; ca.z_std = a->z_std; ca.flags = a->nonfinite;
     if (a->perturb && s1 == 64 && ni == 128) {
-        composite_sample_64_128_kernel<<<(n + 7) / 8, 256, 0, st>>>(ca);
+        if (sig == 0) composite_sample_64_128_kernel<0><<<(n + 7) / 8, 256, 0, st>>>(ca);
+        else if (sig == 1) composite_sample_64_128_kernel<1><<<(n + 7) / 8, 256, 0, st>>>(ca);
+        else composite_sample_64_128_kernel<4><<<(n + 7) / 8, 256, 0, st>>>(ca);
         rc = check_launch("inerf_render_rays_fused[coarse compositor + sampler]");
         if (rc) return rc;
     } else {
         float* w_c = F(w.w_c);
-        rc = inerf_composite_fwd(F(w.raw_c), z_c, rays + 3, stride, a->bc_rgb, nullptr, n, s1, a->white_bkgd, a->rgb0, a->disp0, a->acc0,
-                                 F(w.depth0), w_c, a->rgb_map_fg0, stream);
+        if (sig == 0) {
+            rc = inerf_composite_fwd(F(w.raw_c), z_c, rays + 3, stride, a->bc_rgb, nullptr, n, s1, a->white_bkgd, a->rgb0, a->disp0, a->acc0,
+                                     F(w.depth0), w_c, a->rgb_map_fg0, stream);
+        } else {
+            ca.weights = w_c;
+            if (sig == 1) launch_composite_sigma<1>(ca, st); else launch_composite_sigma<4>(ca, st);
+            rc = check_launch("inerf_render_rays_fused[coarse compositor, sigma only]");
+        }
         if (rc) return rc;
         if (a->last_weight0) {
             cudaError_t e = cudaMemcpy2DAsync(a->last_weight0, 4, w_c + (s1 - 1), (size_t)s1 * 4, 4, (size_t)n, cudaMemcpyDeviceToDevice, st);
@@ -337,7 +378,7 @@ int render_rays_fused(const InerfRenderArgs* a, void* stream, cudaEvent_t* ev) {
     if (a->nonfinite && !(a->perturb && s1 == 64 && ni == 128)) {      // the coarse maps of the stand-alone path
         // inerf_flag_nonfinite sets bit i for tensor i: three empty entries put the maps on INERF_NF_RGB0 / _DISP0 / _ACC0
         const float* xs6[6] = {nullptr, nullptr, nullptr, a->rgb0, a->disp0, a->acc0};
-        const int64_t ns6[6] = {0, 0, 0, (int64_t)n * 3, n, n};
+        const int64_t ns6[6] = {0, 0, 0, a->rgb0 ? (int64_t)n * 3 : 0, n, n};
         rc = inerf_flag_nonfinite(xs6, ns6, 6, a->nonfinite, stream);
         if (rc) return rc;
     }

@@ -612,11 +612,15 @@ def _render_net(net, aud, expr, latent, keep):
 
 def render_rays_fused(net_coarse, net_fine, cond_coarse, cond_fine, bc_rgb, n_samples, n_importance, perturb, rays=None, gen=None,
                       lindisp=False, white_bkgd=False, with_fg=False, want_weights=False, want_z=False, check_numerics=False, state=None,
-                      stage_ms=None):
+                      stage_ms=None, coarse_rgb=True):
     """Network.render_rays under no_grad as ONE C call (inerf_render_rays_fused): five kernel launches in the reference's
     configuration (set-up, coarse FaceNeRF, compositor + sampler, fine FaceNeRF, final compositor).  rays: packed (n, 11), or
     gen = dict(H, W, focal, cx, cy, near, far, c2w, first, count) to generate the rays of pixels [first, first + count) on the fly.
-    cond_*: (aud, expr, latent) of each net.  Returns the render_rays dict (plus '_nonfinite' bits when check_numerics)."""
+    cond_*: (aud, expr, latent) of each net.  coarse_rgb=False: no 'rgb0' (a frame render keeps only the fine colour), so the coarse
+    pass computes densities alone (in bf16 mode the coarse net skips its colour branch); every other output is unchanged, bit for bit.
+    Not with with_fg.  Returns the render_rays dict (plus '_nonfinite' bits when check_numerics)."""
+    if with_fg and not coarse_rgb:
+        raise ValueError("render_rays_fused: the torso extras (with_fg) include a coarse colour; they need coarse_rgb=True")
     mode = net_coarse._mode()
     bc_rgb = f32c(bc_rgb, "bc_rgb")
     dev = bc_rgb.device
@@ -646,9 +650,9 @@ def render_rays_fused(net_coarse, net_fine, cond_coarse, cond_fine, bc_rgb, n_sa
     a.coarse = _render_net(net_coarse, *cond_coarse, keep)
     a.fine = _render_net(net_fine, *cond_fine, keep)
     stot = n_samples + n_importance
-    out = torch.empty((n * (13 + (7 if with_fg else 0)),), device=dev)
-    cuts = [("rgb_map", 3), ("disp_map", 1), ("acc_map", 1), ("depth_map", 1), ("last_weight", 1), ("rgb0", 3), ("disp0", 1), ("acc0", 1),
-            ("z_std", 1)] + ([("rgb_map_fg", 3), ("rgb_map_fg0", 3), ("last_weight0", 1)] if with_fg else [])
+    cuts = [("rgb_map", 3), ("disp_map", 1), ("acc_map", 1), ("depth_map", 1), ("last_weight", 1)] + ([("rgb0", 3)] if coarse_rgb else []) + \
+        [("disp0", 1), ("acc0", 1), ("z_std", 1)] + ([("rgb_map_fg", 3), ("rgb_map_fg0", 3), ("last_weight0", 1)] if with_fg else [])
+    out = torch.empty((n * sum(w for _, w in cuts),), device=dev)
     ret, o = {}, 0
     for k, w in cuts:
         ret[k] = out[o:o + n * w].view(n, 3) if w == 3 else out[o:o + n]

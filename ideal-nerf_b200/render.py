@@ -75,15 +75,16 @@ def _fusable(net_coarse, net_fine, aud, expr, latent, N_samples, N_importance, r
 
 def _render_rays_impl(rays, bc_rgb, net_coarse, net_fine, aud, expr, latent, N_samples, N_importance, retraw=False,
                       lindisp=False, perturb=0., white_bkgd=False, raw_noise_std=0., pytest=False, with_fg=False,
-                      pdf_policy=_lib.INERF_PDF_EXACT_TORCH_CPU, check_numerics=False, gen=None):
+                      pdf_policy=_lib.INERF_PDF_EXACT_TORCH_CPU, check_numerics=False, gen=None, coarse_rgb=True):
     """audio_exp_nerf.py:297-371 (torso extras: train_torso.py:290-363).  gen: instead of `rays`, the frame / camera / pixel range whose
-    rays the fused entry generates itself (frame.FrameRenderer)."""
+    rays the fused entry generates itself (frame.FrameRenderer).  coarse_rgb=False: the caller does not read 'rgb0', so the fused entry
+    leaves it out and skips the coarse colour (ops.render_rays_fused); the stage-by-stage path still returns it."""
     net_f = net_coarse if net_fine is None else net_fine
     if gen is not None or _fusable(net_coarse, net_f, aud, expr, latent, N_samples, N_importance, retraw, raw_noise_std, pytest, pdf_policy):
         # inference: the whole call is ONE C entry point (inerf_render_rays_fused), five launches in the reference's configuration
         ret = ops.render_rays_fused(net_coarse, net_f, (aud, expr, latent), (aud, expr, latent), bc_rgb, N_samples, N_importance, perturb,
                                     rays=rays, gen=gen, lindisp=lindisp, white_bkgd=white_bkgd, with_fg=with_fg,
-                                    check_numerics=check_numerics)
+                                    check_numerics=check_numerics, coarse_rgb=coarse_rgb)
         for k in ret.get('_nonfinite', ()):
             logger.info(f"! [Numerical Error] {k} contains nan or inf.")
         return ret

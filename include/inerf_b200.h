@@ -398,9 +398,11 @@ typedef struct InerfRenderArgs {
     const float* u_vals;             /* torch.linspace(0, 1, n_importance); only read when perturb == 0                    */
     uint64_t* rng_state;             /* {seed, offset}; only used when perturb != 0; the offset is advanced by 1           */
     InerfRenderNet coarse, fine;
-    /* outputs (device).  Required: rgb_map (n,3), disp_map, acc_map, depth_map, last_weight (n), rgb0 (n,3), disp0, acc0, z_std (n).
+    /* outputs (device).  Required: rgb_map (n,3), disp_map, acc_map, depth_map, last_weight (n), disp0, acc0, z_std (n).
+     * rgb0 (n,3): NULL = no coarse colour.  The coarse net then runs its density-only build in INERF_MLP_BF16 mode (the full net in the
+     * others) and the coarse compositor reads sigma alone; every other output keeps its bits.  Not with the torso extras.
      * Optional (NULL to skip): weights (n, S) of the fine pass, z_vals (n, S) merged depths, and the torso extras rgb_map_fg (n,3),
-     * rgb_map_fg0 (n,3), last_weight0 (n) -- the three are given together or not at all. */
+     * rgb_map_fg0 (n,3), last_weight0 (n) -- the three are given together or not at all, and need rgb0. */
     float *rgb_map, *disp_map, *acc_map, *depth_map, *last_weight, *rgb0, *disp0, *acc0, *z_std;
     float *weights, *z_vals, *rgb_map_fg, *rgb_map_fg0, *last_weight0;
     int32_t* nonfinite;              /* NULL or a device int32: INERF_NF_* bits are OR-ed in (not cleared here)            */
@@ -408,8 +410,9 @@ typedef struct InerfRenderArgs {
     size_t workspace_bytes;
 } InerfRenderArgs;
 
-/* Scratch the call needs for these shapes (rays when generated, both conditioning buffers, coarse depths, raw of both passes, merged
- * depths, and the coarse weights / samples of the deterministic path). */
+/* Scratch the call needs for these shapes (rays when generated, both conditioning buffers, coarse depths, raw of both passes -- the
+ * coarse one a float per sample when rgb0 is NULL in INERF_MLP_BF16 mode -- merged depths, and the coarse weights / samples of the
+ * deterministic path). */
 int inerf_render_workspace_bytes(const InerfRenderArgs* args, size_t* bytes);
 int inerf_render_rays_fused(const InerfRenderArgs* args, void* stream);
 /* Measurement twin (the one entry point that SYNCHRONISES): the same call with a CUDA event between the stages; ms_host5 (HOST, 5 floats)
