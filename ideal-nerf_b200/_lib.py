@@ -12,7 +12,7 @@ import subprocess
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 REPO_ROOT = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
-SO_PATH = os.environ.get("INERF_SO") or os.path.join(PKG_DIR, "libinerf_b200.so")     # INERF_SO: profiling builds only
+SO_PATH = os.environ.get("INERF_SO") or os.path.join(PKG_DIR, "libinerf_b200.so")     # INERF_SO: another build (profiles/ab_compare.py)
 SOURCES = ["api.cu", "rays.cu", "composite.cu", "sample_pdf.cu", "mlp_api.cu", "mlp_fp32.cu", "mlp_fp32_bwd.cu", "mlp_bf16.cu", "mlp_bf16_bwd.cu",
            "mlp_bf16_dw.cu", "mlp_f16x2.cu", "audio_net.cu", "render_fused.cu", "pixel_sampler.cu", "image_metrics.cu",
            "lpips.cu"]
@@ -106,7 +106,6 @@ SIGNATURES = {
     "inerf_mlp_packed_bytes": (_I, [_I, _DIMS, _SZP]),
     "inerf_mlp_pack": (_I, [_I, _DIMS, _PARAMS, _P, _P]),
     "inerf_mlp_fwd": (_I, [_I, _DIMS, _PARAMS, _P, _P, _P, _I, _P, _I, _I, _P, _P]),
-    "inerf_mlp_fwd_trace": (_I, [_I, _DIMS, _PARAMS, _P, _P, _P, _I, _P, _I, _I, _P, _P, _P]),
     "inerf_mlp_train_sizes": (_I, [_DIMS, _L, _SZP, _SZP, _SZP]),
     "inerf_mlp_fwd_train": (_I, [_DIMS, _PARAMS, _P, _P, _I, _P, _I, _I, _P, _L, _P, _P, _P]),
     "inerf_mlp_bwd": (_I, [_DIMS, _PARAMS, _PARAMS, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P]),
@@ -118,7 +117,6 @@ SIGNATURES = {
     "inerf_audio_att_fwd": (_I, [_PARAMS, _P, _I, _I, _I, _P, _P]),
     "inerf_audio_net_bwd": (_I, [_PARAMS, _PARAMS, _P, _P, _I, _I, _P]),
     "inerf_audio_att_bwd": (_I, [_PARAMS, _PARAMS, _P, _P, _I, _I, _I, _P, _P]),
-    "inerf_debug_hang_info": (_I, [ctypes.POINTER(ctypes.c_int32)]),
     "inerf_mlp_fwd_embedded": (_I, [_I, _DIMS, _PARAMS, _P, _P, _P, _L, _P, _P]),
     "inerf_pixel_sampler_workspace_bytes": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _SZP]),
     "inerf_sample_train_pixels": (_I, [ctypes.POINTER(InerfPixelSampleArgs), _P, ctypes.c_size_t, _P]),
@@ -148,8 +146,7 @@ def build(force=False, verbose=False):
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         raise RuntimeError("nvcc not found: cannot build libinerf_b200.so")
-    extra = os.environ.get("INERF_EXTRA_NVCC", "").split()
-    objdir = os.path.join(REPO_ROOT, "build", "obj" + ("_" + str(abs(hash(tuple(extra))) % 10 ** 8) if extra else ""))
+    objdir = os.path.join(REPO_ROOT, "build", "obj")
     os.makedirs(objdir, exist_ok=True)
     hdrs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))] + [os.path.join(REPO_ROOT, "include", "inerf_b200.h")]
     t_hdr = max(os.path.getmtime(h) for h in hdrs)
@@ -160,7 +157,7 @@ def build(force=False, verbose=False):
         spath = os.path.join(CSRC, src)
         if not force and os.path.exists(obj) and os.path.getmtime(obj) > max(t_hdr, os.path.getmtime(spath)):
             return obj, ""
-        r = subprocess.run([nvcc] + flags + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", "-o", obj, spath],
+        r = subprocess.run([nvcc] + flags + (["-Xptxas", "-v"] if verbose else []) + ["-c", "-o", obj, spath],
                            cwd=CSRC, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError(f"nvcc failed on {src}:\n" + r.stdout + r.stderr)

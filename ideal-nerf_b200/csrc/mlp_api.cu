@@ -141,20 +141,6 @@ extern "C" int inerf_mlp_fwd(int mode, const InerfNetDims* dims, const float* co
     return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd: unknown mode");
 }
 
-extern "C" int inerf_mlp_fwd_trace(int mode, const InerfNetDims* dims, const float* const* params_host, const void* packed,
-                                   const float* cond, const float* rays, int ray_stride, const float* z, int n, int s,
-                                   float* raw, float* trace, void* stream) {
-    MlpArgs a{};
-    int rc = fill_args(a, dims, params_host, cond);
-    if (rc) return rc;
-    if (mode != INERF_MLP_BF16) return fail(INERF_E_UNSUPPORTED, "inerf_mlp_fwd_trace: only the bf16 kernel has a trace build");
-    if (n <= 0 || s <= 0 || ray_stride < 11) return fail(INERF_E_SHAPE, "inerf_mlp_fwd_trace: bad n/s/ray_stride");
-    if (!rays || !z || !raw || !trace || !packed) return fail(INERF_E_ARG, "inerf_mlp_fwd_trace: NULL pointer");
-    a.rays = rays; a.ray_stride = ray_stride; a.z = z; a.s = s;
-    a.P = (long long)n * s; a.out = raw; a.packed = packed; a.trace = trace;
-    return mlp_bf16_launch(a, false, as_stream(stream));
-}
-
 extern "C" int inerf_mlp_train_sizes(const InerfNetDims* dims, int64_t n_points, size_t* acts_floats, size_t* deltas_floats,
                                      size_t* scratch_bytes) {
     int rc = check_dims(dims);
@@ -200,11 +186,6 @@ extern "C" int inerf_mlp_bwd(const InerfNetDims* dims, const float* const* param
     if (((uintptr_t)acts | (uintptr_t)deltas | (uintptr_t)d_raw) & 15) return fail(INERF_E_ALIGN, "inerf_mlp_bwd: acts/deltas/d_raw must be 16-byte aligned");
     return mlp_fp32_bwd_launch(dims, params_host, grads_host, aud, expr, latent, acts, deltas, d_raw, n_points, d_cond, scratch,
                                as_stream(stream));
-}
-
-extern "C" int inerf_debug_hang_info(int32_t* out8) {
-    if (!out8) return fail(INERF_E_ARG, "inerf_debug_hang_info: NULL");
-    return mlp_bf16_hang_info(out8);
 }
 
 extern "C" int inerf_mlp_fwd_embedded(int mode, const InerfNetDims* dims, const float* const* params_host,

@@ -33,7 +33,6 @@
 // gamma(v) image that the producer warps write into the PE buffer once L5 (the last reader of gamma(p)) has completed; the commit after
 // the last V0 view MMA hands the buffer back for the next iteration's gamma(p).  Packed blob: INERF_MLP_BF16_EMB (two more stages).
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include "mlp_tc.cuh"
 
@@ -86,47 +85,6 @@ struct Bars {
 };
 static_assert(sizeof(Bars) <= 320, "barrier block");
 
-// Hang diagnostics (trace build only): every mbarrier wait has a ~1 s clock64 budget; the first waiter that
-// runs out records {site code, block, thread, aux...} in a host-mapped buffer and traps.  The production build
-// waits unconditionally.
-__device__ int* g_hang_dev = nullptr;
-
-template <bool DBG>
-__device__ __forceinline__ void wait_or_report(uint64_t* bar, uint32_t parity, int code, int aux0, int aux1) {
-    if constexpr (!DBG) {
-        mbar_wait(bar, parity);
-    } else {
-        const long long t0 = clock64();
-        while (!mbar_try_wait(bar, parity)) {
-            if (clock64() - t0 > 2000000000LL) {
-                int* h = g_hang_dev;
-                if (h && atomicCAS(h, 0, code) == 0) {
-                    h[1] = blockIdx.x; h[2] = threadIdx.x; h[3] = aux0; h[4] = aux1; h[5] = (int)parity;
-                    __threadfence_system();
-                }
-                __nanosleep(1000000);
-                __trap();
-            }
-        }
-    }
-}
-
-// Light phase timers of the PRODUCTION kernel (builds with -DINERF_PHASE_TIMERS only; profiles/mlp_phase_timers.py): two clock reads per
-// epilogue half in ONE warp and around the issuer's epilogue-event / weight waits -- the TRACE build's timers inflate an iteration by 50 %.
-#ifdef INERF_PHASE_TIMERS
-__device__ unsigned long long g_phase[148][16];
-#define PH_CLK() clock64()
-#else
-#define PH_CLK() 0ll
-#endif
-
-// issuer-side wait on an event whose arrivals may come from the peer CTA (pair build: cluster-scope acquire)
-template <bool DBG, bool PAIR>
-__device__ __forceinline__ void wait_ev(uint64_t* bar, uint32_t parity, int code, int aux0, int aux1) {
-    if constexpr (DBG && !PAIR) wait_or_report<true>(bar, parity, code, aux0, aux1);
-    else sm100::wait_ev<PAIR>(bar, parity);
-}
-
 struct LayerInfo { int N, bias_off; };
 
 __device__ __forceinline__ LayerInfo layer_info(int l) {
@@ -138,10 +96,10 @@ __device__ __forceinline__ LayerInfo layer_info(int l) {
 
 // One 32-column chunk of an epilogue: +bias (+per-ray view bias), ReLU, bf16 pack; KIND 1 also accumulates
 // alpha_linear, KIND 3 rgb_linear, in fp32 from the un-rounded activations.
-template <int KIND, bool TRACE, bool SAVE>
+template <int KIND, bool SAVE>
 __device__ __forceinline__ void epi_convert(const uint32_t (&r)[32], uint32_t* __restrict__ packed16,
                                             const float* __restrict__ dsrc, const float* __restrict__ aw, const float* __restrict__ rw,
-                                            float& alpha, float& rgb0, float& rgb1, float& rgb2, float* tr, bool dump, uint32_t& neg_bits) {
+                                            float& alpha, float& rgb0, float& rgb1, float& rgb2, uint32_t& neg_bits) {
 #pragma unroll
     for (int j = 0; j < 32; j += 4) {
         float v[4] = {__uint_as_float(r[j]), __uint_as_float(r[j + 1]), __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3])};
@@ -169,9 +127,6 @@ __device__ __forceinline__ void epi_convert(const uint32_t (&r)[32], uint32_t* _
         }
         packed16[(j >> 1)] = pack_bf16x2_relu(v[0], v[1]);
         packed16[(j >> 1) + 1] = pack_bf16x2_relu(v[2], v[3]);
-        if constexpr (TRACE) {
-            if (dump) { tr[j] = relu_nan(v[0]); tr[j + 1] = relu_nan(v[1]); tr[j + 2] = relu_nan(v[2]); tr[j + 3] = relu_nan(v[3]); }
-        }
     }
 }
 
@@ -182,9 +137,6 @@ struct IssueCtx {
     uint32_t stage, wpar;                // weight ring position and the parity of its current round
     uint32_t ones_lo, bt_lo, bslot, bpar;   // bias MMA operands (no-swizzle descriptors) and the bias ring position
     uint32_t layer_ctr, iter_ctr;
-    long long ph_e0, ph_e1, ph_e_other, ph_w;      // INERF_PHASE_TIMERS build: cycles waiting for E0 / E1 of a 256-wide layer after a 256-wide one, other layers' events, weight stages
-    long long t_e, t_w, t_pe;            // trace build: where the issuer waits
-    long long t_e_layer[11];             // ... and the epilogue-event waits per layer
 };
 
 // All MMAs of layer L for both 128-row slots, straight-line: every descriptor offset, wait and commit below is a compile-time
@@ -193,7 +145,7 @@ struct IssueCtx {
 // against the 512 the tensor pipe needs -- profiles/r01_mlp_ablation.txt.)
 // EMB: the embedded-row schedule.  pe_ready and pe_free then complete twice per iteration (gamma(p) for L0 / L5, gamma(v) for V0), so
 // the issuer's waits have fixed parities: 0 before L0, 1 before V0's view K-block.
-template <int L, bool TRACE, int ABL, bool PAIR, bool EMB = false>
+template <int L, bool PAIR, bool EMB = false>
 __device__ __forceinline__ void issue_layer(IssueCtx& c) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
     constexpr int N = lay_N(L), NH = N / 2, NKB = lay_act_kb(L), CNT = NKB + (lay_x(L, EMB) ? 1 : 0);
@@ -208,34 +160,20 @@ __device__ __forceinline__ void issue_layer(IssueCtx& c) {
 #pragma unroll
         for (int i = 0; i < CNT; ++i) {
             const bool is_pe = (i == NKB);                     // the PE block comes last in both halves
-            long long c0 = 0;
-            if constexpr (TRACE) c0 = clock64();
             if (h == 0 && c.layer_ctr > 0) {                   // each epilogue event is waited ONCE per layer, at its first use
                 if (L == 0) {                                  // new iteration: both accumulator halves of V2 drained
-                    if (i == 0) { const long long p0 = PH_CLK();
-                                  wait_ev<TRACE, PAIR>(&bars->ebar[0], par_prev, 201, L, (int)c.layer_ctr);
-                                  wait_ev<TRACE, PAIR>(&bars->ebar[1], par_prev, 202, L, (int)c.layer_ctr);
-                                  c.ph_e_other += PH_CLK() - p0; }
+                    if (i == 0) { wait_ev<PAIR>(&bars->ebar[0], par_prev); wait_ev<PAIR>(&bars->ebar[1], par_prev); }
                 } else if (!is_pe) {
-                    if (i == 0) { const long long p0 = PH_CLK(); wait_ev<TRACE, PAIR>(&bars->ebar[0], par_prev, 201, L, (int)c.layer_ctr);
-                                  if (L == 1) c.ph_e0 += PH_CLK() - p0; else c.ph_e_other += PH_CLK() - p0; }
-                    if (i == KB_PER_HALF_PREV) { const long long p0 = PH_CLK(); wait_ev<TRACE, PAIR>(&bars->ebar[1], par_prev, 202, L, (int)c.layer_ctr);
-                                                 if (L == 1) c.ph_e1 += PH_CLK() - p0; else c.ph_e_other += PH_CLK() - p0; }
+                    if (i == 0) wait_ev<PAIR>(&bars->ebar[0], par_prev);
+                    if (i == KB_PER_HALF_PREV) wait_ev<PAIR>(&bars->ebar[1], par_prev);
                 }
             }
-            if constexpr (TRACE) { const long long c1 = clock64(); c.t_e += c1 - c0; c.t_e_layer[c.layer_ctr % 11] += c1 - c0; c0 = c1; }
-            if (L == 0 && h == 0 && i == 0) wait_ev<TRACE, PAIR>(&bars->pe_ready, EMB ? 0u : c.iter_ctr & 1, 203, L, (int)c.iter_ctr);
-            if (EMB && L == 8 && h == 0 && is_pe) wait_ev<TRACE, PAIR>(&bars->pe_ready, 1u, 206, L, (int)c.iter_ctr);
-            if constexpr (TRACE) { const long long c1 = clock64(); c.t_pe += c1 - c0; c0 = c1; }
-            if (!(ABL & 2) || (c.layer_ctr == 0 && L == 0 && h * CNT + i < NSTAGE)) {
-                const long long p0 = PH_CLK();
-                wait_or_report<TRACE>(&bars->wfull[c.stage], c.wpar, 204, L, (int)c.stage);
-                if constexpr (PAIR) mbar_wait_cluster(&bars->pfull[c.stage], c.wpar);
-                c.ph_w += PH_CLK() - p0;
-            }
-            if constexpr (TRACE) c.t_w += clock64() - c0;
+            if (L == 0 && h == 0 && i == 0) wait_ev<PAIR>(&bars->pe_ready, EMB ? 0u : c.iter_ctr & 1);
+            if (EMB && L == 8 && h == 0 && is_pe) wait_ev<PAIR>(&bars->pe_ready, 1u);
+            mbar_wait(&bars->wfull[c.stage], c.wpar);
+            if constexpr (PAIR) mbar_wait_cluster(&bars->pfull[c.stage], c.wpar);
             if (i == 0) {
-                wait_or_report<TRACE>(&bars->bfull[c.bslot], c.bpar, 205, L, (int)c.bslot);
+                mbar_wait(&bars->bfull[c.bslot], c.bpar);
                 if constexpr (PAIR) mbar_wait_cluster(&bars->pbfull[c.bslot], c.bpar);
             }
             tc_fence_after();
@@ -281,17 +219,15 @@ __device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, ui
 // per kernel + immediates, no layer-kind or chunk-count branch between the chunks.  The general loop below spends a third of its stall
 // samples on instruction fetch and branch resolution around exactly this body (ncu source counters); instantiating that loop twice was
 // slower (register spills), a separate small function is not.  act_row: shared-memory address of this thread's row in K-block 0 of its
-// slot; soff[j] = byte offset of 16-byte chunk j of a 128-byte row after the swizzle.  ph: phase timers (INERF_PHASE_TIMERS builds).
+// slot; soff[j] = byte offset of 16-byte chunk j of a 128-byte row after the swizzle.
 template <int NH, bool PAIR>
 __device__ __forceinline__ void epi_plain_layer(Bars* bars, uint32_t par, uint32_t t_lane, uint32_t act_row, const uint32_t (&soff)[8],
-                                                int lane, long long* ph) {
+                                                int lane) {
     constexpr int NC = NH / 32;      // chunks per half: 4 (N = 256) or 2 (N = 128)
     // ---- first half: convert everything, wait until the second half's MMAs have read the K-blocks it overwrites (C1), store ----------
-    const long long p0 = PH_CLK();
     mbar_wait(&bars->cbar[0], par);
     __syncwarp();
     tc_fence_after();
-    const long long p1 = PH_CLK();
     uint32_t packed[NC * 16];
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
@@ -302,9 +238,7 @@ __device__ __forceinline__ void epi_plain_layer(Bars* bars, uint32_t par, uint32
         for (int j = 0; j < 16; ++j) packed[c * 16 + j] = pack_bf16x2_relu(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1]));
     }
     tc_fence_before();
-    const long long p2 = PH_CLK();
     mbar_wait(&bars->cbar[1], par);
-    ph[4] += PH_CLK() - p2;
     __syncwarp();
 #pragma unroll
     for (int c = 0; c < NC; ++c)
@@ -315,13 +249,10 @@ __device__ __forceinline__ void epi_plain_layer(Bars* bars, uint32_t par, uint32
     fence_proxy_async_smem();
     __syncwarp();
     if (lane == 0) { if constexpr (PAIR) mbar_arrive_remote(&bars->ebar[0], 0); else mbar_arrive(&bars->ebar[0]); }
-    const long long p3 = PH_CLK();
-    ph[0] += p1 - p0; ph[1] += p3 - p1;
     // ---- second half: nothing reads its K-blocks any more, every chunk is stored as soon as it is converted ----------------------------
     mbar_wait(&bars->cbar[2], par);
     __syncwarp();
     tc_fence_after();
-    const long long p4 = PH_CLK();
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
         uint32_t r[32], pk[16];
@@ -337,8 +268,6 @@ __device__ __forceinline__ void epi_plain_layer(Bars* bars, uint32_t par, uint32
     fence_proxy_async_smem();
     __syncwarp();
     if (lane == 0) { if constexpr (PAIR) mbar_arrive_remote(&bars->ebar[1], 0); else mbar_arrive(&bars->ebar[1]); }
-    const long long p5 = PH_CLK();
-    ph[2] += p4 - p3; ph[3] += p5 - p4;
 }
 
 // Epilogue of L7 in the density-only build (DENS): the alpha head alone, in epi_convert<1>'s FMA order.  Nothing reads h7 (V0 does not
@@ -372,16 +301,6 @@ __device__ __forceinline__ void epi_alpha_layer(Bars* bars, uint32_t par, uint32
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
-// ABL (builds with -DINERF_ABLATION only; profiles/ablate_mlp.py): bit 0 = epilogue keeps its barrier protocol but skips the
-// TMEM loads / conversion / smem stores, bit 1 = weights are loaded once (no streaming, no full-barrier waits), bit 2 = the
-// positional-encoding warps skip sincosf, bit 3 = the epilogue skips only its TMEM loads, bit 4 = only its bias/ReLU/convert math.  Outputs are garbage; only the timing is meaningful.
-#ifdef INERF_ABLATION
-__device__ int g_save_abl;      // profiling builds: switch parts of the activation saving off (profiles/ablate_save.py); results are garbage
-#define SAVE_OFF(bit) (g_save_abl & (bit))
-#else
-#define SAVE_OFF(bit) false
-#endif
-
 // PAIR = true (inference build): the kernel runs as clusters of two CTAs.  Every MMA is ONE tcgen05.mma.cta_group::2 over the 2 x 128
 // rows of the pair (issued by the leader's warp 1), and the B operand -- the weight stage -- is split across the pair: each CTA streams
 // and keeps only HALF of the rows of every stage.  Why: the N = 128 MMAs of the single-CTA form read 8 KB of operands per 64 cycles,
@@ -396,12 +315,10 @@ __device__ int g_save_abl;      // profiling builds: switch parts of the activat
 // depends on L0-L7 and the alpha head.  The issuer runs L0-L7 and starts the next iteration (L0 waits E0 / E1 of L7), producer and relay
 // stream the stages of L0-L7 -- the first n_steps of the same schedule and blob -- the PE warps skip the per-ray view bias, and the output
 // is one float per point, alpha + alpha_linear.bias: the .w of the full build, bit for bit.
-template <bool TRACE, int ABL = 0, bool SAVE = false, bool PAIR = false, bool EMB = false, bool DENS = false>
-__global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, int n_steps, int n_rays, float* __restrict__ trace) {
+template <bool SAVE = false, bool PAIR = false, bool EMB = false, bool DENS = false>
+__global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, int n_steps, int n_rays) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
-    static_assert(!(PAIR && (TRACE || ABL != 0)), "the pair build has no trace / ablation variants");
-    static_assert(!(EMB && (TRACE || ABL != 0)), "the embedded-row build has no trace / ablation variants");
-    static_assert(!(DENS && (TRACE || ABL != 0 || SAVE || EMB)), "the density-only build is an inference build of the fused entry");
+    static_assert(!(DENS && (SAVE || EMB)), "the density-only build is an inference build of the fused entry");
     // Dynamic shared memory is the only shared allocation of this kernel, so it starts at offset 0 of the CTA's
     // window: 1024-byte aligned as the 128B-swizzle atoms need.  (No pointer re-alignment arithmetic here: it would
     // make the compiler lose the shared address space and emit generic LD/ST for every epilogue access.)
@@ -469,13 +386,12 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         const uint32_t slot = bh & 1, l = step_at<EMB>(s).layer, h = step_at<EMB>(s).half;
                         const uint32_t bytes = (uint32_t)step_at<EMB>(s).n8 * 8u * 32u / SPLIT;
                         const uint32_t off = bias_tile_offset(l, h) + rank * bytes;
-                        wait_or_report<TRACE>(&bars->bempty[slot], ((bh >> 1) & 1) ^ 1, 102, s, (int)bh);
+                        mbar_wait(&bars->bempty[slot], ((bh >> 1) & 1) ^ 1);
                         mbar_arrive_expect_tx(&bars->bfull[slot], bytes);
                         bulk_g2s(sm + OFF_BT + slot * 4096, tiles + off, bytes, &bars->bfull[slot]);
                         ++bh;
                     }
-                    if ((ABL & 2) && g >= NSTAGE) continue;
-                    wait_or_report<TRACE>(&bars->wempty[stage], (round & 1) ^ 1, 101, s, (int)g);
+                    mbar_wait(&bars->wempty[stage], (round & 1) ^ 1);
                     const uint32_t bytes = (uint32_t)step_at<EMB>(s).n8 * 8u * 128u / SPLIT;
                     mbar_arrive_expect_tx(&bars->wfull[stage], bytes);
                     bulk_g2s(sm + OFF_W + stage * STAGE_BYTES, blob + step_at<EMB>(s).offset + rank * bytes, bytes, &bars->wfull[stage]);
@@ -510,40 +426,21 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
         c.bt_lo = desc_lo_noswz(smem_u32(sm + OFF_BT));
         c.bslot = 0; c.bpar = 0;
         c.stage = 0; c.wpar = 0; c.layer_ctr = 0; c.iter_ctr = 0;
-        c.t_e = c.t_w = c.t_pe = 0;
-        c.ph_e0 = c.ph_e1 = c.ph_e_other = c.ph_w = 0;
-        const long long ph_t0 = PH_CLK();
-        for (int j = 0; j < 11; ++j) c.t_e_layer[j] = 0;
-        const long long t_tot = clock64();
         for (long long it = it_first; it < n_iter; it += it_step, ++c.iter_ctr) {
             // Layers of equal geometry share ONE copy of the straight-line issue code (L1-L4, L6, L7 are 256 x 256 after a 256-wide
             // layer; V1, V2 are 128 x 128 after a 128-wide one): 11 inlined copies were 78 KB of SASS streamed once per iteration, which
             // together with the epilogue and PE code overflowed the instruction cache the epilogue warps live in (ncu: stall_no_inst).
-            issue_layer<0, TRACE, ABL, PAIR, EMB>(c);
+            issue_layer<0, PAIR, EMB>(c);
 #pragma unroll 1
             for (int seg = 0; seg < 2; ++seg) {
 #pragma unroll 1
-                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, TRACE, ABL, PAIR, EMB>(c);
-                if (seg == 0) issue_layer<5, TRACE, ABL, PAIR, EMB>(c);
+                for (int r = 0; r < (seg ? 2 : 4); ++r) issue_layer<1, PAIR, EMB>(c);
+                if (seg == 0) issue_layer<5, PAIR, EMB>(c);
             }
             if constexpr (!DENS) {
-                issue_layer<8, TRACE, ABL, PAIR, EMB>(c);
+                issue_layer<8, PAIR, EMB>(c);
 #pragma unroll 1
-                for (int r = 0; r < 2; ++r) issue_layer<9, TRACE, ABL, PAIR, EMB>(c);
-            }
-        }
-#ifdef INERF_PHASE_TIMERS
-        if (lane == 0) {
-            unsigned long long* g = g_phase[blockIdx.x];
-            g[0] = (unsigned long long)(PH_CLK() - ph_t0); g[1] = c.iter_ctr; g[2] = c.ph_e0; g[3] = c.ph_e1; g[4] = c.ph_e_other; g[5] = c.ph_w;
-        }
-#endif
-        if constexpr (TRACE) {      // per-CTA issuer timing after the activation trace: {total, wait E, wait PE, wait weights, iterations}
-            if (lane == 0) {
-                float* t = trace + (size_t)11 * 256 * 256 + blockIdx.x * 8;
-                t[0] = (float)(clock64() - t_tot); t[1] = (float)c.t_e; t[2] = (float)c.t_pe; t[3] = (float)c.t_w; t[4] = (float)c.iter_ctr;
-                float* tl = trace + (size_t)11 * 256 * 256 + 2 * 148 * 8 + blockIdx.x * 16;
-                for (int j = 0; j < 11; ++j) tl[j] = (float)c.t_e_layer[j];
+                for (int r = 0; r < 2; ++r) issue_layer<9, PAIR, EMB>(c);
             }
         }
     } else if (warp >= 4 && warp < 12) {
@@ -559,8 +456,6 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 #pragma unroll
         for (int j = 0; j < 8; ++j) soff[j] = ((uint32_t)j ^ rsw) << 4;
         uint32_t layer_ctr = 0, iter_ctr = 0;
-        long long te_wait = 0, te_ld = 0, te_c1 = 0, te_st = 0;       // trace build: epilogue phase cycles (warp 4)
-        long long ph_wait[2] = {0, 0}, ph_dur[2] = {0, 0}, ph_c1 = 0;  // INERF_PHASE_TIMERS build: L1..L7, per half: wait for the commit / work until the arrival; wait for C1
         for (long long it = it_first; it < n_iter; it += it_step, ++iter_ctr) {
             const long long chunk = CHUNK_OF(it);
             const bool chunk_ok = !PAIR || chunk * 256 < a.P;      // pair build: the peer's last chunk may lie wholly past the end (nothing is saved for it)
@@ -574,27 +469,17 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 const LayerInfo li = layer_info(l);
                 const int NH = li.N >> 1;
                 const uint32_t par = layer_ctr & 1;
-                if constexpr (!SAVE && !TRACE && ABL == 0) {      // inference: the layers without head / view-bias work take the straight-line epilogue
-                    long long phl[5] = {0, 0, 0, 0, 0};
-                    if (l <= 6) {
-                        epi_plain_layer<128, PAIR>(bars, par, t_lane, act_row_u32, soff, lane, phl);
-                        if (l >= 1) { ph_wait[0] += phl[0]; ph_dur[0] += phl[1]; ph_wait[1] += phl[2]; ph_dur[1] += phl[3]; ph_c1 += phl[4]; }
-                        continue;
-                    }
+                if constexpr (!SAVE) {      // inference: the layers without head / view-bias work take the straight-line epilogue
+                    if (l <= 6) { epi_plain_layer<128, PAIR>(bars, par, t_lane, act_row_u32, soff, lane); continue; }
                     if constexpr (DENS) { epi_alpha_layer<PAIR>(bars, par, t_lane, s_aw, lane, alpha); continue; }
-                    if (l == 9 || (EMB && l == 8)) { epi_plain_layer<64, PAIR>(bars, par, t_lane, act_row_u32, soff, lane, phl); continue; }
+                    if (l == 9 || (EMB && l == 8)) { epi_plain_layer<64, PAIR>(bars, par, t_lane, act_row_u32, soff, lane); continue; }
                 }
-                if (!EMB && l == 8) wait_or_report<TRACE>(&bars->dirb_ready, iter_ctr & 1, 301, l, (int)iter_ctr);
+                if (!EMB && l == 8) mbar_wait(&bars->dirb_ready, iter_ctr & 1);
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
-                    long long q0 = 0;
-                    if constexpr (TRACE) q0 = clock64();
-                    const long long ph0 = PH_CLK();
-                    wait_or_report<TRACE>(&bars->cbar[h == 0 ? 0 : 2], par, 302 + h, l, (int)layer_ctr);
+                    mbar_wait(&bars->cbar[h == 0 ? 0 : 2], par);
                     __syncwarp();
                     tc_fence_after();
-                    const long long ph1 = PH_CLK();
-                    if constexpr (TRACE) { const long long q1 = clock64(); te_wait += q1 - q0; q0 = q1; }
                     uint32_t packed[64];
                     const int nchunk = NH >> 5;      // 4 (N=256) or 2 (N=128)
                     // training: this row's mask words of the half (one pointer per half instead of a 64-bit index product per chunk)
@@ -602,34 +487,22 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                                                : nullptr;
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
-                        if (c < nchunk && !(ABL & 1)) {
+                        if (c < nchunk) {
                             uint32_t r[32];
-                            if constexpr (ABL & 8) {
-#pragma unroll
-                                for (int j = 0; j < 32; ++j) r[j] = (uint32_t)(lane + j + l);
-                            } else {
-                                tmem_ld32(t_lane + h * NH + c * 32, r);
-                                tmem_wait_ld();
-                            }
-                            if constexpr (ABL & 16) {
-#pragma unroll
-                                for (int j = 0; j < 16; ++j) packed[c * 16 + j] = r[j] ^ r[j + 16];
-                                continue;
-                            }
+                            tmem_ld32(t_lane + h * NH + c * 32, r);
+                            tmem_wait_ld();
                             const int f0 = h * NH + c * 32;                 // first output feature of the chunk
                             uint32_t neg = 0;
-                            float* tr = TRACE ? trace + ((size_t)l * 256 + slot * 128 + row) * 256 + f0 : nullptr;
-                            const bool dump = TRACE && chunk == 0;
                             switch (l) {                                    // layer kind is warp-uniform: one specialised body per chunk
-                                case 7: epi_convert<1, TRACE, SAVE>(r, &packed[c * 16], nullptr, s_aw + f0, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
+                                case 7: epi_convert<1, SAVE>(r, &packed[c * 16], nullptr, s_aw + f0, nullptr, alpha, rgb0, rgb1, rgb2, neg); break;
                                 case 8:
-                                    if constexpr (EMB) epi_convert<0, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg);
-                                    else epi_convert<2, TRACE, SAVE>(r, &packed[c * 16], s_dirb + (slot * RMAX + ray_local) * 128 + f0, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg);
+                                    if constexpr (EMB) epi_convert<0, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, neg);
+                                    else epi_convert<2, SAVE>(r, &packed[c * 16], s_dirb + (slot * RMAX + ray_local) * 128 + f0, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, neg);
                                     break;
-                                case 10: epi_convert<3, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, s_rw + f0, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
-                                default: epi_convert<0, TRACE, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, tr, dump, neg); break;
+                                case 10: epi_convert<3, SAVE>(r, &packed[c * 16], nullptr, nullptr, s_rw + f0, alpha, rgb0, rgb1, rgb2, neg); break;
+                                default: epi_convert<0, SAVE>(r, &packed[c * 16], nullptr, nullptr, nullptr, alpha, rgb0, rgb1, rgb2, neg); break;
                             }
-                            if (SAVE && !SAVE_OFF(1) && chunk_ok)      // training: the ReLU mask word of the chunk (the activations follow as a bulk copy of the smem image)
+                            if (SAVE && chunk_ok)      // training: the ReLU mask word of the chunk (the activations follow as a bulk copy of the smem image)
                                 mask_half[c * 128] = ~neg;
                             if (!SAVE && h == 1 && l != 10) {
                                 // second half: nothing reads these K-blocks any more (its own MMAs are complete), so each chunk goes to shared
@@ -644,23 +517,19 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         }
                     }
                     tc_fence_before();
-                    if constexpr (TRACE) { const long long q1 = clock64(); te_ld += q1 - q0; q0 = q1; }
                     if (l != 10 || SAVE) {
-                        const long long ph2 = PH_CLK();
-                        if (h == 0) wait_or_report<TRACE>(&bars->cbar[1], par, 304, l, (int)layer_ctr);
-                        ph_c1 += PH_CLK() - ph2;
+                        if (h == 0) mbar_wait(&bars->cbar[1], par);
                         if constexpr (SAVE) {
                             // training: each warp bulk-copies its own 32 rows of the K-blocks it writes (4 KB per K-block image) to HBM, so no
                             // barrier couples the warps.  Before overwriting them, lane 0 waits until the copy that last read these rows has
                             // left shared memory: that is two copies back (this half's K-blocks were written by the same half of the previous
                             // layer) unless the layer widens (l == 0 after the 128-wide rgb layer), where it is the latest one.
-                            if (lane == 0 && !SAVE_OFF(8)) { if (h == 0 && l == 0) bulk_wait_read_all(); else bulk_wait_read_but_one(); }
+                            if (lane == 0) { if (h == 0 && l == 0) bulk_wait_read_all(); else bulk_wait_read_but_one(); }
                         }
                         __syncwarp();      // h1 has finished reading the K-blocks written below
-                        if constexpr (TRACE) { const long long q1 = clock64(); te_c1 += q1 - q0; q0 = q1; }
 #pragma unroll
                         for (int c = 0; c < 4; ++c) {
-                            if (c < nchunk && !(ABL & 1) && (SAVE || h == 0)) {
+                            if (c < nchunk && (SAVE || h == 0)) {
                                 const int f0 = h * NH + c * 32;
                                 uint8_t* kb = act + (f0 >> 6) * 16384 + row_off;
                                 const int ch0 = (f0 & 63) >> 3;                // first 16-byte chunk inside the 128-byte row
@@ -675,7 +544,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         fence_proxy_async_smem();
                         if constexpr (SAVE) {
                             __syncwarp();
-                            if (lane == 0 && !SAVE_OFF(2) && chunk_ok) {
+                            if (lane == 0 && chunk_ok) {
                                 const int kb0 = (h * NH) >> 6, nkb = NH >> 6;      // 2 K-blocks per half (N = 256) or 1 (N = 128)
                                 const uint32_t wrow = (uint32_t)(warp & 3) * 4096u;      // 32 rows = 4 row groups of 1 KB
                                 uint8_t* g = a.save_img + (((size_t)chunk * 2 + slot) * TRAIN_IMGS + train_img_of(l) + kb0) * 16384 + wrow;
@@ -688,8 +557,6 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                     // the layer-to-layer critical path (E1 gates the next layer's third K-block)
                     __syncwarp();
                     if (lane == 0) { if constexpr (PAIR) mbar_arrive_remote(&bars->ebar[h], 0); else mbar_arrive(&bars->ebar[h]); }
-                    if (l >= 1 && l <= 7) { const long long ph3 = PH_CLK(); ph_wait[h] += ph1 - ph0; ph_dur[h] += ph3 - ph1; }
-                    if constexpr (TRACE) te_st += clock64() - q0;
                 }
                 if (!EMB && l == 8) {
                     __syncwarp();
@@ -709,18 +576,6 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
         }
         if constexpr (SAVE) {
             if (lane == 0) bulk_wait_all();
-        }
-#ifdef INERF_PHASE_TIMERS
-        if ((warp == 4 || warp == 11) && lane == 0) {
-            unsigned long long* g = g_phase[blockIdx.x] + (warp == 4 ? 6 : 11);
-            g[0] = ph_wait[0]; g[1] = ph_dur[0]; g[2] = ph_wait[1]; g[3] = ph_dur[1]; g[4] = ph_c1;
-        }
-#endif
-        if constexpr (TRACE) {
-            if (warp == 4 && lane == 0) {
-                float* t = trace + (size_t)11 * 256 * 256 + (148 + blockIdx.x) * 8;
-                t[0] = (float)te_wait; t[1] = (float)te_ld; t[2] = (float)te_c1; t[3] = (float)te_st; t[4] = (float)iter_ctr;
-            }
         }
     } else if (EMB && warp >= 12) {
         // ================= embedded rows: gamma(p), then gamma(v), of row t of both slots, copied from x into the PE buffer ======
@@ -765,7 +620,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 }
                 pk[sl][31] = pack_bf16x2(__ldg(xr[sl] + 62), 0.f);
             }
-            if (it != it_first) wait_or_report<TRACE>(&bars->pe_free, 1u, 401, 0, 0);
+            if (it != it_first) mbar_wait(&bars->pe_free, 1u);
 #pragma unroll
             for (int sl = 0; sl < 2; ++sl) store_img(sm + OFF_PE + sl * 16384, pk[sl], 8);
             arrive_ready();
@@ -789,7 +644,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 for (int j = 0; j < 14; ++j) pv[sl][j] = pack_bf16x2(g[2 * j], g[2 * j + 1]);
                 pv[sl][14] = pv[sl][15] = 0u;
             }
-            wait_or_report<TRACE>(&bars->pe_free, 0u, 402, 0, 0);
+            mbar_wait(&bars->pe_free, 0u);
 #pragma unroll
             for (int sl = 0; sl < 2; ++sl) store_img(sm + OFF_PE + sl * 16384, pv[sl], 4);
             arrive_ready();
@@ -833,8 +688,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                     // and it costs 27 short FMA chains instead of 27 range reductions.  (mlp_f16x2.cu and mlp_fp32.cu call sincosf
                     // per octave.)
                     float sn, cs;
-                    if constexpr (ABL & 4) { sn = v[c]; cs = zz; }
-                    else sincosf(v[c], &sn, &cs);
+                    sincosf(v[c], &sn, &cs);
                     v[3 + c] = sn;
                     v[6 + c] = cs;
 #pragma unroll
@@ -849,7 +703,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 #pragma unroll
                 for (int j = 0; j < 32; ++j) pk[sl][j] = pack_bf16x2(v[2 * j], v[2 * j + 1]);
             }
-            if (iter_ctr > 0) wait_or_report<TRACE>(&bars->pe_free, (iter_ctr - 1) & 1, 401, 0, (int)iter_ctr);
+            if (iter_ctr > 0) mbar_wait(&bars->pe_free, (iter_ctr - 1) & 1);
 #pragma unroll
             for (int sl = 0; sl < 2; ++sl) {
                 uint8_t* dst = sm + OFF_PE + sl * 16384 + (t >> 3) * 1024 + (t & 7) * 128;
@@ -866,7 +720,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                 mbar_arrive(&bars->pe_ready);
             }
             const bool chunk_ok = !PAIR || chunk * 256 < a.P;
-            if (SAVE && !SAVE_OFF(4) && chunk_ok) {          // training: gamma(p) is the X operand of dW for pts_linears.0 / .5
+            if (SAVE && chunk_ok) {          // training: gamma(p) is the X operand of dW for pts_linears.0 / .5
 #pragma unroll
                 for (int sl = 0; sl < 2; ++sl) {
                     uint8_t* dst = a.save_img + (((size_t)chunk * 2 + sl) * TRAIN_IMGS + TRAIN_IMG_PE) * 16384 + (t >> 3) * 1024 + (t & 7) * 128;
@@ -901,7 +755,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
 #pragma unroll
                     for (int j = 0; j < 27; ++j) enc[j] = 0.f;
                 }
-                if (SAVE && !SAVE_OFF(4) && chunk_ok) {      // training: gamma(v) per POINT, the X operand of dW for the view columns of views_linears.0
+                if (SAVE && chunk_ok) {      // training: gamma(v) per POINT, the X operand of dW for the view columns of views_linears.0
 #pragma unroll
                     for (int sl = 0; sl < 2; ++sl) {
                         long long p = chunk * 256 + sl * 128 + t, pfirst = chunk * 256 + sl * 128;
@@ -925,7 +779,7 @@ __global__ void __launch_bounds__(NTHREADS_BF16, 1) mlp_bf16_kernel(MlpArgs a, i
                         }
                     }
                 }
-                if (iter_ctr > 0) wait_or_report<TRACE>(&bars->dirb_free, (iter_ctr - 1) & 1, 402, 0, (int)iter_ctr);
+                if (iter_ctr > 0) mbar_wait(&bars->dirb_free, (iter_ctr - 1) & 1);
                 for (int q2 = 0; q2 < 2 * RMAX; ++q2) {
                     float acc = 0.f;
 #pragma unroll
@@ -962,27 +816,9 @@ int mlp_bf16_pack(const InerfNetDims* d, const float* const* params_host, void* 
     return pack_tc_schedule<false>(build_tc_schedule(d, embedded, 1), params_host, packed, st, "inerf_mlp_pack");
 }
 
-#ifdef INERF_PHASE_TIMERS
-}  // namespace inerf
-// profiling builds only (not part of include/inerf_b200.h): the phase timers of the last launch, [148][16] uint64
-extern "C" int inerf_debug_phase_timers(unsigned long long* out_host) {
-    return (int)cudaMemcpyFromSymbol(out_host, g_phase, sizeof(unsigned long long) * 148 * 16);
-}
-namespace inerf {
-#endif
-
-static int* g_hang_host = nullptr;
-
-int mlp_bf16_hang_info(int32_t* out8) {
-    for (int i = 0; i < 8; ++i) out8[i] = g_hang_host ? g_hang_host[i] : 0;
-    return INERF_OK;
-}
-
-// the production builds: no trace, no ablation
 template <bool SAVE, bool PAIR, bool EMB, bool DENS = false>
 static int launch(const MlpArgs& a, int n_steps, int n_rays, cudaStream_t st, const char* what) {
-    return launch_tc(mlp_bf16_kernel<false, 0, SAVE, PAIR, EMB, DENS>, PAIR, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, what, a, n_steps, n_rays,
-                     (float*)nullptr);
+    return launch_tc(mlp_bf16_kernel<SAVE, PAIR, EMB, DENS>, PAIR, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, what, a, n_steps, n_rays);
 }
 
 // FaceNeRF.forward on embedded rows x (P, 90): a.packed is an INERF_MLP_BF16_EMB blob, a.save_img != NULL selects the saving build
@@ -992,8 +828,8 @@ static int launch_embedded(const MlpArgs& a, cudaStream_t st) {
     static thread_local int configured_dev = -1;
     static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, true, 1); }();
     int rc = setup_once(configured_dev,
-                        {(const void*)mlp_bf16_kernel<false, 0, false, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, false, true>,
-                         (const void*)mlp_bf16_kernel<false, 0, false, true, true>, (const void*)mlp_bf16_kernel<false, 0, true, true, true>},
+                        {(const void*)mlp_bf16_kernel<false, false, true>, (const void*)mlp_bf16_kernel<true, false, true>,
+                         (const void*)mlp_bf16_kernel<false, true, true>, (const void*)mlp_bf16_kernel<true, true, true>},
                         SMEM_ALLOC, "mlp_bf16", [] { return cudaMemcpyToSymbol(c_steps_emb, S.st, sizeof(TcStage) * MAX_STEPS); });
     if (rc) return rc;
     if (mlp_pair_enabled())
@@ -1012,63 +848,24 @@ int mlp_bf16_launch(const MlpArgs& a, bool embedded, cudaStream_t st, bool densi
     static const TcSchedule S = [] { InerfNetDims d{64, 76, 32, 256, 8, 63, 27}; return build_tc_schedule(&d, false, 1); }();
     static const int n_steps_dens = tc_stages_before(S, 8);      // the stages of L0-L7
     int rc = setup_once(configured_dev,
-                        {(const void*)mlp_bf16_kernel<false>, (const void*)mlp_bf16_kernel<true>, (const void*)mlp_bf16_kernel<false, 0, true>,
-                         (const void*)mlp_bf16_kernel<false, 0, false, true>, (const void*)mlp_bf16_kernel<false, 0, true, true>,
-                         (const void*)mlp_bf16_kernel<false, 0, false, false, false, true>,
-                         (const void*)mlp_bf16_kernel<false, 0, false, true, false, true>},
+                        {(const void*)mlp_bf16_kernel<false>, (const void*)mlp_bf16_kernel<true>, (const void*)mlp_bf16_kernel<false, true>,
+                         (const void*)mlp_bf16_kernel<true, true>, (const void*)mlp_bf16_kernel<false, false, false, true>,
+                         (const void*)mlp_bf16_kernel<false, true, false, true>},
                         SMEM_ALLOC, "mlp_bf16", [] { return cudaMemcpyToSymbol(c_steps, S.st, sizeof(TcStage) * MAX_STEPS); });
     if (rc) return rc;
     const int n_rays = (int)(a.P / a.s);
-    const bool use_pair = mlp_pair_enabled() && !a.trace;
     if (density) {
-        if (a.trace || a.save_img) return fail(INERF_E_ARG, "mlp_bf16: the density-only build has no trace / saving form");
-        return use_pair ? launch<false, true, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16 pair, density only]")
-                        : launch<false, false, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16, density only]");
+        if (a.save_img) return fail(INERF_E_ARG, "mlp_bf16: the density-only build has no saving form");
+        return mlp_pair_enabled() ? launch<false, true, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16 pair, density only]")
+                                  : launch<false, false, false, true>(a, n_steps_dens, n_rays, st, "inerf_mlp_fwd[bf16, density only]");
     }
-    if (a.trace) {
-        if (!g_hang_host) {
-            int* dptr = nullptr;
-            if (cudaHostAlloc(&g_hang_host, 64, cudaHostAllocMapped) == cudaSuccess &&
-                cudaHostGetDevicePointer(&dptr, g_hang_host, 0) == cudaSuccess)
-                cudaMemcpyToSymbol(g_hang_dev, &dptr, sizeof(dptr));
-        }
-        if (g_hang_host) for (int i = 0; i < 8; ++i) g_hang_host[i] = 0;
-    }
-#ifdef INERF_ABLATION
-    const long long n_iter = (a.P + 255) / 256;
-    const int grid = (int)(n_iter < (long long)num_sms() ? n_iter : (long long)num_sms());
-    if (const char* e = a.save_img ? nullptr : getenv("INERF_ABL")) {
-        const int abl = atoi(e);
-#define ABL_CASE(N_) case N_: cudaFuncSetAttribute(mlp_bf16_kernel<false, N_>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC); \
-                              mlp_bf16_kernel<false, N_><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); break;
-        switch (abl) { ABL_CASE(1) ABL_CASE(2) ABL_CASE(3) ABL_CASE(4) ABL_CASE(5) ABL_CASE(6) ABL_CASE(7) ABL_CASE(8) ABL_CASE(16) ABL_CASE(24) default: break; }
-#undef ABL_CASE
-        if (abl >= 1 && abl <= 24) return check_launch("inerf_mlp_fwd[bf16,ablation]");
-    }
-#endif
     if (a.save_img) {
         if (!a.save_mask) return fail(INERF_E_ARG, "mlp_bf16: save_mask is NULL");
-#ifdef INERF_ABLATION
-        { const char* e = getenv("INERF_SAVE_ABL"); const int v = e ? atoi(e) : 0; cudaMemcpyToSymbolAsync(g_save_abl, &v, sizeof(v), 0, cudaMemcpyHostToDevice, st); cudaStreamSynchronize(st); }
-        if (const char* e = getenv("INERF_ABL")) {      // weight streaming (2) / sincosf (4) off on top of the saving switches
-            const int abl = atoi(e);
-            if (abl == 2 || abl == 4) {
-                if (abl == 2) { cudaFuncSetAttribute(mlp_bf16_kernel<false, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-                                mlp_bf16_kernel<false, 2, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); }
-                else { cudaFuncSetAttribute(mlp_bf16_kernel<false, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC);
-                       mlp_bf16_kernel<false, 4, true><<<grid, NTHREADS_BF16, SMEM_ALLOC, st>>>(a, S.n_stages, n_rays, nullptr); }
-                return check_launch("inerf_mlp_fwd_train[bf16,ablation]");
-            }
-        }
-#endif
-        return use_pair ? launch<true, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16 pair]")
-                        : launch<true, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16]");
+        return mlp_pair_enabled() ? launch<true, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16 pair]")
+                                  : launch<true, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd_train[bf16]");
     }
-    if (a.trace)
-        return launch_tc(mlp_bf16_kernel<true>, false, (a.P + 255) / 256, NTHREADS_BF16, SMEM_ALLOC, st, "inerf_mlp_fwd[bf16]", a, S.n_stages, n_rays,
-                         a.trace);
-    return use_pair ? launch<false, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16 pair]")
-                    : launch<false, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16]");
+    return mlp_pair_enabled() ? launch<false, true, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16 pair]")
+                              : launch<false, false, false>(a, S.n_stages, n_rays, st, "inerf_mlp_fwd[bf16]");
 }
 
 }  // namespace inerf

@@ -29,13 +29,10 @@ struct MlpArgs {
     int cond_dim;                     // dim_aud + dim_expr + dim_latent
     int dim_expr;
     float* save;                      // optional (fp32 path, training): activation store [ceil(P/64)*64][SAVE_W]
-    float* trace;                     // optional (bf16 path): post-activation values of the first 256 points, [11][256][256]
     // optional (bf16 path, training): per 128-point tile T = point/128, the activations as the forward kernel holds them in shared
     // memory -- TRAIN_IMGS 16 KB images [128 points][64 features] bf16, K-major, 128-byte swizzle -- and the ReLU masks
     uint8_t* save_img;                // [n_tiles][TRAIN_IMGS][16384]
     uint32_t* save_mask;              // [n_tiles][TRAIN_MASK_WORDS][128]: bit (31-j) of word w = pre-activation 32w+j of the row is >= 0
-    float tc_comp;                    // fp16x2 kernel, calibration runs only: uniform main-accumulator scale - 1 (< 0: use tc_ulps)
-    float tc_ulps[4];                 // fp16x2 kernel: main-accumulator compensation in ulps of 1.0 for {L0, L1-7, V0, V1-2}
 };
 
 // image index inside a tile: h0..h7 at 4l+kb, v0..v2 at 32+2v+kb, gamma(p) (63 cols) at 38, gamma(v) (27 cols) at 39; the backward
@@ -46,7 +43,7 @@ __host__ __device__ constexpr int train_mask_of(int l) { return l < 8 ? 8 * l : 
 
 // ---- launch plumbing of the tensor-core kernels ----------------------------------------------------------------------------------
 // The CTA-pair builds (clusters of two, tcgen05 cta_group::2) run by default; INERF_MLP_PAIR=0, read once per process, keeps the
-// single-CTA builds: the bit-exact reference of the pair builds, and what the trace / ablation builds run.
+// single-CTA builds: the bit-exact reference of the pair builds.
 inline bool mlp_pair_enabled() {
     static const bool env = [] { const char* e = getenv("INERF_MLP_PAIR"); return !e || atoi(e) != 0; }();
     return env && num_sms() >= 2;
@@ -106,7 +103,6 @@ size_t mlp_fp32_bwd_args_bytes();
 int mlp_f16x2_packed_bytes(const InerfNetDims* d, size_t* bytes, bool embedded = false);
 int mlp_f16x2_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st, bool embedded = false);
 int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st);
-int mlp_bf16_hang_info(int32_t* out8);
 // bf16 training path (mlp_bf16_bwd.cu, mlp_bf16_dw.cu, mlp_fp32_bwd.cu)
 int mlp_bf16_bwd_packed_bytes(const InerfNetDims* d, size_t* bytes);
 int mlp_bf16_bwd_pack(const InerfNetDims* d, const float* const* params_host, void* packed, cudaStream_t st);

@@ -38,7 +38,6 @@
 // buffer once L5 (the last reader of gamma(p)) has completed; the commit after the last V0 view MMA hands the buffer back for the next
 // iteration's gamma(p).  pe_ready / pe_free therefore complete twice per iteration.  Packed blob: INERF_MLP_F16X2_EMB (four more stages).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "mlp_tc.cuh"
 
@@ -115,7 +114,6 @@ constexpr uint32_t CORR_COL = 256;      // first TMEM column of the correction a
 // shrink: n/3 ulps of the final sum, a random walk of partial sums) rounded to fp32 ulps of 1.0 (2^-23): 1 for L0, 4 for the 256-wide
 // layers, 2 for V0 / V1-2 (V0's theoretical 4 is indistinguishable in the sweep; the landscape is flat to 5 % around this point).  It
 // brings raw to 2.0e-6 max / 5e-7 rms of scale, against 1.5e-6 / 3.3e-7 for the FFMA kernel and 3.5e-6 / 1.0e-6 uncompensated.
-// INERF_F16X2_COMP (uniform comp) / INERF_F16X2_ULPS ("l0,trunk,v0,v12") re-run the calibration (tests/native/f16x2_comp_sweep.py).
 __host__ __device__ constexpr float tc_comp_ulps(int l) { return l == 0 ? 1.0f : (l < 8 ? 4.0f : 2.0f); }
 
 // (hi, lo) fp16x2 words of two fp32 values, ReLU applied: hi = the value truncated to 11 significant bits, lo = the exact remainder
@@ -252,13 +250,11 @@ __device__ __forceinline__ void epi16(const uint32_t (&r)[16], const uint32_t (&
     }
 }
 
-// abl (profiling only, INERF_F16X2_ABL; results are garbage): bit 0 = the weight ring is filled once and never reloaded, bit 1 = the
-// epilogue keeps its barrier protocol but skips the TMEM loads / conversion / stores, bit 2 = the positional-encoding warps skip sincosf
 // PAIR = true: clusters of two CTAs, one tcgen05.mma.cta_group::2 over the 2 x 128 rows of the pair, the weight stages split across the
 // pair (the bf16 kernel's pair build, mlp_bf16.cu; a pair iteration is two 128-point slots, CTA r takes slot 2 it + r).
-// EMB = true: rows of a.x (P, 90) with the INERF_MLP_F16X2_EMB schedule (see the header); launched with abl = 0.
+// EMB = true: rows of a.x (P, 90) with the INERF_MLP_F16X2_EMB schedule (see the header).
 template <bool PAIR, bool EMB = false>
-__global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n_stages, int n_rays, int abl) {
+__global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n_stages, int n_rays) {
     constexpr int NSTAGE = RingOf<PAIR>::N, STAGE_BYTES = RingOf<PAIR>::BYTES;
     extern __shared__ __align__(1024) uint8_t sm[];
     if ((smem_u32(sm) & 1023u) != 0) __trap();
@@ -330,7 +326,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                     }
                     wait_b(&bars->wempty[stage], (round & 1) ^ 1);
                     const uint32_t bytes = (uint32_t)fs.n8 * 8u * 128u / SPLIT;
-                    if ((abl & 1) && g >= NSTAGE) { mbar_arrive(&bars->wfull[stage]); continue; }
                     mbar_arrive_expect_tx(&bars->wfull[stage], bytes);
                     bulk_g2s(sm + OFF_W + stage * STAGE_BYTES, blob + fs.offset + rank * bytes, bytes, &bars->wfull[stage]);
                 }
@@ -396,7 +391,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                 const int NH = (l < 8 ? 256 : 128) >> 1;
                 const int npg = NH >> 6;                       // chunks per group and half: 2 (N = 256) or 1 (N = 128)
                 const uint32_t par = layer_ctr & 1;
-                const float ms = a.tc_comp >= 0.f ? 1.0f + a.tc_comp : 1.0f + a.tc_ulps[l == 0 ? 0 : (l < 8 ? 1 : (l == 8 ? 2 : 3))] * 1.1920928955078125e-07f;
+                // 1 + tc_comp_ulps(l) ulps of 1.0, exactly.  Written as float arithmetic the same value let the compiler specialise the
+                // epilogue per scale: 3 % slower (profiles/r13_scaffolding_removal_ab.txt)
+                const float ms = __uint_as_float(0x3F800000u + (uint32_t)tc_comp_ulps(l));
                 if (!EMB && l == 8) wait_b(&bars->dirb_ready, iter_ctr & 1);
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) {
@@ -406,7 +403,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                     uint32_t ph[32], pl[32];
 #pragma unroll
                     for (int cc = 0; cc < 2; ++cc) {
-                        if (cc < npg && !(abl & 2)) {
+                        if (cc < npg) {
                             const int f0 = h * NH + (grp * npg + cc) * 32;       // first output feature of the chunk
 #pragma unroll
                             for (int q16 = 0; q16 < 2; ++q16) {
@@ -435,7 +432,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
                         __syncwarp();
 #pragma unroll
                         for (int cc = 0; cc < 2; ++cc) {
-                            if (cc < npg && !(abl & 2)) {
+                            if (cc < npg) {
                                 const int f0 = h * NH + (grp * npg + cc) * 32;
                                 uint8_t* kb = act + (f0 >> 6) * 16384 + row_off;
                                 const int ch0 = (f0 & 63) >> 3;
@@ -557,8 +554,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) mlp_f16x2_kernel(MlpArgs a, int n
 #pragma unroll
                     for (int c = 0; c < 3; ++c) {
                         float sn, cs;
-                        if (abl & 4) { sn = v[c]; cs = zz; }
-                        else sincosf(v[c] * (float)(1 << f), &sn, &cs);
+                        sincosf(v[c] * (float)(1 << f), &sn, &cs);
                         v[3 + 6 * f + c] = sn;
                         v[6 + 6 * f + c] = cs;
                     }
@@ -662,13 +658,6 @@ int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
                             return e == cudaSuccess ? cudaMemcpyToSymbol(c_fstages_emb, SE.st, sizeof(TcStage) * MAX_FSTAGES) : e;
                         });
     if (rc) return rc;
-    MlpArgs b = a;
-    b.tc_comp = -1.0f;                                                                // < 0: the per-layer table tc_comp_ulps
-    b.tc_ulps[0] = tc_comp_ulps(0); b.tc_ulps[1] = tc_comp_ulps(1); b.tc_ulps[2] = tc_comp_ulps(8); b.tc_ulps[3] = tc_comp_ulps(9);
-    if (const char* e = getenv("INERF_F16X2_COMP")) b.tc_comp = (float)atof(e);      // calibration sweeps (tests/native/f16x2_comp_sweep.py)
-    if (const char* e = getenv("INERF_F16X2_ULPS")) sscanf(e, "%f,%f,%f,%f", &b.tc_ulps[0], &b.tc_ulps[1], &b.tc_ulps[2], &b.tc_ulps[3]);
-    int abl = 0;
-    if (const char* e = getenv("INERF_F16X2_ABL"); e && !embedded) abl = atoi(e);   // the embedded-row build has no ablation variants
     const int n_stages = embedded ? SE.n_stages : S.n_stages;
     const int n_rays = embedded ? 0 : (int)(a.P / a.s);
     const bool pair = mlp_pair_enabled();
@@ -676,7 +665,7 @@ int mlp_f16x2_launch(const MlpArgs& a, bool embedded, cudaStream_t st) {
                              : (embedded ? mlp_f16x2_kernel<false, true> : mlp_f16x2_kernel<false>);
     const char* what = embedded ? (pair ? "inerf_mlp_fwd_embedded[fp16x2 pair]" : "inerf_mlp_fwd_embedded[fp16x2]")
                                 : (pair ? "inerf_mlp_fwd[fp16x2 pair]" : "inerf_mlp_fwd[fp16x2]");
-    return launch_tc(kernel, pair, (a.P + 127) / 128, NTHREADS, SMEM_BYTES, st, what, b, n_stages, n_rays, abl);
+    return launch_tc(kernel, pair, (a.P + 127) / 128, NTHREADS, SMEM_BYTES, st, what, a, n_stages, n_rays);
 }
 
 }  // namespace inerf

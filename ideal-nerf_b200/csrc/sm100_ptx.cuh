@@ -13,10 +13,7 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 // Suspend-time hint of mbarrier.try_wait: the waiting thread may sleep in hardware until the phase completes (it is woken as soon as it
 // does) instead of returning after the short default window.  Without it the role warps of the MLP kernels spent ~30 % of all issued
 // instructions on try_wait / branch pairs (ncu source counters) -- issue slots the epilogue warps of the same scheduler need.
-#ifndef INERF_MBAR_HINT
-#define INERF_MBAR_HINT 0x989680u
-#endif
-constexpr uint32_t MBAR_SUSPEND_HINT = INERF_MBAR_HINT;
+constexpr uint32_t MBAR_SUSPEND_HINT = 0x989680u;
 
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");

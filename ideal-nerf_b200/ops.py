@@ -861,21 +861,6 @@ def decode_images(buf, n_tiles, n_imgs=40):
     return out.reshape(n_tiles, n_imgs, 128, 64).float()
 
 
-def mlp_fwd_trace(mode, dims, params, packed, cond, rays, z):
-    """bf16 kernel with the per-layer activation trace of the first 256 points: returns (raw, trace[11,256,256])."""
-    rays, z = f32c(rays, "rays"), f32c(z, "z_vals")
-    n, s = z.shape
-    raw = torch.empty((n, s, 4), device=z.device)
-    trace = torch.zeros((11 * 256 * 256 + 148 * 8 * 2 + 148 * 16,), device=z.device)     # activations + per-CTA issuer / epilogue timing
-    arr = param_array(params)
-    with torch.cuda.device(z.device):
-        call("inerf_mlp_fwd_trace", _lib.lib().inerf_mlp_fwd_trace, mode, ctypes.byref(dims), arr, ptr(packed), ptr(cond),
-             ptr(rays), rays.shape[1], ptr(z), n, s, ptr(raw), ptr(trace), stream())
-    mlp_fwd_trace.timing = trace[11 * 256 * 256:11 * 256 * 256 + 148 * 16].reshape(-1, 8)
-    mlp_fwd_trace.layer_waits = trace[11 * 256 * 256 + 148 * 16:].reshape(148, 16)
-    return raw, trace[:11 * 256 * 256].reshape(11, 256, 256)
-
-
 def _rows90(x):
     """x as the embedded-row kernels read it: contiguous fp32 (P, 90), 16-byte aligned as the bf16 kernel needs (a row slice may start off
     alignment)."""

@@ -453,14 +453,6 @@ int inerf_mlp_fwd(int mode, const InerfNetDims* dims, const float* const* params
                   const float* cond, const float* rays, int ray_stride, const float* z, int n, int s,
                   float* raw, void* stream);
 
-/* Diagnostic twin of inerf_mlp_fwd for the bf16 kernel: additionally writes the post-ReLU activations of
- * every layer (L0..L7, V0..V2; fp32, before the bf16 rounding) of the FIRST 256 points to
- * trace [11][256][256] (columns >= 128 of V0..V2 are not written).  Used by the parity tests to localise
- * a mismatch to a layer. */
-int inerf_mlp_fwd_trace(int mode, const InerfNetDims* dims, const float* const* params_host, const void* packed,
-                        const float* cond, const float* rays, int ray_stride, const float* z, int n, int s,
-                        float* raw, float* trace, void* stream);
-
 /* ---- training (fp32 mode): forward that keeps activations + analytic backward ------------------------------- */
 
 /* Buffer sizes for n_points = n*s points: acts (floats), deltas (floats), scratch (bytes, device). */
@@ -521,11 +513,6 @@ int inerf_audio_net_bwd(const float* const* params_host, float* const* grads_hos
                         void* stream);
 int inerf_audio_att_bwd(const float* const* params_host, float* const* grads_host, const float* x, const float* dy, int seq_len,
                         int dim_feat, int dim_att, float* dx, void* stream);
-
-/* After a failed inerf_mlp_fwd_trace (the trace build bounds every mbarrier wait to ~1 s and traps): the record
- * of the first waiter that timed out, {site code, block, thread, aux0, aux1, parity, 0, 0}; all zero otherwise.
- * HOST pointer to 8 ints. */
-int inerf_debug_hang_info(int32_t* out8);
 
 /* FaceNeRF.forward on already-embedded inputs x (p, in_xyz+in_views) -- the reference module's own
  * call signature (face_nerf.py:40).  out (p, 4).  Any p >= 0 (0 enqueues nothing).

@@ -1,7 +1,7 @@
 """FaceNeRF.forward on embedded rows (x (P, 63+27), the reference module's own signature) against the fused (rays, z) entry.
 
     python profiles/embedded_mlp.py                      # card, power limit, points/s of the paths below, query hashes
-    python profiles/embedded_mlp.py --hash-only --root T # only the sha256 of the bf16 and fp16x2 fused-query raw, with the package of tree T
+    python profiles/embedded_mlp.py --hash-only --root T # only the sha256 of the bf16 and fp16x2 outputs below, with the package of tree T
 
 On P = 202 500 x 64 rows (one 450 x 450 frame, 64 samples per ray; x is 4.7 GB, far larger than L2, and read once per call):
   * FaceNeRF.forward(x), mlp_mode="fp32" (FFMA kernel), "bf16" and "fp16x2" (tcgen05 embedded-row kernels);
@@ -11,8 +11,8 @@ On P = 202 500 x 64 rows (one 450 x 450 frame, 64 samples per ray; x is 4.7 GB, 
 Times are CUDA-event times of whole calls after a warm-up.  TFLOP/s are algorithmic: 560 640 MAC per point for the fused form (view
 columns folded into a per-ray bias), 560 640 + 3 456 for the embedded form, against the sustained cuBLAS bf16 figure of DESIGN.md §3;
 for fp16x2 the issued rate of its three MMA passes (hi.hi + lo.hi + hi.lo) is printed as well.
-The hashes are of raw from a seeded FaceNeRF.query (137 rays x {64, 192} samples) in bf16 and in fp16x2: equal hashes from two trees =
-the fused paths are unchanged bit for bit.
+The hashes are of raw from a seeded FaceNeRF.query (137 rays x {64, 192} samples) and of FaceNeRF.forward on the embedded rows of the
+same points, each in bf16 and in fp16x2: equal hashes from two trees = the fused and embedded-row paths are unchanged bit for bit.
 """
 import argparse
 import hashlib
@@ -48,20 +48,28 @@ cam, fr = S.camera(), S.frame_inputs(0)
 aud, expr, lat = fr["aud"].to(dev), fr["expr"].to(dev), fr["latent"].to(dev)
 
 
-def query_hash(mode):
+def raw_hashes(mode):
+    """sha256 of FaceNeRF.query(rays, z) and of FaceNeRF.forward(x) on the embedded rows of the same points."""
     torch.manual_seed(3)
     net = M.FaceNeRF(dim_aud=64, dim_latent=32, dim_expr=76, mlp_mode=mode).apply(M.init_weights).to(dev)
     rays = ops.get_rays_range(450, 450, cam["focal"], cam["c2w"].to(dev), S.NEAR, S.FAR, 90000, 137)
-    h = hashlib.sha256()
+    e10, _ = M.get_embedder(10, 0)
+    e4, _ = M.get_embedder(4, 0)
+    hq, he = hashlib.sha256(), hashlib.sha256()
     with torch.no_grad():
         for s in (64, 192):
             z = torch.sort(S.NEAR + (S.FAR - S.NEAR) * torch.rand(137, s, device=dev, generator=torch.Generator(dev).manual_seed(s)), -1)[0]
-            h.update(net.query(rays, z.contiguous(), aud, expr, lat).cpu().numpy().tobytes())
-    return h.hexdigest()
+            hq.update(net.query(rays, z.contiguous(), aud, expr, lat).cpu().numpy().tobytes())
+            pts = (rays[:, None, 0:3] + rays[:, None, 3:6] * z[..., None]).reshape(-1, 3)
+            x = torch.cat([e10(pts), e4(rays[:, None, 8:11].expand(137, s, 3).reshape(-1, 3))], -1).contiguous()
+            he.update(net(x, aud, expr, lat).cpu().numpy().tobytes())
+    return hq.hexdigest(), he.hexdigest()
 
 
-say(f"query_raw_sha256 {query_hash('bf16')}  (package of {os.path.abspath(args.root)})")
-say(f"query_raw_sha256_fp16x2 {query_hash('fp16x2')}  (package of {os.path.abspath(args.root)})")
+for mode, tag in (("bf16", ""), ("fp16x2", "_fp16x2")):
+    hq, he = raw_hashes(mode)
+    say(f"query_raw_sha256{tag} {hq}  (package of {os.path.abspath(args.root)})")
+    say(f"embedded_raw_sha256{tag} {he}  (package of {os.path.abspath(args.root)})")
 if args.hash_only:
     sys.exit(0)
 

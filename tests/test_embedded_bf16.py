@@ -52,7 +52,7 @@ def _state(preset, dims, seed, b):
 
 
 def _bf16_bars(got, ref, what, max_rel=6e-2, rms_rel=3e-2):
-    """The bars of test_bf16_mlp_trace_and_raw, per channel, relative to the channel's scale over the whole batch `ref`."""
+    """The bars of test_bf16_mlp_layers_and_raw, per channel, relative to the channel's scale over the whole batch `ref`."""
     got, ref = got.double(), ref.double()
     scale, rms_ref = ref.abs().amax(0), (ref ** 2).mean(0).sqrt()
     d = got - ref[:got.shape[0]]

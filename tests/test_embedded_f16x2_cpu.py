@@ -52,11 +52,10 @@ def test_embedded_entry_argument_checks(L):
     assert b"INERF_MLP_F16X2_EMB" in L.inerf_last_error()
 
 
-def test_other_entries_reject_the_embedded_mode(L):
+def test_fused_entries_reject_the_embedded_mode(L):
     d = InerfNetDims(64, 76, 32, 256, 8, 63, 27)
     P = _params()
     assert L.inerf_mlp_fwd(_lib.INERF_MLP_F16X2_EMB, ctypes.byref(d), P, A16, A16, A16, 11, A16, 4, 64, A16, None) == -4
-    assert L.inerf_mlp_fwd_trace(_lib.INERF_MLP_F16X2_EMB, ctypes.byref(d), P, A16, A16, A16, 11, A16, 4, 64, A16, A16, None) == -4
     a = _lib.InerfRenderArgs(mode=_lib.INERF_MLP_F16X2_EMB, n=0, n_samples=64, n_importance=128)
     a.coarse.dims = a.fine.dims = d
     assert L.inerf_render_rays_fused(ctypes.byref(a), None) == -4

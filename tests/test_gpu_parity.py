@@ -397,7 +397,7 @@ def test_cpu_tensor_is_rejected(M):
 # bf16 tensor-core MLP (tcgen05) -- gate: PSNR delta <= 0.05 dB vs the reference render
 # ------------------------------------------------------------------------------------------------
 def _folded_layers_fp32(sd, x_pe, x_dir, aud, expr, lat):
-    """Per-layer post-ReLU activations of FaceNeRF (fp64 torch on CPU) for the trace comparison."""
+    """Per-layer post-ReLU activations of FaceNeRF (fp64 torch on CPU) for the layer-by-layer comparison."""
     sd = {k: v.double() for k, v in sd.items()}
     cond = torch.cat([aud, expr / 3, lat]).double()
     first = torch.cat([x_pe.double(), cond[None].expand(x_pe.shape[0], -1)], -1)
@@ -415,8 +415,9 @@ def _folded_layers_fp32(sd, x_pe, x_dir, aud, expr, lat):
 
 
 @pytest.mark.parametrize("s", [64, 192, 45])
-def test_bf16_mlp_trace_and_raw(M, s):
-    """Layer-by-layer check of the fused tcgen05 kernel on the first 256 points, then raw (n,s,4) vs the fp32 kernel."""
+def test_bf16_mlp_layers_and_raw(M, s):
+    """Layer-by-layer check of the fused tcgen05 kernel on the first 256 points (the activation images of the saving build), then raw
+    (n,s,4) vs the fp32 kernel."""
     b = O.synthetic_train_batch(0)
     n = 3072 * 64 // s // 4 + 3                                        # ragged: n*s is not a multiple of 256
     rays = b["rays"][:n].to(DEV)
@@ -428,16 +429,17 @@ def test_bf16_mlp_trace_and_raw(M, s):
         params = [p.detach() for p in net16.kernel_params()]
         cond = M.ops.fold_cond(net16._dims, params, aud, expr, lat)
         packed = net16.packed_weights(net16.kernel_params())
-        raw16, trace = M.ops.mlp_fwd_trace(M._lib.INERF_MLP_BF16, net16._dims, params, packed, cond, rays, z)
+        raw16, acts16, _, _ = M.ops.mlp_fwd_train_bf16(net16._dims, params, packed, cond, rays, z)
         raw32 = net32.query(rays, z, aud, expr, lat)
         raw16b = net16.query(rays, z, aud, expr, lat)
-    assert torch.equal(raw16, raw16b), "trace build and production build must agree bit for bit"
-    # reference activations of the first 256 points
+    assert torch.equal(raw16, raw16b), "saving build and inference build must agree bit for bit"
+    # reference activations of the first 256 points (tiles 0 and 1 of the saved images)
+    A = M.ops.decode_images(acts16, 2)
     pts = (rays[:, None, 0:3] + rays[:, None, 3:6] * z[..., None]).reshape(-1, 3)[:256].cpu()
     dirs = rays[:, None, 8:11].expand(n, s, 3).reshape(-1, 3)[:256].cpu()
     acts = _folded_layers_fp32(sd, O.positional_encoding(pts, 10), O.positional_encoding(dirs, 4), b["aud"], b["expr"], b["latent"])
     for l, ref in enumerate(acts):
-        got = trace[l, :, :ref.shape[1]].cpu().double()
+        got = _img_cols(A, *_lay_img(l)).cpu().double()
         scale = float(ref.abs().max()) + 1e-6
         err = float((got - ref).abs().max()) / scale
         print(f"[s={s}] layer {l}: max-abs/scale {err:.3e} (scale {scale:.3f})")
