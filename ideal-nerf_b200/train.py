@@ -90,14 +90,27 @@ class _AdamStep:
 
     cuda_graph=True with world > 1 needs an NCCL process group: the all-reduce of the flat gradient is recorded in each rank's graph
     (a gloo collective cannot be).  The ranks compare their graph keys once, on the capturing call (_check_ranks_agree); replays add no
-    collective and no host work."""
-    _FIXED = "batch shapes and perturb"
+    collective and no host work.
 
-    def __init__(self, params, args, world, group, cuda_graph):
+    max_graphs (graph mode): how many captured graphs the step may hold, one per key; they share the flat parameters and Adam's state.
+    With the default 1 a second key raises.  log_rows > 0 (graph mode): every iteration also writes one row of LOG_COLUMNS -- its losses,
+    the PSNR of img_loss and the learning rate it leaves for the next step -- into the device tensor log_ring (log_rows, len(LOG_COLUMNS)),
+    at row global_step % log_rows (global_step before the iteration), inside the graph: a reader copies the ring to the host once per
+    log_rows steps instead of reading a loss every step."""
+    _FIXED = "batch shapes and perturb"
+    LOG_COLUMNS = ()
+
+    def __init__(self, params, args, world, group, cuda_graph, max_graphs=1, log_rows=0):
         self.args, self.world, self.group = args, world, group
         self.flat = FlatParams(params)
         self.cuda_graph = bool(cuda_graph)
-        self._static = None
+        if int(max_graphs) < 1:
+            raise ValueError(f"max_graphs must be >= 1, got {max_graphs}")
+        if (int(max_graphs) > 1 or int(log_rows) > 0) and not self.cuda_graph:
+            raise ValueError("max_graphs and log_rows are options of the CUDA-graph mode (cuda_graph=True)")
+        self.max_graphs = int(max_graphs)
+        self._graphs = {}                                                  # key -> static buffers, graph and outputs of that key
+        self._static = None                                                # the entry of the last call's key
         name = type(self).__name__
         on_cuda = self.flat.flat.is_cuda
         if self.cuda_graph:
@@ -111,8 +124,10 @@ class _AdamStep:
             self._lr_t = torch.tensor(float(args.lrate), device=dev)          # the learning rate and the step count live on the device
             self._gs_t = torch.zeros((), device=dev)
             self.optimizer = torch.optim.Adam([self.flat.flat], lr=self._lr_t, betas=(0.9, 0.999), fused=True, capturable=True)
+            self.log_ring = torch.zeros((int(log_rows), len(self.LOG_COLUMNS)), device=dev) if int(log_rows) > 0 else None
         else:
             self.optimizer = torch.optim.Adam([self.flat.flat], lr=args.lrate, betas=(0.9, 0.999), fused=on_cuda)
+            self.log_ring = None
         self.global_step = 0
 
     # -- checkpoint interchange with the reference's per-parameter Adam -----------------------------------------------------------
@@ -162,7 +177,7 @@ class _AdamStep:
 
     def _check_loadable(self):
         """load() replaces weights the captured graph reads: it is refused, before anything is changed, once the graph exists."""
-        if self.cuda_graph and self._static is not None and self._static["graph"] is not None:
+        if self.cuda_graph and any(st["graph"] is not None for st in self._graphs.values()):
             name = type(self).__name__
             raise RuntimeError(f"{name}.load() after the CUDA graph was captured: load before the first graphed step")
 
@@ -196,27 +211,35 @@ class _AdamStep:
         self.global_step += 1
         return lr
 
-    def _graph_step(self, key, make_static, fill, body):
+    def _graph_step(self, key, make_static, fill, body, log_row):
         """One call of the CUDA-graph mode.  `key` is what a captured graph fixes; make_static() returns the static input buffers,
-        fill(st) copies this call's inputs into them, body(st) is the iteration (its tensors are the outputs the replays refresh).  The
-        learning-rate schedule runs on the device after body.  The first call runs eagerly (it initialises Adam's state and the kernels'
-        per-device constants; with world > 1 its eager all-reduce also sets up the NCCL communicator the capture records into), the
-        second call captures, every later call replays.  With world > 1 the capturing call first checks that every rank has the same key
+        fill(st) copies this call's inputs into them, body(st) is the iteration (its tensors are the outputs the replays refresh),
+        log_row(out) the losses of LOG_COLUMNS[:-2] among body's outputs.  The learning-rate schedule (and the log_ring row) runs on the
+        device after body.  The first call of a key runs eagerly (it initialises Adam's state and the kernels' per-device constants; with
+        world > 1 its eager all-reduce also sets up the NCCL communicator the capture records into), the second captures, every later
+        call replays.  A key beyond max_graphs raises.  With world > 1 each capturing call first checks that every rank has the same key
         (_check_ranks_agree); a key that changes on one rank after the capture raises on that rank only, and the other ranks then wait in
         their next replay's all-reduce, as in any data-parallel program whose ranks stop taking the same steps."""
-        if self._static is None or self._static["key"] != key:
-            if self._static is not None:
+        st = self._graphs.get(key)
+        if st is None:
+            if len(self._graphs) >= self.max_graphs:
                 name = type(self).__name__
-                raise RuntimeError(f"{name}(cuda_graph=True) was captured for {self._static['key']}, got {key}: {self._FIXED} are fixed "
-                                   f"per {name}")
-            self._static = dict(make_static(), key=key, graph=None, out=None, calls=0)
-        st = self._static
+                held = "; ".join(str(k) for k in self._graphs)
+                raise RuntimeError(f"{name}(cuda_graph=True) was captured for {held}, got {key}: {self._FIXED} are fixed "
+                                   f"per {name} (max_graphs={self.max_graphs})")
+            st = self._graphs[key] = dict(make_static(), key=key, graph=None, out=None, calls=0)
+        self._static = st
         fill(st)
 
         def run():
             out = body(st)
             # new_lrate = lrate * 0.1 ** (global_step / (lrate_decay * 1500)); global_step += 1      (:554-558), on the device
             self._lr_t.copy_(self.args.lrate * torch.pow(0.1, self._gs_t / (self.args.lrate_decay * 1500)))
+            if self.log_ring is not None:
+                losses = log_row(out)
+                row = torch.stack([*losses, -10. * torch.log10(losses[1]), self._lr_t])
+                slot = torch.remainder(self._gs_t, self.log_ring.shape[0]).long().reshape(1)
+                self.log_ring.index_copy_(0, slot, row[None])
             self._gs_t.add_(1.0)
             return out
 
@@ -263,17 +286,20 @@ class TrainStep(_AdamStep):
     identical replicas stay identical.  The returned losses are the rank's own.
 
     cuda_graph=True: the first call runs eagerly, the second captures the whole iteration, later calls replay it; a graph fixes the
-    batch shapes, the aud_window / aud_feature choice and perturb (a change raises).  With world > 1 (NCCL only) each rank captures its
-    own graph with the all-reduce recorded in it, after the ranks have checked once that their keys agree -- so in this mode every rank
-    takes a band of the same shape.  For the ranks to draw complementary bands of one batch (DeviceHeadDataset.sample(i, rank, world)),
-    seed the in-kernel Philox stream the same way on every rank (ops.seed_rng(seed) on each rank's device) and make the same sequence of
-    stochastic calls."""
-    _FIXED = "batch shapes, the aud_window / aud_feature choice and perturb"
+    batch shapes, the aud_window / aud_feature choice, `smooth` and perturb.  A call with another key raises, unless max_graphs > 1 lets
+    the step capture one graph per key (e.g. max_graphs=2 for the two audio phases of the reference's schedule, smooth=False before
+    nosmo_iters and smooth=True after); the graphs share the flat parameters and Adam's state.  With world > 1 (NCCL only) each rank
+    captures its own graph with the all-reduce recorded in it, after the ranks have checked that their keys agree (again before each
+    further capture) -- so in this mode every rank takes a band of the same shape.  For the ranks to draw complementary bands of one
+    batch (DeviceHeadDataset.sample(i, rank, world)), seed the in-kernel Philox stream the same way on every rank (ops.seed_rng(seed) on
+    each rank's device) and make the same sequence of stochastic calls.  log_rows: the device log ring of _AdamStep, LOG_COLUMNS."""
+    _FIXED = "batch shapes, the aud_window / aud_feature choice, smooth and perturb"
+    LOG_COLUMNS = ("loss", "img_loss", "latent_code_loss", "psnr", "lr")
 
-    def __init__(self, network, latent_codes, args, world=1, group=None, cuda_graph=False):
+    def __init__(self, network, latent_codes, args, world=1, group=None, cuda_graph=False, max_graphs=1, log_rows=0):
         self.net, self.latent_codes = network, latent_codes
         latent_codes.requires_grad_(True)
-        super().__init__(list(network.parameters()) + [latent_codes], args, world, group, cuda_graph)
+        super().__init__(list(network.parameters()) + [latent_codes], args, world, group, cuda_graph, max_graphs, log_rows)
 
     def save(self, path):
         """head.tar as the reference writes it (audio_exp_nerf.py:584-591), loadable by the reference's resume code (:516-525)."""
@@ -294,19 +320,28 @@ class TrainStep(_AdamStep):
                 m.invalidate_packed()
         return self.global_step
 
-    def __call__(self, rays, bc_rgb, target, aud_feature, expr, index, perturb=None, aud_window=None):
+    def __call__(self, rays, bc_rgb, target, aud_feature, expr, index, perturb=None, aud_window=None, smooth=True):
         """aud_feature: the (dim_aud,) audio code (a constant, or a tensor with a graph into the conditioning nets); or pass
-        aud_window = the (smo_size, 16, 29) DeepSpeech window (Network.audio_window) and the code is computed -- and the two
-        conditioning nets are trained -- inside the step, as the reference's forward does (audio_exp_nerf.py:241-266)."""
+        aud_window = the (smo_size, 16, 29) DeepSpeech window (Network.audio_window) and the code is computed -- and the conditioning
+        nets are trained -- inside the step, as the reference's forward does (audio_exp_nerf.py:241-266): with smooth=True the whole
+        window through AudioNet, then AudioAttNet; with smooth=False the frame's own DeepSpeech features alone through AudioNet (row
+        smo_size // 2 of the window, which audio_window's padding makes auds[index]), Network.audio_feature before nosmo_iters --
+        AudioAttNet then gets no gradient."""
         perturb = self.args.perturb if perturb is None else perturb
         if self.cuda_graph:
-            return self._graphed(rays, bc_rgb, target, aud_feature, expr, index, perturb, aud_window)
+            return self._graphed(rays, bc_rgb, target, aud_feature, expr, index, perturb, aud_window, smooth)
         latent_code = self.latent_codes[index]
         if aud_window is not None:
-            aud_feature = self.net.aud_att_net(self.net.aud_net(aud_window))
+            aud_feature = self._audio_code(aud_window, smooth)
         loss, img_loss, latent_loss = self._body(rays, bc_rgb, target, aud_feature, expr, latent_code, perturb)
         lr = self._advance_lr()
         return {"loss": loss.detach(), "img_loss": img_loss.detach(), "latent_code_loss": latent_loss.detach(), "lr": lr}
+
+    def _audio_code(self, aud_window, smooth):
+        if smooth:
+            return self.net.aud_att_net(self.net.aud_net(aud_window))
+        half = aud_window.shape[0] // 2
+        return self.net.aud_net(aud_window[half:half + 1])
 
     def _body(self, rays, bc_rgb, target, aud_feature, expr, latent_code, perturb):
         """Forward, loss, backward, gradient gather (+ all-reduce), Adam: everything between two learning-rate updates."""
@@ -318,7 +353,7 @@ class TrainStep(_AdamStep):
         return loss, img_loss, latent_loss
 
     # -- CUDA-graph mode (SURVEY.md 8f-2) ------------------------------------------------------------------------------------------
-    def _graphed(self, rays, bc_rgb, target, aud_feature, expr, index, perturb, aud_window):
+    def _graphed(self, rays, bc_rgb, target, aud_feature, expr, index, perturb, aud_window, smooth):
         """The whole iteration -- conditioning nets, both render passes, loss, backward, gradient gather, Adam, learning-rate schedule, RNG
         offset -- as ONE cudaGraphLaunch.  Inputs are copied into static buffers; the latent-code row is selected on the device from a
         one-element index tensor; the learning rate and Adam's step count live in device tensors updated inside the graph; the
@@ -326,7 +361,7 @@ class TrainStep(_AdamStep):
         dev = self.flat.flat.device
         use_win = aud_window is not None
         aud_src = aud_window if use_win else aud_feature
-        key = (tuple(rays.shape), tuple(bc_rgb.shape), use_win, float(perturb))
+        key = (tuple(rays.shape), tuple(bc_rgb.shape), use_win, bool(smooth), float(perturb))
 
         def make_static():
             return {"rays": torch.empty_like(rays), "bc": torch.empty_like(bc_rgb), "target": torch.empty_like(target),
@@ -343,11 +378,11 @@ class TrainStep(_AdamStep):
 
         def body(st):
             latent_code = self.latent_codes.index_select(0, st["idx"]).squeeze(0)
-            aud = self.net.aud_att_net(self.net.aud_net(st["aud"])) if use_win else st["aud"]
+            aud = self._audio_code(st["aud"], smooth) if use_win else st["aud"]
             loss, img_loss, latent_loss = self._body(st["rays"], st["bc"], st["target"], aud, st["expr"], latent_code, perturb)
             return loss.detach(), img_loss.detach(), latent_loss.detach()
 
-        loss, img_loss, latent_loss = self._graph_step(key, make_static, fill, body)
+        loss, img_loss, latent_loss = self._graph_step(key, make_static, fill, body, lambda out: out)
         return {"loss": loss, "img_loss": img_loss, "latent_code_loss": latent_loss, "lr": self._lr_t}
 
 
@@ -379,17 +414,19 @@ class TorsoTrainStep(_AdamStep):
       TrainStep; seed the Philox stream alike on every rank for DeviceTorsoDataset.sample(i, rank, world) to give complementary bands.
       Each rank's step owns the head pair's packed blobs its graph reads; when the nets' caches were dropped (train() / eval(),
       invalidate_packed(), checkpoint.load_head_into_torso) the next call re-packs the current head weights into that same memory.
-      load() after the capture raises before it changes anything.
+      load() after the capture raises before it changes anything.  log_rows (LOG_COLUMNS) as in _AdamStep.
 
     save() / load() write and read {'global_step', 'model_state_dict': torso_network.state_dict(), 'optimizer': the per-parameter Adam
     state over the trained parameters}, the key set and per-parameter layout of head.tar.  Whether that equals the reference's
     {:06d}_torso.tar (train_torso.py:565-572) is not verified."""
 
-    def __init__(self, torso_network, args, world=1, group=None, cuda_graph=False):
+    LOG_COLUMNS = ("loss", "img_loss", "img_loss0", "psnr", "lr")
+
+    def __init__(self, torso_network, args, world=1, group=None, cuda_graph=False, log_rows=0):
         self.net = torso_network
         self.trained = (torso_network.torso_coarse_nerf, torso_network.torso_fine_nerf)
         mine = {id(p) for m in self.trained for p in m.parameters()}
-        super().__init__([p for p in torso_network.parameters() if id(p) in mine], args, world, group, cuda_graph)
+        super().__init__([p for p in torso_network.parameters() if id(p) in mine], args, world, group, cuda_graph, log_rows=log_rows)
 
     def save(self, path):
         torch.save({"global_step": int(self.global_step), "model_state_dict": self.net.state_dict(),
@@ -454,5 +491,5 @@ class TorsoTrainStep(_AdamStep):
                                   perturb)
             return loss.detach(), l2
 
-        loss, l2 = self._graph_step(key, make_static, fill, body)
+        loss, l2 = self._graph_step(key, make_static, fill, body, lambda out: (out[0], out[1][0], out[1][1]))
         return {"loss": loss, "img_loss": l2[0], "img_loss0": l2[1], "lr": self._lr_t}
